@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the headline benchmark: WindowTransformer 720p -> 1080p frames/s in bf16 (BASELINE.json configs[1]).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 N = 1: one "step" = one TransformerModel.forward over a batch of 8 synthetic 720p frames (configs[1]).
@@ -17,6 +17,14 @@ HBM fractions of the memory-bound kernels; `cpu_baseline` = the reference's own 
 
 --impl reference: times the reference's CPU implementation (baseline/_ref, unmodified; else the oracle port) on one
 frame of the same workload per step, on all host threads.
+
+--dump-outputs DIR: after the timing, writes what the last of the K headline steps returned (rank 0's frames, bf16 widened to
+float32, exactly): DIR/upscaled_frame0.npy, the first frame whole (3, 1080, 1920), and DIR/upscaled_sample.npy, the values at a
+fixed, seeded set of DUMP_SAMPLE flat indices of the whole (frames, 3, 1080, 1920) output (sorted).  Weights and frames are seeded,
+so two builds run with the same arguments can be compared output for output.  Compare with a tolerance of one bf16 ulp
+(2^-8 in [0.5, 1)), not bitwise: with four forwards in flight on the headline's four streams, the engine's output varies from run
+to run by up to one bf16 ulp over whole 128-token tiles (measured on a B200 at its 1000 W power limit: 34 to 44 of 60 steps,
+up to about 1 % of a step's values; with one or two streams every step repeats bitwise).
 """
 import argparse
 import json
@@ -44,6 +52,18 @@ HBM_BYTES_PER_FRAME = {
     "patch_unembed": 3840 * 128 * 2 + 2 * 360 * 640 * 64 * 2,                                # bf16 tokens + skip map in, sum out
     "bicubic_add_clamp": 3 * 720 * 1280 * 2 + 3 * 360 * 640 * 4 + 3 * 1080 * 1920 * 2,       # frame + fp32 residual in, frame out
 }
+DUMP_SAMPLE = 4 * 1024 * 1024      # --dump-outputs: 16 MB of sampled values beside the 25 MB first frame
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, y):
+    """y: the last headline step's output on the host (frames, 3, OH, OW), float32"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    flat = y.reshape(-1).numpy()
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(flat.size, size=min(DUMP_SAMPLE, flat.size), replace=False))
+    np.save(os.path.join(out_dir, "upscaled_frame0.npy"), y[0].numpy())
+    np.save(os.path.join(out_dir, "upscaled_sample.npy"), flat[idx])
 
 
 def peaks():
@@ -152,7 +172,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 2 s back-to-back run (config.sustained)")
     ap.add_argument("--no-tcgen05", action="store_true", help="force the CUDA-core bf16 path (A/B only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output to DIR as .npy (see the module docstring)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the engine (--impl engine)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -239,7 +262,7 @@ def main():
 
     def timed_forwards(n, profile_dominant=True, multi=False):
         """n back-to-back forwards bracketed by barrier + synchronize; returns (ms total on this rank, launches, dominant-kernel
-        (ms, count))"""
+        (ms, count), conv1 fused?, the last forward's output)"""
         barrier()
         if profile_dominant:
             lib.tu_profile_enable(1)
@@ -252,12 +275,12 @@ def main():
                 st_.wait_event(e0)
             for i in range(n):
                 with torch.cuda.stream(side[i % nstreams]):
-                    model(xs[i & 1])
+                    y_last = model(xs[i & 1])
             for st_ in side:
                 cur.wait_stream(st_)
         else:
             for i in range(n):
-                model(xs[i & 1])
+                y_last = model(xs[i & 1])
         e1.record()
         barrier()
         launches = lib.tu_launch_count() - n0
@@ -268,7 +291,7 @@ def main():
         if not fused:
             lib.tu_profile_collect(b"conv2", C.byref(kms), C.byref(kn))
         lib.tu_profile_reset()
-        return e0.elapsed_time(e1), launches, kms.value, kn.value, fused
+        return e0.elapsed_time(e1), launches, kms.value, kn.value, fused, y_last
 
     # ---------------- device-resident throughput (`value`)
     with torch.no_grad():
@@ -278,9 +301,12 @@ def main():
             with torch.cuda.stream(side[i % nstreams]):
                 model(xs[i & 1])
         torch.cuda.synchronize()
-        ms_single, _, kms, kn, fused12 = timed_forwards(steps)                     # one stream: clean per-kernel timings
+        ms_single, _, kms, kn, fused12, _ = timed_forwards(steps)                  # one stream: clean per-kernel timings
         time.sleep(0.5)
-        ms_total, launches, _, _, _ = timed_forwards(steps, profile_dominant=False, multi=True)     # the headline: EXACTLY `steps` steps
+        ms_total, launches, _, _, _, y_last = timed_forwards(steps, profile_dominant=False, multi=True)  # the headline: EXACTLY `steps` steps
+        # the output of the headline's last step (the timed region ended in a synchronize); written out after every measurement
+        y_dump = y_last.float().cpu() if args.dump_outputs and rank == 0 else None
+        del y_last
         # per-kernel breakdown: a separate, untimed pass with every launch bracketed (the extra event records would perturb
         # the timed region: they sit between kernels that otherwise chain through programmatic dependent launch)
         lib.tu_profile_enable(2)
@@ -395,7 +421,7 @@ def main():
         if not args.no_sustained:
             n_sus = max(int(2200.0 / (ms_total / steps)), steps)
             t_mark = time.time()
-            s_ms, _, s_kms, s_kn, _ = timed_forwards(n_sus)                        # single stream (kernel timings stay clean)
+            s_ms, _, s_kms, s_kn, _, _ = timed_forwards(n_sus)                     # single stream (kernel timings stay clean)
             s_ms = max_over_ranks(s_ms)
             sustained = {"frames_per_s": total_frames * n_sus / (s_ms * 1e-3), "ms_per_step": s_ms / n_sus, "steps": n_sus,
                          "seconds": s_ms * 1e-3, "streams": 1, "dominant_kernel_ms": (s_kms / s_kn) if s_kn else None,
@@ -497,6 +523,8 @@ def main():
             cfps, cms, kind, cores = reference_cpu_fps(3, 1)
             line["cpu_baseline"] = {"value": cfps, "unit": "frames/s", "cores": cores, "kind": kind,
                                     "sample": "1 frame (B=1) of the same 720p->1080p workload, fp32, mean of 3 after 1 warm-up"}
+        if y_dump is not None:
+            dump_outputs(args.dump_outputs, y_dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

@@ -66,6 +66,25 @@ def sample_fullsize(t, c):
     return t[..., ::st, ::st], crops
 
 
+# the seeded ragged-shape sweep (tests/golden/make_ragged.py): pre-clamp output on the lattice of the smallest stride among
+# RAGGED_STRIDES that keeps it within RAGGED_LATTICE values (1, or a prime >= 5: coprime to every sub-pixel factor 2/3/4/6 and to
+# the 8-pixel patch, so all phases are sampled), plus dense 8x8 crops of the four corners
+RAGGED_LATTICE = 2048
+RAGGED_STRIDES = (1, 5, 7, 11, 13, 17, 19, 23, 29, 31, 37, 41)
+RAGGED_CORNERS = ((0, 0), (0, -8), (-8, 0), (-8, -8))
+
+
+def ragged_sample(t):
+    """(stride, lattice, [crops]) of a (B, 3, H, W) array the way the ragged-sweep goldens store it"""
+    B, C, H, W = t.shape
+    st = next(s for s in RAGGED_STRIDES if B * C * -(-H // s) * -(-W // s) <= RAGGED_LATTICE)
+    crops = []
+    for y0, x0 in RAGGED_CORNERS:
+        y0, x0 = (H + y0 if y0 < 0 else y0), (W + x0 if x0 < 0 else x0)
+        crops.append(t[..., y0:y0 + 8, x0:x0 + 8])
+    return st, t[..., ::st, ::st], crops
+
+
 # natural-image fixtures (tests/golden/make_natural.py): uint8 LR frame, uint8 HR target, the reference's fp32 output as fp16
 NATURAL = {
     "natural_window_96x176_r1p5": dict(model="WindowTransformer", wseed=31, kw=dict(res_out=(144, 264))),

@@ -160,15 +160,37 @@ def test_fold_up1_matches_the_op_chain(r):
         assert bias[ch * NO + q * r + j] == bf[1, 1, o]
 
 
-def test_reference_loader_resolves_to_the_reference_not_to_the_drop_in_alias():
-    """bench.py's reference arm / cpu_baseline must time the UNMODIFIED reference modules (baseline/_ref), although this
-    repository ships a `models` package with the same module paths"""
+# A stand-in for the reference's models/ tree, same layout: namespace directories (no __init__.py), model.py per model, and the
+# relative import of FastTransformer/model.py (`from .utils import ...`).  Its forward runs on CPU, as the reference's does.
+_STAND_IN_MODEL = """import torch
+import torch.nn.functional as F
+{extra}
+
+class TransformerModel(torch.nn.Module):
+    def __init__(self):
+        super().__init__()
+        self.conv1 = torch.nn.Conv2d(3, 3, 3, padding=1)
+
+    def forward(self, x, res_out=(1080, 1920)):
+        return F.interpolate(self.conv1(x), size=res_out, mode="bicubic", align_corners=False)
+"""
+
+
+def test_reference_loader_resolves_to_the_reference_not_to_the_drop_in_alias(tmp_path):
+    """bench.py's reference arm / cpu_baseline must time the UNMODIFIED reference modules (a copy of the reference's models/ in
+    baseline/_ref), although this repository ships a `models` package with the same module paths.  The reference's sources are
+    not part of this repository, so the loader is pointed at a stand-in tree of the same layout."""
     import os
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref = os.path.join(root, "baseline", "_ref", "models")
-    if not os.path.isdir(os.path.join(ref, "WindowTransformer")):
-        pytest.skip("baseline/_ref not present")
+    ref = str(tmp_path / "models")
+    for name in MODELS:
+        os.makedirs(os.path.join(ref, name))
+        extra = "from .utils import default_conv  # noqa: F401" if name == "FastTransformer" else ""
+        with open(os.path.join(ref, name, "model.py"), "w") as fh:
+            fh.write(_STAND_IN_MODEL.format(extra=extra))
+    with open(os.path.join(ref, "FastTransformer", "utils.py"), "w") as fh:
+        fh.write("def default_conv(*args):\n    return None\n")
     if root not in sys.path:
         sys.path.insert(0, root)
     from baseline.refload import reference_model_class

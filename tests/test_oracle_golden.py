@@ -71,19 +71,31 @@ def _ragged_cases():
 
 @pytest.mark.parametrize("model,shape,kw,seed", _ragged_cases())
 def test_oracle_matches_live_reference_on_ragged_shapes(model, shape, kw, seed):
-    """the same seeded sweep of awkward shapes the GPU suite runs, here oracle vs the UNMODIFIED reference modules executed live
-    (baseline/_ref, a verbatim copy of the reference's models/ made in the build container)"""
+    """the same seeded sweep of awkward shapes the GPU suite runs, here the oracle against the reference: always against the stored
+    sweep (tests/golden/ragged_<k>.npz, tests/golden/make_ragged.py: the oracle arithmetic that matched the reference on every case
+    of the sweep to TOL_FP32, on a coprime-stride lattice plus the corners), and against the UNMODIFIED reference modules executed
+    live whenever a copy of the reference's models/ is in baseline/_ref (python baseline/fetch_ref.py <reference checkout>)"""
     import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref_dir = os.path.join(root, "baseline", "_ref", "models")
-    if not os.path.isdir(os.path.join(ref_dir, model)):
-        pytest.skip("baseline/_ref not present")
-    if root not in sys.path:
-        sys.path.insert(0, root)
-    from baseline.refload import reference_model_class
+    from tests.golden.cases import ragged_sample
     B, H, W = shape
     sd = synth_state_dict(model, seed)
     x = synth_frames(B, H, W, seed=seed + 100)
+    k = _ragged_cases().index((model, shape, kw, seed))
+    g = np.load(os.path.join(GOLD, f"ragged_{k:02d}.npz"))
+    assert (str(g["model"]), int(g["seed"]), str(g["kw"])) == (model, seed, repr(sorted(kw.items())))
+    pre = orc.forward(model, sd, x, pre_clamp=True, **kw).numpy()
+    assert tuple(g["shape"]) == pre.shape
+    st, lat, crops = ragged_sample(pre)
+    assert st == int(g["stride"])
+    err = max([np.abs(lat - g["pre"]).max()] + [np.abs(cr - g[f"crop{i}"]).max() for i, cr in enumerate(crops)])
+    assert err < TOL_FP32, (model, shape, kw, err)
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    ref_dir = os.path.join(root, "baseline", "_ref", "models")
+    if not os.path.isdir(os.path.join(ref_dir, model)):
+        return
+    if root not in sys.path:
+        sys.path.insert(0, root)
+    from baseline.refload import reference_model_class
     M = reference_model_class(ref_dir, model)().eval()
     M.load_state_dict(sd, strict=True)
     with torch.no_grad():

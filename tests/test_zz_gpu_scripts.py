@@ -26,8 +26,9 @@ def _env(extra=()):
 
 
 def _need(script):
+    # the reference's sources are not part of this repository: without a copy in baseline/_ref there is nothing to run
     if not os.path.exists(os.path.join(REF, script)):
-        pytest.skip(f"baseline/_ref/{script} not present (run baseline/fetch_ref.py in the build container)")
+        pytest.skip(f"needs the reference's {script} in baseline/_ref (python baseline/fetch_ref.py <reference checkout>)")
 
 
 def _png(path, h, w, seed):
@@ -35,6 +36,36 @@ def _png(path, h, w, seed):
     yy, xx = np.meshgrid(np.linspace(0, 1, h), np.linspace(0, 1, w), indexing="ij")
     img = np.stack([0.5 + 0.4 * np.sin(6.28 * (rs.uniform(1, 4) * xx + rs.uniform(1, 4) * yy)) for _ in range(3)], -1)
     Image.fromarray((img * 255).astype(np.uint8)).save(path)
+
+
+@pytest.mark.parametrize("model,shape,kw,autocast_fp16", [
+    ("WindowTransformer", (90, 160), dict(res_out=(2160, 3840)), False),      # speed_test.py:60-67
+    ("FastTransformer", (120, 200), dict(upscale_factor=3), True),             # inference.py:117-123
+    ("FastTransformer", (120, 200), dict(upscale_factor=4), True),
+    ("WindowTransformer", (120, 200), dict(upscale_factor=2), True)])
+def test_reference_call_patterns_run_on_the_drop_in_models(tmp_path, model, shape, kw, autocast_fp16):
+    """The scripts' call patterns without the scripts (the two tests below run the reference's own files when they are present):
+    the class found through importlib.import_module("models.<M>.model"), a checkpoint saved as a state_dict with the reference's
+    keys and loaded with torch.load(map_location=device), then model(lr, res_out=(2160, 3840)) under no_grad, or
+    model(x, upscale_factor=s) under torch.autocast(float16); the result against the CPU oracle."""
+    import importlib
+    from oracle import upscaler_oracle as orc
+    from oracle.weights import synth_frames
+    ckpt = tmp_path / "model_epoch_1.pth"
+    torch.save(synth_state_dict(model, 5), str(ckpt))
+    cls = importlib.import_module(f"models.{model}.model").TransformerModel
+    assert cls.__module__.startswith("transformerupscaler_b200.")
+    M = cls().to("cuda")
+    M.load_state_dict(torch.load(str(ckpt), map_location="cuda"))
+    M.eval()
+    x = synth_frames(1, *shape, seed=6)
+    with torch.no_grad(), torch.autocast("cuda", dtype=torch.float16, enabled=autocast_fp16):
+        y = M(x.cuda(), **kw)
+    ref = orc.forward(model, synth_state_dict(model, 5), x, **kw)
+    assert tuple(y.shape) == tuple(ref.shape)
+    # under autocast the reference's FastTransformer ends in convs (low-precision output); the other two end in fp32 ops
+    assert y.dtype == (torch.float16 if autocast_fp16 and model == "FastTransformer" else torch.float32)
+    assert (y.float().cpu() - ref).abs().max().item() < (2e-2 if autocast_fp16 else 1e-4)
 
 
 def test_reference_speed_test_script_runs_on_the_drop_in_models(tmp_path):

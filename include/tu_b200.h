@@ -10,7 +10,7 @@
  *   - the caller owns every buffer; the library never allocates or frees device memory, never
  *     synchronises the device, and enqueues all work on `stream` (a cudaStream_t passed as void*);
  *   - return value 0 = success, negative = error; tu_last_error() gives the message (thread-local);
- *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 (image input / output only);
+ *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 and TU_F16 = 3 (both image input / output only);
  *   - activations inside the engine are NHWC (64 channels); images at the boundary are NCHW, like
  *     the reference's tensors.
  */
@@ -28,6 +28,10 @@ extern "C" {
 #define TU_BF16 1
 #define TU_U8 2   /* image I/O only (in_dtype / out_dtype of tu_forward, tu_stem_conv, tu_bicubic_add_clamp,        */
                   /* tu_final_conv_add): uint8 frames, x/255 on read (ToTensor), trunc(clamp(v*255,0,255)) on write  */
+#define TU_F16 3  /* image I/O only (in_dtype / out_dtype of tu_forward, tu_stem_conv, tu_conv12_fused, tu_bicubic_add_clamp,  */
+                  /* tu_subpixel_conv_add, tu_final_conv_add, tu_resize_bilinear_aa[_to]); never a compute dtype: an fp16    */
+                  /* model runs on the TU_BF16 (or TU_F32) path.  Read exactly into fp32 registers; the fp32 result is        */
+                  /* rounded to fp16 once, at the store, so fp16 output == (the fp32-output call on the same values).half() */
 
 /* uint8 frame layouts (OR-ed into TU_U8 for the image input / output of tu_forward, and for the output of tu_bicubic_add_clamp,
  * tu_subpixel_conv_add and tu_resize_bilinear_aa_to): planar CHW is the default (the reference's tensors); HWC is what PIL /
@@ -179,7 +183,8 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
 /* ---- whole-model forward (what TransformerModel.forward calls) --------------------------------
  * x:   (B,3,H,W) NCHW, dtype in_dtype.     out: (B,3,outH,outW) NCHW, dtype out_dtype, clamped to [0,1]
  *      (or un-clamped when clamp == 0; tests compare pre-clamp tensors).
- * compute_dtype: TU_F32 (exact fp32 FFMA path) or TU_BF16 (bf16 operands, fp32 accumulate).
+ * compute_dtype: TU_F32 (exact fp32 FFMA path) or TU_BF16 (bf16 operands, fp32 accumulate); TU_F16 is rejected (TU_ERR_ARG,
+ *      and a workspace size of 0).  in_dtype / out_dtype: TU_F32, TU_BF16, TU_F16 or TU_U8 [| layout] for either compute dtype.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.

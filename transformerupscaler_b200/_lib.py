@@ -11,7 +11,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libtu_b200.so")
 
-TU_F32, TU_BF16, TU_U8 = 0, 1, 2
+TU_F32, TU_BF16, TU_U8, TU_F16 = 0, 1, 2, 3      # TU_U8 and TU_F16: image input / output only, never a compute dtype
 TU_LAYOUT_HWC, TU_LAYOUT_HWC_BGR = 0x100, 0x200      # OR-ed into TU_U8 for interleaved uint8 frames
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}

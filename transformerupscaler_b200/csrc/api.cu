@@ -2,6 +2,7 @@
 // forward drivers that enqueue every kernel of a TransformerModel.forward on the caller's stream.
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <vector>
@@ -101,6 +102,14 @@ static int patch_unembed(const float *tok, const T *w, const float *b, const T *
     return launch_gemm_simt<T>(a, wd, M, 4096, dim, e, st, "patch_unembed");
 }
 
+// fp16 frame -> fp32 frame (exact).  Used where an fp16 frame's rows cannot be addressed by TMA but fp32 rows can (W % 8 == 4), so
+// that the frame takes the fused conv1+conv2 kernel like the fp32 frame of the same values, and gives its bits.
+__global__ void __launch_bounds__(256) widen_f16_kernel(const f16 *__restrict__ in, float *__restrict__ out, long n) {
+    pdl_trigger();
+    pdl_wait();
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) out[i] = __half2float(in[i]);
+}
+
 // ------------------------------------------------------------------ workspace arena
 struct Arena {
     char *base;
@@ -158,6 +167,17 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
         if ((rc = tu_frames_to_planar(x, dtype_layout(in_dtype) << 8, xplanar, B, H, W, stv))) return rc;
         x = xplanar;
         in_dtype = TU_U8;
+    }
+    // (sized on every pass whose width needs it: the workspace queries do not know the input dtype)
+    float *xwide = (W % 8) == 4 ? (float *)a.get((size_t)B * 3 * H * W * sizeof(float)) : nullptr;
+    if (!dry && xwide && dtype_base(in_dtype) == TU_F16 && tc_on(dt) && w->conv1_w64) {
+        const long n = (long)B * 3 * H * W;
+        const cudaError_t e = launch_pdl(widen_f16_kernel, dim3((unsigned)std::min<long>((n + 255) / 256, 4096)), dim3(256), 0, st,
+                                         (const f16 *)x, xwide, n);
+        if (e != cudaSuccess) return cuda_fail(e, "widen_f16");
+        count_launch();
+        x = xwide;
+        in_dtype = TU_F32;
     }
     const size_t full = (size_t)B * H * W * 64 * sizeof(T);
     T *f1 = (T *)a.get(full);
@@ -562,7 +582,7 @@ extern "C" int tu_dec12_fused(const void *in, const void *w1, const float *b1, c
 extern "C" int tu_conv12_fused(const void *x, int in_dtype, const void *w64, const float *b1, const void *w2, const float *b2, void *out,
                                int B, int H, int W, void *stream) {
     TU_CHECK_ARG(x && w64 && b1 && w2 && out && B > 0 && H > 0 && W > 0, "conv12_fused: bad argument");
-    TU_CHECK_ARG(in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_U8, "conv12_fused: bad input dtype");
+    TU_CHECK_ARG(in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_F16 || in_dtype == TU_U8, "conv12_fused: bad input dtype");
     TU_CHECK_ARG(tc_enabled(), "conv12_fused: tcgen05 kernels are unavailable or switched off");
     int rc = tc_conv12_fused(x, in_dtype, (const bf16 *)w64, b1, (const bf16 *)w2, b2, (bf16 *)out, B, H, W, (cudaStream_t)stream);
     TU_CHECK_ARG(rc != TU_TC_UNSUPPORTED, "conv12_fused: unsupported alignment (image row pitch must be a multiple of 16 bytes) or switched off");
@@ -673,7 +693,8 @@ extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, 
     TU_CHECK_ARG(x && out && workspace, "forward: null buffer");
     {
         const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype), il = dtype_layout(in_dtype), ol = dtype_layout(out_dtype);
-        TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_U8) && (ob == TU_F32 || ob == TU_BF16 || ob == TU_U8), "forward: bad i/o dtype");
+        TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8) && (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8),
+                     "forward: bad i/o dtype");
         TU_CHECK_ARG((il == 0 || (ib == TU_U8 && il <= 2)) && (ol == 0 || (ob == TU_U8 && ol <= 2)),
                      "forward: interleaved layouts (TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR) are for uint8 frames");
     }

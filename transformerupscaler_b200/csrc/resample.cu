@@ -58,6 +58,7 @@ constexpr int BS_W = 128, BS_H = 32;
 // element as stored -> float, and the factor applied once per 4-tap sum (uint8 frames: 1/255, ToTensor)
 __device__ __forceinline__ float raw_f(float v) { return v; }
 __device__ __forceinline__ float raw_f(bf16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float raw_f(f16 v) { return __half2float(v); }
 __device__ __forceinline__ float raw_f(uint8_t v) { return u8_to_float(v); }
 template <typename TS> __device__ __forceinline__ float src_scale(float t) { return t; }
 template <> __device__ __forceinline__ float src_scale<uint8_t>(float t) { return t * 0.00392156862745098f; }
@@ -147,6 +148,11 @@ template <int OFF> __device__ __forceinline__ float lds_raw(uint32_t a, bf16) {
     unsigned short h;
     asm("ld.shared.u16 %0, [%1+%2];" : "=h"(h) : "r"(a), "n"(OFF * 2));
     return __uint_as_float((uint32_t)h << 16);
+}
+template <int OFF> __device__ __forceinline__ float lds_raw(uint32_t a, f16) {
+    unsigned short h;
+    asm("ld.shared.u16 %0, [%1+%2];" : "=h"(h) : "r"(a), "n"(OFF * 2));
+    return __half2float(__ushort_as_half(h));
 }
 template <int OFF> __device__ __forceinline__ float lds_raw(uint32_t a, uint8_t) {
     unsigned short h;
@@ -356,6 +362,7 @@ __device__ __forceinline__ void slide_pair(ptx::f32x2 (&win)[3][4], int &cur, in
 }
 __device__ __forceinline__ void store_pair(float *o, float a, float b) { *reinterpret_cast<float2 *>(o) = make_float2(a, b); }
 __device__ __forceinline__ void store_pair(bf16 *o, float a, float b) { *reinterpret_cast<__nv_bfloat162 *>(o) = __floats2bfloat162_rn(a, b); }
+__device__ __forceinline__ void store_pair(f16 *o, float a, float b) { *reinterpret_cast<__half2 *>(o) = __floats2half2_rn(a, b); }
 __device__ __forceinline__ void store_pair(uint8_t *o, float a, float b) {
     *reinterpret_cast<unsigned short *>(o) = (unsigned short)((unsigned)from_f<uint8_t>(a) | ((unsigned)from_f<uint8_t>(b) << 8));
 }
@@ -481,6 +488,13 @@ template <> __device__ __forceinline__ void clamp_store_pair<bf16>(bf16 *o, floa
     asm("min.bf16x2 %0, %0, %1;" : "+r"(d) : "r"(0x3f803f80u));
     *reinterpret_cast<uint32_t *>(o) = d;
 }
+// fp16: the same identity (1.0 = 0x3c00 is an fp16 and rounding to fp16 is monotonic as well)
+template <> __device__ __forceinline__ void clamp_store_pair<f16>(f16 *o, float lo, float hi) {
+    uint32_t d;
+    asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
+    asm("min.f16x2 %0, %0, %1;" : "+r"(d) : "r"(0x3c003c00u));
+    *reinterpret_cast<uint32_t *>(o) = d;
+}
 
 // one value already clamped to [0, 1] -> the output element (uint8: the same product and round-down add as from_f<uint8_t>, whose clamp
 // is a no-op here; the low byte of the sum is the result)
@@ -511,6 +525,17 @@ template <> __device__ __forceinline__ void ld6<bf16>(uint32_t a, float (&e)[6])
     e[0] = __uint_as_float(__byte_perm(w0, 0u, 0x1044)); e[1] = __uint_as_float(w0 & 0xffff0000u);
     e[2] = __uint_as_float(__byte_perm(w1, 0u, 0x1044)); e[3] = __uint_as_float(w1 & 0xffff0000u);
     e[4] = __uint_as_float(__byte_perm(w2, 0u, 0x1044)); e[5] = __uint_as_float(w2 & 0xffff0000u);
+}
+// fp16: the same three aligned words, each half converted exactly (cvt.f32.f16; fp16 -> fp32 never rounds)
+template <> __device__ __forceinline__ void ld6<f16>(uint32_t a, float (&e)[6]) {
+    uint32_t w0, w1, w2;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w0) : "r"(a));
+    asm volatile("ld.shared.u32 %0, [%1+4];" : "=r"(w1) : "r"(a));
+    asm volatile("ld.shared.u32 %0, [%1+8];" : "=r"(w2) : "r"(a));
+    const float2 f0 = __half22float2(*reinterpret_cast<const __half2 *>(&w0));
+    const float2 f1 = __half22float2(*reinterpret_cast<const __half2 *>(&w1));
+    const float2 f2 = __half22float2(*reinterpret_cast<const __half2 *>(&w2));
+    e[0] = f0.x; e[1] = f0.y; e[2] = f1.x; e[3] = f1.y; e[4] = f2.x; e[5] = f2.y;
 }
 template <> __device__ __forceinline__ void ld6<uint8_t>(uint32_t a, float (&e)[6]) {
     unsigned short h0, h1, h2;
@@ -1002,14 +1027,15 @@ using namespace tu;
 thread_local int tu::g_bicubic_tile = 0;      // debug key "bicubic_tile": rows per CTA of the row-schedule kernel: 0 = by grid size (default), 1 = the smaller tile, 2 = the larger
 thread_local int tu::g_bicubic_pair = 2;      // debug key "bicubic_pair": 2 = two output columns per thread + the unrolled fixed-row-pattern kernel where it applies (default), 3 = the same with the streaming form of that kernel (measured slower), 1 = the pair kernel only, 0 = the one-column strip kernel
 
-// (W, H, 3, B) view of an NCHW image for the tile loads; box = (cols, rows, 3, 1)
-static bool encode_image_map(CUtensorMap *tm, const void *ptr, int elem_bytes, int B, int H, int W, int box_rows, int box_cols) {
+// (W, H, 3, B) view of an NCHW image of dtype code `dtype` for the tile loads; box = (cols, rows, 3, 1)
+static bool encode_image_map(CUtensorMap *tm, const void *ptr, int dtype, int B, int H, int W, int box_rows, int box_cols) {
     TcEncodeFn enc = tc_encode_fn();
+    const int elem_bytes = (int)dtype_size(dtype);
     if (!enc || box_rows > 256 || box_cols > 256) return false;
     cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
     cuuint64_t strides[3] = {(cuuint64_t)W * elem_bytes, (cuuint64_t)H * W * elem_bytes, (cuuint64_t)3 * H * W * elem_bytes};
     cuuint32_t box[4] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, 3, 1}, es[4] = {1, 1, 1, 1};
-    return enc(tm, elem_bytes == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void *)ptr, dims, strides,
+    return enc(tm, tc_image_map_dtype(dtype), 4, (void *)ptr, dims, strides,
                box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -1019,7 +1045,8 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
     TU_CHECK_ARG(x && out && B > 0 && H > 0 && W > 0 && outH > 0 && outW > 0, "bicubic_add_clamp: bad argument");
     const int layout = dtype_layout(out_dtype);
     out_dtype = dtype_base(out_dtype);
-    TU_CHECK_ARG((in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_U8) && (out_dtype == TU_F32 || out_dtype == TU_BF16 || out_dtype == TU_U8),
+    TU_CHECK_ARG((in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_F16 || in_dtype == TU_U8) &&
+                     (out_dtype == TU_F32 || out_dtype == TU_BF16 || out_dtype == TU_F16 || out_dtype == TU_U8),
                  "bicubic_add_clamp: bad dtype");
     TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout <= 2), "bicubic_add_clamp: interleaved layouts are for uint8 frames");
     cudaStream_t st = (cudaStream_t)stream;
@@ -1041,12 +1068,12 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
         memset(&tr, 0, sizeof(tr));
         bool ok = tile_bytes <= 96 * 1024 && ((size_t)W * eb) % 16 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
                   (!res || (((size_t)rW * 4) % 16 == 0 && (reinterpret_cast<uintptr_t>(res) & 15) == 0));
-        return ok && encode_image_map(&tx, x, eb, B, H, W, g.xr, g.xc) && (!res || encode_image_map(&tr, res, 4, B, rH, rW, g.rr, g.rc));
+        return ok && encode_image_map(&tx, x, in_dtype, B, H, W, g.xr, g.xc) && (!res || encode_image_map(&tr, res, TU_F32, B, rH, rW, g.rr, g.rc));
     };
     // two output columns per thread: TMA tiles, even output width, pair stores aligned
     const bool pair = g_bicubic_pair && (outW % 2) == 0 && (reinterpret_cast<uintptr_t>(out) % (2 * ob)) == 0 && plan(PAIR_H);
     // periodic row schedules (x1.5 outputs such as 720p -> 1080p, x3 outputs such as 720p -> 4K): the unrolled circular-window kernel
-    const int pat = pair && g_bicubic_pair >= 2 && res && clamp && (in_dtype == TU_BF16 || in_dtype == TU_U8) &&
+    const int pat = pair && g_bicubic_pair >= 2 && res && clamp && (in_dtype == TU_BF16 || in_dtype == TU_F16 || in_dtype == TU_U8) &&
                             W <= outW && rW <= outW
                         ? row_pattern(H, rH, outH)
                         : -1;
@@ -1133,7 +1160,7 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
         else TU_BIC_R32_P(TI, TO, 6, HWC);                                                                                      \
     } while (0)
 #define TU_BIC_R32(TI, TO) TU_BIC_R32_L(TI, TO, false)
-    if (r32 && pat == 0 && layout == 0 && g_bicubic_pair >= 3) {
+    if (r32 && pat == 0 && layout == 0 && g_bicubic_pair >= 3 && in_dtype != TU_F16 && out_dtype != TU_F16) {
         // streaming variant: strips x segments co-resident (5 CTAs per SM), <= 16 blocks of 12 rows per segment
         const int nblk = outH / 12, strips = (int)grid.x * B;
         const size_t stage = (((size_t)3 * 8 * g.xc * eb + 127) & ~(size_t)127) + (((size_t)3 * 4 * g.rc * 4 + 127) & ~(size_t)127);
@@ -1146,7 +1173,7 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
         CUtensorMap sx, sr;
         memset(&sx, 0, sizeof(sx));
         memset(&sr, 0, sizeof(sr));
-        if (ring_bytes <= 96 * 1024 && encode_image_map(&sx, x, eb, B, H, W, 8, g.xc) && encode_image_map(&sr, res, 4, B, rH, rW, 4, g.rc)) {
+        if (ring_bytes <= 96 * 1024 && encode_image_map(&sx, x, in_dtype, B, H, W, 8, g.xc) && encode_image_map(&sr, res, TU_F32, B, rH, rW, 4, g.rc)) {
             dim3 sgrid(grid.x, nseg, B);
 #define TU_BIC_R32S(TI, TO)                                                                                                     \
     do {                                                                                                                        \
@@ -1173,13 +1200,20 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
     }
     if (r32 && layout != 0) {           // interleaved uint8 frames (layouts are accepted for uint8 output only)
         if (in_dtype == TU_BF16) TU_BIC_R32_L(bf16, uint8_t, true);
+        else if (in_dtype == TU_F16) TU_BIC_R32_L(f16, uint8_t, true);
         else TU_BIC_R32_L(uint8_t, uint8_t, true);
     } else if (r32) {
         if (in_dtype == TU_BF16 && out_dtype == TU_BF16) TU_BIC_R32(bf16, bf16);
         else if (in_dtype == TU_BF16 && out_dtype == TU_F32) TU_BIC_R32(bf16, float);
+        else if (in_dtype == TU_BF16 && out_dtype == TU_F16) TU_BIC_R32(bf16, f16);
         else if (in_dtype == TU_BF16) TU_BIC_R32(bf16, uint8_t);
+        else if (in_dtype == TU_F16 && out_dtype == TU_F16) TU_BIC_R32(f16, f16);
+        else if (in_dtype == TU_F16 && out_dtype == TU_F32) TU_BIC_R32(f16, float);
+        else if (in_dtype == TU_F16 && out_dtype == TU_BF16) TU_BIC_R32(f16, bf16);
+        else if (in_dtype == TU_F16) TU_BIC_R32(f16, uint8_t);
         else if (out_dtype == TU_U8) TU_BIC_R32(uint8_t, uint8_t);
         else if (out_dtype == TU_BF16) TU_BIC_R32(uint8_t, bf16);
+        else if (out_dtype == TU_F16) TU_BIC_R32(uint8_t, f16);
         else TU_BIC_R32(uint8_t, float);
     } else
     if (in_dtype == TU_F32 && out_dtype == TU_F32) TU_BIC2(float, float);
@@ -1190,6 +1224,13 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
     else if (in_dtype == TU_U8 && out_dtype == TU_F32) TU_BIC2(uint8_t, float);
     else if (in_dtype == TU_U8 && out_dtype == TU_BF16) TU_BIC2(uint8_t, bf16);
     else if (in_dtype == TU_F32 && out_dtype == TU_U8) TU_BIC2(float, uint8_t);
+    else if (in_dtype == TU_F16 && out_dtype == TU_F16) TU_BIC2(f16, f16);
+    else if (in_dtype == TU_F16 && out_dtype == TU_F32) TU_BIC2(f16, float);
+    else if (in_dtype == TU_F16 && out_dtype == TU_BF16) TU_BIC2(f16, bf16);
+    else if (in_dtype == TU_F16 && out_dtype == TU_U8) TU_BIC2(f16, uint8_t);
+    else if (in_dtype == TU_F32 && out_dtype == TU_F16) TU_BIC2(float, f16);
+    else if (in_dtype == TU_BF16 && out_dtype == TU_F16) TU_BIC2(bf16, f16);
+    else if (in_dtype == TU_U8 && out_dtype == TU_F16) TU_BIC2(uint8_t, f16);
     else TU_BIC2(bf16, uint8_t);
 #undef TU_BIC2
 #undef TU_BIC_R32
@@ -1218,6 +1259,12 @@ extern "C" int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out,
     else if (in_dtype == TU_BF16 && out_dtype == TU_F32) TU_RS(bf16, float);
     else if (in_dtype == TU_F32 && out_dtype == TU_U8) TU_RS(float, uint8_t);
     else if (in_dtype == TU_BF16 && out_dtype == TU_U8) TU_RS(bf16, uint8_t);
+    else if (in_dtype == TU_F16 && out_dtype == TU_F16) TU_RS(f16, f16);
+    else if (in_dtype == TU_F16 && out_dtype == TU_F32) TU_RS(f16, float);
+    else if (in_dtype == TU_F16 && out_dtype == TU_BF16) TU_RS(f16, bf16);
+    else if (in_dtype == TU_F16 && out_dtype == TU_U8) TU_RS(f16, uint8_t);
+    else if (in_dtype == TU_F32 && out_dtype == TU_F16) TU_RS(float, f16);
+    else if (in_dtype == TU_BF16 && out_dtype == TU_F16) TU_RS(bf16, f16);
     else TU_CHECK_ARG(false, "resize_bilinear_aa: bad dtype");
 #undef TU_RS
     TU_CHECK_LAUNCH("resize_bilinear_aa");
@@ -1226,7 +1273,7 @@ extern "C" int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out,
 
 extern "C" int tu_resize_bilinear_aa(const void *in, int dtype, void *out, int B, int H, int W, int outH, int outW,
                                      int clamp, void *stream) {
-    TU_CHECK_ARG(dtype == TU_F32 || dtype == TU_BF16, "resize_bilinear_aa: bad dtype");
+    TU_CHECK_ARG(dtype == TU_F32 || dtype == TU_BF16 || dtype == TU_F16, "resize_bilinear_aa: bad dtype");
     return tu_resize_bilinear_aa_to(in, dtype, out, dtype, B, H, W, outH, outW, clamp, stream);
 }
 

@@ -172,7 +172,7 @@ using namespace tu;
 extern "C" int tu_stem_conv(const void *x, int in_dtype, const float *w27x64, const void *w64, const float *b, void *out,
                             int dtype, int B, int H, int W, void *stream) {
     TU_CHECK_ARG(x && w27x64 && b && out && B > 0 && H > 0 && W > 0, "stem_conv: bad argument");
-    TU_CHECK_ARG(in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_U8, "stem_conv: bad input dtype");
+    TU_CHECK_ARG(in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_F16 || in_dtype == TU_U8, "stem_conv: bad input dtype");
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == TU_BF16 && w64 && tc_enabled()) {
         int rc = tc_stem_conv(x, in_dtype, (const bf16 *)w64, b, (bf16 *)out, B, H, W, st);
@@ -191,6 +191,10 @@ extern "C" int tu_stem_conv(const void *x, int in_dtype, const float *w27x64, co
         stem_conv_kernel<uint8_t, float><<<grid, 256, 0, st>>>((const uint8_t *)x, w27x64, b, (float *)out, H, W);
     else if (in_dtype == TU_U8 && dtype == TU_BF16)
         stem_conv_kernel<uint8_t, bf16><<<grid, 256, 0, st>>>((const uint8_t *)x, w27x64, b, (bf16 *)out, H, W);
+    else if (in_dtype == TU_F16 && dtype == TU_F32)
+        stem_conv_kernel<f16, float><<<grid, 256, 0, st>>>((const f16 *)x, w27x64, b, (float *)out, H, W);
+    else if (in_dtype == TU_F16 && dtype == TU_BF16)
+        stem_conv_kernel<f16, bf16><<<grid, 256, 0, st>>>((const f16 *)x, w27x64, b, (bf16 *)out, H, W);
     else
         TU_CHECK_ARG(false, "stem_conv: bad dtype");
     TU_CHECK_LAUNCH("stem_conv");
@@ -238,6 +242,8 @@ extern "C" int tu_final_conv_add(const float *in, const float *w, const float *b
         final_conv_add_kernel<bf16><<<grid, 256, 0, st>>>(in, w, b, addend, (bf16 *)out, H, W, clamp);
     else if (out_dtype == TU_U8)
         final_conv_add_kernel<uint8_t><<<grid, 256, 0, st>>>(in, w, b, addend, (uint8_t *)out, H, W, clamp);
+    else if (out_dtype == TU_F16)
+        final_conv_add_kernel<f16><<<grid, 256, 0, st>>>(in, w, b, addend, (f16 *)out, H, W, clamp);
     else
         TU_CHECK_ARG(false, "final_conv_add: bad dtype");
     TU_CHECK_LAUNCH("final_conv_add");

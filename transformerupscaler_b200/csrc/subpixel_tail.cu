@@ -272,5 +272,6 @@ extern "C" int tu_subpixel_conv_add(const float *in, const float *w_ps, const fl
     if (out_dtype == TU_F32) return tail_by_r<float>(r, in, w_ps, b_ps, addend, (float *)out, B, H, W, clamp, layout, fin, st);
     if (out_dtype == TU_BF16) return tail_by_r<bf16>(r, in, w_ps, b_ps, addend, (bf16 *)out, B, H, W, clamp, layout, fin, st);
     if (out_dtype == TU_U8) return tail_by_r<uint8_t>(r, in, w_ps, b_ps, addend, (uint8_t *)out, B, H, W, clamp, layout, fin, st);
+    if (out_dtype == TU_F16) return tail_by_r<f16>(r, in, w_ps, b_ps, addend, (f16 *)out, B, H, W, clamp, layout, fin, st);
     TU_CHECK_ARG(false, "subpixel_conv_add: bad dtype");
 }

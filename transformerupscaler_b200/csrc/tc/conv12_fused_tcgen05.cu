@@ -78,6 +78,7 @@ static_assert(sizeof(FusedBarriers) <= 384, "barrier block too large (the last 2
 
 __device__ __forceinline__ float ldx(float v) { return v; }
 __device__ __forceinline__ float ldx(bf16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float ldx(f16 v) { return __half2float(v); }
 __device__ __forceinline__ float ldx(uint8_t v) { return u8_to_float(v) * 0.00392156862745098f; }
 __device__ __forceinline__ uint32_t pack2_relu(float lo, float hi) {
     uint32_t d;
@@ -510,12 +511,12 @@ thread_local int g_enable_fused = 1;
 
 void tc_set_conv12_fused(int on) { g_enable_fused = on; }
 
-// relu(conv2(relu(conv1(x)))): NCHW image (fp32 | bf16 | uint8) -> NHWC bf16 (B,H,W,64).  w64: conv1 filter bf16 (64 co, 64 k);
+// relu(conv2(relu(conv1(x)))): NCHW image (fp32 | bf16 | fp16 | uint8) -> NHWC bf16 (B,H,W,64).  w64: conv1 filter bf16 (64 co, 64 k);
 // w2: conv2 filter bf16 [9 taps][64 co][64 ci].  Needs an image row pitch that is a multiple of 16 bytes (raw rows arrive by TMA).
 int tc_conv12_fused(const void *x, int in_dtype, const bf16 *w64, const float *bias1, const bf16 *w2, const float *bias2, bf16 *out,
                     int B, int H, int W, cudaStream_t st) {
     if (!g_enable_fused) return TU_TC_UNSUPPORTED;
-    const int eb = in_dtype == TU_F32 ? 4 : in_dtype == TU_BF16 ? 2 : 1;
+    const int eb = (int)dtype_size(in_dtype);
     if (((size_t)W * eb) % 16 || (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(w64) & 127) ||
         (reinterpret_cast<uintptr_t>(w2) & 127) || (reinterpret_cast<uintptr_t>(out) & 15))
         return TU_TC_UNSUPPORTED;
@@ -526,6 +527,7 @@ int tc_conv12_fused(const void *x, int in_dtype, const bf16 *w64, const float *b
         cudaError_t e = cudaFuncSetAttribute(conv12_fused_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(conv12_fused_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(conv12_fused_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(conv12_fused_kernel<f16>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
         if (e != cudaSuccess) return cuda_fail(e, "conv12_fused smem attribute");
         g_attr_set_c.set();
     }
@@ -535,8 +537,7 @@ int tc_conv12_fused(const void *x, int in_dtype, const bf16 *w64, const float *b
         cuuint64_t xd[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
         cuuint64_t xs[3] = {(cuuint64_t)W * eb, (cuuint64_t)H * W * eb, (cuuint64_t)3 * H * W * eb};
         cuuint32_t xb[4] = {(cuuint32_t)rw, 1, 3, 1}, e1[4] = {1, 1, 1, 1};
-        CUresult r = enc(&tm_x, eb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : eb == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8,
-                         4, const_cast<void *>(x), xd, xs, xb, e1, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+        CUresult r = enc(&tm_x, tc_image_map_dtype(in_dtype), 4, const_cast<void *>(x), xd, xs, xb, e1, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
                          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         cuuint64_t w1d[2] = {64, 64}, wst[1] = {128};
         cuuint32_t wb[2] = {64, 64};
@@ -576,6 +577,7 @@ int tc_conv12_fused(const void *x, int in_dtype, const bf16 *w64, const float *b
     const int grid = p.total_items < g_sm_count_c ? p.total_items : g_sm_count_c;
     if (in_dtype == TU_F32) launch_pdl(conv12_fused_kernel<float>, dim3(grid), dim3(NUM_THREADS), SMEM_BYTES, st, tm_x, tm_w1, tm_w2, tm_out, p);
     else if (in_dtype == TU_BF16) launch_pdl(conv12_fused_kernel<bf16>, dim3(grid), dim3(NUM_THREADS), SMEM_BYTES, st, tm_x, tm_w1, tm_w2, tm_out, p);
+    else if (in_dtype == TU_F16) launch_pdl(conv12_fused_kernel<f16>, dim3(grid), dim3(NUM_THREADS), SMEM_BYTES, st, tm_x, tm_w1, tm_w2, tm_out, p);
     else launch_pdl(conv12_fused_kernel<uint8_t>, dim3(grid), dim3(NUM_THREADS), SMEM_BYTES, st, tm_x, tm_w1, tm_w2, tm_out, p);
     TU_CHECK_LAUNCH("conv12_fused");
     return TU_OK;

@@ -51,6 +51,7 @@ struct Barriers {
 // image element -> float for the bf16 operand (uint8 frames: x * (1/255); the product is rounded to bf16 right after)
 __device__ __forceinline__ float ldx(float v) { return v; }
 __device__ __forceinline__ float ldx(bf16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float ldx(f16 v) { return __half2float(v); }
 __device__ __forceinline__ float ldx(uint8_t v) { return u8_to_float(v) * 0.00392156862745098f; }
 
 // (lo, hi) -> bf16x2 with ReLU in the same instruction
@@ -318,6 +319,7 @@ int tc_stem_conv(const void *x, int in_dtype, const bf16 *w64, const float *bias
         TU_STEM_ATTR(float, false); TU_STEM_ATTR(float, true);
         TU_STEM_ATTR(bf16, false); TU_STEM_ATTR(bf16, true);
         TU_STEM_ATTR(uint8_t, false); TU_STEM_ATTR(uint8_t, true);
+        TU_STEM_ATTR(f16, false); TU_STEM_ATTR(f16, true);
 #undef TU_STEM_ATTR
         if (e != cudaSuccess) return cuda_fail(e, "stem_tc smem attribute");
         g_attr_set.set();
@@ -350,7 +352,7 @@ int tc_stem_conv(const void *x, int in_dtype, const bf16 *w64, const float *bias
     p.bias = bias; p.out = out;
     const int grid = p.total_tiles < 2 * g_sm_count ? p.total_tiles : 2 * g_sm_count;
     // raw image tiles by TMA when the row pitch allows it: (W, H, 3, B) view, box (RW, ROWS + 2, 3, 1)
-    const int eb = in_dtype == TU_F32 ? 4 : in_dtype == TU_BF16 ? 2 : 1;
+    const int eb = (int)dtype_size(in_dtype);
     const int rw = 128 + 2 * (16 / eb);
     CUtensorMap tx;
     memset(&tx, 0, sizeof(tx));
@@ -359,7 +361,7 @@ int tc_stem_conv(const void *x, int in_dtype, const bf16 *w64, const float *bias
         cuuint64_t xd[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
         cuuint64_t xs[3] = {(cuuint64_t)W * eb, (cuuint64_t)H * W * eb, (cuuint64_t)3 * H * W * eb};
         cuuint32_t xb[4] = {(cuuint32_t)rw, ROWS + 2, 3, 1}, xe[4] = {1, 1, 1, 1};
-        raw_tma = enc(&tx, eb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : eb == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8,
+        raw_tma = enc(&tx, tc_image_map_dtype(in_dtype),
                       4, const_cast<void *>(x), xd, xs, xb, xe, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
     }
@@ -372,6 +374,7 @@ int tc_stem_conv(const void *x, int in_dtype, const bf16 *w64, const float *bias
     } while (0)
     if (in_dtype == TU_F32) TU_STEM_LAUNCH(float);
     else if (in_dtype == TU_U8) TU_STEM_LAUNCH(uint8_t);
+    else if (in_dtype == TU_F16) TU_STEM_LAUNCH(f16);
     else TU_STEM_LAUNCH(bf16);
 #undef TU_STEM_LAUNCH
     TU_CHECK_LAUNCH("stem_tc");

@@ -39,6 +39,15 @@ typedef CUresult (*TcEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, v
                                const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 TcEncodeFn tc_encode_fn();
+// TMA element type of an image at the boundary, chosen by dtype code: fp16 and bf16 are both 2 bytes wide and must not share it
+static inline CUtensorMapDataType tc_image_map_dtype(int dtype) {
+    switch (dtype_base(dtype)) {
+        case TU_F32: return CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+        case TU_BF16: return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        case TU_F16: return CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+        default: return CU_TENSOR_MAP_DATA_TYPE_UINT8;
+    }
+}
 
 // C = A W^T GEMMs of the transformer part (gemm_tcgen05.cu).  All return TU_OK, an error, or TU_TC_UNSUPPORTED.
 //   out != nullptr : out[M][N] = act(A W^T + bias) as bf16 (act 0 none, 2 exact GELU)

@@ -1,6 +1,7 @@
 // Shared device/host helpers for libtu_b200 (sm_100a only).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -12,6 +13,7 @@
 namespace tu {
 
 typedef __nv_bfloat16 bf16;
+typedef __half f16;
 
 // ---- error plumbing (host) -------------------------------------------------------------------
 void set_error(const std::string &msg);
@@ -72,6 +74,7 @@ inline int device_sm_count() {                          // SM count of the CURRE
 // ---- scalar load/store with dtype conversion --------------------------------------------------
 __device__ __forceinline__ float to_f(float v) { return v; }
 __device__ __forceinline__ float to_f(bf16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float to_f(f16 v) { return __half2float(v); }      // exact: every fp16 value is an fp32 value
 // uint8 frames: ToTensor semantics on the way in (x / 255 in fp32, inference.py:65-70, app_overlay.py:298) and
 // (out * 255).clamp(0, 255).to(uint8) on the way out (truncation, app_overlay.py:383)
 // exact uint8 -> float without the conversion pipe: 2^23 + v has v in its low mantissa bits
@@ -80,6 +83,7 @@ __device__ __forceinline__ float to_f(uint8_t v) { return u8_to_float(v) / 255.f
 template <typename T> __device__ __forceinline__ T from_f(float v);
 template <> __device__ __forceinline__ float from_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ bf16 from_f<bf16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ f16 from_f<f16>(float v) { return __float2half_rn(v); }
 // trunc(clamp(v * 255, 0, 255)): adding 2^23 with round-down leaves floor(t) in the low mantissa bits (t >= 0)
 template <> __device__ __forceinline__ uint8_t from_f<uint8_t>(float v) {
     return (uint8_t)(__float_as_uint(__fadd_rd(fminf(fmaxf(v * 255.f, 0.f), 255.f), 8388608.f)) & 0xFFu);
@@ -152,6 +156,9 @@ __device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + e
 
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-static inline size_t dtype_size(int dtype) { return (dtype & 0xFF) == TU_BF16 ? 2 : (dtype & 0xFF) == TU_U8 ? 1 : 4; }
+static inline size_t dtype_size(int dtype) {
+    const int d = dtype & 0xFF;
+    return d == TU_BF16 || d == TU_F16 ? 2 : d == TU_U8 ? 1 : 4;
+}
 
 }  // namespace tu

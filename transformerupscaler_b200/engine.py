@@ -18,7 +18,7 @@ import torch
 from . import _lib
 from .packing import PackedWeights
 
-_DT = {torch.float32: _lib.TU_F32, torch.bfloat16: _lib.TU_BF16, torch.uint8: _lib.TU_U8}
+_DT = {torch.float32: _lib.TU_F32, torch.bfloat16: _lib.TU_BF16, torch.float16: _lib.TU_F16, torch.uint8: _lib.TU_U8}
 _TORCH_DT = {v: k for k, v in _DT.items()}
 # handle -> PackedWeights, WEAK: the owner (EngineModel._tu_cache, or a test) keeps the object alive; a handle whose owner is gone
 # simply disappears, so a copied / unpickled module can never release another module's weights and nothing leaks
@@ -49,7 +49,7 @@ def _require_cuda(*ts: torch.Tensor) -> None:
 
 def _code(dt: torch.dtype) -> int:
     if dt not in _DT:
-        raise TypeError(f"unsupported dtype {dt}; the engine handles float32, bfloat16 and (frames only) uint8")
+        raise TypeError(f"unsupported dtype {dt}; the engine handles float32, bfloat16, float16 and (frames only) uint8")
     return _DT[dt]
 
 
@@ -157,7 +157,8 @@ def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int,
     if not need_resize:
         return tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, out_code, clamp, il)
     # Resize is the last op: the un-clamped full-size image stays in the compute dtype and the Resize kernel writes the requested
-    # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store)
-    mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype != torch.float32 else torch.float32)
+    # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store).  fp16 output keeps an fp32
+    # intermediate, so that it is the fp32 result rounded once, at the Resize's store
+    mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) else torch.float32)
     full = tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, mid_code, False, il)
     return tu_resize_aa(full, res_out[0], res_out[1], clamp, out_code)

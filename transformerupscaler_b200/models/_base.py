@@ -126,19 +126,21 @@ class EngineModel(nn.Module):
         return hit[2]
 
     def _select_precision(self, x: torch.Tensor) -> Tuple[bool, torch.dtype]:
-        """(compute in bf16?, output dtype) mirroring what the reference returns for this input/autocast state."""
+        """(compute in bf16?, output dtype) mirroring what the reference returns for this input/autocast state.  An fp16 module
+        runs on the bf16 tensor-core path (or the fp32 one under engine_precision="fp32") and returns fp16: fp16 is an I/O dtype
+        here, and the fp16 result is the fp32 result of that path rounded once."""
         pdt = self.conv1.weight.dtype
-        if pdt not in (torch.float32, torch.bfloat16):
-            raise TypeError(f"unsupported parameter dtype {pdt}: the engine runs fp32 or bf16 modules")
+        if pdt not in (torch.float32, torch.bfloat16, torch.float16):
+            raise TypeError(f"unsupported parameter dtype {pdt}: the engine runs fp32, bf16 or fp16 modules")
         autocast = x.is_cuda and torch.is_autocast_enabled("cuda")
         if self.engine_precision == "fp32":
             bf16 = False
         elif self.engine_precision == "bf16":
             bf16 = True
         else:
-            bf16 = autocast or pdt == torch.bfloat16
-        if pdt == torch.bfloat16:
-            out_dt = torch.bfloat16
+            bf16 = autocast or pdt != torch.float32
+        if pdt != torch.float32:
+            out_dt = pdt
         elif autocast and not self.AUTOCAST_OUT_FP32:
             out_dt = torch.bfloat16
         else:
@@ -160,7 +162,7 @@ class EngineModel(nn.Module):
         # uint8 frames in -> uint8 frames out (ToTensor scaling on read, (out*255).clamp(0,255).to(uint8) on write, fused into
         # the first and last kernels): the video-pipeline entry, an extension of the reference's float-only signature
         frames_u8 = x.dtype == torch.uint8
-        if x.dtype not in (torch.float32, torch.bfloat16, torch.uint8):
+        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8):
             x = x.float()
         bf16, out_dt = self._select_precision(x)
         if frames_u8:

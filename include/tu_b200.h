@@ -41,6 +41,16 @@ extern "C" {
 #define TU_LAYOUT_HWC_BGR 0x200
 #define TU_U8_HWC (TU_U8 | TU_LAYOUT_HWC)
 #define TU_U8_HWC_BGR (TU_U8 | TU_LAYOUT_HWC_BGR)
+/* NV12 video frames (OR-ed into TU_U8 for the image input and / or output of tu_forward, and the code of tu_nv12_to_rgb /
+ * tu_rgb_to_nv12): one uint8 buffer of (3H/2) x W bytes per frame, (B, 3H/2, W) for a batch.  Rows 0..H-1 are the Y plane, the next
+ * H/2 rows hold interleaved chroma pairs (U first) of the 4:2:0 "type 0" siting: chroma co-sited with even luma columns, midway
+ * between luma rows 2i and 2i+1.  H and W must be even.  The colour bits below are valid with TU_LAYOUT_NV12 only, and the input and
+ * output codes carry their own; neither bit = BT.709 limited range.  The frame is converted to / from planar fp16 RGB (the TU_F16
+ * image I/O path) at both ends of the forward. */
+#define TU_LAYOUT_NV12 0x400
+#define TU_YUV_BT601 0x1000         /* BT.601 matrix (Kr, Kb = 0.299, 0.114) instead of BT.709 (0.2126, 0.0722) */
+#define TU_YUV_FULL_RANGE 0x2000    /* full range (Y, C in 0..255) instead of limited (Y 16..235, C 16..240) */
+#define TU_U8_NV12 (TU_U8 | TU_LAYOUT_NV12)
 
 #define TU_OK 0
 #define TU_ERR_ARG (-1)      /* bad argument (shape / dtype / null pointer)              */
@@ -64,7 +74,7 @@ long long tu_launch_count(void);
  * events on the caller's stream (two event records per forward: cheap enough for the timed region); tu_profile_enable(2)
  * brackets EVERY kernel, tagged with the reference op it implements ("conv1", "conv2" (or "conv1_conv2" when fused), "downsample", "patch_embed",
  * "transformer_blocks", "patch_unembed", "decoder_conv1", "decoder_conv2", "bicubic_add_clamp", "up1", "up1_conv",
- * "final_upscale", "final_conv_add").  tu_profile_collect / tu_profile_report synchronise those events (the only
+ * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end).  tu_profile_collect / tu_profile_report synchronise those events (the only
  * calls in the library that wait on the device): collect sums the milliseconds and launches recorded under `name`
  * (NULL = all); report writes "name total_ms launches\n" lines into buf (returns the needed size when buf is NULL);
  * tu_profile_reset drops the records. */
@@ -185,6 +195,9 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      (or un-clamped when clamp == 0; tests compare pre-clamp tensors).
  * compute_dtype: TU_F32 (exact fp32 FFMA path) or TU_BF16 (bf16 operands, fp32 accumulate); TU_F16 is rejected (TU_ERR_ARG,
  *      and a workspace size of 0).  in_dtype / out_dtype: TU_F32, TU_BF16, TU_F16 or TU_U8 [| layout] for either compute dtype.
+ *      TU_U8 | TU_LAYOUT_NV12 [| colour bits]: x is (B, 3H/2, W) and / or out is (B, 3 outH/2, outW), H, W (outH, outW) even; the
+ *      frame is converted to planar fp16 first (the forward is then the TU_F16 one) / the last image kernel writes planar fp16 that
+ *      is converted last (codes saturate at 0 / 255 with clamp == 0 too).  Size the workspace with tu_forward_workspace_bytes_io.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
@@ -192,6 +205,10 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
 size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
 /* the same, sized from the packed weights actually used (non-default dim / heads / n_blocks; which fused kernels are packed) */
 size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
+/* the same for the image input / output codes of the call: equal to tu_forward_workspace_bytes_for for every code pair without
+ * TU_LAYOUT_NV12, larger by the planar fp16 frames of the side(s) that are NV12 (tu_forward needs it then); 0 for a bad code */
+size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype,
+                                     int in_dtype, int out_dtype);
 int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype,
                int B, int H, int W, int outH, int outW, int scale, int compute_dtype, int clamp,
                void *workspace, size_t workspace_bytes, void *stream);
@@ -287,6 +304,17 @@ int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out, int out_dt
 /* uint8 frames (B,H,W,3) interleaved (layout TU_LAYOUT_HWC or TU_LAYOUT_HWC_BGR) -> planar RGB (B,3,H,W) uint8; tu_forward does
  * this itself for an in_dtype that carries a layout (into its workspace) */
 int tu_frames_to_planar(const void *in, int layout, void *out, int B, int H, int W, void *stream);
+/* NV12 frames (B, 3H/2, W) uint8 -> planar RGB (B, 3, H, W) fp16, and back.  code = TU_U8 | TU_LAYOUT_NV12 | colour bits (anything else,
+ * an odd H or W, or B > 65535: TU_ERR_ARG).  Every step is one correctly rounded fp32 operation (no contraction), so the results are exactly
+ * those of the formulas below, with (yo, ys, cs) = (16, 219, 224) limited / (0, 255, 255) full range, Kg = 1 - Kr - Kb and every
+ * coefficient computed in double and rounded once to float:
+ *   to RGB:  chroma upsampled bilinearly (type-0 siting, edges clamped), y' = (Y - yo) / ys, u' = (U - 128) / cs, v' = (V - 128) / cs,
+ *            R = y' + a_rv v', G = (y' + a_gu u') + a_gv v', B = y' + a_bu u', each clamped to [0, 1] and rounded to fp16;
+ *   to NV12: Y' = (Kr R + Kg G) + Kb B per pixel; chroma from the 2-row column sums v(c) filtered (v(2j-1) + 2 v(2j) + v(2j+1)) / 8
+ *            (column 2j-1 clamped at 0), Cb' = (cbR R + cbG G) + 0.5 B, Cr' = (0.5 R + crG G) + crB B; a code is
+ *            min(max(floor(s Y' + o + 0.5), 0), 255) with (s, o) = (219, 16) / (224, 128) limited, (255, 0) / (255, 128) full range. */
+int tu_nv12_to_rgb(const void *nv12, int code, void *rgb_f16, int B, int H, int W, void *stream);
+int tu_rgb_to_nv12(const void *rgb_f16, void *nv12, int code, int B, int H, int W, void *stream);
 
 #ifdef __cplusplus
 }

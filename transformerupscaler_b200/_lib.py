@@ -13,6 +13,8 @@ LIB_PATH = os.path.join(HERE, "libtu_b200.so")
 
 TU_F32, TU_BF16, TU_U8, TU_F16 = 0, 1, 2, 3      # TU_U8 and TU_F16: image input / output only, never a compute dtype
 TU_LAYOUT_HWC, TU_LAYOUT_HWC_BGR = 0x100, 0x200      # OR-ed into TU_U8 for interleaved uint8 frames
+TU_LAYOUT_NV12 = 0x400                               # OR-ed into TU_U8 for NV12 (4:2:0) video frames, (B, 3H/2, W)
+TU_YUV_BT601, TU_YUV_FULL_RANGE = 0x1000, 0x2000     # colour bits of an NV12 code; neither = BT.709 limited range
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}
 
@@ -85,6 +87,7 @@ SIGNATURES = {
     "tu_pack_weights": (i32, [i32, C.POINTER(TuNamedTensor), i32, i32, vp, sz, C.POINTER(TuPackedModel), vp]),
     "tu_forward_workspace_bytes": (sz, [i32] * 8),
     "tu_forward_workspace_bytes_for": (sz, [C.POINTER(TuModelWeights)] + [i32] * 7),
+    "tu_forward_workspace_bytes_io": (sz, [C.POINTER(TuModelWeights)] + [i32] * 9),
     "tu_forward": (i32, [C.POINTER(TuModelWeights), vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp, sz, vp]),
     "tu_stem_conv": (i32, [vp, i32, fp, vp, fp, vp, i32, i32, i32, i32, vp]),
     "tu_conv3x3_c64": (i32, [vp, vp, fp, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp]),
@@ -110,7 +113,16 @@ SIGNATURES = {
     "tu_resize_bilinear_aa_to": (i32, [vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
     "tu_frames_to_planar": (i32, [vp, i32, vp, i32, i32, i32, vp]),
     "tu_bicubic_row_schedule": (i32, [i32, i32, i32]),
+    "tu_nv12_to_rgb": (i32, [vp, i32, vp, i32, i32, i32, vp]),
+    "tu_rgb_to_nv12": (i32, [vp, vp, i32, i32, i32, i32, vp]),
 }
+
+
+
+def dtype_size(code: int) -> int:
+    """bytes per element of an image dtype code (a layout or colour bits do not change it: every uint8 frame is bytes)"""
+    return {TU_F32: 4, TU_BF16: 2, TU_U8: 1, TU_F16: 2}[code & 0xFF]
+
 
 _lib = None
 

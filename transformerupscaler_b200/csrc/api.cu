@@ -161,6 +161,21 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
     const int Mtok = window ? B * nWy * nWx * 64 : B * Ht * Wt;
     const int Hc = fast ? H : min(Hd, 8 * Ht), Wc = fast ? W : min(Wd, 8 * Wt);
 
+    // NV12 frames are converted to planar fp16 first: from then on the frame is an fp16 frame (the W % 8 == 4 widening below
+    // included), and the final bicubic reads the same buffer
+    if (dtype_is_nv12(in_dtype)) {
+        f16 *rgb = (f16 *)a.get((size_t)B * 3 * H * W * sizeof(f16));
+        if (!dry) TU_STEP("nv12_to_rgb", tu_nv12_to_rgb(x, in_dtype, rgb, B, H, W, stv));
+        x = rgb;
+        in_dtype = TU_F16;
+    }
+    // NV12 output: the last image kernel writes planar fp16 here, and tu_rgb_to_nv12 writes `out` from it
+    const bool nv12_out = dtype_is_nv12(out_dtype);
+    void *img = nv12_out ? a.get((size_t)B * 3 * outH * outW * sizeof(f16)) : out;
+    const int img_dtype = nv12_out ? TU_F16 : out_dtype;
+#define TU_NV12_OUT() \
+    if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv))
+
     // interleaved uint8 frames (HWC RGB / BGR) are made planar once; the stem and the final bicubic both read the planar copy
     uint8_t *xplanar = (uint8_t *)a.get((size_t)B * 3 * H * W);
     if (!dry && dtype_layout(in_dtype)) {
@@ -340,7 +355,10 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
     }
 
     if (!fast) {
-        if (!dry) TU_STEP("bicubic_add_clamp", tu_bicubic_add_clamp(x, in_dtype, H, W, res, Hc, Wc, out, out_dtype, B, outH, outW, clamp, stv));
+        if (!dry) {
+            TU_STEP("bicubic_add_clamp", tu_bicubic_add_clamp(x, in_dtype, H, W, res, Hc, Wc, img, img_dtype, B, outH, outW, clamp, stv));
+            TU_NV12_OUT();
+        }
         return TU_OK;
     }
     // ---- FastTransformer branch B: sub-pixel upsample of the residual image, 3->3 conv, sum, clamp
@@ -359,8 +377,9 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
                         set_error("tu: FastTransformer output buffer must be (scale*H, scale*W)");
                         return TU_ERR_ARG;
                     }
-                    TU_STEP("final_upscale_conv_add", tu_subpixel_conv_add(cur, (const float *)sg.w, sg.b, r, w->host_finconv_wb, upA, out,
-                                                                           out_dtype, B, ch, cw, clamp, stv));
+                    TU_STEP("final_upscale_conv_add", tu_subpixel_conv_add(cur, (const float *)sg.w, sg.b, r, w->host_finconv_wb, upA, img,
+                                                                           img_dtype, B, ch, cw, clamp, stv));
+                    TU_NV12_OUT();
                 }
                 return TU_OK;
             }
@@ -375,10 +394,12 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
                 set_error("tu: FastTransformer output buffer must be (scale*H, scale*W)");
                 return TU_ERR_ARG;
             }
-            TU_STEP("final_conv_add", tu_final_conv_add(cur, w->finconv_w, w->finconv_b, upA, out, out_dtype, B, ch, cw, clamp, stv));
+            TU_STEP("final_conv_add", tu_final_conv_add(cur, w->finconv_w, w->finconv_b, upA, img, img_dtype, B, ch, cw, clamp, stv));
+            TU_NV12_OUT();
         }
     }
     return TU_OK;
+#undef TU_NV12_OUT
 }
 
 }  // namespace tu
@@ -685,14 +706,41 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
     return rc == TU_OK ? a.off : 0;
 }
 
+// NV12 codes are TU_U8 | TU_LAYOUT_NV12 [| colour bits]; NV12 frames have an even height and width
+static int check_nv12_codes(int in_dtype, int out_dtype, int H, int W, int outH, int outW) {
+    const bool in12 = dtype_is_nv12(in_dtype), out12 = dtype_is_nv12(out_dtype);
+    TU_CHECK_ARG(in12 || !(in_dtype & (TU_LAYOUT_NV12 | TU_YUV_BT601 | TU_YUV_FULL_RANGE)),
+                 "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), and the colour bits TU_YUV_* go with TU_LAYOUT_NV12 only (input)");
+    TU_CHECK_ARG(out12 || !(out_dtype & (TU_LAYOUT_NV12 | TU_YUV_BT601 | TU_YUV_FULL_RANGE)),
+                 "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), and the colour bits TU_YUV_* go with TU_LAYOUT_NV12 only (output)");
+    TU_CHECK_ARG(!in12 || (H % 2 == 0 && W % 2 == 0), "forward: NV12 input frames need an even height and width");
+    TU_CHECK_ARG(!out12 || (outH % 2 == 0 && outW % 2 == 0), "forward: NV12 output frames need an even height and width");
+    return TU_OK;
+}
+
+extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale,
+                                                int compute_dtype, int in_dtype, int out_dtype) {
+    if (check_forward_args(w, B, H, W, outH, outW, compute_dtype) || check_nv12_codes(in_dtype, out_dtype, H, W, outH, outW)) return 0;
+    // only the NV12 sides change the arena; every other code sizes exactly as tu_forward_workspace_bytes_for
+    in_dtype = dtype_is_nv12(in_dtype) ? in_dtype : TU_F32;
+    out_dtype = dtype_is_nv12(out_dtype) ? out_dtype : TU_F32;
+    Arena a{nullptr, 0, 0, true};
+    int rc = compute_dtype == TU_F32
+                 ? forward_impl<float>(w, nullptr, in_dtype, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0)
+                 : forward_impl<bf16>(w, nullptr, in_dtype, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0);
+    return rc == TU_OK ? a.off : 0;
+}
+
 extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype, int B, int H,
                           int W, int outH, int outW, int scale, int compute_dtype, int clamp, void *workspace,
                           size_t workspace_bytes, void *stream) {
     int rc = check_forward_args(w, B, H, W, outH, outW, compute_dtype);
     if (rc) return rc;
     TU_CHECK_ARG(x && out && workspace, "forward: null buffer");
+    if ((rc = check_nv12_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
     {
-        const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype), il = dtype_layout(in_dtype), ol = dtype_layout(out_dtype);
+        const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype);
+        const int il = dtype_is_nv12(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_nv12(out_dtype) ? 0 : dtype_layout(out_dtype);
         TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8) && (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8),
                      "forward: bad i/o dtype");
         TU_CHECK_ARG((il == 0 || (ib == TU_U8 && il <= 2)) && (ol == 0 || (ob == TU_U8 && ol <= 2)),

@@ -92,8 +92,12 @@ template <> __device__ __forceinline__ uint8_t from_f<uint8_t>(float v) {
 // ---- uint8 frame layouts at the boundary ---------------------------------------------------------------------------
 // A dtype code of the image input / output may carry a layout in bits 8..: TU_U8 | TU_LAYOUT_HWC (interleaved RGB, what PIL /
 // OpenCV hand over: inference.py:65-70) or TU_U8 | TU_LAYOUT_HWC_BGR (channel order reversed: app_overlay.py:384-386).
+// TU_U8 | TU_LAYOUT_NV12 (4:2:0 video frames) may add the colour bits TU_YUV_BT601 / TU_YUV_FULL_RANGE in bits 12..13.
 __host__ __device__ __forceinline__ int dtype_base(int d) { return d & 0xFF; }
-__host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }          // 0 planar CHW, 1 HWC RGB, 2 HWC BGR
+__host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }          // 0 planar CHW, 1 HWC RGB, 2 HWC BGR; NV12: >= 4
+__host__ __device__ __forceinline__ bool dtype_is_nv12(int d) {                        // TU_U8 | TU_LAYOUT_NV12 [| colour bits]
+    return (d & ~(TU_YUV_BT601 | TU_YUV_FULL_RANGE)) == (TU_U8 | TU_LAYOUT_NV12);
+}
 // one RGB pixel of frame b -> out, in the requested layout.  pix = y * W + x, plane = H * W
 template <typename TO>
 __device__ __forceinline__ void store_rgb(TO *out, long b, long plane, long pix, int layout, float r, float g, float bl) {

@@ -53,13 +53,45 @@ def _code(dt: torch.dtype) -> int:
     return _DT[dt]
 
 
-LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR}
+LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR, "nv12": _lib.TU_LAYOUT_NV12}
+# colour of NV12 frames: matrix and range
+YUV = {"bt709": 0, "bt601": _lib.TU_YUV_BT601, "bt709_full": _lib.TU_YUV_FULL_RANGE,
+       "bt601_full": _lib.TU_YUV_BT601 | _lib.TU_YUV_FULL_RANGE}
 
 
 def layout_code(name: str) -> int:
     if name not in LAYOUTS:
-        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc' or 'hwc_bgr'")
+        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr' or 'nv12'")
     return LAYOUTS[name]
+
+
+def yuv_code(name: str) -> int:
+    if name not in YUV:
+        raise ValueError(f"unknown NV12 colour {name!r}: use 'bt709', 'bt601', 'bt709_full' or 'bt601_full'")
+    return YUV[name]
+
+
+def _is_nv12(code: int) -> bool:
+    return code & 0xF00 == _lib.TU_LAYOUT_NV12
+
+
+def _image_shape(B: int, C_: int, h: int, w: int, code: int) -> Tuple[int, ...]:
+    """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3) or NV12 (B,3h/2,w)"""
+    if _is_nv12(code):
+        return (B, 3 * h // 2, w)
+    return (B, h, w, 3) if code >> 8 else (B, C_, h, w)
+
+
+def _nv12_hw(x: torch.Tensor) -> Tuple[int, int]:
+    """(H, W) of NV12 frames (B, 3H/2, W); raises ValueError for a shape that is not one"""
+    if x.dim() != 3 or x.dtype != torch.uint8:
+        raise ValueError(f"NV12 frames must be uint8 of shape (B, 3H/2, W), got {x.dtype} {tuple(x.shape)}")
+    if x.shape[1] % 3:
+        raise ValueError(f"NV12 frames (B, 3H/2, W) need a row count divisible by 3, got {tuple(x.shape)}")
+    H, W = int(x.shape[1]) * 2 // 3, int(x.shape[2])
+    if H % 2 or W % 2:
+        raise ValueError(f"NV12 frames need an even height and width, got H={H} W={W}")
+    return H, W
 
 
 def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: int, compute_bf16: bool,
@@ -69,7 +101,11 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
     if pw is None:
         raise RuntimeError(f"tu::forward: packed-weights handle {handle} is not alive (its TransformerModel was deleted or repacked)")
     _require_cuda(x)
-    if in_layout:
+    if _is_nv12(in_layout):
+        H, W = _nv12_hw(x)
+        x = x.contiguous()
+        B = x.shape[0]
+    elif in_layout:
         if x.dim() != 4 or x.shape[3] != 3 or x.dtype != torch.uint8:
             raise RuntimeError(f"interleaved frames must be uint8 of shape (B,H,W,3), got {x.dtype} {tuple(x.shape)}")
         x = x.contiguous()
@@ -80,16 +116,17 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
         x = x.contiguous()
         B, _, H, W = x.shape
     cdt = _lib.TU_BF16 if compute_bf16 else _lib.TU_F32
-    out_shape = (B, out_h, out_w, 3) if out_code >> 8 else (B, 3, out_h, out_w)
+    out_shape = _image_shape(B, 3, out_h, out_w, out_code)
     if out_code >> 8 and (out_code & 0xFF) != _lib.TU_U8:
-        raise RuntimeError("interleaved output layouts are for uint8 frames")
+        raise RuntimeError("interleaved and NV12 output layouts are for uint8 frames")
     out = torch.empty(out_shape, dtype=_TORCH_DT[out_code & 0xFF], device=x.device)
-    nbytes = lib.tu_forward_workspace_bytes_for(C.byref(pw.struct), B, H, W, out_h, out_w, scale, cdt)
+    in_code = _code(x.dtype) | in_layout
+    nbytes = lib.tu_forward_workspace_bytes_io(C.byref(pw.struct), B, H, W, out_h, out_w, scale, cdt, in_code, out_code)
     if nbytes == 0:
         _lib.check(_lib.TU_ERR_SCALE if "was not built" in _lib.last_error() else _lib.TU_ERR_ARG)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
     with torch.cuda.device(x.device):
-        rc = lib.tu_forward(C.byref(pw.struct), x.data_ptr(), _code(x.dtype) | in_layout, out.data_ptr(), out_code,
+        rc = lib.tu_forward(C.byref(pw.struct), x.data_ptr(), in_code, out.data_ptr(), out_code,
                             B, H, W, out_h, out_w, scale, cdt, int(clamp), ws.data_ptr(), nbytes, _stream())
     _lib.check(rc)
     return out
@@ -103,8 +140,7 @@ def tu_forward(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: int,
 
 @tu_forward.register_fake
 def _(x, handle, out_h, out_w, scale, compute_bf16, out_code, clamp, in_layout=0):
-    shape = (x.shape[0], out_h, out_w, 3) if out_code >> 8 else (x.shape[0], 3, out_h, out_w)
-    return x.new_empty(shape, dtype=_TORCH_DT[out_code & 0xFF])
+    return x.new_empty(_image_shape(x.shape[0], 3, out_h, out_w, out_code), dtype=_TORCH_DT[out_code & 0xFF])
 
 
 @torch.library.custom_op("tu::resize_aa", mutates_args=(), device_types="cuda")
@@ -134,18 +170,55 @@ def _(x, out_h, out_w, clamp, out_code=-1):
     return x.new_empty(shape, dtype=_TORCH_DT[out_code & 0xFF])
 
 
+@torch.library.custom_op("tu::rgb_to_nv12", mutates_args=(), device_types="cuda")
+def tu_rgb_to_nv12(x: torch.Tensor, code: int) -> torch.Tensor:
+    """planar fp16 RGB (B,3,H,W) -> NV12 frames (B,3H/2,W) uint8; code = TU_U8 | TU_LAYOUT_NV12 | colour bits"""
+    lib = _lib.load()
+    _require_cuda(x)
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != torch.float16:
+        raise RuntimeError(f"rgb_to_nv12 takes planar fp16 RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    out = torch.empty((B, 3 * H // 2, W), dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_nv12(x.data_ptr(), out.data_ptr(), code, B, H, W, _stream()))
+    return out
+
+
+@tu_rgb_to_nv12.register_fake
+def _(x, code):
+    return x.new_empty((x.shape[0], 3 * x.shape[2] // 2, x.shape[3]), dtype=torch.uint8)
+
+
 def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int, int], upscale_factor: Optional[int],
                 require_ratio: bool, compute_bf16: bool, out_dtype: torch.dtype, clamp: bool = True,
-                in_layout: str = "chw", out_layout: str = "chw") -> torch.Tensor:
+                in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709") -> torch.Tensor:
     """Shape logic of the three reference forwards (W:237-238, F:245-248,323-327, R:121-122) around tu::forward.
-    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr'): uint8 frames may be interleaved (B,H,W,3) on either side."""
+    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'nv12'): uint8 frames may be interleaved (B,H,W,3) or NV12 (B,3H/2,W) on
+    either side; yuv ('bt709' | 'bt601' | 'bt709_full' | 'bt601_full') is the colour of the NV12 side(s)."""
     il, ol = layout_code(in_layout), layout_code(out_layout)
-    H, W = (int(x.shape[1]), int(x.shape[2])) if il else (int(x.shape[2]), int(x.shape[3]))
+    nv12_in, nv12_out = in_layout == "nv12", out_layout == "nv12"
+    if yuv != "bt709" and not (nv12_in or nv12_out):
+        raise ValueError(f"yuv={yuv!r} applies to NV12 frames only: pass in_layout='nv12' and / or out_layout='nv12'")
+    yc = yuv_code(yuv)
+    if nv12_out and out_dtype != torch.uint8:
+        raise ValueError("out_layout='nv12' writes uint8 frames")
+    il |= yc if nv12_in else 0
+    if nv12_in:
+        H, W = _nv12_hw(x)
+    else:
+        H, W = (int(x.shape[1]), int(x.shape[2])) if il else (int(x.shape[2]), int(x.shape[3]))
     if upscale_factor is not None:
         res_out = (H * upscale_factor, W * upscale_factor)
     res_out = (int(res_out[0]), int(res_out[1]))
-    out_code = _code(out_dtype) | ol
+    out_code = _code(out_dtype) | ol | (yc if nv12_out else 0)
+
+    def even_out(oh, ow):
+        if nv12_out and (oh % 2 or ow % 2):
+            raise ValueError(f"NV12 output frames need an even height and width, got {oh}x{ow}")
+
     if model != "FastTransformer":
+        even_out(*res_out)
         return tu_forward(x, pw_handle, res_out[0], res_out[1], 0, compute_bf16, out_code, clamp, il)
     scale = upscale_factor if upscale_factor is not None else math.ceil(max(res_out[0] / H, res_out[1] / W))
     if scale not in (2, 3, 4, 6):
@@ -155,10 +228,14 @@ def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int,
     # output and is the identity when the size already matches
     need_resize = require_ratio and res_out != (oh, oh) and res_out != (oh, ow)
     if not need_resize:
+        even_out(oh, ow)
         return tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, out_code, clamp, il)
+    even_out(*res_out)
     # Resize is the last op: the un-clamped full-size image stays in the compute dtype and the Resize kernel writes the requested
     # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store).  fp16 output keeps an fp32
-    # intermediate, so that it is the fp32 result rounded once, at the Resize's store
-    mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) else torch.float32)
+    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  NV12 output is the fp16 output converted
+    mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) and not nv12_out else torch.float32)
     full = tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, mid_code, False, il)
+    if nv12_out:
+        return tu_rgb_to_nv12(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16), out_code)
     return tu_resize_aa(full, res_out[0], res_out[1], clamp, out_code)

@@ -148,10 +148,12 @@ class EngineModel(nn.Module):
         return bf16, out_dt
 
     def forward(self, x: torch.Tensor, res_out: Tuple[int, int] = (1080, 1920), upscale_factor: int = None,
-                require_ratio: bool = True, in_layout: str = "chw", out_layout: str = "chw") -> torch.Tensor:
-        """The reference's signature (W:224, F:231, R:114) plus two keyword-only-in-spirit extensions for uint8 video frames:
-        in_layout / out_layout in {'chw', 'hwc', 'hwc_bgr'} — uint8 frames may arrive / leave interleaved (B,H,W,3), the form PIL
-        and OpenCV hold them in (inference.py:65-70, app_overlay.py:382-386), with the channel swap done in the last kernel."""
+                require_ratio: bool = True, in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709") -> torch.Tensor:
+        """The reference's signature (W:224, F:231, R:114) plus keyword-only-in-spirit extensions for uint8 video frames:
+        in_layout / out_layout in {'chw', 'hwc', 'hwc_bgr', 'nv12'} — uint8 frames may arrive / leave interleaved (B,H,W,3), the form PIL
+        and OpenCV hold them in (inference.py:65-70, app_overlay.py:382-386), with the channel swap done in the last kernel, or as
+        NV12 video frames (B,3H/2,W), the form video decoders hand out and encoders take, converted on the GPU at both ends.
+        yuv in {'bt709', 'bt601', 'bt709_full', 'bt601_full'} is the colour matrix and range of the NV12 side(s)."""
         if self.training:
             raise RuntimeError("transformerupscaler_b200 is a forward-only inference engine: call .eval() first "
                                "(dropout is treated as identity; there is no backward)")
@@ -171,7 +173,7 @@ class EngineModel(nn.Module):
         if (in_layout != "chw" or out_layout != "chw") and not frames_u8:
             raise ValueError("in_layout / out_layout other than 'chw' apply to uint8 frames only")
         out = engine.run_forward(handle, self.ENGINE_MODEL, x, res_out, upscale_factor, require_ratio, bf16, out_dt,
-                                 in_layout=in_layout, out_layout=out_layout)
+                                 in_layout=in_layout, out_layout=out_layout, yuv=yuv)
         if not frames_u8 and x.is_cuda and torch.is_autocast_enabled("cuda") and not self.AUTOCAST_OUT_FP32:
             want = torch.get_autocast_dtype("cuda")
             if out.dtype != want:

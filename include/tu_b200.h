@@ -10,7 +10,8 @@
  *   - the caller owns every buffer; the library never allocates or frees device memory, never
  *     synchronises the device, and enqueues all work on `stream` (a cudaStream_t passed as void*);
  *   - return value 0 = success, negative = error; tu_last_error() gives the message (thread-local);
- *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 and TU_F16 = 3 (both image input / output only);
+ *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 and TU_F16 = 3 (both image input / output only), TU_U16 = 4 (P010
+ *     frames only);
  *   - activations inside the engine are NHWC (64 channels); images at the boundary are NCHW, like
  *     the reference's tensors.
  */
@@ -51,6 +52,19 @@ extern "C" {
 #define TU_YUV_BT601 0x1000         /* BT.601 matrix (Kr, Kb = 0.299, 0.114) instead of BT.709 (0.2126, 0.0722) */
 #define TU_YUV_FULL_RANGE 0x2000    /* full range (Y, C in 0..255) instead of limited (Y 16..235, C 16..240) */
 #define TU_U8_NV12 (TU_U8 | TU_LAYOUT_NV12)
+/* P010 video frames (10-bit 4:2:0; TU_U16 | TU_LAYOUT_P010 for the image input and / or output of tu_forward, and the code of
+ * tu_p010_to_rgb / tu_rgb_to_p010): one buffer of (3H/2) x W little-endian uint16 words per frame, (B, 3H/2, W) for a batch, laid
+ * out and sited like NV12 (Y plane, then H/2 rows of interleaved (U, V) pairs, U first; H and W even).  A word holds its 10-bit
+ * code in the HIGH 10 bits, as video decoders write it and encoders read it: the code is word >> 6 on read (the low 6 bits are
+ * ignored) and code << 6 on write (the low 6 bits are zero).  TU_U16 is valid with TU_LAYOUT_P010 only, and never a compute dtype.
+ * The colour bits: TU_YUV_BT601 or TU_YUV_BT2020 (not both), TU_YUV_FULL_RANGE; none = BT.709 limited range.  Limited range is
+ * Y 64..940, C 64..960; full range (BT.2100) is Y, C 0..1023.  The frame is converted to / from planar fp32 RGB (the TU_F32 image
+ * I/O path) at both ends of the forward: fp16 would move a 10-bit output code by one on many bright samples.  RGB values outside
+ * [0, 1] are clamped on the way in, which matters for wide-gamut BT.2020 content. */
+#define TU_U16 4
+#define TU_LAYOUT_P010 0x800
+#define TU_YUV_BT2020 0x4000        /* BT.2020 non-constant-luminance matrix (Kr, Kb = 0.2627, 0.0593); with TU_LAYOUT_P010 only */
+#define TU_U16_P010 (TU_U16 | TU_LAYOUT_P010)
 
 #define TU_OK 0
 #define TU_ERR_ARG (-1)      /* bad argument (shape / dtype / null pointer)              */
@@ -74,7 +88,7 @@ long long tu_launch_count(void);
  * events on the caller's stream (two event records per forward: cheap enough for the timed region); tu_profile_enable(2)
  * brackets EVERY kernel, tagged with the reference op it implements ("conv1", "conv2" (or "conv1_conv2" when fused), "downsample", "patch_embed",
  * "transformer_blocks", "patch_unembed", "decoder_conv1", "decoder_conv2", "bicubic_add_clamp", "up1", "up1_conv",
- * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end).  tu_profile_collect / tu_profile_report synchronise those events (the only
+ * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end).  tu_profile_collect / tu_profile_report synchronise those events (the only
  * calls in the library that wait on the device): collect sums the milliseconds and launches recorded under `name`
  * (NULL = all); report writes "name total_ms launches\n" lines into buf (returns the needed size when buf is NULL);
  * tu_profile_reset drops the records. */
@@ -198,6 +212,9 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      TU_U8 | TU_LAYOUT_NV12 [| colour bits]: x is (B, 3H/2, W) and / or out is (B, 3 outH/2, outW), H, W (outH, outW) even; the
  *      frame is converted to planar fp16 first (the forward is then the TU_F16 one) / the last image kernel writes planar fp16 that
  *      is converted last (codes saturate at 0 / 255 with clamp == 0 too).  Size the workspace with tu_forward_workspace_bytes_io.
+ *      TU_U16 | TU_LAYOUT_P010 [| colour bits]: the same with 16-bit words and planar fp32: a P010 input is converted to planar fp32
+ *      first (the forward is then the TU_F32-input one), a P010 output is the converted TU_F32 output (codes saturate at 0 / 1023
+ *      with clamp == 0 too).  Either side may be NV12, P010 or any other code independently of the other.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
@@ -206,7 +223,8 @@ size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int outH, int 
 /* the same, sized from the packed weights actually used (non-default dim / heads / n_blocks; which fused kernels are packed) */
 size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
 /* the same for the image input / output codes of the call: equal to tu_forward_workspace_bytes_for for every code pair without
- * TU_LAYOUT_NV12, larger by the planar fp16 frames of the side(s) that are NV12 (tu_forward needs it then); 0 for a bad code */
+ * TU_LAYOUT_NV12 or TU_LAYOUT_P010, larger by the planar fp16 frames of the side(s) that are NV12 and the planar fp32 frames of the
+ * side(s) that are P010 (tu_forward needs it then); 0 for a bad code */
 size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype,
                                      int in_dtype, int out_dtype);
 int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype,
@@ -315,6 +333,15 @@ int tu_frames_to_planar(const void *in, int layout, void *out, int B, int H, int
  *            min(max(floor(s Y' + o + 0.5), 0), 255) with (s, o) = (219, 16) / (224, 128) limited, (255, 0) / (255, 128) full range. */
 int tu_nv12_to_rgb(const void *nv12, int code, void *rgb_f16, int B, int H, int W, void *stream);
 int tu_rgb_to_nv12(const void *rgb_f16, void *nv12, int code, int B, int H, int W, void *stream);
+/* P010 frames (B, 3H/2, W) of uint16 words -> planar RGB (B, 3, H, W) fp32, and back.  code = TU_U16 | TU_LAYOUT_P010 | colour bits
+ * (anything else, an odd H or W, or B > 65535: TU_ERR_ARG); the P010 buffer must be 4-byte and the RGB buffer 8-byte aligned.  The
+ * formulas are those of the NV12 ops above, on 10-bit codes (Y = word >> 6, and so on) with chroma midpoint 512 instead of 128,
+ * (yo, ys, cs) = (64, 876, 896) limited / (0, 1023, 1023) full range, and (Kr, Kb) = (0.2627, 0.0593) for TU_YUV_BT2020:
+ *   to RGB:  y' = (Y - yo) / ys, u' = (U - 512) / cs, v' = (V - 512) / cs, R, G, B as for NV12, each clamped to [0, 1] (fp32 out);
+ *   to P010: Y', Cb', Cr' as for NV12; a code is min(max(floor(s Y' + o + 0.5), 0), 1023) with (s, o) = (876, 64) / (896, 512)
+ *            limited, (1023, 0) / (1023, 512) full range, stored as code << 6. */
+int tu_p010_to_rgb(const void *p010, int code, void *rgb_f32, int B, int H, int W, void *stream);
+int tu_rgb_to_p010(const void *rgb_f32, void *p010, int code, int B, int H, int W, void *stream);
 
 #ifdef __cplusplus
 }

@@ -15,6 +15,9 @@ TU_F32, TU_BF16, TU_U8, TU_F16 = 0, 1, 2, 3      # TU_U8 and TU_F16: image input
 TU_LAYOUT_HWC, TU_LAYOUT_HWC_BGR = 0x100, 0x200      # OR-ed into TU_U8 for interleaved uint8 frames
 TU_LAYOUT_NV12 = 0x400                               # OR-ed into TU_U8 for NV12 (4:2:0) video frames, (B, 3H/2, W)
 TU_YUV_BT601, TU_YUV_FULL_RANGE = 0x1000, 0x2000     # colour bits of an NV12 code; neither = BT.709 limited range
+TU_U16 = 4                                           # 16-bit frame words: valid only as TU_U16 | TU_LAYOUT_P010
+TU_LAYOUT_P010 = 0x800                               # OR-ed into TU_U16 for P010 (10-bit 4:2:0) video frames, (B, 3H/2, W)
+TU_YUV_BT2020 = 0x4000                               # BT.2020 matrix: a colour bit of P010 codes only (not with TU_YUV_BT601)
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}
 
@@ -115,13 +118,16 @@ SIGNATURES = {
     "tu_bicubic_row_schedule": (i32, [i32, i32, i32]),
     "tu_nv12_to_rgb": (i32, [vp, i32, vp, i32, i32, i32, vp]),
     "tu_rgb_to_nv12": (i32, [vp, vp, i32, i32, i32, i32, vp]),
+    "tu_p010_to_rgb": (i32, [vp, i32, vp, i32, i32, i32, vp]),
+    "tu_rgb_to_p010": (i32, [vp, vp, i32, i32, i32, i32, vp]),
 }
 
 
 
 def dtype_size(code: int) -> int:
-    """bytes per element of an image dtype code (a layout or colour bits do not change it: every uint8 frame is bytes)"""
-    return {TU_F32: 4, TU_BF16: 2, TU_U8: 1, TU_F16: 2}[code & 0xFF]
+    """bytes per element of an image dtype code (a layout or colour bits do not change it: every uint8 frame is bytes, every P010
+    frame 16-bit words)"""
+    return {TU_F32: 4, TU_BF16: 2, TU_U8: 1, TU_F16: 2, TU_U16: 2}[code & 0xFF]
 
 
 _lib = None

@@ -168,13 +168,21 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
         if (!dry) TU_STEP("nv12_to_rgb", tu_nv12_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F16;
+    } else if (dtype_is_p010(in_dtype)) {
+        // P010 frames are converted to planar fp32 (fp16 cannot hold every 10-bit step exactly): the forward is then the fp32-input one
+        float *rgb = (float *)a.get((size_t)B * 3 * H * W * sizeof(float));
+        if (!dry) TU_STEP("p010_to_rgb", tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
+        x = rgb;
+        in_dtype = TU_F32;
     }
-    // NV12 output: the last image kernel writes planar fp16 here, and tu_rgb_to_nv12 writes `out` from it
-    const bool nv12_out = dtype_is_nv12(out_dtype);
-    void *img = nv12_out ? a.get((size_t)B * 3 * outH * outW * sizeof(f16)) : out;
-    const int img_dtype = nv12_out ? TU_F16 : out_dtype;
-#define TU_NV12_OUT() \
-    if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv))
+    // NV12 / P010 output: the last image kernel writes planar fp16 / fp32 here, and tu_rgb_to_nv12 / tu_rgb_to_p010 writes `out` from it
+    const bool nv12_out = dtype_is_nv12(out_dtype), p010_out = dtype_is_p010(out_dtype);
+    void *img = nv12_out ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
+                : p010_out ? a.get((size_t)B * 3 * outH * outW * sizeof(float)) : out;
+    const int img_dtype = nv12_out ? TU_F16 : p010_out ? TU_F32 : out_dtype;
+#define TU_YUV_OUT()                                                                    \
+    if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv)); \
+    else if (p010_out) TU_STEP("rgb_to_p010", tu_rgb_to_p010(img, out, out_dtype, B, outH, outW, stv))
 
     // interleaved uint8 frames (HWC RGB / BGR) are made planar once; the stem and the final bicubic both read the planar copy
     uint8_t *xplanar = (uint8_t *)a.get((size_t)B * 3 * H * W);
@@ -357,7 +365,7 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
     if (!fast) {
         if (!dry) {
             TU_STEP("bicubic_add_clamp", tu_bicubic_add_clamp(x, in_dtype, H, W, res, Hc, Wc, img, img_dtype, B, outH, outW, clamp, stv));
-            TU_NV12_OUT();
+            TU_YUV_OUT();
         }
         return TU_OK;
     }
@@ -379,7 +387,7 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
                     }
                     TU_STEP("final_upscale_conv_add", tu_subpixel_conv_add(cur, (const float *)sg.w, sg.b, r, w->host_finconv_wb, upA, img,
                                                                            img_dtype, B, ch, cw, clamp, stv));
-                    TU_NV12_OUT();
+                    TU_YUV_OUT();
                 }
                 return TU_OK;
             }
@@ -395,11 +403,11 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
                 return TU_ERR_ARG;
             }
             TU_STEP("final_conv_add", tu_final_conv_add(cur, w->finconv_w, w->finconv_b, upA, img, img_dtype, B, ch, cw, clamp, stv));
-            TU_NV12_OUT();
+            TU_YUV_OUT();
         }
     }
     return TU_OK;
-#undef TU_NV12_OUT
+#undef TU_YUV_OUT
 }
 
 }  // namespace tu
@@ -706,24 +714,30 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
     return rc == TU_OK ? a.off : 0;
 }
 
-// NV12 codes are TU_U8 | TU_LAYOUT_NV12 [| colour bits]; NV12 frames have an even height and width
-static int check_nv12_codes(int in_dtype, int out_dtype, int H, int W, int outH, int outW) {
-    const bool in12 = dtype_is_nv12(in_dtype), out12 = dtype_is_nv12(out_dtype);
-    TU_CHECK_ARG(in12 || !(in_dtype & (TU_LAYOUT_NV12 | TU_YUV_BT601 | TU_YUV_FULL_RANGE)),
-                 "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), and the colour bits TU_YUV_* go with TU_LAYOUT_NV12 only (input)");
-    TU_CHECK_ARG(out12 || !(out_dtype & (TU_LAYOUT_NV12 | TU_YUV_BT601 | TU_YUV_FULL_RANGE)),
-                 "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), and the colour bits TU_YUV_* go with TU_LAYOUT_NV12 only (output)");
-    TU_CHECK_ARG(!in12 || (H % 2 == 0 && W % 2 == 0), "forward: NV12 input frames need an even height and width");
-    TU_CHECK_ARG(!out12 || (outH % 2 == 0 && outW % 2 == 0), "forward: NV12 output frames need an even height and width");
+// 4:2:0 codes: TU_U8 | TU_LAYOUT_NV12 [| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_P010 [| TU_YUV_BT601 or
+// TU_YUV_BT2020] [| TU_YUV_FULL_RANGE].  TU_U16 is a P010 word and nothing else.  Such frames have an even height and width.
+static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int outH, int outW) {
+    const int bits = TU_LAYOUT_NV12 | TU_LAYOUT_P010 | TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE;
+    const bool in420 = dtype_is_yuv420(in_dtype), out420 = dtype_is_yuv420(out_dtype);
+    TU_CHECK_ARG(in420 || (!(in_dtype & bits) && dtype_base(in_dtype) != TU_U16),
+                 "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
+                 "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (input)");
+    TU_CHECK_ARG(out420 || (!(out_dtype & bits) && dtype_base(out_dtype) != TU_U16),
+                 "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
+                 "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (output)");
+    TU_CHECK_ARG(!in420 || (H % 2 == 0 && W % 2 == 0),
+                 std::string("forward: ") + (dtype_is_p010(in_dtype) ? "P010" : "NV12") + " input frames need an even height and width");
+    TU_CHECK_ARG(!out420 || (outH % 2 == 0 && outW % 2 == 0),
+                 std::string("forward: ") + (dtype_is_p010(out_dtype) ? "P010" : "NV12") + " output frames need an even height and width");
     return TU_OK;
 }
 
 extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale,
                                                 int compute_dtype, int in_dtype, int out_dtype) {
-    if (check_forward_args(w, B, H, W, outH, outW, compute_dtype) || check_nv12_codes(in_dtype, out_dtype, H, W, outH, outW)) return 0;
-    // only the NV12 sides change the arena; every other code sizes exactly as tu_forward_workspace_bytes_for
-    in_dtype = dtype_is_nv12(in_dtype) ? in_dtype : TU_F32;
-    out_dtype = dtype_is_nv12(out_dtype) ? out_dtype : TU_F32;
+    if (check_forward_args(w, B, H, W, outH, outW, compute_dtype) || check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW)) return 0;
+    // only the NV12 / P010 sides change the arena; every other code sizes exactly as tu_forward_workspace_bytes_for
+    in_dtype = dtype_is_yuv420(in_dtype) ? in_dtype : TU_F32;
+    out_dtype = dtype_is_yuv420(out_dtype) ? out_dtype : TU_F32;
     Arena a{nullptr, 0, 0, true};
     int rc = compute_dtype == TU_F32
                  ? forward_impl<float>(w, nullptr, in_dtype, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0)
@@ -737,11 +751,13 @@ extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, 
     int rc = check_forward_args(w, B, H, W, outH, outW, compute_dtype);
     if (rc) return rc;
     TU_CHECK_ARG(x && out && workspace, "forward: null buffer");
-    if ((rc = check_nv12_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
+    if ((rc = check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
     {
         const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype);
-        const int il = dtype_is_nv12(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_nv12(out_dtype) ? 0 : dtype_layout(out_dtype);
-        TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8) && (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8),
+        const int il = dtype_is_yuv420(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_yuv420(out_dtype) ? 0 : dtype_layout(out_dtype);
+        // (TU_U16 has passed check_yuv420_codes only as a P010 word)
+        TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8 || ib == TU_U16) &&
+                         (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8 || ob == TU_U16),
                      "forward: bad i/o dtype");
         TU_CHECK_ARG((il == 0 || (ib == TU_U8 && il <= 2)) && (ol == 0 || (ob == TU_U8 && ol <= 2)),
                      "forward: interleaved layouts (TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR) are for uint8 frames");

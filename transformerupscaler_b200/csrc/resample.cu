@@ -1020,24 +1020,26 @@ __global__ void __launch_bounds__(256) frames_to_planar_kernel(const uint8_t *__
     }
 }
 
-// ---- NV12 (4:2:0, type-0 chroma siting) <-> planar fp16 RGB -------------------------------------------------------------------
+// ---- 4:2:0 video frames (NV12 / P010, type-0 chroma siting) <-> planar RGB (fp16 / fp32) ------------------------------------------
 // Every step is one correctly rounded fp32 operation (__fmul_rn / __fadd_rn / __fdiv_rn: -O3 would contract a*b+c into an FMA), in
 // the order include/tu_b200.h states, so that the kernels give the bits of a plain fp32 evaluation of the formulas.
 struct YuvCoef {
-    float yo, ys, cs;                   // y' = (Y - yo) / ys, c' = (C - 128) / cs
+    float yo, ys, cs;                   // y' = (Y - yo) / ys, c' = (C - mid) / cs (mid: Yuv420<TS>::mid)
     float a_rv, a_gu, a_gv, a_bu;       // YUV -> RGB
     float kr, kg, kb;                   // RGB -> Y'
-    float cb_r, cb_g, cr_g, cr_b;       // RGB -> Cb', Cr' (the 0.5 terms are exact); codes: ys Y' + yo, cs C' + 128
+    float cb_r, cb_g, cr_g, cr_b;       // RGB -> Cb', Cr' (the 0.5 terms are exact); codes: ys Y' + yo, cs C' + mid
 };
 
-// coefficients of a colour code, each computed in double and rounded once to float
+// coefficients of a colour code, each computed in double and rounded once to float.  P010 codes (TU_U16) take the 10-bit offsets
+// and scales, and may name the BT.2020 matrix
 static YuvCoef yuv_coef(int code) {
-    const double kr = (code & TU_YUV_BT601) ? 0.299 : 0.2126, kb = (code & TU_YUV_BT601) ? 0.114 : 0.0722, kg = 1.0 - kr - kb;
-    const bool full = code & TU_YUV_FULL_RANGE;
+    const bool bt601 = code & TU_YUV_BT601, bt2020 = code & TU_YUV_BT2020, full = code & TU_YUV_FULL_RANGE;
+    const bool p010 = dtype_base(code) == TU_U16;
+    const double kr = bt2020 ? 0.2627 : bt601 ? 0.299 : 0.2126, kb = bt2020 ? 0.0593 : bt601 ? 0.114 : 0.0722, kg = 1.0 - kr - kb;
     YuvCoef k;
-    k.yo = full ? 0.f : 16.f;
-    k.ys = full ? 255.f : 219.f;
-    k.cs = full ? 255.f : 224.f;
+    k.yo = full ? 0.f : p010 ? 64.f : 16.f;
+    k.ys = full ? (p010 ? 1023.f : 255.f) : p010 ? 876.f : 219.f;
+    k.cs = full ? (p010 ? 1023.f : 255.f) : p010 ? 896.f : 224.f;
     k.a_rv = (float)(2.0 * (1.0 - kr));
     k.a_bu = (float)(2.0 * (1.0 - kb));
     k.a_gu = (float)(-2.0 * (1.0 - kb) * kb / kg);
@@ -1052,12 +1054,37 @@ static YuvCoef yuv_coef(int code) {
     return k;
 }
 
+// sample formats: NV12 holds one 8-bit code per byte; P010 one 10-bit code in the high bits of a little-endian uint16 word (the low
+// 6 bits are ignored on read and zero on write).  A pair of samples (two luma, or U then V) is one 2-byte / 4-byte access.
+template <typename TS> struct Yuv420;
+template <> struct Yuv420<uint8_t> {
+    typedef uchar2 Pair;
+    static constexpr int shift = 0;
+    static constexpr float mid = 128.f, cmax = 255.f;
+    static __device__ __forceinline__ Pair pair(uint8_t a, uint8_t b) { return make_uchar2(a, b); }
+};
+template <> struct Yuv420<uint16_t> {
+    typedef ushort2 Pair;
+    static constexpr int shift = 6;
+    static constexpr float mid = 512.f, cmax = 1023.f;
+    static __device__ __forceinline__ Pair pair(uint16_t a, uint16_t b) { return make_ushort2(a, b); }
+};
+
 __device__ __forceinline__ float clamp01(float v) { return fminf(fmaxf(v, 0.f), 1.f); }
+// two horizontally adjacent RGB values of one plane (an aligned half2 / float2)
+__device__ __forceinline__ void store_rgb2(f16 *p, float a, float b) { *reinterpret_cast<__half2 *>(p) = __floats2half2_rn(a, b); }
+__device__ __forceinline__ void store_rgb2(float *p, float a, float b) { *reinterpret_cast<float2 *>(p) = make_float2(a, b); }
+__device__ __forceinline__ float2 load_rgb2(const f16 *p) { return __half22float2(*reinterpret_cast<const __half2 *>(p)); }
+__device__ __forceinline__ float2 load_rgb2(const float *p) { return *reinterpret_cast<const float2 *>(p); }
 
 // One thread per chroma sample (i, j): the 2x2 luma block rows 2i..2i+1, columns 2j..2j+1.  Bilinear chroma: luma row 2i takes
 // (C[i-1] + 3 C[i]) / 4, row 2i+1 (3 C[i] + C[i+1]) / 4; column 2j takes chroma column j, column 2j+1 the mean of j and j+1 (edges
-// clamped).  These are integer sums times 1/4 or 1/8: exact in fp32.
-__global__ void __launch_bounds__(256) nv12_to_rgb_kernel(const uint8_t *__restrict__ in, f16 *__restrict__ out, int H, int W, YuvCoef k) {
+// clamped).  These are integer sums (at most 8 * 1023) times 1/4 or 1/8: exact in fp32.
+template <typename TS, typename TR>
+__global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(const TS *__restrict__ in, TR *__restrict__ out, int H, int W, YuvCoef k) {
+    typedef Yuv420<TS> F;
+    typedef typename F::Pair P;
+    constexpr int s = F::shift;
     pdl_trigger();
     pdl_wait();
     const int Hc = H >> 1, Wc = W >> 1;
@@ -1065,45 +1092,51 @@ __global__ void __launch_bounds__(256) nv12_to_rgb_kernel(const uint8_t *__restr
     if (t >= Hc * Wc) return;
     const int i = t / Wc, j = t - i * Wc;
     const long plane = (long)H * W;
-    const uint8_t *f = in + (long)blockIdx.y * (plane + plane / 2);
-    const uint8_t *ch = f + plane;
+    const TS *f = in + (long)blockIdx.y * (plane + plane / 2);
+    const TS *ch = f + plane;
     const int im = max(i - 1, 0), ip = min(i + 1, Hc - 1), jp = min(j + 1, Wc - 1);
-    const uchar2 cm0 = *reinterpret_cast<const uchar2 *>(ch + (long)im * W + 2 * j), cm1 = *reinterpret_cast<const uchar2 *>(ch + (long)im * W + 2 * jp);
-    const uchar2 c00 = *reinterpret_cast<const uchar2 *>(ch + (long)i * W + 2 * j), c01 = *reinterpret_cast<const uchar2 *>(ch + (long)i * W + 2 * jp);
-    const uchar2 cp0 = *reinterpret_cast<const uchar2 *>(ch + (long)ip * W + 2 * j), cp1 = *reinterpret_cast<const uchar2 *>(ch + (long)ip * W + 2 * jp);
+    const P cm0 = *reinterpret_cast<const P *>(ch + (long)im * W + 2 * j), cm1 = *reinterpret_cast<const P *>(ch + (long)im * W + 2 * jp);
+    const P c00 = *reinterpret_cast<const P *>(ch + (long)i * W + 2 * j), c01 = *reinterpret_cast<const P *>(ch + (long)i * W + 2 * jp);
+    const P cp0 = *reinterpret_cast<const P *>(ch + (long)ip * W + 2 * j), cp1 = *reinterpret_cast<const P *>(ch + (long)ip * W + 2 * jp);
     // vertical sums (x4) of U and V for the top (2i) and bottom (2i+1) luma rows, at chroma columns j and j+1
-    const int ut0 = cm0.x + 3 * c00.x, ut1 = cm1.x + 3 * c01.x, ub0 = 3 * c00.x + cp0.x, ub1 = 3 * c01.x + cp1.x;
-    const int vt0 = cm0.y + 3 * c00.y, vt1 = cm1.y + 3 * c01.y, vb0 = 3 * c00.y + cp0.y, vb1 = 3 * c01.y + cp1.y;
+    const int ut0 = (cm0.x >> s) + 3 * (c00.x >> s), ut1 = (cm1.x >> s) + 3 * (c01.x >> s);
+    const int ub0 = 3 * (c00.x >> s) + (cp0.x >> s), ub1 = 3 * (c01.x >> s) + (cp1.x >> s);
+    const int vt0 = (cm0.y >> s) + 3 * (c00.y >> s), vt1 = (cm1.y >> s) + 3 * (c01.y >> s);
+    const int vb0 = 3 * (c00.y >> s) + (cp0.y >> s), vb1 = 3 * (c01.y >> s) + (cp1.y >> s);
     const int us[4] = {2 * ut0, ut0 + ut1, 2 * ub0, ub0 + ub1}, vs[4] = {2 * vt0, vt0 + vt1, 2 * vb0, vb0 + vb1};   // x8
-    const uchar2 y0 = *reinterpret_cast<const uchar2 *>(f + (long)(2 * i) * W + 2 * j);
-    const uchar2 y1 = *reinterpret_cast<const uchar2 *>(f + (long)(2 * i + 1) * W + 2 * j);
-    const int ys[4] = {y0.x, y0.y, y1.x, y1.y};
+    const P y0 = *reinterpret_cast<const P *>(f + (long)(2 * i) * W + 2 * j);
+    const P y1 = *reinterpret_cast<const P *>(f + (long)(2 * i + 1) * W + 2 * j);
+    const int ys[4] = {y0.x >> s, y0.y >> s, y1.x >> s, y1.y >> s};
     float r[4], g[4], bl[4];
 #pragma unroll
     for (int p = 0; p < 4; ++p) {
         const float yn = __fdiv_rn(__fadd_rn((float)ys[p], -k.yo), k.ys);
-        const float un = __fdiv_rn(__fadd_rn(__fmul_rn((float)us[p], 0.125f), -128.f), k.cs);
-        const float vn = __fdiv_rn(__fadd_rn(__fmul_rn((float)vs[p], 0.125f), -128.f), k.cs);
+        const float un = __fdiv_rn(__fadd_rn(__fmul_rn((float)us[p], 0.125f), -F::mid), k.cs);
+        const float vn = __fdiv_rn(__fadd_rn(__fmul_rn((float)vs[p], 0.125f), -F::mid), k.cs);
         r[p] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_rv, vn)));
         g[p] = clamp01(__fadd_rn(__fadd_rn(yn, __fmul_rn(k.a_gu, un)), __fmul_rn(k.a_gv, vn)));
         bl[p] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_bu, un)));
     }
-    f16 *o = out + (long)blockIdx.y * 3 * plane + (long)(2 * i) * W + 2 * j;
-    *reinterpret_cast<__half2 *>(o) = __floats2half2_rn(r[0], r[1]);
-    *reinterpret_cast<__half2 *>(o + W) = __floats2half2_rn(r[2], r[3]);
-    *reinterpret_cast<__half2 *>(o + plane) = __floats2half2_rn(g[0], g[1]);
-    *reinterpret_cast<__half2 *>(o + plane + W) = __floats2half2_rn(g[2], g[3]);
-    *reinterpret_cast<__half2 *>(o + 2 * plane) = __floats2half2_rn(bl[0], bl[1]);
-    *reinterpret_cast<__half2 *>(o + 2 * plane + W) = __floats2half2_rn(bl[2], bl[3]);
+    TR *o = out + (long)blockIdx.y * 3 * plane + (long)(2 * i) * W + 2 * j;
+    store_rgb2(o, r[0], r[1]);
+    store_rgb2(o + W, r[2], r[3]);
+    store_rgb2(o + plane, g[0], g[1]);
+    store_rgb2(o + plane + W, g[2], g[3]);
+    store_rgb2(o + 2 * plane, bl[0], bl[1]);
+    store_rgb2(o + 2 * plane + W, bl[2], bl[3]);
 }
 
-__device__ __forceinline__ uint8_t yuv_code(float v) {         // min(max(floor(v + 0.5), 0), 255)
-    return (uint8_t)(int)fminf(fmaxf(floorf(__fadd_rn(v, 0.5f)), 0.f), 255.f);
+template <typename TS>
+__device__ __forceinline__ TS yuv_code(float v) {         // min(max(floor(v + 0.5), 0), cmax), stored << shift
+    return (TS)((int)fminf(fmaxf(floorf(__fadd_rn(v, 0.5f)), 0.f), Yuv420<TS>::cmax) << Yuv420<TS>::shift);
 }
 
 // One thread per chroma sample (i, j): its (U, V) pair and its 2x2 luma block.  Chroma filter (type-0 siting): the column sums
 // v(c) = P[2i][c] + P[2i+1][c] weighted 1, 2, 1 over columns 2j-1 (clamped at 0), 2j, 2j+1, times 1/8, per channel.
-__global__ void __launch_bounds__(256) rgb_to_nv12_kernel(const f16 *__restrict__ in, uint8_t *__restrict__ out, int H, int W, YuvCoef k) {
+template <typename TR, typename TS>
+__global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict__ in, TS *__restrict__ out, int H, int W, YuvCoef k) {
+    typedef Yuv420<TS> F;
+    typedef typename F::Pair P;
     pdl_trigger();
     pdl_wait();
     const int Hc = H >> 1, Wc = W >> 1;
@@ -1111,32 +1144,32 @@ __global__ void __launch_bounds__(256) rgb_to_nv12_kernel(const f16 *__restrict_
     if (t >= Hc * Wc) return;
     const int i = t / Wc, j = t - i * Wc;
     const long plane = (long)H * W;
-    const f16 *src = in + (long)blockIdx.y * 3 * plane + (long)(2 * i) * W;
+    const TR *src = in + (long)blockIdx.y * 3 * plane + (long)(2 * i) * W;
     const int cl = max(2 * j - 1, 0);
     float px[3][4], bar[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        const f16 *s = src + c * plane;
-        const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(s + 2 * j));
-        const float2 b = __half22float2(*reinterpret_cast<const __half2 *>(s + W + 2 * j));
-        const float v0 = __fadd_rn(__half2float(s[cl]), __half2float(s[W + cl]));
+        const TR *s = src + c * plane;
+        const float2 a = load_rgb2(s + 2 * j);
+        const float2 b = load_rgb2(s + W + 2 * j);
+        const float v0 = __fadd_rn(to_f(s[cl]), to_f(s[W + cl]));
         const float v1 = __fadd_rn(a.x, b.x), v2 = __fadd_rn(a.y, b.y);
         px[c][0] = a.x; px[c][1] = a.y; px[c][2] = b.x; px[c][3] = b.y;
         bar[c] = __fmul_rn(__fadd_rn(__fadd_rn(v0, __fmul_rn(2.f, v1)), v2), 0.125f);
     }
-    uint8_t yq[4];
+    TS yq[4];
 #pragma unroll
     for (int p = 0; p < 4; ++p) {
         const float yl = __fadd_rn(__fadd_rn(__fmul_rn(k.kr, px[0][p]), __fmul_rn(k.kg, px[1][p])), __fmul_rn(k.kb, px[2][p]));
-        yq[p] = yuv_code(__fadd_rn(__fmul_rn(k.ys, yl), k.yo));
+        yq[p] = yuv_code<TS>(__fadd_rn(__fmul_rn(k.ys, yl), k.yo));
     }
     const float cb = __fadd_rn(__fadd_rn(__fmul_rn(k.cb_r, bar[0]), __fmul_rn(k.cb_g, bar[1])), __fmul_rn(0.5f, bar[2]));
     const float cr = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, bar[0]), __fmul_rn(k.cr_g, bar[1])), __fmul_rn(k.cr_b, bar[2]));
-    uint8_t *f = out + (long)blockIdx.y * (plane + plane / 2);
-    *reinterpret_cast<uchar2 *>(f + (long)(2 * i) * W + 2 * j) = make_uchar2(yq[0], yq[1]);
-    *reinterpret_cast<uchar2 *>(f + (long)(2 * i + 1) * W + 2 * j) = make_uchar2(yq[2], yq[3]);
-    *reinterpret_cast<uchar2 *>(f + plane + (long)i * W + 2 * j) =
-        make_uchar2(yuv_code(__fadd_rn(__fmul_rn(k.cs, cb), 128.f)), yuv_code(__fadd_rn(__fmul_rn(k.cs, cr), 128.f)));
+    TS *f = out + (long)blockIdx.y * (plane + plane / 2);
+    *reinterpret_cast<P *>(f + (long)(2 * i) * W + 2 * j) = F::pair(yq[0], yq[1]);
+    *reinterpret_cast<P *>(f + (long)(2 * i + 1) * W + 2 * j) = F::pair(yq[2], yq[3]);
+    *reinterpret_cast<P *>(f + plane + (long)i * W + 2 * j) =
+        F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid)));
 }
 
 }  // namespace tu
@@ -1407,30 +1440,56 @@ extern "C" int tu_frames_to_planar(const void *in, int layout, void *out, int B,
     return TU_OK;
 }
 
-static int check_nv12_args(const void *nv12, int code, const void *rgb, int B, int H, int W, const char *op) {
-    TU_CHECK_ARG(nv12 && rgb && B > 0 && B <= 65535 && H > 0 && W > 0, std::string(op) + ": bad argument");
-    TU_CHECK_ARG(dtype_is_nv12(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_NV12 [| TU_YUV_BT601] [| TU_YUV_FULL_RANGE]");
-    TU_CHECK_ARG(H % 2 == 0 && W % 2 == 0, std::string(op) + ": NV12 frames need an even height and width");
+// NV12: code TU_U8 | TU_LAYOUT_NV12 [| colour bits], RGB fp16; P010: code TU_U16 | TU_LAYOUT_P010 [| colour bits], RGB fp32
+static int check_yuv420_args(const void *frames, int code, bool p010, const void *rgb, int B, int H, int W, const char *op) {
+    const std::string fmt = p010 ? "P010" : "NV12";
+    TU_CHECK_ARG(frames && rgb && B > 0 && B <= 65535 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    if (p010)
+        TU_CHECK_ARG(dtype_is_p010(code), std::string(op) + ": code must be TU_U16 | TU_LAYOUT_P010 [| TU_YUV_BT601 or TU_YUV_BT2020] "
+                                                            "[| TU_YUV_FULL_RANGE]");
+    else
+        TU_CHECK_ARG(dtype_is_nv12(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_NV12 [| TU_YUV_BT601] [| TU_YUV_FULL_RANGE]");
+    TU_CHECK_ARG(H % 2 == 0 && W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even height and width");
     TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
-    TU_CHECK_ARG((reinterpret_cast<uintptr_t>(nv12) & 1) == 0 && (reinterpret_cast<uintptr_t>(rgb) & 3) == 0,
-                 std::string(op) + ": buffers must be 2-byte (NV12) and 4-byte (fp16) aligned");
+    const uintptr_t fa = p010 ? 3 : 1, ra = p010 ? 7 : 3;      // a pair of samples / of RGB values is one access
+    TU_CHECK_ARG((reinterpret_cast<uintptr_t>(frames) & fa) == 0 && (reinterpret_cast<uintptr_t>(rgb) & ra) == 0,
+                 std::string(op) + (p010 ? ": buffers must be 4-byte (P010) and 8-byte (fp32) aligned"
+                                         : ": buffers must be 2-byte (NV12) and 4-byte (fp16) aligned"));
     return TU_OK;
 }
 
 extern "C" int tu_nv12_to_rgb(const void *nv12, int code, void *rgb_f16, int B, int H, int W, void *stream) {
-    if (int rc = check_nv12_args(nv12, code, rgb_f16, B, H, W, "nv12_to_rgb")) return rc;
+    if (int rc = check_yuv420_args(nv12, code, false, rgb_f16, B, H, W, "nv12_to_rgb")) return rc;
     const int n = (H / 2) * (W / 2);
-    launch_pdl(nv12_to_rgb_kernel, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream, (const uint8_t *)nv12,
-               (f16 *)rgb_f16, H, W, yuv_coef(code));
+    launch_pdl(yuv420_to_rgb_kernel<uint8_t, f16>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+               (const uint8_t *)nv12, (f16 *)rgb_f16, H, W, yuv_coef(code));
     TU_CHECK_LAUNCH("nv12_to_rgb");
     return TU_OK;
 }
 
 extern "C" int tu_rgb_to_nv12(const void *rgb_f16, void *nv12, int code, int B, int H, int W, void *stream) {
-    if (int rc = check_nv12_args(nv12, code, rgb_f16, B, H, W, "rgb_to_nv12")) return rc;
+    if (int rc = check_yuv420_args(nv12, code, false, rgb_f16, B, H, W, "rgb_to_nv12")) return rc;
     const int n = (H / 2) * (W / 2);
-    launch_pdl(rgb_to_nv12_kernel, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream, (const f16 *)rgb_f16,
-               (uint8_t *)nv12, H, W, yuv_coef(code));
+    launch_pdl(rgb_to_yuv420_kernel<f16, uint8_t>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+               (const f16 *)rgb_f16, (uint8_t *)nv12, H, W, yuv_coef(code));
     TU_CHECK_LAUNCH("rgb_to_nv12");
+    return TU_OK;
+}
+
+extern "C" int tu_p010_to_rgb(const void *p010, int code, void *rgb_f32, int B, int H, int W, void *stream) {
+    if (int rc = check_yuv420_args(p010, code, true, rgb_f32, B, H, W, "p010_to_rgb")) return rc;
+    const int n = (H / 2) * (W / 2);
+    launch_pdl(yuv420_to_rgb_kernel<uint16_t, float>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+               (const uint16_t *)p010, (float *)rgb_f32, H, W, yuv_coef(code));
+    TU_CHECK_LAUNCH("p010_to_rgb");
+    return TU_OK;
+}
+
+extern "C" int tu_rgb_to_p010(const void *rgb_f32, void *p010, int code, int B, int H, int W, void *stream) {
+    if (int rc = check_yuv420_args(p010, code, true, rgb_f32, B, H, W, "rgb_to_p010")) return rc;
+    const int n = (H / 2) * (W / 2);
+    launch_pdl(rgb_to_yuv420_kernel<float, uint16_t>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+               (const float *)rgb_f32, (uint16_t *)p010, H, W, yuv_coef(code));
+    TU_CHECK_LAUNCH("rgb_to_p010");
     return TU_OK;
 }

@@ -264,6 +264,7 @@ extern "C" int tu_subpixel_conv_add(const float *in, const float *w_ps, const fl
     const int layout = dtype_layout(out_dtype);
     out_dtype = dtype_base(out_dtype);
     TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout <= 2), "subpixel_conv_add: interleaved layouts are for uint8 frames");
+    TU_CHECK_ARG(out_dtype == TU_F32 || out_dtype == TU_BF16 || out_dtype == TU_U8 || out_dtype == TU_F16, "subpixel_conv_add: bad dtype");
     cudaStream_t st = (cudaStream_t)stream;
     FinFilter fin;
     for (int cp = 0; cp < 3; ++cp)

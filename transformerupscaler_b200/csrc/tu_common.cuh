@@ -93,11 +93,17 @@ template <> __device__ __forceinline__ uint8_t from_f<uint8_t>(float v) {
 // A dtype code of the image input / output may carry a layout in bits 8..: TU_U8 | TU_LAYOUT_HWC (interleaved RGB, what PIL /
 // OpenCV hand over: inference.py:65-70) or TU_U8 | TU_LAYOUT_HWC_BGR (channel order reversed: app_overlay.py:384-386).
 // TU_U8 | TU_LAYOUT_NV12 (4:2:0 video frames) may add the colour bits TU_YUV_BT601 / TU_YUV_FULL_RANGE in bits 12..13.
+// TU_U16 | TU_LAYOUT_P010 (10-bit 4:2:0 frames) may add the same bits, or TU_YUV_BT2020 (bit 14) instead of TU_YUV_BT601.
 __host__ __device__ __forceinline__ int dtype_base(int d) { return d & 0xFF; }
-__host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }          // 0 planar CHW, 1 HWC RGB, 2 HWC BGR; NV12: >= 4
+__host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }          // 0 planar CHW, 1 HWC RGB, 2 HWC BGR; NV12 / P010: >= 4
 __host__ __device__ __forceinline__ bool dtype_is_nv12(int d) {                        // TU_U8 | TU_LAYOUT_NV12 [| colour bits]
     return (d & ~(TU_YUV_BT601 | TU_YUV_FULL_RANGE)) == (TU_U8 | TU_LAYOUT_NV12);
 }
+__host__ __device__ __forceinline__ bool dtype_is_p010(int d) {                        // TU_U16 | TU_LAYOUT_P010 [| colour bits]
+    const int c = d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE);
+    return (d & ~c) == (TU_U16 | TU_LAYOUT_P010) && (c & (TU_YUV_BT601 | TU_YUV_BT2020)) != (TU_YUV_BT601 | TU_YUV_BT2020);
+}
+__host__ __device__ __forceinline__ bool dtype_is_yuv420(int d) { return dtype_is_nv12(d) || dtype_is_p010(d); }
 // one RGB pixel of frame b -> out, in the requested layout.  pix = y * W + x, plane = H * W
 template <typename TO>
 __device__ __forceinline__ void store_rgb(TO *out, long b, long plane, long pix, int layout, float r, float g, float bl) {
@@ -162,7 +168,7 @@ static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 static inline size_t dtype_size(int dtype) {
     const int d = dtype & 0xFF;
-    return d == TU_BF16 || d == TU_F16 ? 2 : d == TU_U8 ? 1 : 4;
+    return d == TU_BF16 || d == TU_F16 || d == TU_U16 ? 2 : d == TU_U8 ? 1 : 4;
 }
 
 }  // namespace tu

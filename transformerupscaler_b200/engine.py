@@ -18,7 +18,8 @@ import torch
 from . import _lib
 from .packing import PackedWeights
 
-_DT = {torch.float32: _lib.TU_F32, torch.bfloat16: _lib.TU_BF16, torch.float16: _lib.TU_F16, torch.uint8: _lib.TU_U8}
+_DT = {torch.float32: _lib.TU_F32, torch.bfloat16: _lib.TU_BF16, torch.float16: _lib.TU_F16, torch.uint8: _lib.TU_U8,
+       torch.uint16: _lib.TU_U16}
 _TORCH_DT = {v: k for k, v in _DT.items()}
 # handle -> PackedWeights, WEAK: the owner (EngineModel._tu_cache, or a test) keeps the object alive; a handle whose owner is gone
 # simply disappears, so a copied / unpickled module can never release another module's weights and nothing leaks
@@ -49,49 +50,70 @@ def _require_cuda(*ts: torch.Tensor) -> None:
 
 def _code(dt: torch.dtype) -> int:
     if dt not in _DT:
-        raise TypeError(f"unsupported dtype {dt}; the engine handles float32, bfloat16, float16 and (frames only) uint8")
+        raise TypeError(f"unsupported dtype {dt}; the engine handles float32, bfloat16, float16 and (frames only) uint8 / uint16")
     return _DT[dt]
 
 
-LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR, "nv12": _lib.TU_LAYOUT_NV12}
-# colour of NV12 frames: matrix and range
+LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR, "nv12": _lib.TU_LAYOUT_NV12,
+           "p010": _lib.TU_LAYOUT_P010}
+# colour of NV12 and P010 frames: matrix and range
 YUV = {"bt709": 0, "bt601": _lib.TU_YUV_BT601, "bt709_full": _lib.TU_YUV_FULL_RANGE,
        "bt601_full": _lib.TU_YUV_BT601 | _lib.TU_YUV_FULL_RANGE}
+# BT.2020 (HDR10 / HLG, 10-bit UHD): defined for 10-bit coding, so P010 frames only
+YUV_P010 = {"bt2020": _lib.TU_YUV_BT2020, "bt2020_full": _lib.TU_YUV_BT2020 | _lib.TU_YUV_FULL_RANGE}
 
 
 def layout_code(name: str) -> int:
     if name not in LAYOUTS:
-        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr' or 'nv12'")
+        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr', 'nv12' or 'p010'")
     return LAYOUTS[name]
 
 
 def yuv_code(name: str) -> int:
-    if name not in YUV:
-        raise ValueError(f"unknown NV12 colour {name!r}: use 'bt709', 'bt601', 'bt709_full' or 'bt601_full'")
-    return YUV[name]
+    if name in YUV:
+        return YUV[name]
+    if name in YUV_P010:
+        return YUV_P010[name]
+    raise ValueError(f"unknown YUV colour {name!r}: use 'bt709', 'bt601', 'bt709_full', 'bt601_full' or, for P010 frames, "
+                     "'bt2020', 'bt2020_full'")
 
 
 def _is_nv12(code: int) -> bool:
     return code & 0xF00 == _lib.TU_LAYOUT_NV12
 
 
+def _is_p010(code: int) -> bool:
+    return code & 0xF00 == _lib.TU_LAYOUT_P010
+
+
 def _image_shape(B: int, C_: int, h: int, w: int, code: int) -> Tuple[int, ...]:
-    """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3) or NV12 (B,3h/2,w)"""
-    if _is_nv12(code):
+    """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3) or NV12 / P010
+    (B,3h/2,w)"""
+    if _is_nv12(code) or _is_p010(code):
         return (B, 3 * h // 2, w)
     return (B, h, w, 3) if code >> 8 else (B, C_, h, w)
 
 
-def _nv12_hw(x: torch.Tensor) -> Tuple[int, int]:
-    """(H, W) of NV12 frames (B, 3H/2, W); raises ValueError for a shape that is not one"""
-    if x.dim() != 3 or x.dtype != torch.uint8:
-        raise ValueError(f"NV12 frames must be uint8 of shape (B, 3H/2, W), got {x.dtype} {tuple(x.shape)}")
+def _yuv420_hw(x: torch.Tensor, fmt: str, dtype: torch.dtype) -> Tuple[int, int]:
+    """(H, W) of 4:2:0 frames (B, 3H/2, W); raises ValueError for a shape or dtype that is not one"""
+    if x.dim() != 3 or x.dtype != dtype:
+        raise ValueError(f"{fmt} frames must be {str(dtype)[6:]} of shape (B, 3H/2, W), got {x.dtype} {tuple(x.shape)}")
     if x.shape[1] % 3:
-        raise ValueError(f"NV12 frames (B, 3H/2, W) need a row count divisible by 3, got {tuple(x.shape)}")
+        raise ValueError(f"{fmt} frames (B, 3H/2, W) need a row count divisible by 3, got {tuple(x.shape)}")
     H, W = int(x.shape[1]) * 2 // 3, int(x.shape[2])
     if H % 2 or W % 2:
-        raise ValueError(f"NV12 frames need an even height and width, got H={H} W={W}")
+        raise ValueError(f"{fmt} frames need an even height and width, got H={H} W={W}")
     return H, W
+
+
+def _nv12_hw(x: torch.Tensor) -> Tuple[int, int]:
+    """(H, W) of NV12 frames (B, 3H/2, W) uint8"""
+    return _yuv420_hw(x, "NV12", torch.uint8)
+
+
+def _p010_hw(x: torch.Tensor) -> Tuple[int, int]:
+    """(H, W) of P010 frames (B, 3H/2, W) uint16"""
+    return _yuv420_hw(x, "P010", torch.uint16)
 
 
 def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: int, compute_bf16: bool,
@@ -101,8 +123,8 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
     if pw is None:
         raise RuntimeError(f"tu::forward: packed-weights handle {handle} is not alive (its TransformerModel was deleted or repacked)")
     _require_cuda(x)
-    if _is_nv12(in_layout):
-        H, W = _nv12_hw(x)
+    if _is_nv12(in_layout) or _is_p010(in_layout):
+        H, W = _nv12_hw(x) if _is_nv12(in_layout) else _p010_hw(x)
         x = x.contiguous()
         B = x.shape[0]
     elif in_layout:
@@ -117,7 +139,9 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
         B, _, H, W = x.shape
     cdt = _lib.TU_BF16 if compute_bf16 else _lib.TU_F32
     out_shape = _image_shape(B, 3, out_h, out_w, out_code)
-    if out_code >> 8 and (out_code & 0xFF) != _lib.TU_U8:
+    if _is_p010(out_code) != ((out_code & 0xFF) == _lib.TU_U16):
+        raise RuntimeError("the P010 output layout is for uint16 frames, and uint16 output is P010 only")
+    if out_code >> 8 and not _is_p010(out_code) and (out_code & 0xFF) != _lib.TU_U8:
         raise RuntimeError("interleaved and NV12 output layouts are for uint8 frames")
     out = torch.empty(out_shape, dtype=_TORCH_DT[out_code & 0xFF], device=x.device)
     in_code = _code(x.dtype) | in_layout
@@ -190,32 +214,60 @@ def _(x, code):
     return x.new_empty((x.shape[0], 3 * x.shape[2] // 2, x.shape[3]), dtype=torch.uint8)
 
 
+@torch.library.custom_op("tu::rgb_to_p010", mutates_args=(), device_types="cuda")
+def tu_rgb_to_p010(x: torch.Tensor, code: int) -> torch.Tensor:
+    """planar fp32 RGB (B,3,H,W) -> P010 frames (B,3H/2,W) uint16; code = TU_U16 | TU_LAYOUT_P010 | colour bits"""
+    lib = _lib.load()
+    _require_cuda(x)
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != torch.float32:
+        raise RuntimeError(f"rgb_to_p010 takes planar fp32 RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    out = torch.empty((B, 3 * H // 2, W), dtype=torch.uint16, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_p010(x.data_ptr(), out.data_ptr(), code, B, H, W, _stream()))
+    return out
+
+
+@tu_rgb_to_p010.register_fake
+def _(x, code):
+    return x.new_empty((x.shape[0], 3 * x.shape[2] // 2, x.shape[3]), dtype=torch.uint16)
+
+
 def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int, int], upscale_factor: Optional[int],
                 require_ratio: bool, compute_bf16: bool, out_dtype: torch.dtype, clamp: bool = True,
                 in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709") -> torch.Tensor:
     """Shape logic of the three reference forwards (W:237-238, F:245-248,323-327, R:121-122) around tu::forward.
-    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'nv12'): uint8 frames may be interleaved (B,H,W,3) or NV12 (B,3H/2,W) on
-    either side; yuv ('bt709' | 'bt601' | 'bt709_full' | 'bt601_full') is the colour of the NV12 side(s)."""
+    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'nv12' | 'p010'): uint8 frames may be interleaved (B,H,W,3) or NV12
+    (B,3H/2,W) on either side, and either side may be P010 (B,3H/2,W) uint16 frames; yuv ('bt709' | 'bt601' | 'bt709_full' |
+    'bt601_full', and 'bt2020' | 'bt2020_full' for P010 only) is the colour of the NV12 / P010 side(s)."""
     il, ol = layout_code(in_layout), layout_code(out_layout)
     nv12_in, nv12_out = in_layout == "nv12", out_layout == "nv12"
-    if yuv != "bt709" and not (nv12_in or nv12_out):
-        raise ValueError(f"yuv={yuv!r} applies to NV12 frames only: pass in_layout='nv12' and / or out_layout='nv12'")
+    p010_in, p010_out = in_layout == "p010", out_layout == "p010"
+    if yuv != "bt709" and not (nv12_in or nv12_out or p010_in or p010_out):
+        raise ValueError(f"yuv={yuv!r} applies to NV12 / P010 frames only: pass in_layout / out_layout 'nv12' or 'p010'")
     yc = yuv_code(yuv)
+    if yuv in YUV_P010 and (nv12_in or nv12_out or not (p010_in or p010_out)):
+        raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a P010 side and no NV12 side")
     if nv12_out and out_dtype != torch.uint8:
         raise ValueError("out_layout='nv12' writes uint8 frames")
-    il |= yc if nv12_in else 0
+    if p010_out and out_dtype != torch.uint16:
+        raise ValueError("out_layout='p010' writes uint16 frames")
+    il |= yc if nv12_in or p010_in else 0
     if nv12_in:
         H, W = _nv12_hw(x)
+    elif p010_in:
+        H, W = _p010_hw(x)
     else:
         H, W = (int(x.shape[1]), int(x.shape[2])) if il else (int(x.shape[2]), int(x.shape[3]))
     if upscale_factor is not None:
         res_out = (H * upscale_factor, W * upscale_factor)
     res_out = (int(res_out[0]), int(res_out[1]))
-    out_code = _code(out_dtype) | ol | (yc if nv12_out else 0)
+    out_code = _code(out_dtype) | ol | (yc if nv12_out or p010_out else 0)
 
     def even_out(oh, ow):
-        if nv12_out and (oh % 2 or ow % 2):
-            raise ValueError(f"NV12 output frames need an even height and width, got {oh}x{ow}")
+        if (nv12_out or p010_out) and (oh % 2 or ow % 2):
+            raise ValueError(f"{'NV12' if nv12_out else 'P010'} output frames need an even height and width, got {oh}x{ow}")
 
     if model != "FastTransformer":
         even_out(*res_out)
@@ -233,9 +285,12 @@ def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int,
     even_out(*res_out)
     # Resize is the last op: the un-clamped full-size image stays in the compute dtype and the Resize kernel writes the requested
     # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store).  fp16 output keeps an fp32
-    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  NV12 output is the fp16 output converted
+    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  NV12 output is the fp16 output converted,
+    # P010 output the fp32 output converted
     mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) and not nv12_out else torch.float32)
     full = tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, mid_code, False, il)
     if nv12_out:
         return tu_rgb_to_nv12(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16), out_code)
+    if p010_out:
+        return tu_rgb_to_p010(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F32), out_code)
     return tu_resize_aa(full, res_out[0], res_out[1], clamp, out_code)

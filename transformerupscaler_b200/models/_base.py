@@ -153,7 +153,11 @@ class EngineModel(nn.Module):
         in_layout / out_layout in {'chw', 'hwc', 'hwc_bgr', 'nv12'} — uint8 frames may arrive / leave interleaved (B,H,W,3), the form PIL
         and OpenCV hold them in (inference.py:65-70, app_overlay.py:382-386), with the channel swap done in the last kernel, or as
         NV12 video frames (B,3H/2,W), the form video decoders hand out and encoders take, converted on the GPU at both ends.
-        yuv in {'bt709', 'bt601', 'bt709_full', 'bt601_full'} is the colour matrix and range of the NV12 side(s)."""
+        'p010' on either side: 10-bit P010 video frames (B,3H/2,W) uint16 (HEVC Main10, AV1, VP9 profile 2, HDR), code in the high
+        10 bits of each word.  in_layout='p010' takes uint16 frames; out_layout='p010' returns uint16 frames for any frame input
+        (uint8 in any layout, or P010), and a P010 input with any other out_layout returns uint8 frames.
+        yuv in {'bt709', 'bt601', 'bt709_full', 'bt601_full'} is the colour matrix and range of the NV12 / P010 side(s); 'bt2020' and
+        'bt2020_full' (BT.2020 / BT.2100) need a P010 side and no NV12 side."""
         if self.training:
             raise RuntimeError("transformerupscaler_b200 is a forward-only inference engine: call .eval() first "
                                "(dropout is treated as identity; there is no backward)")
@@ -163,18 +167,22 @@ class EngineModel(nn.Module):
             raise RuntimeError("transformerupscaler_b200 is forward-only (no autograd): the input requires grad; call under torch.no_grad()")
         # uint8 frames in -> uint8 frames out (ToTensor scaling on read, (out*255).clamp(0,255).to(uint8) on write, fused into
         # the first and last kernels): the video-pipeline entry, an extension of the reference's float-only signature
+        # P010 frames are uint16; any other uint16 tensor is an image like any other and is read as float32
+        if in_layout == "p010" and x.dtype != torch.uint16:
+            raise ValueError(f"in_layout='p010' takes uint16 frames (B, 3H/2, W), got {x.dtype}")
         frames_u8 = x.dtype == torch.uint8
-        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8):
+        frames = frames_u8 or in_layout == "p010"
+        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8) and not frames:
             x = x.float()
         bf16, out_dt = self._select_precision(x)
-        if frames_u8:
-            out_dt = torch.uint8
+        if frames:
+            out_dt = torch.uint16 if out_layout == "p010" else torch.uint8
         handle = self._packed(bf16, x.device)
-        if (in_layout != "chw" or out_layout != "chw") and not frames_u8:
-            raise ValueError("in_layout / out_layout other than 'chw' apply to uint8 frames only")
+        if (in_layout != "chw" or out_layout != "chw") and not frames:
+            raise ValueError("in_layout / out_layout other than 'chw' apply to uint8 / P010 frames only")
         out = engine.run_forward(handle, self.ENGINE_MODEL, x, res_out, upscale_factor, require_ratio, bf16, out_dt,
                                  in_layout=in_layout, out_layout=out_layout, yuv=yuv)
-        if not frames_u8 and x.is_cuda and torch.is_autocast_enabled("cuda") and not self.AUTOCAST_OUT_FP32:
+        if not frames and x.is_cuda and torch.is_autocast_enabled("cuda") and not self.AUTOCAST_OUT_FP32:
             want = torch.get_autocast_dtype("cuda")
             if out.dtype != want:
                 out = out.to(want)

@@ -219,6 +219,21 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
  */
+/* one NV12 / P010 frame as a video decoder maps it or an encoder registers it: two planes, each with its own row pitch, anywhere in
+ * device memory.  A sample is 1 byte (NV12) or one 2-byte word (P010, the code in the high 10 bits as above).
+ *   y:  H rows of W samples; row r starts at y + r * y_pitch bytes;
+ *   uv: H/2 rows of W samples (W/2 interleaved (U, V) pairs, U first); row r starts at uv + r * uv_pitch bytes;
+ *   y_pitch, uv_pitch: bytes between rows, >= W samples.
+ * The kernels access a pair of samples at a time, so both plane pointers and both pitches must be multiples of 2 bytes (NV12) or
+ * 4 bytes (P010).  A write touches only the W samples of each row: pitch padding and the bytes between or after the planes are never
+ * written.  The surfaces of one call must not overlap each other or the other side's buffers; the library does not check that. */
+typedef struct TuFramePlanes {
+    void *y;
+    void *uv;
+    long long y_pitch;
+    long long uv_pitch;
+} TuFramePlanes;
+
 size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
 /* the same, sized from the packed weights actually used (non-default dim / heads / n_blocks; which fused kernels are packed) */
 size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
@@ -230,6 +245,16 @@ size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int 
 int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype,
                int B, int H, int W, int outH, int outW, int scale, int compute_dtype, int clamp,
                void *workspace, size_t workspace_bytes, void *stream);
+/* tu_forward with per-frame decoder / encoder surfaces on an NV12 or P010 side.  On each side exactly one of the dense buffer (x, out)
+ * and x_frames / out_frames, a HOST array of B TuFramePlanes, is non-NULL; a frames array is valid only when that side's code is NV12 or
+ * P010.  Frame b of the batch is x_frames[b] / out_frames[b].  The arrays are read during the call (the descriptors travel in kernel
+ * parameters), so the caller may reuse them once it returns, and a captured CUDA graph replays the same surfaces.  Every descriptor is
+ * checked before anything is enqueued (TU_ERR_ARG, with the frame index and field in tu_last_error).  The workspace is the one
+ * tu_forward_workspace_bytes_io gives for the same codes: surfaces do not change it.  The results are bitwise those of tu_forward on the
+ * dense frames of the same contents.  tu_forward(...) is tu_forward_planes with both arrays NULL. */
+int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlanes *x_frames, int in_dtype, void *out,
+                      const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
+                      int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---- single ops (exported for the per-op parity tests and for composition) ---------------------- */
 /* conv1: 3->64 3x3 p1 + ReLU, NCHW in -> NHWC out.  w64 (optional, bf16 (64,64)) enables the tensor-core kernel
@@ -342,6 +367,11 @@ int tu_rgb_to_nv12(const void *rgb_f16, void *nv12, int code, int B, int H, int 
  *            limited, (1023, 0) / (1023, 512) full range, stored as code << 6. */
 int tu_p010_to_rgb(const void *p010, int code, void *rgb_f32, int B, int H, int W, void *stream);
 int tu_rgb_to_p010(const void *rgb_f32, void *p010, int code, int B, int H, int W, void *stream);
+/* the four ops above on per-frame surfaces: frames is a HOST array of B TuFramePlanes (see tu_forward_planes), read during the call.
+ * code = TU_U8 | TU_LAYOUT_NV12 [| colour bits] with planar fp16 RGB (4-byte aligned), or TU_U16 | TU_LAYOUT_P010 [| colour bits] with
+ * planar fp32 RGB (8-byte aligned); rgb is a dense (B, 3, H, W) buffer.  Same bits as the dense ops on the same frame contents. */
+int tu_yuv420_planes_to_rgb(const TuFramePlanes *frames, int code, void *rgb, int B, int H, int W, void *stream);
+int tu_rgb_to_yuv420_planes(const void *rgb, const TuFramePlanes *frames, int code, int B, int H, int W, void *stream);
 
 #ifdef __cplusplus
 }

@@ -73,6 +73,11 @@ class TuPackedModel(C.Structure):
                 ("device_bytes_used", C.c_size_t)]
 
 
+class TuFramePlanes(C.Structure):
+    """one NV12 / P010 frame as two device planes with row pitches in bytes (decoder / encoder surfaces)"""
+    _fields_ = [("y", C.c_void_p), ("uv", C.c_void_p), ("y_pitch", C.c_longlong), ("uv_pitch", C.c_longlong)]
+
+
 # name -> (restype, argtypes); must list every symbol include/tu_b200.h declares
 SIGNATURES = {
     "tu_version": (i32, []),
@@ -92,6 +97,8 @@ SIGNATURES = {
     "tu_forward_workspace_bytes_for": (sz, [C.POINTER(TuModelWeights)] + [i32] * 7),
     "tu_forward_workspace_bytes_io": (sz, [C.POINTER(TuModelWeights)] + [i32] * 9),
     "tu_forward": (i32, [C.POINTER(TuModelWeights), vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp, sz, vp]),
+    "tu_forward_planes": (i32, [C.POINTER(TuModelWeights), vp, C.POINTER(TuFramePlanes), i32, vp, C.POINTER(TuFramePlanes), i32,
+                                i32, i32, i32, i32, i32, i32, i32, i32, vp, sz, vp]),
     "tu_stem_conv": (i32, [vp, i32, fp, vp, fp, vp, i32, i32, i32, i32, vp]),
     "tu_conv3x3_c64": (i32, [vp, vp, fp, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp]),
     "tu_conv3x3_c64_to3": (i32, [vp, i32, fp, vp, fp, fp, i32, i32, i32, i32, vp]),
@@ -120,6 +127,8 @@ SIGNATURES = {
     "tu_rgb_to_nv12": (i32, [vp, vp, i32, i32, i32, i32, vp]),
     "tu_p010_to_rgb": (i32, [vp, i32, vp, i32, i32, i32, vp]),
     "tu_rgb_to_p010": (i32, [vp, vp, i32, i32, i32, i32, vp]),
+    "tu_yuv420_planes_to_rgb": (i32, [C.POINTER(TuFramePlanes), i32, vp, i32, i32, i32, vp]),
+    "tu_rgb_to_yuv420_planes": (i32, [vp, C.POINTER(TuFramePlanes), i32, i32, i32, i32, vp]),
 }
 
 

@@ -125,9 +125,10 @@ struct Arena {
 static int scale_slot(int s) { return s == 2 ? 0 : s == 3 ? 1 : s == 4 ? 2 : s == 6 ? 3 : -1; }
 
 // Runs (or, with a.dry, only sizes) one forward.  TI/TO are handled by dtype codes in the leaf launchers.
+// xf / of: the input / output frame surfaces of an NV12 / P010 side, or NULL for the dense buffer x / out.
 template <typename T>
-static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype, int B, int H,
-                        int W, int outH, int outW, int scale, int clamp, Arena &a, cudaStream_t st) {
+static int forward_impl(const TuModelWeights *w, const void *x, const TuFramePlanes *xf, int in_dtype, void *out, const TuFramePlanes *of,
+                        int out_dtype, int B, int H, int W, int outH, int outW, int scale, int clamp, Arena &a, cudaStream_t st) {
     const int dt = sizeof(T) == 2 ? TU_BF16 : TU_F32;
     const bool dry = a.dry;
     const int model = w->model, dim = w->dim, heads = w->heads;
@@ -165,13 +166,13 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
     // included), and the final bicubic reads the same buffer
     if (dtype_is_nv12(in_dtype)) {
         f16 *rgb = (f16 *)a.get((size_t)B * 3 * H * W * sizeof(f16));
-        if (!dry) TU_STEP("nv12_to_rgb", tu_nv12_to_rgb(x, in_dtype, rgb, B, H, W, stv));
+        if (!dry) TU_STEP("nv12_to_rgb", xf ? tu_yuv420_planes_to_rgb(xf, in_dtype, rgb, B, H, W, stv) : tu_nv12_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F16;
     } else if (dtype_is_p010(in_dtype)) {
         // P010 frames are converted to planar fp32 (fp16 cannot hold every 10-bit step exactly): the forward is then the fp32-input one
         float *rgb = (float *)a.get((size_t)B * 3 * H * W * sizeof(float));
-        if (!dry) TU_STEP("p010_to_rgb", tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
+        if (!dry) TU_STEP("p010_to_rgb", xf ? tu_yuv420_planes_to_rgb(xf, in_dtype, rgb, B, H, W, stv) : tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F32;
     }
@@ -180,8 +181,9 @@ static int forward_impl(const TuModelWeights *w, const void *x, int in_dtype, vo
     void *img = nv12_out ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
                 : p010_out ? a.get((size_t)B * 3 * outH * outW * sizeof(float)) : out;
     const int img_dtype = nv12_out ? TU_F16 : p010_out ? TU_F32 : out_dtype;
-#define TU_YUV_OUT()                                                                    \
-    if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv)); \
+#define TU_YUV_OUT()                                                                                                    \
+    if (of) TU_STEP(nv12_out ? "rgb_to_nv12" : "rgb_to_p010", tu_rgb_to_yuv420_planes(img, of, out_dtype, B, outH, outW, stv)); \
+    else if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv));                    \
     else if (p010_out) TU_STEP("rgb_to_p010", tu_rgb_to_p010(img, out, out_dtype, B, outH, outW, stv))
 
     // interleaved uint8 frames (HWC RGB / BGR) are made planar once; the stem and the final bicubic both read the planar copy
@@ -699,8 +701,8 @@ extern "C" size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int
     if (check_forward_args(&w, B, H, W, outH, outW, compute_dtype)) return 0;
     Arena a{nullptr, 0, 0, true};
     int rc = compute_dtype == TU_F32
-                 ? forward_impl<float>(&w, nullptr, TU_F32, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0)
-                 : forward_impl<bf16>(&w, nullptr, TU_F32, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0);
+                 ? forward_impl<float>(&w, nullptr, nullptr, TU_F32, nullptr, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0)
+                 : forward_impl<bf16>(&w, nullptr, nullptr, TU_F32, nullptr, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0);
     return rc == TU_OK ? a.off : 0;
 }
 
@@ -709,8 +711,8 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
     if (check_forward_args(w, B, H, W, outH, outW, compute_dtype)) return 0;
     Arena a{nullptr, 0, 0, true};
     int rc = compute_dtype == TU_F32
-                 ? forward_impl<float>(w, nullptr, TU_F32, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0)
-                 : forward_impl<bf16>(w, nullptr, TU_F32, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0);
+                 ? forward_impl<float>(w, nullptr, nullptr, TU_F32, nullptr, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0)
+                 : forward_impl<bf16>(w, nullptr, nullptr, TU_F32, nullptr, nullptr, TU_F32, B, H, W, outH, outW, scale, 1, a, 0);
     return rc == TU_OK ? a.off : 0;
 }
 
@@ -740,18 +742,25 @@ extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, 
     out_dtype = dtype_is_yuv420(out_dtype) ? out_dtype : TU_F32;
     Arena a{nullptr, 0, 0, true};
     int rc = compute_dtype == TU_F32
-                 ? forward_impl<float>(w, nullptr, in_dtype, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0)
-                 : forward_impl<bf16>(w, nullptr, in_dtype, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0);
+                 ? forward_impl<float>(w, nullptr, nullptr, in_dtype, nullptr, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0)
+                 : forward_impl<bf16>(w, nullptr, nullptr, in_dtype, nullptr, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0);
     return rc == TU_OK ? a.off : 0;
 }
 
-extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype, int B, int H,
-                          int W, int outH, int outW, int scale, int compute_dtype, int clamp, void *workspace,
-                          size_t workspace_bytes, void *stream) {
+extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlanes *x_frames, int in_dtype, void *out,
+                                 const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
+                                 int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream) {
     int rc = check_forward_args(w, B, H, W, outH, outW, compute_dtype);
     if (rc) return rc;
-    TU_CHECK_ARG(x && out && workspace, "forward: null buffer");
+    TU_CHECK_ARG((x || x_frames) && (out || out_frames) && workspace, "forward: null buffer");
+    TU_CHECK_ARG(!(x && x_frames), "forward: give the input as either x or x_frames, not both");
+    TU_CHECK_ARG(!(out && out_frames), "forward: give the output as either out or out_frames, not both");
     if ((rc = check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
+    TU_CHECK_ARG(!x_frames || dtype_is_yuv420(in_dtype), "forward: x_frames (frame planes) are for NV12 / P010 input only");
+    TU_CHECK_ARG(!out_frames || dtype_is_yuv420(out_dtype), "forward: out_frames (frame planes) are for NV12 / P010 output only");
+    // every descriptor is checked here, before the first kernel of the forward is enqueued
+    if (x_frames && (rc = check_yuv420_planes(x_frames, in_dtype, B, H, W, "forward: x_frames"))) return rc;
+    if (out_frames && (rc = check_yuv420_planes(out_frames, out_dtype, B, outH, outW, "forward: out_frames"))) return rc;
     {
         const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype);
         const int il = dtype_is_yuv420(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_yuv420(out_dtype) ? 0 : dtype_layout(out_dtype);
@@ -766,8 +775,8 @@ extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, 
     // size pass, then the real pass
     Arena dry{nullptr, 0, 0, true};
     rc = compute_dtype == TU_F32
-             ? forward_impl<float>(w, x, in_dtype, out, out_dtype, B, H, W, outH, outW, scale, clamp, dry, 0)
-             : forward_impl<bf16>(w, x, in_dtype, out, out_dtype, B, H, W, outH, outW, scale, clamp, dry, 0);
+             ? forward_impl<float>(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, clamp, dry, 0)
+             : forward_impl<bf16>(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, clamp, dry, 0);
     if (rc) return rc;
     if (dry.off > workspace_bytes) {
         set_error("tu: forward workspace too small: need " + std::to_string(dry.off) + " bytes");
@@ -776,6 +785,13 @@ extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, 
     Arena a{(char *)workspace, 0, workspace_bytes, false};
     cudaStream_t st = (cudaStream_t)stream;
     return compute_dtype == TU_F32
-               ? forward_impl<float>(w, x, in_dtype, out, out_dtype, B, H, W, outH, outW, scale, clamp, a, st)
-               : forward_impl<bf16>(w, x, in_dtype, out, out_dtype, B, H, W, outH, outW, scale, clamp, a, st);
+               ? forward_impl<float>(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, clamp, a, st)
+               : forward_impl<bf16>(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, clamp, a, st);
+}
+
+extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype, int B, int H,
+                          int W, int outH, int outW, int scale, int compute_dtype, int clamp, void *workspace,
+                          size_t workspace_bytes, void *stream) {
+    return tu_forward_planes(w, x, nullptr, in_dtype, out, nullptr, out_dtype, B, H, W, outH, outW, scale, compute_dtype, clamp, workspace,
+                             workspace_bytes, stream);
 }

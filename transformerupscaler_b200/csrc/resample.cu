@@ -10,6 +10,7 @@
 #include <cuda.h>
 
 #include <algorithm>
+#include <type_traits>
 
 #include "tc/ptx.cuh"
 #include "tc/tc_api.cuh"
@@ -1070,6 +1071,37 @@ template <> struct Yuv420<uint16_t> {
     static __device__ __forceinline__ Pair pair(uint16_t a, uint16_t b) { return make_ushort2(a, b); }
 };
 
+// Frame addressing of the 4:2:0 kernels: where row r of a frame's luma and chroma planes starts.  blockIdx.y is the frame of the launch
+// (the RGB side is always a dense (B, 3, H, W) batch indexed by it).  Param is the kernel parameter that carries the frames.
+// Dense: one (B, 3H/2, W) buffer, row pitch W samples, the chroma plane right after the luma plane, frame b at b * 3HW/2.
+template <typename TS> struct Dense420 {
+    typedef TS *__restrict__ Param;
+    TS *y, *uv;
+    int W;
+    static __device__ __forceinline__ Dense420 frame(Param p, int H, int W) {
+        const long plane = (long)H * W;
+        TS *f = p + (long)blockIdx.y * (plane + plane / 2);
+        return {f, f + plane, W};
+    }
+    __device__ __forceinline__ TS *yrow(int r) const { return y + (long)r * W; }
+    __device__ __forceinline__ TS *uvrow(int r) const { return uv + (long)r * W; }
+};
+// Surfaces: frame blockIdx.y of a table of up to kPlanesPerLaunch TuFramePlanes passed by value in the kernel parameters (no copy of
+// descriptors to the device, so a captured graph needs no host memory alive); a larger batch is several launches.  64 x 32 bytes keeps
+// the parameters of a launch at about 2 KB, within the classic 4 KB limit.
+constexpr int kPlanesPerLaunch = 64;
+template <typename TS> struct Planes420 {
+    struct Param { TuFramePlanes f[kPlanesPerLaunch]; };
+    TS *y, *uv;
+    long long yp, uvp;
+    static __device__ __forceinline__ Planes420 frame(const Param &p, int, int) {
+        const TuFramePlanes &d = p.f[blockIdx.y];
+        return {(TS *)d.y, (TS *)d.uv, d.y_pitch, d.uv_pitch};
+    }
+    __device__ __forceinline__ TS *yrow(int r) const { return (TS *)((char *)y + (long long)r * yp); }
+    __device__ __forceinline__ TS *uvrow(int r) const { return (TS *)((char *)uv + (long long)r * uvp); }
+};
+
 __device__ __forceinline__ float clamp01(float v) { return fminf(fmaxf(v, 0.f), 1.f); }
 // two horizontally adjacent RGB values of one plane (an aligned half2 / float2)
 __device__ __forceinline__ void store_rgb2(f16 *p, float a, float b) { *reinterpret_cast<__half2 *>(p) = __floats2half2_rn(a, b); }
@@ -1080,8 +1112,8 @@ __device__ __forceinline__ float2 load_rgb2(const float *p) { return *reinterpre
 // One thread per chroma sample (i, j): the 2x2 luma block rows 2i..2i+1, columns 2j..2j+1.  Bilinear chroma: luma row 2i takes
 // (C[i-1] + 3 C[i]) / 4, row 2i+1 (3 C[i] + C[i+1]) / 4; column 2j takes chroma column j, column 2j+1 the mean of j and j+1 (edges
 // clamped).  These are integer sums (at most 8 * 1023) times 1/4 or 1/8: exact in fp32.
-template <typename TS, typename TR>
-__global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(const TS *__restrict__ in, TR *__restrict__ out, int H, int W, YuvCoef k) {
+template <typename TS, typename TR, typename A>
+__global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(typename A::Param in, TR *__restrict__ out, int H, int W, YuvCoef k) {
     typedef Yuv420<TS> F;
     typedef typename F::Pair P;
     constexpr int s = F::shift;
@@ -1092,20 +1124,19 @@ __global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(const TS *__restrict
     if (t >= Hc * Wc) return;
     const int i = t / Wc, j = t - i * Wc;
     const long plane = (long)H * W;
-    const TS *f = in + (long)blockIdx.y * (plane + plane / 2);
-    const TS *ch = f + plane;
+    const A f = A::frame(in, H, W);
     const int im = max(i - 1, 0), ip = min(i + 1, Hc - 1), jp = min(j + 1, Wc - 1);
-    const P cm0 = *reinterpret_cast<const P *>(ch + (long)im * W + 2 * j), cm1 = *reinterpret_cast<const P *>(ch + (long)im * W + 2 * jp);
-    const P c00 = *reinterpret_cast<const P *>(ch + (long)i * W + 2 * j), c01 = *reinterpret_cast<const P *>(ch + (long)i * W + 2 * jp);
-    const P cp0 = *reinterpret_cast<const P *>(ch + (long)ip * W + 2 * j), cp1 = *reinterpret_cast<const P *>(ch + (long)ip * W + 2 * jp);
+    const P cm0 = *reinterpret_cast<const P *>(f.uvrow(im) + 2 * j), cm1 = *reinterpret_cast<const P *>(f.uvrow(im) + 2 * jp);
+    const P c00 = *reinterpret_cast<const P *>(f.uvrow(i) + 2 * j), c01 = *reinterpret_cast<const P *>(f.uvrow(i) + 2 * jp);
+    const P cp0 = *reinterpret_cast<const P *>(f.uvrow(ip) + 2 * j), cp1 = *reinterpret_cast<const P *>(f.uvrow(ip) + 2 * jp);
     // vertical sums (x4) of U and V for the top (2i) and bottom (2i+1) luma rows, at chroma columns j and j+1
     const int ut0 = (cm0.x >> s) + 3 * (c00.x >> s), ut1 = (cm1.x >> s) + 3 * (c01.x >> s);
     const int ub0 = 3 * (c00.x >> s) + (cp0.x >> s), ub1 = 3 * (c01.x >> s) + (cp1.x >> s);
     const int vt0 = (cm0.y >> s) + 3 * (c00.y >> s), vt1 = (cm1.y >> s) + 3 * (c01.y >> s);
     const int vb0 = 3 * (c00.y >> s) + (cp0.y >> s), vb1 = 3 * (c01.y >> s) + (cp1.y >> s);
     const int us[4] = {2 * ut0, ut0 + ut1, 2 * ub0, ub0 + ub1}, vs[4] = {2 * vt0, vt0 + vt1, 2 * vb0, vb0 + vb1};   // x8
-    const P y0 = *reinterpret_cast<const P *>(f + (long)(2 * i) * W + 2 * j);
-    const P y1 = *reinterpret_cast<const P *>(f + (long)(2 * i + 1) * W + 2 * j);
+    const P y0 = *reinterpret_cast<const P *>(f.yrow(2 * i) + 2 * j);
+    const P y1 = *reinterpret_cast<const P *>(f.yrow(2 * i + 1) + 2 * j);
     const int ys[4] = {y0.x >> s, y0.y >> s, y1.x >> s, y1.y >> s};
     float r[4], g[4], bl[4];
 #pragma unroll
@@ -1133,8 +1164,8 @@ __device__ __forceinline__ TS yuv_code(float v) {         // min(max(floor(v + 0
 
 // One thread per chroma sample (i, j): its (U, V) pair and its 2x2 luma block.  Chroma filter (type-0 siting): the column sums
 // v(c) = P[2i][c] + P[2i+1][c] weighted 1, 2, 1 over columns 2j-1 (clamped at 0), 2j, 2j+1, times 1/8, per channel.
-template <typename TR, typename TS>
-__global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict__ in, TS *__restrict__ out, int H, int W, YuvCoef k) {
+template <typename TR, typename TS, typename A>
+__global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict__ in, typename A::Param out, int H, int W, YuvCoef k) {
     typedef Yuv420<TS> F;
     typedef typename F::Pair P;
     pdl_trigger();
@@ -1165,10 +1196,10 @@ __global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict
     }
     const float cb = __fadd_rn(__fadd_rn(__fmul_rn(k.cb_r, bar[0]), __fmul_rn(k.cb_g, bar[1])), __fmul_rn(0.5f, bar[2]));
     const float cr = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, bar[0]), __fmul_rn(k.cr_g, bar[1])), __fmul_rn(k.cr_b, bar[2]));
-    TS *f = out + (long)blockIdx.y * (plane + plane / 2);
-    *reinterpret_cast<P *>(f + (long)(2 * i) * W + 2 * j) = F::pair(yq[0], yq[1]);
-    *reinterpret_cast<P *>(f + (long)(2 * i + 1) * W + 2 * j) = F::pair(yq[2], yq[3]);
-    *reinterpret_cast<P *>(f + plane + (long)i * W + 2 * j) =
+    const A f = A::frame(out, H, W);
+    *reinterpret_cast<P *>(f.yrow(2 * i) + 2 * j) = F::pair(yq[0], yq[1]);
+    *reinterpret_cast<P *>(f.yrow(2 * i + 1) + 2 * j) = F::pair(yq[2], yq[3]);
+    *reinterpret_cast<P *>(f.uvrow(i) + 2 * j) =
         F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid)));
 }
 
@@ -1461,7 +1492,7 @@ static int check_yuv420_args(const void *frames, int code, bool p010, const void
 extern "C" int tu_nv12_to_rgb(const void *nv12, int code, void *rgb_f16, int B, int H, int W, void *stream) {
     if (int rc = check_yuv420_args(nv12, code, false, rgb_f16, B, H, W, "nv12_to_rgb")) return rc;
     const int n = (H / 2) * (W / 2);
-    launch_pdl(yuv420_to_rgb_kernel<uint8_t, f16>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+    launch_pdl(yuv420_to_rgb_kernel<uint8_t, f16, Dense420<const uint8_t>>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
                (const uint8_t *)nv12, (f16 *)rgb_f16, H, W, yuv_coef(code));
     TU_CHECK_LAUNCH("nv12_to_rgb");
     return TU_OK;
@@ -1470,7 +1501,7 @@ extern "C" int tu_nv12_to_rgb(const void *nv12, int code, void *rgb_f16, int B, 
 extern "C" int tu_rgb_to_nv12(const void *rgb_f16, void *nv12, int code, int B, int H, int W, void *stream) {
     if (int rc = check_yuv420_args(nv12, code, false, rgb_f16, B, H, W, "rgb_to_nv12")) return rc;
     const int n = (H / 2) * (W / 2);
-    launch_pdl(rgb_to_yuv420_kernel<f16, uint8_t>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+    launch_pdl(rgb_to_yuv420_kernel<f16, uint8_t, Dense420<uint8_t>>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
                (const f16 *)rgb_f16, (uint8_t *)nv12, H, W, yuv_coef(code));
     TU_CHECK_LAUNCH("rgb_to_nv12");
     return TU_OK;
@@ -1479,7 +1510,7 @@ extern "C" int tu_rgb_to_nv12(const void *rgb_f16, void *nv12, int code, int B, 
 extern "C" int tu_p010_to_rgb(const void *p010, int code, void *rgb_f32, int B, int H, int W, void *stream) {
     if (int rc = check_yuv420_args(p010, code, true, rgb_f32, B, H, W, "p010_to_rgb")) return rc;
     const int n = (H / 2) * (W / 2);
-    launch_pdl(yuv420_to_rgb_kernel<uint16_t, float>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+    launch_pdl(yuv420_to_rgb_kernel<uint16_t, float, Dense420<const uint16_t>>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
                (const uint16_t *)p010, (float *)rgb_f32, H, W, yuv_coef(code));
     TU_CHECK_LAUNCH("p010_to_rgb");
     return TU_OK;
@@ -1488,8 +1519,79 @@ extern "C" int tu_p010_to_rgb(const void *p010, int code, void *rgb_f32, int B, 
 extern "C" int tu_rgb_to_p010(const void *rgb_f32, void *p010, int code, int B, int H, int W, void *stream) {
     if (int rc = check_yuv420_args(p010, code, true, rgb_f32, B, H, W, "rgb_to_p010")) return rc;
     const int n = (H / 2) * (W / 2);
-    launch_pdl(rgb_to_yuv420_kernel<float, uint16_t>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
+    launch_pdl(rgb_to_yuv420_kernel<float, uint16_t, Dense420<uint16_t>>, dim3((unsigned)ceil_div(n, 256), B), dim3(256), 0, (cudaStream_t)stream,
                (const float *)rgb_f32, (uint16_t *)p010, H, W, yuv_coef(code));
     TU_CHECK_LAUNCH("rgb_to_p010");
     return TU_OK;
+}
+
+// B frame surfaces of an NV12 (code TU_U8 | TU_LAYOUT_NV12 ...) or P010 (TU_U16 | TU_LAYOUT_P010 ...) side: host-side checks of the
+// code, the sizes and every descriptor, made before anything is enqueued (tu_forward_planes runs them ahead of its first kernel)
+int tu::check_yuv420_planes(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op) {
+    TU_CHECK_ARG(frames && B > 0 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_yuv420(code), std::string(op) + ": frame planes are for NV12 (TU_U8 | TU_LAYOUT_NV12 [| colour bits]) or P010 "
+                                                          "(TU_U16 | TU_LAYOUT_P010 [| colour bits]) frames only");
+    const bool p010 = dtype_is_p010(code);
+    const std::string fmt = p010 ? "P010" : "NV12";
+    TU_CHECK_ARG(H % 2 == 0 && W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even height and width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    const long long row = (long long)W * (p010 ? 2 : 1);
+    const uintptr_t al = p010 ? 4 : 2;                              // a pair of samples is one access
+    const char *al_msg = p010 ? "a multiple of 4 bytes (P010)" : "a multiple of 2 bytes (NV12)";
+    for (int b = 0; b < B; ++b) {
+        const TuFramePlanes &d = frames[b];
+        const std::string at = std::string(op) + ": frame " + std::to_string(b) + ": ";
+        TU_CHECK_ARG(d.y, at + "y is NULL");
+        TU_CHECK_ARG(d.uv, at + "uv is NULL");
+        TU_CHECK_ARG(d.y_pitch >= row, at + "y_pitch " + std::to_string(d.y_pitch) + " is smaller than W samples (" + std::to_string(row) + " bytes)");
+        TU_CHECK_ARG(d.uv_pitch >= row, at + "uv_pitch " + std::to_string(d.uv_pitch) + " is smaller than W samples (" + std::to_string(row) + " bytes)");
+        TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.y) % al == 0, at + "y must be " + al_msg);
+        TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.uv) % al == 0, at + "uv must be " + al_msg);
+        TU_CHECK_ARG(d.y_pitch % (long long)al == 0, at + "y_pitch must be " + al_msg);
+        TU_CHECK_ARG(d.uv_pitch % (long long)al == 0, at + "uv_pitch must be " + al_msg);
+    }
+    return TU_OK;
+}
+
+// one launch per kPlanesPerLaunch frames; the RGB side is the dense batch, offset to the first frame of the launch
+template <typename TS, typename TR, bool ToRgb>
+static int launch_planes(const TuFramePlanes *frames, int code, TR *rgb, int B, int H, int W, cudaStream_t st, const char *what) {
+    typedef Planes420<typename std::conditional<ToRgb, const TS, TS>::type> A;
+    const int n = (H / 2) * (W / 2);
+    const long frame = 3L * H * W;
+    for (int b0 = 0; b0 < B; b0 += kPlanesPerLaunch) {
+        const int nb = std::min(kPlanesPerLaunch, B - b0);
+        typename A::Param p = {};
+        for (int b = 0; b < nb; ++b) p.f[b] = frames[b0 + b];
+        const dim3 grid((unsigned)ceil_div(n, 256), nb);
+        if constexpr (ToRgb)
+            launch_pdl(yuv420_to_rgb_kernel<TS, TR, A>, grid, dim3(256), 0, st, p, rgb + b0 * frame, H, W, yuv_coef(code));
+        else
+            launch_pdl(rgb_to_yuv420_kernel<TR, TS, A>, grid, dim3(256), 0, st, (const TR *)rgb + b0 * frame, p, H, W,
+                       yuv_coef(code));
+        TU_CHECK_LAUNCH(what);
+    }
+    return TU_OK;
+}
+
+extern "C" int tu_yuv420_planes_to_rgb(const TuFramePlanes *frames, int code, void *rgb, int B, int H, int W, void *stream) {
+    if (int rc = check_yuv420_planes(frames, code, B, H, W, "yuv420_planes_to_rgb")) return rc;
+    const bool p010 = dtype_is_p010(code);
+    TU_CHECK_ARG(rgb && (reinterpret_cast<uintptr_t>(rgb) & (p010 ? 7 : 3)) == 0,
+                 std::string(p010 ? "yuv420_planes_to_rgb: the fp32 RGB buffer must be non-NULL and 8-byte aligned"
+                                  : "yuv420_planes_to_rgb: the fp16 RGB buffer must be non-NULL and 4-byte aligned"));
+    cudaStream_t st = (cudaStream_t)stream;
+    return p010 ? launch_planes<uint16_t, float, true>(frames, code, (float *)rgb, B, H, W, st, "p010_to_rgb")
+                : launch_planes<uint8_t, f16, true>(frames, code, (f16 *)rgb, B, H, W, st, "nv12_to_rgb");
+}
+
+extern "C" int tu_rgb_to_yuv420_planes(const void *rgb, const TuFramePlanes *frames, int code, int B, int H, int W, void *stream) {
+    if (int rc = check_yuv420_planes(frames, code, B, H, W, "rgb_to_yuv420_planes")) return rc;
+    const bool p010 = dtype_is_p010(code);
+    TU_CHECK_ARG(rgb && (reinterpret_cast<uintptr_t>(rgb) & (p010 ? 7 : 3)) == 0,
+                 std::string(p010 ? "rgb_to_yuv420_planes: the fp32 RGB buffer must be non-NULL and 8-byte aligned"
+                                  : "rgb_to_yuv420_planes: the fp16 RGB buffer must be non-NULL and 4-byte aligned"));
+    cudaStream_t st = (cudaStream_t)stream;
+    return p010 ? launch_planes<uint16_t, float, false>(frames, code, (float *)rgb, B, H, W, st, "rgb_to_p010")
+                : launch_planes<uint8_t, f16, false>(frames, code, (f16 *)rgb, B, H, W, st, "rgb_to_nv12");
 }

@@ -19,6 +19,8 @@ typedef __half f16;
 void set_error(const std::string &msg);
 int cuda_fail(cudaError_t e, const char *what);
 void count_launch();   // every kernel launch of the library is counted (tu_launch_count)
+// checks B NV12 / P010 frame surfaces (resample.cu): TU_ERR_ARG with the frame index and field in the message
+int check_yuv420_planes(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op);
 
 #define TU_CHECK_ARG(cond, msg)                         \
     do {                                                \

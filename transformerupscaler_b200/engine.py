@@ -11,7 +11,7 @@ import ctypes as C
 import itertools
 import math
 import weakref
-from typing import Dict, Optional, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
 
@@ -116,6 +116,49 @@ def _p010_hw(x: torch.Tensor) -> Tuple[int, int]:
     return _yuv420_hw(x, "P010", torch.uint16)
 
 
+def plane_pairs(frames, fmt: str, what: str) -> Tuple[int, int, int]:
+    """(B, H, W) of 4:2:0 frames given as a list / tuple of B (y, uv) plane pairs -- strided views of a decoder's or encoder's pitched
+    surfaces: y (H, W) and uv (H/2, W), uint8 for NV12 and uint16 for P010, unit stride along W, any row stride, all CUDA tensors on
+    one device.  Raises ValueError for anything else."""
+    dtype = torch.uint8 if fmt == "NV12" else torch.uint16
+    if not isinstance(frames, (list, tuple)) or not frames:
+        raise ValueError(f"{what}: {fmt} frame planes are a non-empty list of (y, uv) tensor pairs")
+    dev, hw = None, None
+    for b, pair in enumerate(frames):
+        if not isinstance(pair, (list, tuple)) or len(pair) != 2 or not all(isinstance(t, torch.Tensor) for t in pair):
+            raise ValueError(f"{what}[{b}] must be a (y, uv) pair of tensors")
+        for name, t in zip(("y", "uv"), pair):
+            if t.dim() != 2 or t.dtype != dtype:
+                raise ValueError(f"{what}[{b}].{name}: {fmt} planes are 2-D {str(dtype)[6:]} tensors, got {t.dtype} {tuple(t.shape)}")
+            if t.stride(1) != 1 and t.shape[1] > 1:
+                raise ValueError(f"{what}[{b}].{name}: a plane needs unit stride along its rows, got strides {t.stride()}")
+            if not t.is_cuda or (dev is not None and t.device != dev):
+                raise ValueError(f"{what}[{b}].{name}: every plane must be a CUDA tensor on one device, got {t.device}")
+            dev = t.device
+        y, uv = pair
+        H, W = int(y.shape[0]), int(y.shape[1])
+        if H % 2 or W % 2 or tuple(uv.shape) != (H // 2, W):
+            raise ValueError(f"{what}[{b}]: {fmt} planes are y (H, W) and uv (H/2, W) with H and W even, got {tuple(y.shape)} and "
+                             f"{tuple(uv.shape)}")
+        if hw is not None and hw != (H, W):
+            raise ValueError(f"{what}[{b}]: every frame of a batch has the same size, got {(H, W)} after {hw}")
+        hw = (H, W)
+    return len(frames), hw[0], hw[1]
+
+
+def _flat(frames) -> List[torch.Tensor]:
+    return [t for pair in frames for t in pair]
+
+
+def _descriptors(flat: Sequence[torch.Tensor]):
+    """TuFramePlanes array of the flattened planes [y0, uv0, y1, uv1, ...]; a plane of one row has no meaningful row stride"""
+    def pitch(t):
+        return (t.stride(0) if t.shape[0] > 1 else t.shape[1]) * t.element_size()
+    n = len(flat) // 2
+    return (_lib.TuFramePlanes * n)(*[_lib.TuFramePlanes(flat[2 * b].data_ptr(), flat[2 * b + 1].data_ptr(), pitch(flat[2 * b]),
+                                                          pitch(flat[2 * b + 1])) for b in range(n)])
+
+
 def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: int, compute_bf16: bool,
                   out_code: int, clamp: bool, in_layout: int = 0) -> torch.Tensor:
     lib = _lib.load()
@@ -165,6 +208,54 @@ def tu_forward(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: int,
 @tu_forward.register_fake
 def _(x, handle, out_h, out_w, scale, compute_bf16, out_code, clamp, in_layout=0):
     return x.new_empty(_image_shape(x.shape[0], 3, out_h, out_w, out_code), dtype=_TORCH_DT[out_code & 0xFF])
+
+
+@torch.library.custom_op("tu::forward_planes", mutates_args=("out_planes",), device_types="cuda")
+def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], out_planes: List[torch.Tensor], handle: int, out_h: int,
+                      out_w: int, scale: int, compute_bf16: bool, out_code: int, clamp: bool, in_layout: int) -> torch.Tensor:
+    """tu::forward with frame surfaces on an NV12 / P010 side: the input is x (dense) or x_planes ([y0, uv0, y1, uv1, ...]); the output
+    is written into out_planes (and an empty tensor returned), or returned as a new dense tensor when out_planes is empty"""
+    lib = _lib.load()
+    pw = _REGISTRY.get(handle)
+    if pw is None:
+        raise RuntimeError(f"tu::forward_planes: packed-weights handle {handle} is not alive (its TransformerModel was deleted or repacked)")
+    ref = x if x is not None else x_planes[0]
+    _require_cuda(ref)
+    if x is not None:
+        if _is_nv12(in_layout) or _is_p010(in_layout):
+            H, W = _nv12_hw(x) if _is_nv12(in_layout) else _p010_hw(x)
+            B = x.shape[0]
+        elif in_layout:
+            B, H, W = x.shape[0], x.shape[1], x.shape[2]
+        else:
+            B, H, W = x.shape[0], x.shape[2], x.shape[3]
+        x = x.contiguous()
+        in_code = _code(x.dtype) | in_layout
+    else:
+        B, (H, W) = len(x_planes) // 2, x_planes[0].shape
+        in_code = _code(x_planes[0].dtype) | in_layout
+    cdt = _lib.TU_BF16 if compute_bf16 else _lib.TU_F32
+    odt = _TORCH_DT[out_code & 0xFF]
+    out = ref.new_empty((0,) if out_planes else _image_shape(B, 3, out_h, out_w, out_code), dtype=odt)
+    nbytes = lib.tu_forward_workspace_bytes_io(C.byref(pw.struct), B, H, W, out_h, out_w, scale, cdt, in_code, out_code)
+    if nbytes == 0:
+        _lib.check(_lib.TU_ERR_SCALE if "was not built" in _lib.last_error() else _lib.TU_ERR_ARG)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=ref.device)
+    xd = _descriptors(x_planes) if x is None else None
+    od = _descriptors(out_planes) if out_planes else None
+    with torch.cuda.device(ref.device):
+        rc = lib.tu_forward_planes(C.byref(pw.struct), x.data_ptr() if x is not None else None, xd, in_code,
+                                   None if out_planes else out.data_ptr(), od, out_code, B, H, W, out_h, out_w, scale, cdt, int(clamp),
+                                   ws.data_ptr(), nbytes, _stream())
+    _lib.check(rc)
+    return out
+
+
+@tu_forward_planes.register_fake
+def _(x, x_planes, out_planes, handle, out_h, out_w, scale, compute_bf16, out_code, clamp, in_layout):
+    ref = x if x is not None else x_planes[0]
+    B = x.shape[0] if x is not None else len(x_planes) // 2
+    return ref.new_empty((0,) if out_planes else _image_shape(B, 3, out_h, out_w, out_code), dtype=_TORCH_DT[out_code & 0xFF])
 
 
 @torch.library.custom_op("tu::resize_aa", mutates_args=(), device_types="cuda")
@@ -234,13 +325,34 @@ def _(x, code):
     return x.new_empty((x.shape[0], 3 * x.shape[2] // 2, x.shape[3]), dtype=torch.uint16)
 
 
-def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int, int], upscale_factor: Optional[int],
+@torch.library.custom_op("tu::rgb_to_yuv420_planes", mutates_args=("planes",), device_types="cuda")
+def tu_rgb_to_yuv420_planes(x: torch.Tensor, planes: List[torch.Tensor], code: int) -> None:
+    """planar RGB (B,3,H,W) -> NV12 (fp16 RGB) or P010 (fp32 RGB) frames written into the surfaces [y0, uv0, y1, uv1, ...]"""
+    lib = _lib.load()
+    _require_cuda(x)
+    want = torch.float32 if _is_p010(code) else torch.float16
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != want:
+        raise RuntimeError(f"rgb_to_yuv420_planes takes planar {str(want)[6:]} RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_yuv420_planes(x.data_ptr(), _descriptors(planes), code, B, H, W, _stream()))
+
+
+@tu_rgb_to_yuv420_planes.register_fake
+def _(x, planes, code):
+    return None
+
+
+def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale_factor: Optional[int],
                 require_ratio: bool, compute_bf16: bool, out_dtype: torch.dtype, clamp: bool = True,
-                in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709") -> torch.Tensor:
+                in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709", out=None):
     """Shape logic of the three reference forwards (W:237-238, F:245-248,323-327, R:121-122) around tu::forward.
     in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'nv12' | 'p010'): uint8 frames may be interleaved (B,H,W,3) or NV12
     (B,3H/2,W) on either side, and either side may be P010 (B,3H/2,W) uint16 frames; yuv ('bt709' | 'bt601' | 'bt709_full' |
-    'bt601_full', and 'bt2020' | 'bt2020_full' for P010 only) is the colour of the NV12 / P010 side(s)."""
+    'bt601_full', and 'bt2020' | 'bt2020_full' for P010 only) is the colour of the NV12 / P010 side(s).
+    Frame surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs (see plane_pairs); with out_layout
+    'nv12' / 'p010', out= a list of B (y, uv) pairs receives the result and is returned."""
     il, ol = layout_code(in_layout), layout_code(out_layout)
     nv12_in, nv12_out = in_layout == "nv12", out_layout == "nv12"
     p010_in, p010_out = in_layout == "p010", out_layout == "p010"
@@ -254,7 +366,14 @@ def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int,
     if p010_out and out_dtype != torch.uint16:
         raise ValueError("out_layout='p010' writes uint16 frames")
     il |= yc if nv12_in or p010_in else 0
-    if nv12_in:
+    planes_in = isinstance(x, (list, tuple))
+    if planes_in and not (nv12_in or p010_in):
+        raise ValueError("a list of (y, uv) frame planes is NV12 / P010 input: pass in_layout='nv12' or 'p010'")
+    if out is not None and not (nv12_out or p010_out):
+        raise ValueError("out= takes NV12 / P010 frame planes: pass out_layout='nv12' or 'p010'")
+    if planes_in:
+        B, H, W = plane_pairs(x, "NV12" if nv12_in else "P010", "frames")
+    elif nv12_in:
         H, W = _nv12_hw(x)
     elif p010_in:
         H, W = _p010_hw(x)
@@ -268,10 +387,26 @@ def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int,
     def even_out(oh, ow):
         if (nv12_out or p010_out) and (oh % 2 or ow % 2):
             raise ValueError(f"{'NV12' if nv12_out else 'P010'} output frames need an even height and width, got {oh}x{ow}")
+        if out is not None:
+            fmt = "NV12" if nv12_out else "P010"
+            if not isinstance(out, (list, tuple)) or len(out) != (len(x) if planes_in else x.shape[0]):
+                raise ValueError("out= must be a list of one (y, uv) plane pair per input frame")
+            n, h, w = plane_pairs(out, fmt, "out")
+            dev = (x[0][0] if planes_in else x).device
+            if (h, w) != (oh, ow) or out[0][0].device != dev:
+                raise ValueError(f"out= planes must be {fmt} frames of {oh}x{ow} on {dev}, got {h}x{w} on {out[0][0].device}")
+
+    def forward(oh, ow, scale_, code, clamp_):
+        if not planes_in and out is None:
+            return tu_forward(x, pw_handle, oh, ow, scale_, compute_bf16, code, clamp_, il)
+        oplanes = _flat(out) if out is not None and code == out_code else []
+        y = tu_forward_planes(None if planes_in else x, _flat(x) if planes_in else [], oplanes, pw_handle, oh, ow, scale_, compute_bf16,
+                              code, clamp_, il)
+        return out if oplanes else y
 
     if model != "FastTransformer":
         even_out(*res_out)
-        return tu_forward(x, pw_handle, res_out[0], res_out[1], 0, compute_bf16, out_code, clamp, il)
+        return forward(res_out[0], res_out[1], 0, out_code, clamp)
     scale = upscale_factor if upscale_factor is not None else math.ceil(max(res_out[0] / H, res_out[1] / W))
     if scale not in (2, 3, 4, 6):
         raise ValueError(f"Requested scale={scale} was not built.")
@@ -281,14 +416,18 @@ def run_forward(pw_handle: int, model: str, x: torch.Tensor, res_out: Tuple[int,
     need_resize = require_ratio and res_out != (oh, oh) and res_out != (oh, ow)
     if not need_resize:
         even_out(oh, ow)
-        return tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, out_code, clamp, il)
+        return forward(oh, ow, scale, out_code, clamp)
     even_out(*res_out)
     # Resize is the last op: the un-clamped full-size image stays in the compute dtype and the Resize kernel writes the requested
     # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store).  fp16 output keeps an fp32
     # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  NV12 output is the fp16 output converted,
     # P010 output the fp32 output converted
     mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) and not nv12_out else torch.float32)
-    full = tu_forward(x, pw_handle, oh, ow, scale, compute_bf16, mid_code, False, il)
+    full = forward(oh, ow, scale, mid_code, False)
+    if out is not None:
+        tu_rgb_to_yuv420_planes(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16 if nv12_out else _lib.TU_F32), _flat(out),
+                                out_code)
+        return out
     if nv12_out:
         return tu_rgb_to_nv12(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16), out_code)
     if p010_out:

@@ -31,6 +31,10 @@ class GraphedModel:
 
     @torch.no_grad()
     def __call__(self, x: torch.Tensor, **kw) -> torch.Tensor:
+        if isinstance(x, (list, tuple)) or kw.get("out") is not None:
+            # a graph replays from a static input buffer, so frame planes would be copied into it: call the model directly instead
+            raise TypeError("GraphedModel takes dense frame tensors only, not lists of (y, uv) frame planes or out=; call the model "
+                            "itself with frame planes")
         if not x.is_cuda:
             raise RuntimeError("transformerupscaler_b200 has no CPU path: move the input to a CUDA device")
         key = self._key(x, kw)

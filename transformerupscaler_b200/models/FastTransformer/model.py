@@ -39,5 +39,5 @@ class TransformerModel(EngineModel):
         self.decoder_conv2 = nn.Conv2d(base_channels, in_channels, kernel_size=3, stride=1, padding=1)
 
     def forward(self, x: torch.Tensor, res_out: Tuple[int, int] = (1080, 1920), upscale_factor: int = None,
-                require_ratio: bool = True, in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709") -> torch.Tensor:
-        return super().forward(x, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv)
+                require_ratio: bool = True, in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709", out=None):
+        return super().forward(x, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)

@@ -148,7 +148,7 @@ class EngineModel(nn.Module):
         return bf16, out_dt
 
     def forward(self, x: torch.Tensor, res_out: Tuple[int, int] = (1080, 1920), upscale_factor: int = None,
-                require_ratio: bool = True, in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709") -> torch.Tensor:
+                require_ratio: bool = True, in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709", out=None):
         """The reference's signature (W:224, F:231, R:114) plus keyword-only-in-spirit extensions for uint8 video frames:
         in_layout / out_layout in {'chw', 'hwc', 'hwc_bgr', 'nv12'} — uint8 frames may arrive / leave interleaved (B,H,W,3), the form PIL
         and OpenCV hold them in (inference.py:65-70, app_overlay.py:382-386), with the channel swap done in the last kernel, or as
@@ -157,32 +157,50 @@ class EngineModel(nn.Module):
         10 bits of each word.  in_layout='p010' takes uint16 frames; out_layout='p010' returns uint16 frames for any frame input
         (uint8 in any layout, or P010), and a P010 input with any other out_layout returns uint8 frames.
         yuv in {'bt709', 'bt601', 'bt709_full', 'bt601_full'} is the colour matrix and range of the NV12 / P010 side(s); 'bt2020' and
-        'bt2020_full' (BT.2020 / BT.2100) need a P010 side and no NV12 side."""
+        'bt2020_full' (BT.2020 / BT.2100) need a P010 side and no NV12 side.
+        Decoder / encoder surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs -- y (H, W), uv (H/2, W),
+        uint8 (NV12) or uint16 (P010), unit stride along W and any row stride (strided views of a pitched surface pool) -- and with
+        out_layout 'nv12' / 'p010', out= a list of B such pairs of the output size receives the result and is returned.  Each side is
+        independent of the other; pitch padding and the bytes around the planes are never written."""
+        if isinstance(x, (list, tuple)):
+            if in_layout not in ("nv12", "p010"):
+                raise ValueError("a list of (y, uv) frame planes is NV12 / P010 input: pass in_layout='nv12' or 'p010'")
+            engine.plane_pairs(x, in_layout.upper(), "frames")
+            return self._forward(x, x[0][0], res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
+        return self._forward(x, x, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
+
+    def _forward(self, x, x0: torch.Tensor, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out):
+        """x0: x, or the first plane of a list of frame planes (device, dtype and autocast state of the call)"""
         if self.training:
             raise RuntimeError("transformerupscaler_b200 is a forward-only inference engine: call .eval() first "
                                "(dropout is treated as identity; there is no backward)")
-        if not x.is_cuda:
+        if not x0.is_cuda:
             raise RuntimeError("transformerupscaler_b200 has no CPU path: move the model and the input to a CUDA device")
-        if x.requires_grad and torch.is_grad_enabled():
+        if x0.requires_grad and torch.is_grad_enabled():
             raise RuntimeError("transformerupscaler_b200 is forward-only (no autograd): the input requires grad; call under torch.no_grad()")
         # uint8 frames in -> uint8 frames out (ToTensor scaling on read, (out*255).clamp(0,255).to(uint8) on write, fused into
         # the first and last kernels): the video-pipeline entry, an extension of the reference's float-only signature
         # P010 frames are uint16; any other uint16 tensor is an image like any other and is read as float32
-        if in_layout == "p010" and x.dtype != torch.uint16:
-            raise ValueError(f"in_layout='p010' takes uint16 frames (B, 3H/2, W), got {x.dtype}")
-        frames_u8 = x.dtype == torch.uint8
+        if in_layout == "p010" and x0.dtype != torch.uint16:
+            raise ValueError(f"in_layout='p010' takes uint16 frames (B, 3H/2, W), got {x0.dtype}")
+        frames_u8 = x0.dtype == torch.uint8
         frames = frames_u8 or in_layout == "p010"
-        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8) and not frames:
-            x = x.float()
-        bf16, out_dt = self._select_precision(x)
+        if x0.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8) and not frames:
+            x = x0 = x.float()
+        bf16, out_dt = self._select_precision(x0)
         if frames:
             out_dt = torch.uint16 if out_layout == "p010" else torch.uint8
-        handle = self._packed(bf16, x.device)
+        handle = self._packed(bf16, x0.device)
         if (in_layout != "chw" or out_layout != "chw") and not frames:
             raise ValueError("in_layout / out_layout other than 'chw' apply to uint8 / P010 frames only")
-        out = engine.run_forward(handle, self.ENGINE_MODEL, x, res_out, upscale_factor, require_ratio, bf16, out_dt,
-                                 in_layout=in_layout, out_layout=out_layout, yuv=yuv)
-        if not frames and x.is_cuda and torch.is_autocast_enabled("cuda") and not self.AUTOCAST_OUT_FP32:
+        if out is not None and out_layout not in ("nv12", "p010"):
+            raise ValueError("out= takes NV12 / P010 frame planes: pass out_layout='nv12' or 'p010'")
+        y = engine.run_forward(handle, self.ENGINE_MODEL, x, res_out, upscale_factor, require_ratio, bf16, out_dt,
+                               in_layout=in_layout, out_layout=out_layout, yuv=yuv, out=out)
+        if out is not None:
+            return y
+        out = y
+        if not frames and x0.is_cuda and torch.is_autocast_enabled("cuda") and not self.AUTOCAST_OUT_FP32:
             want = torch.get_autocast_dtype("cuda")
             if out.dtype != want:
                 out = out.to(want)

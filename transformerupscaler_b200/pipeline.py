@@ -42,6 +42,8 @@ class FramePipeline:
     def __init__(self, model, depth: int = 2, device: Optional[torch.device] = None, compute_streams: int = 2, **forward_kw):
         """compute_streams > 1: consecutive batches run their forwards on alternating streams, so the kernels of one batch
         can fill the SMs the other batch's partly filled waves leave idle (needs depth >= compute_streams)"""
+        if forward_kw.get("out") is not None:
+            raise TypeError("FramePipeline writes dense host frames: out= (frame planes) is not supported; call the model itself")
         self.model, self.kw, self.depth = model, forward_kw, depth
         self.device = device or next(model.parameters()).device
         self.s_in, self.s_out = (torch.cuda.Stream(self.device) for _ in range(2))
@@ -56,6 +58,8 @@ class FramePipeline:
     def submit(self, host_in: torch.Tensor, host_out: torch.Tensor) -> Ticket:
         """Enqueue one batch: host_in (pinned) is upscaled into host_out (pinned).  Returns immediately with the batch's Ticket
         (see the buffer lifetime contract in the module docstring)."""
+        if not isinstance(host_in, torch.Tensor) or not isinstance(host_out, torch.Tensor):
+            raise TypeError("FramePipeline takes dense pinned frame tensors only, not lists of (y, uv) frame planes")
         slot = self.n % self.depth
         if self.tickets[slot] is not None:
             self.tickets[slot].wait()                # slot's previous result has left the device

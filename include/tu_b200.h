@@ -42,6 +42,18 @@ extern "C" {
 #define TU_LAYOUT_HWC_BGR 0x200
 #define TU_U8_HWC (TU_U8 | TU_LAYOUT_HWC)
 #define TU_U8_HWC_BGR (TU_U8 | TU_LAYOUT_HWC_BGR)
+/* 32-bit pixels with an alpha byte (OR-ed into TU_U8 for the image input and / or output of tu_forward, the output of
+ * tu_bicubic_add_clamp, tu_subpixel_conv_add and tu_resize_bilinear_aa_to[_alpha], and the input of tu_frames_to_planar and
+ * tu_resample_alpha): (B,H,W,4) uint8, bytes R G B A (TU_LAYOUT_RGBA) or B G R A (TU_LAYOUT_BGRA: DXGI_FORMAT_B8G8R8A8_UNORM, what
+ * screen capture returns).  Alpha is straight (not premultiplied).  R, G, B are read and written exactly as TU_LAYOUT_HWC /
+ * TU_LAYOUT_HWC_BGR read and write them; the alpha bytes never reach the network.  A 4-byte output buffer must be 4-byte aligned.
+ * The alpha byte of an output pixel is the input alpha resampled to the output size when the input is 4-byte too (tu_resample_alpha),
+ * 255 otherwise; a 4-byte input going to an output without alpha loses its alpha.  TU_U8 only; never with colour bits.
+ * The layout bits 8..11 are an enumeration: 0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 8 P010. */
+#define TU_LAYOUT_RGBA 0x300
+#define TU_LAYOUT_BGRA 0x500
+#define TU_U8_RGBA (TU_U8 | TU_LAYOUT_RGBA)
+#define TU_U8_BGRA (TU_U8 | TU_LAYOUT_BGRA)
 /* NV12 video frames (OR-ed into TU_U8 for the image input and / or output of tu_forward, and the code of tu_nv12_to_rgb /
  * tu_rgb_to_nv12): one uint8 buffer of (3H/2) x W bytes per frame, (B, 3H/2, W) for a batch.  Rows 0..H-1 are the Y plane, the next
  * H/2 rows hold interleaved chroma pairs (U first) of the 4:2:0 "type 0" siting: chroma co-sited with even luma columns, midway
@@ -88,7 +100,7 @@ long long tu_launch_count(void);
  * events on the caller's stream (two event records per forward: cheap enough for the timed region); tu_profile_enable(2)
  * brackets EVERY kernel, tagged with the reference op it implements ("conv1", "conv2" (or "conv1_conv2" when fused), "downsample", "patch_embed",
  * "transformer_blocks", "patch_unembed", "decoder_conv1", "decoder_conv2", "bicubic_add_clamp", "up1", "up1_conv",
- * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end).  tu_profile_collect / tu_profile_report synchronise those events (the only
+ * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
  * calls in the library that wait on the device): collect sums the milliseconds and launches recorded under `name`
  * (NULL = all); report writes "name total_ms launches\n" lines into buf (returns the needed size when buf is NULL);
  * tu_profile_reset drops the records. */
@@ -215,6 +227,9 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      TU_U16 | TU_LAYOUT_P010 [| colour bits]: the same with 16-bit words and planar fp32: a P010 input is converted to planar fp32
  *      first (the forward is then the TU_F32-input one), a P010 output is the converted TU_F32 output (codes saturate at 0 / 1023
  *      with clamp == 0 too).  Either side may be NV12, P010 or any other code independently of the other.
+ *      TU_U8 | TU_LAYOUT_RGBA / TU_LAYOUT_BGRA: (B,H,W,4) frames on either side; an input is read as the same pixels given as
+ *      TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR.  With 4-byte frames on BOTH sides the output alpha is the input alpha resampled
+ *      (tu_resample_alpha; the workspace of tu_forward_workspace_bytes_io then holds that (B, outH, outW) plane), else 255.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
@@ -239,7 +254,8 @@ size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int outH, int 
 size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
 /* the same for the image input / output codes of the call: equal to tu_forward_workspace_bytes_for for every code pair without
  * TU_LAYOUT_NV12 or TU_LAYOUT_P010, larger by the planar fp16 frames of the side(s) that are NV12 and the planar fp32 frames of the
- * side(s) that are P010 (tu_forward needs it then); 0 for a bad code */
+ * side(s) that are P010, and by the (B, outH, outW) alpha plane when both sides are RGBA / BGRA (tu_forward needs it then); 0 for a
+ * bad code */
 size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype,
                                      int in_dtype, int out_dtype);
 int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype,
@@ -341,12 +357,25 @@ int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, const float 
 int tu_resize_bilinear_aa(const void *in, int dtype, void *out, int B, int H, int W, int outH, int outW,
                           int clamp, void *stream);
 /* the same with an output dtype of its own (TU_F32 / TU_BF16 / TU_U8 [| layout]): FastTransformer's Resize as the LAST op of a
- * uint8-frame forward (FastTransformer/model.py:323-327 followed by app_overlay.py:382-386) */
+ * uint8-frame forward (FastTransformer/model.py:323-327 followed by app_overlay.py:382-386); a 4-byte layout gets alpha 255 */
 int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out, int out_dtype, int B, int H, int W, int outH, int outW,
                              int clamp, void *stream);
-/* uint8 frames (B,H,W,3) interleaved (layout TU_LAYOUT_HWC or TU_LAYOUT_HWC_BGR) -> planar RGB (B,3,H,W) uint8; tu_forward does
- * this itself for an in_dtype that carries a layout (into its workspace) */
+/* the same with the alpha byte of a 4-byte output (TU_U8 | TU_LAYOUT_RGBA / TU_LAYOUT_BGRA) taken from `alpha`, a (B, outH, outW) uint8
+ * plane (tu_resample_alpha); alpha == NULL writes 255.  tu_resize_bilinear_aa_to is this function with alpha == NULL. */
+int tu_resize_bilinear_aa_to_alpha(const void *in, int in_dtype, const void *alpha, void *out, int out_dtype, int B, int H, int W,
+                                   int outH, int outW, int clamp, void *stream);
+/* uint8 frames (B,H,W,3) interleaved (layout TU_LAYOUT_HWC or TU_LAYOUT_HWC_BGR), or (B,H,W,4) with alpha (TU_LAYOUT_RGBA or
+ * TU_LAYOUT_BGRA; the alpha is dropped) -> planar RGB (B,3,H,W) uint8; tu_forward does this itself for an in_dtype that carries a
+ * layout (into its workspace) */
 int tu_frames_to_planar(const void *in, int layout, void *out, int B, int H, int W, void *stream);
+/* the alpha bytes of 4-byte frames (B,H,W,4), code TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA, resampled to a (B, outH, outW) uint8
+ * plane: bicubic, ATen's F.interpolate(mode="bicubic", align_corners=False) -- A = -0.75, half-pixel centres, taps clamped to the
+ * edge, the taps ty_i / tx_j and weights wy_i / wx_j of the engine's bicubic kernels (scale = (float)in / out,
+ * src = fma(scale, dst + 0.5, -0.5) in fp32) -- on the codes 0..255 as floats, every step one correctly rounded fp32 operation
+ * (no contraction), sums left to right from 0:
+ *   acc_i = sum_j A[ty_i, tx_j] * wx_j,   a = sum_i acc_i * wy_i,   alpha = min(max(floor(a + 0.5), 0), 255).
+ * A constant plane stays exactly constant.  tu_forward runs this on its input when both sides are 4-byte frames (into its workspace). */
+int tu_resample_alpha(const void *frames, int code, void *alpha, int B, int H, int W, int outH, int outW, void *stream);
 /* NV12 frames (B, 3H/2, W) uint8 -> planar RGB (B, 3, H, W) fp16, and back.  code = TU_U8 | TU_LAYOUT_NV12 | colour bits (anything else,
  * an odd H or W, or B > 65535: TU_ERR_ARG).  Every step is one correctly rounded fp32 operation (no contraction), so the results are exactly
  * those of the formulas below, with (yo, ys, cs) = (16, 219, 224) limited / (0, 255, 255) full range, Kg = 1 - Kr - Kb and every

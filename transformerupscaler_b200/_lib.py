@@ -18,6 +18,9 @@ TU_YUV_BT601, TU_YUV_FULL_RANGE = 0x1000, 0x2000     # colour bits of an NV12 co
 TU_U16 = 4                                           # 16-bit frame words: valid only as TU_U16 | TU_LAYOUT_P010
 TU_LAYOUT_P010 = 0x800                               # OR-ed into TU_U16 for P010 (10-bit 4:2:0) video frames, (B, 3H/2, W)
 TU_YUV_BT2020 = 0x4000                               # BT.2020 matrix: a colour bit of P010 codes only (not with TU_YUV_BT601)
+# OR-ed into TU_U8 for 4-byte pixels with a straight alpha byte, (B, H, W, 4): R G B A / B G R A.  The layout bits 8..11 are an
+# enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 8 P010): compare whole values, never single bits
+TU_LAYOUT_RGBA, TU_LAYOUT_BGRA = 0x300, 0x500
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}
 
@@ -121,7 +124,9 @@ SIGNATURES = {
     "tu_bicubic_add_clamp": (i32, [vp, i32, i32, i32, fp, i32, i32, vp, i32, i32, i32, i32, i32, vp]),
     "tu_resize_bilinear_aa": (i32, [vp, i32, vp, i32, i32, i32, i32, i32, i32, vp]),
     "tu_resize_bilinear_aa_to": (i32, [vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
+    "tu_resize_bilinear_aa_to_alpha": (i32, [vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
     "tu_frames_to_planar": (i32, [vp, i32, vp, i32, i32, i32, vp]),
+    "tu_resample_alpha": (i32, [vp, i32, vp, i32, i32, i32, i32, i32, vp]),
     "tu_bicubic_row_schedule": (i32, [i32, i32, i32]),
     "tu_nv12_to_rgb": (i32, [vp, i32, vp, i32, i32, i32, vp]),
     "tu_rgb_to_nv12": (i32, [vp, vp, i32, i32, i32, i32, vp]),

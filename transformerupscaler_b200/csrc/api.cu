@@ -186,8 +186,12 @@ static int forward_impl(const TuModelWeights *w, const void *x, const TuFramePla
     else if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv));                    \
     else if (p010_out) TU_STEP("rgb_to_p010", tu_rgb_to_p010(img, out, out_dtype, B, outH, outW, stv))
 
-    // interleaved uint8 frames (HWC RGB / BGR) are made planar once; the stem and the final bicubic both read the planar copy
+    // interleaved uint8 frames (HWC RGB / BGR, RGBA / BGRA) are made planar once; the stem and the final bicubic both read the planar copy
     uint8_t *xplanar = (uint8_t *)a.get((size_t)B * 3 * H * W);
+    // 4-byte frames on both sides: the input alpha, resampled to the output size, is the output alpha (read by the last image kernel)
+    const bool alpha_io = dtype_is_px4(in_dtype) && dtype_is_px4(out_dtype);
+    uint8_t *aplane = alpha_io ? (uint8_t *)a.get((size_t)B * outH * outW) : nullptr;
+    if (!dry && alpha_io) TU_STEP("resample_alpha", tu_resample_alpha(x, in_dtype, aplane, B, H, W, outH, outW, stv));
     if (!dry && dtype_layout(in_dtype)) {
         if ((rc = tu_frames_to_planar(x, dtype_layout(in_dtype) << 8, xplanar, B, H, W, stv))) return rc;
         x = xplanar;
@@ -366,7 +370,7 @@ static int forward_impl(const TuModelWeights *w, const void *x, const TuFramePla
 
     if (!fast) {
         if (!dry) {
-            TU_STEP("bicubic_add_clamp", tu_bicubic_add_clamp(x, in_dtype, H, W, res, Hc, Wc, img, img_dtype, B, outH, outW, clamp, stv));
+            TU_STEP("bicubic_add_clamp", bicubic_add_clamp_alpha(x, in_dtype, H, W, res, Hc, Wc, img, img_dtype, B, outH, outW, clamp, aplane, st));
             TU_YUV_OUT();
         }
         return TU_OK;
@@ -387,8 +391,8 @@ static int forward_impl(const TuModelWeights *w, const void *x, const TuFramePla
                         set_error("tu: FastTransformer output buffer must be (scale*H, scale*W)");
                         return TU_ERR_ARG;
                     }
-                    TU_STEP("final_upscale_conv_add", tu_subpixel_conv_add(cur, (const float *)sg.w, sg.b, r, w->host_finconv_wb, upA, img,
-                                                                           img_dtype, B, ch, cw, clamp, stv));
+                    TU_STEP("final_upscale_conv_add", subpixel_conv_add_alpha(cur, (const float *)sg.w, sg.b, r, w->host_finconv_wb, upA, img,
+                                                                              img_dtype, B, ch, cw, clamp, aplane, st));
                     TU_YUV_OUT();
                 }
                 return TU_OK;
@@ -718,13 +722,20 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
 
 // 4:2:0 codes: TU_U8 | TU_LAYOUT_NV12 [| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_P010 [| TU_YUV_BT601 or
 // TU_YUV_BT2020] [| TU_YUV_FULL_RANGE].  TU_U16 is a P010 word and nothing else.  Such frames have an even height and width.
+// 4-byte frames: exactly TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA.  Other codes have a layout nibble below 4 and no colour bit.
+static bool plain_code(int d) {
+    const int nib = (d >> 8) & 0xF;
+    return dtype_is_px4(d) || (!(d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE)) && nib < 4 && dtype_base(d) != TU_U16);
+}
 static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int outH, int outW) {
-    const int bits = TU_LAYOUT_NV12 | TU_LAYOUT_P010 | TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE;
     const bool in420 = dtype_is_yuv420(in_dtype), out420 = dtype_is_yuv420(out_dtype);
-    TU_CHECK_ARG(in420 || (!(in_dtype & bits) && dtype_base(in_dtype) != TU_U16),
+    for (int d : {in_dtype, out_dtype})
+        TU_CHECK_ARG(dtype_is_px4(d) || !layout_is_px4((d >> 8) & 0xF),
+                     "forward: TU_LAYOUT_RGBA / TU_LAYOUT_BGRA are for uint8 frames (TU_U8) only, without colour bits");
+    TU_CHECK_ARG(in420 || plain_code(in_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
                  "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (input)");
-    TU_CHECK_ARG(out420 || (!(out_dtype & bits) && dtype_base(out_dtype) != TU_U16),
+    TU_CHECK_ARG(out420 || plain_code(out_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
                  "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (output)");
     TU_CHECK_ARG(!in420 || (H % 2 == 0 && W % 2 == 0),
@@ -737,9 +748,11 @@ static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int out
 extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale,
                                                 int compute_dtype, int in_dtype, int out_dtype) {
     if (check_forward_args(w, B, H, W, outH, outW, compute_dtype) || check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW)) return 0;
-    // only the NV12 / P010 sides change the arena; every other code sizes exactly as tu_forward_workspace_bytes_for
-    in_dtype = dtype_is_yuv420(in_dtype) ? in_dtype : TU_F32;
-    out_dtype = dtype_is_yuv420(out_dtype) ? out_dtype : TU_F32;
+    // only the NV12 / P010 sides and a 4-byte pair of sides (its alpha plane) change the arena; every other code sizes exactly as
+    // tu_forward_workspace_bytes_for
+    const bool alpha_io = dtype_is_px4(in_dtype) && dtype_is_px4(out_dtype);
+    in_dtype = dtype_is_yuv420(in_dtype) || alpha_io ? in_dtype : TU_F32;
+    out_dtype = dtype_is_yuv420(out_dtype) || alpha_io ? out_dtype : TU_F32;
     Arena a{nullptr, 0, 0, true};
     int rc = compute_dtype == TU_F32
                  ? forward_impl<float>(w, nullptr, nullptr, in_dtype, nullptr, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0)
@@ -768,8 +781,9 @@ extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const T
         TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8 || ib == TU_U16) &&
                          (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8 || ob == TU_U16),
                      "forward: bad i/o dtype");
-        TU_CHECK_ARG((il == 0 || (ib == TU_U8 && il <= 2)) && (ol == 0 || (ob == TU_U8 && ol <= 2)),
-                     "forward: interleaved layouts (TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR) are for uint8 frames");
+        TU_CHECK_ARG((il == 0 || (ib == TU_U8 && layout_is_interleaved(il))) && (ol == 0 || (ob == TU_U8 && layout_is_interleaved(ol))),
+                     "forward: interleaved layouts (TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR / TU_LAYOUT_RGBA / TU_LAYOUT_BGRA) are for uint8 frames");
+        TU_CHECK_ARG(!layout_is_px4(ol) || (reinterpret_cast<uintptr_t>(out) & 3) == 0, "forward: a 4-byte (RGBA / BGRA) output must be 4-byte aligned");
     }
     TU_CHECK_ARG(w->blocks && w->n_blocks > 0 && w->dim == w->heads * 16, "forward: bad transformer configuration");
     // size pass, then the real pass

@@ -195,13 +195,15 @@ __device__ __forceinline__ void slide_tile(float (&win)[3][4], int &cur, int bas
 }
 
 // MODE 0: taps from global memory (any shape, residual optional at run time); MODE 1 / 2: TMA-staged tile with / without
-// the residual source (compile-time, so the strip loop has no dead branches)
-template <typename TI, typename TO, int MODE>
+// the residual source (compile-time, so the strip loop has no dead branches).  PX4: 4-byte uint8 pixels (layout 3 / 5) whose alpha
+// comes from the plane `alpha` (NULL: 255); the other instantiations never read `alpha`
+template <typename TI, typename TO, int MODE, bool PX4 = false>
 __global__ void __launch_bounds__(BS_W) bicubic_add_clamp_strip_kernel(const __grid_constant__ CUtensorMap tmap_x,
                                                                        const __grid_constant__ CUtensorMap tmap_r,
                                                                        const BicubicTileGeom g, const TI *__restrict__ x, int H, int W,
                                                                        const float *__restrict__ res, int rH, int rW,
-                                                                       TO *__restrict__ out, int oH, int oW, int clamp, int layout) {
+                                                                       TO *__restrict__ out, int oH, int oW, int clamp, int layout,
+                                                                       const uint8_t *__restrict__ alpha) {
     pdl_trigger();
     pdl_wait();          // the residual image is written by the previous kernel of the stream
     __shared__ float yw[2][BS_H][4];
@@ -277,7 +279,8 @@ __global__ void __launch_bounds__(BS_W) bicubic_add_clamp_strip_kernel(const __g
                 if (clamp) v = fminf(fmaxf(v, 0.f), 1.f);
                 v3[c] = v;
             }
-            store_rgb<TO>(out, b, oplane, (long)(oy0 + r) * oW + ox, layout, v3[0], v3[1], v3[2]);
+            if constexpr (PX4) store_px4(out, b * oplane + (long)(oy0 + r) * oW + ox, layout, v3[0], v3[1], v3[2], alpha);
+            else store_rgb<TO>(out, b, oplane, (long)(oy0 + r) * oW + ox, layout, v3[0], v3[1], v3[2]);
         }
     };
     if (TMA) {
@@ -309,7 +312,9 @@ __global__ void __launch_bounds__(BS_W) bicubic_add_clamp_strip_kernel(const __g
                 }
                 if (clamp) v[c] = fminf(fmaxf(v[c], 0.f), 1.f);
             }
-            if (layout == 0) {
+            if constexpr (PX4) {
+                store_px4(out, b * oplane + (long)(oy0 + r) * oW + ox, layout, v[0], v[1], v[2], alpha);
+            } else if (layout == 0) {
                 *o0 = from_f<TO>(v[0]); *o1 = from_f<TO>(v[1]); *o2 = from_f<TO>(v[2]);
                 o0 += oW; o1 += oW; o2 += oW;
             } else {
@@ -368,11 +373,13 @@ __device__ __forceinline__ void store_pair(uint8_t *o, float a, float b) {
     *reinterpret_cast<unsigned short *>(o) = (unsigned short)((unsigned)from_f<uint8_t>(a) | ((unsigned)from_f<uint8_t>(b) << 8));
 }
 
-template <typename TI, typename TO, bool RES>
+// PX4: 4-byte uint8 pixels (layout 3 / 5), the pair's two pixels one 8-byte store, alpha from the plane `alpha` (NULL: 255)
+template <typename TI, typename TO, bool RES, bool PX4 = false>
 __global__ void __launch_bounds__(BS_W / 2) bicubic_add_clamp_pair_kernel(const __grid_constant__ CUtensorMap tmap_x,
                                                                           const __grid_constant__ CUtensorMap tmap_r,
                                                                           const BicubicTileGeom g, int H, int W, int rH, int rW,
-                                                                          TO *__restrict__ out, int oH, int oW, int clamp, int layout) {
+                                                                          TO *__restrict__ out, int oH, int oW, int clamp, int layout,
+                                                                          const uint8_t *__restrict__ alpha) {
     pdl_trigger();
     pdl_wait();          // the residual image is written by the previous kernel of the stream
     __shared__ __align__(16) float yw[2][PAIR_H][4];
@@ -457,7 +464,17 @@ __global__ void __launch_bounds__(BS_W / 2) bicubic_add_clamp_pair_kernel(const 
             ptx::up2(v, lo[c], hi[c]);
             if (clamp) { lo[c] = fminf(fmaxf(lo[c], 0.f), 1.f); hi[c] = fminf(fmaxf(hi[c], 0.f), 1.f); }
         }
-        if (layout == 0) {
+        if constexpr (PX4) {
+            // the pair's two pixels are eight consecutive bytes (ox even, the buffer 8-byte aligned: host); their alphas two bytes
+            const long pix = ((long)b * oH + oy0 + r) * oW + ox;
+            const uint32_t a2 = alpha ? (uint32_t)*reinterpret_cast<const unsigned short *>(alpha + pix) : 0xFFFFu;
+            const int c0 = layout == 5 ? 2 : 0, c2 = 2 - c0;
+            uint2 px;
+            px.x = (uint32_t)from_f<uint8_t>(lo[c0]) | (uint32_t)from_f<uint8_t>(lo[1]) << 8 | (uint32_t)from_f<uint8_t>(lo[c2]) << 16 | (a2 & 0xFFu) << 24;
+            px.y = (uint32_t)from_f<uint8_t>(hi[c0]) | (uint32_t)from_f<uint8_t>(hi[1]) << 8 | (uint32_t)from_f<uint8_t>(hi[c2]) << 16 |
+                   (a2 >> 8) << 24;
+            *reinterpret_cast<uint2 *>(out + pix * 4) = px;
+        } else if (layout == 0) {
             store_pair(o0, lo[0], hi[0]); store_pair(o1, lo[1], hi[1]); store_pair(o2, lo[2], hi[2]);
             o0 += oW; o1 += oW; o2 += oW;
         } else {
@@ -617,12 +634,18 @@ static inline int sched_tile(int pat, bool big) {
     }
 }
 
-// HWC (uint8 frames only): interleaved output pixels, `layout` 1 = RGB, 2 = BGR; a thread stores its channel's two bytes
-template <typename TI, typename TO, int PAT, bool HWC>
+// PX (uint8 frames only when not 0): 0 planar; 3 interleaved output pixels, `layout` 1 = RGB, 2 = BGR, a thread stores its channel's
+// two bytes; 4 four-byte pixels, `layout` 3 = RGBA, 5 = BGRA: the three channels of a pixel belong to three warps, so each period of
+// rows is staged in shared memory (PX4_STAGE bytes behind the tile) and written as whole pixels, with the alpha of the plane `alpha`
+// (NULL: 255).  PX 0 / 3 never read `alpha`.
+template <int PAT> constexpr int px4_stage_bytes() { return RowSched<PAT>::P * BS_W * 4; }
+template <typename TI, typename TO, int PAT, int PX>
 __global__ void __launch_bounds__(R32_T, 5) bicubic_add_clamp_r32_kernel(const __grid_constant__ CUtensorMap tmap_x,
                                                                          const __grid_constant__ CUtensorMap tmap_r,
                                                                          const BicubicTileGeom g, int H, int W, int rH, int rW,
-                                                                         TO *__restrict__ out, int oH, int oW, int layout, int TILE) {
+                                                                         TO *__restrict__ out, int oH, int oW, int layout, int TILE,
+                                                                         const uint8_t *__restrict__ alpha) {
+    constexpr bool HWC = PX == 3;
     pdl_trigger();
     pdl_wait();          // the residual image is written by the previous kernel of the stream
     constexpr int P = RowSched<PAT>::P;             // TILE (rows per CTA, a multiple of P, <= R32_MAXTILE) is chosen per launch
@@ -673,7 +696,9 @@ __global__ void __launch_bounds__(R32_T, 5) bicubic_add_clamp_r32_kernel(const _
     replicate_pad(reinterpret_cast<TI *>(tile_raw), xr0, xc0, g.xr, g.xc, H, W);
     replicate_pad(reinterpret_cast<float *>(tile_raw + x_bytes_al), rr0, rc0, g.rr, g.rc, rH, rW);
     const int ch = t / (BS_W / 2), pair = t % (BS_W / 2), ox = ox0 + 2 * pair;
-    if (ox >= oW) return;           // oW is even: a pair is inside or outside as a whole
+    // oW is even: a pair is inside or outside as a whole.  PX 4: every thread stays for the block barriers of the staging; a pair
+    // right of the image computes from clamped taps inside the tile, and its pixels are not written
+    if (PX != 4 && ox >= oW) return;
 
     // ---- horizontal filters of the pair: six (x) / five (residual) consecutive elements, zero-padded weights
     const uint32_t xpitch = g.xc * sizeof(TI), rpitch = g.rc * 4u;
@@ -705,6 +730,9 @@ __global__ void __launch_bounds__(R32_T, 5) bicubic_add_clamp_r32_kernel(const _
     TO *o = HWC ? out + (((long)b * oH + oy0) * oW + ox) * 3 + (layout == 2 ? 2 - ch : ch) : out + ((long)b * 3 + ch) * oplane + (long)oy0 * oW + ox;
     const int orow = HWC ? 3 * oW : oW;
     const int nrows = min(TILE, oH - oy0);
+    // PX 4: the staged period, [row q][column 0..127][byte]; the thread's channel byte (reversed for BGRA) of its pair in row 0
+    const uint32_t stage = ptx::smem_u32(tile_raw) + x_bytes_al + ((3u * g.rr * g.rc * 4u + 15u) & ~15u);
+    const uint32_t sbyte = stage + (uint32_t)(2 * pair) * 4u + (uint32_t)(layout == 5 ? 2 - ch : ch);
 
     // window rows live in fixed registers: tile row n of a source sits in slot n & 3
     ptx::f32x2 wx[4], wr[4];
@@ -743,9 +771,27 @@ __global__ void __launch_bounds__(R32_T, 5) bicubic_add_clamp_r32_kernel(const _
             v = ptx::add2(v, u);
             float lo, hi;
             ptx::up2(v, lo, hi);
-            if (HWC) { o[0] = unit_to_u8<TO>(fminf(fmaxf(lo, 0.f), 1.f)); o[3] = unit_to_u8<TO>(fminf(fmaxf(hi, 0.f), 1.f)); }
-            else clamp_store_pair(o, lo, hi);       // outH % P == 0 (host): whole periods of rows
-            o += orow;
+            if constexpr (PX == 4) {
+                const uint32_t q_lo = unit_to_u8<TO>(fminf(fmaxf(lo, 0.f), 1.f)), q_hi = unit_to_u8<TO>(fminf(fmaxf(hi, 0.f), 1.f));
+                asm volatile("st.shared.u8 [%0], %1;" ::"r"(sbyte + (uint32_t)q * BS_W * 4u), "r"(q_lo) : "memory");
+                asm volatile("st.shared.u8 [%0], %1;" ::"r"(sbyte + (uint32_t)q * BS_W * 4u + 4u), "r"(q_hi) : "memory");
+            } else {
+                if (HWC) { o[0] = unit_to_u8<TO>(fminf(fmaxf(lo, 0.f), 1.f)); o[3] = unit_to_u8<TO>(fminf(fmaxf(hi, 0.f), 1.f)); }
+                else clamp_store_pair(o, lo, hi);       // outH % P == 0 (host): whole periods of rows
+                o += orow;
+            }
+        }
+        if constexpr (PX == 4) {        // the period's pixels, each written once as a 32-bit word with its alpha
+            __syncthreads();
+            for (int i = t; i < P * BS_W; i += R32_T) {
+                const int q = i / BS_W, x = ox0 + (i % BS_W);
+                if (x >= oW) continue;
+                const long pix = ((long)b * oH + oy0 + r0 + q) * oW + x;
+                uint32_t w;
+                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w) : "r"(stage + (uint32_t)i * 4u) : "memory");
+                reinterpret_cast<uint32_t *>(out)[pix] = (w & 0x00FFFFFFu) | (alpha ? (uint32_t)alpha[pix] : 255u) << 24;
+            }
+            __syncthreads();            // the next period overwrites the stage
         }
     }
 }
@@ -959,18 +1005,10 @@ __device__ __forceinline__ void aa_range(int dst, int in_size, int out_size, int
     norm = tot != 0.f ? 1.f / tot : 0.f;
 }
 
-template <typename T, typename TO>
-__global__ void __launch_bounds__(256) resize_aa_kernel(const T *__restrict__ in, TO *__restrict__ out, int H, int W, int oH,
-                                                        int oW, int clamp, int layout) {
-    const int ox = blockIdx.x * 64 + (threadIdx.x & 63);
-    const int oy = blockIdx.y * 4 + (threadIdx.x >> 6);
-    const long plane = blockIdx.z;
-    if (ox >= oW || oy >= oH) return;
-    int ylo, yn, xlo, xn;
-    float yc, yi, ynorm, xc, xi, xnorm;
-    aa_range(oy, H, oH, ylo, yn, yc, yi, ynorm);
-    aa_range(ox, W, oW, xlo, xn, xc, xi, xnorm);
-    const T *p = in + plane * H * W;
+// one output value of one plane p (the same operations, in the same order, for every output form)
+template <typename T>
+__device__ __forceinline__ float resize_aa_value(const T *__restrict__ p, int W, int ylo, int yn, float yc, float yi, float ynorm, int xlo,
+                                                 int xn, float xc, float xi, float xnorm) {
     float acc = 0.f;
     for (int a = 0; a < yn; ++a) {
         const float wy = fmaxf(0.f, 1.f - fabsf(((float)(a + ylo) - yc + 0.5f) * yi)) * ynorm;
@@ -981,6 +1019,33 @@ __global__ void __launch_bounds__(256) resize_aa_kernel(const T *__restrict__ in
         }
         acc = fmaf(wy, t, acc);
     }
+    return acc;
+}
+
+// PX4 = false: a thread per (plane = b * 3 + c, pixel); PX4 = true (4-byte uint8 pixels, layout 3 / 5): a thread per (frame b, pixel)
+// computes the three planes and writes the pixel once, its alpha from the plane `alpha` (NULL: 255)
+template <typename T, typename TO, bool PX4 = false>
+__global__ void __launch_bounds__(256) resize_aa_kernel(const T *__restrict__ in, TO *__restrict__ out, int H, int W, int oH,
+                                                        int oW, int clamp, int layout, const uint8_t *__restrict__ alpha) {
+    const int ox = blockIdx.x * 64 + (threadIdx.x & 63);
+    const int oy = blockIdx.y * 4 + (threadIdx.x >> 6);
+    const long plane = blockIdx.z;
+    if (ox >= oW || oy >= oH) return;
+    int ylo, yn, xlo, xn;
+    float yc, yi, ynorm, xc, xi, xnorm;
+    aa_range(oy, H, oH, ylo, yn, yc, yi, ynorm);
+    aa_range(ox, W, oW, xlo, xn, xc, xi, xnorm);
+    if constexpr (PX4) {
+        float v[3];
+#pragma unroll 1
+        for (int c = 0; c < 3; ++c) {
+            v[c] = resize_aa_value(in + (plane * 3 + c) * H * W, W, ylo, yn, yc, yi, ynorm, xlo, xn, xc, xi, xnorm);
+            if (clamp) v[c] = fminf(fmaxf(v[c], 0.f), 1.f);
+        }
+        store_px4(out, (plane * oH + oy) * oW + ox, layout, v[0], v[1], v[2], alpha);
+        return;
+    }
+    float acc = resize_aa_value(in + plane * H * W, W, ylo, yn, yc, yi, ynorm, xlo, xn, xc, xi, xnorm);
     if (clamp) acc = fminf(fmaxf(acc, 0.f), 1.f);
     if (layout == 0) {
         out[(plane * oH + oy) * oW + ox] = from_f<TO>(acc);
@@ -991,7 +1056,9 @@ __global__ void __launch_bounds__(256) resize_aa_kernel(const T *__restrict__ in
     }
 }
 
-// interleaved uint8 frames (B,H,W,3) -> planar RGB (B,3,H,W): four pixels per thread, 12 bytes in, 3 x 4 bytes out
+// interleaved uint8 frames (B,H,W,PX) -> planar RGB (B,3,H,W): four pixels per thread, 4 PX bytes in, 3 x 4 bytes out.  PX = 3: RGB /
+// BGR; PX = 4: RGBA / BGRA, one aligned 32-bit load per pixel, the alpha bytes are not read into the result
+template <int PX>
 __global__ void __launch_bounds__(256) frames_to_planar_kernel(const uint8_t *__restrict__ in, uint8_t *__restrict__ out, long plane,
                                                                int swap) {
     pdl_trigger();
@@ -999,25 +1066,90 @@ __global__ void __launch_bounds__(256) frames_to_planar_kernel(const uint8_t *__
     const long b = blockIdx.y;
     const long q = ((long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (q >= plane) return;
-    const uint8_t *src = in + (b * plane + q) * 3;
+    const uint8_t *src = in + (b * plane + q) * PX;
     uint8_t *dst = out + b * 3 * plane + q;
     const int c0 = swap ? 2 : 0, c2 = 2 - c0;
     if (q + 4 <= plane && ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst) | (uintptr_t)plane) & 3) == 0) {
         const uint32_t w0 = reinterpret_cast<const uint32_t *>(src)[0], w1 = reinterpret_cast<const uint32_t *>(src)[1],
                        w2 = reinterpret_cast<const uint32_t *>(src)[2];
-        // bytes: w0 = p0c0 p0c1 p0c2 p1c0 | w1 = p1c1 p1c2 p2c0 p2c1 | w2 = p2c2 p3c0 p3c1 p3c2
-        const uint32_t ch0 = __byte_perm(__byte_perm(w0, w1, 0x0630), w2, 0x5210);      // p0c0 p1c0 p2c0 p3c0
-        const uint32_t ch1 = __byte_perm(__byte_perm(w0, w1, 0x0741), w2, 0x6210);      // p0c1 p1c1 p2c1 p3c1
-        const uint32_t ch2 = __byte_perm(__byte_perm(w0, w1, 0x0052), w2, 0x7410);      // p0c2 p1c2 p2c2 p3c2
+        uint32_t ch0, ch1, ch2;
+        if constexpr (PX == 3) {
+            // bytes: w0 = p0c0 p0c1 p0c2 p1c0 | w1 = p1c1 p1c2 p2c0 p2c1 | w2 = p2c2 p3c0 p3c1 p3c2
+            ch0 = __byte_perm(__byte_perm(w0, w1, 0x0630), w2, 0x5210);      // p0c0 p1c0 p2c0 p3c0
+            ch1 = __byte_perm(__byte_perm(w0, w1, 0x0741), w2, 0x6210);      // p0c1 p1c1 p2c1 p3c1
+            ch2 = __byte_perm(__byte_perm(w0, w1, 0x0052), w2, 0x7410);      // p0c2 p1c2 p2c2 p3c2
+        } else {
+            // word i = pixel i: pic0 pic1 pic2 alpha; channel c of pixels 0, 1 and of pixels 2, 3, then the two halves
+            const uint32_t w3 = reinterpret_cast<const uint32_t *>(src)[3];
+            ch0 = __byte_perm(__byte_perm(w0, w1, 0x0040), __byte_perm(w2, w3, 0x0040), 0x5410);
+            ch1 = __byte_perm(__byte_perm(w0, w1, 0x0051), __byte_perm(w2, w3, 0x0051), 0x5410);
+            ch2 = __byte_perm(__byte_perm(w0, w1, 0x0062), __byte_perm(w2, w3, 0x0062), 0x5410);
+        }
         reinterpret_cast<uint32_t *>(dst + c0 * plane)[0] = ch0;
         reinterpret_cast<uint32_t *>(dst + plane)[0] = ch1;
         reinterpret_cast<uint32_t *>(dst + c2 * plane)[0] = ch2;
     } else {
         for (int i = 0; i < 4 && q + i < plane; ++i) {
-            dst[c0 * plane + i] = src[3 * i];
-            dst[plane + i] = src[3 * i + 1];
-            dst[c2 * plane + i] = src[3 * i + 2];
+            dst[c0 * plane + i] = src[PX * i];
+            dst[plane + i] = src[PX * i + 1];
+            dst[c2 * plane + i] = src[PX * i + 2];
         }
+    }
+}
+
+// ---- the alpha plane of 4-byte frames, resampled (bicubic, ATen's taps and weights; include/tu_b200.h: tu_resample_alpha) -------
+// Every step is one correctly rounded fp32 operation, the tap weights included: they are the fp32 tensor arithmetic of
+// oracle/upscaler_oracle.py::_cubic_taps, operation for operation, so that a CPU evaluation gives the same bits.
+__device__ __forceinline__ float cubic1_rn(float x) {          // ((A + 2) x - (A + 3)) x x + 1, A = -0.75
+    return __fadd_rn(__fmul_rn(__fmul_rn(__fadd_rn(__fmul_rn(1.25f, x), -2.25f), x), x), 1.f);
+}
+__device__ __forceinline__ float cubic2_rn(float x) {          // ((A x - 5 A) x + 8 A) x - 4 A
+    return __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(-0.75f, x), 3.75f), x), -6.f), x), 3.f);
+}
+__device__ __forceinline__ void cubic_taps_rn(int dst, int in_size, float scale, int (&idx)[4], float (&w)[4]) {
+    const float src = fmaf(scale, (float)dst + 0.5f, -0.5f);
+    const int i0 = min((int)floorf(src), in_size - 1);
+    const float t = fminf(fmaxf(__fadd_rn(src, -(float)i0), 0.f), 1.f), u = __fadd_rn(1.f, -t);
+    w[0] = cubic2_rn(__fadd_rn(t, 1.f)); w[1] = cubic1_rn(t); w[2] = cubic1_rn(u); w[3] = cubic2_rn(__fadd_rn(u, 1.f));
+#pragma unroll
+    for (int j = 0; j < 4; ++j) idx[j] = min(max(i0 + j - 1, 0), in_size - 1);
+}
+
+// A thread writes four consecutive output bytes of one row (one 32-bit store where the row allows it).  Memory bound: the 16 taps
+// of an output are mostly L1 / L2 hits of the 4-byte input pixels (only their alpha byte is used).
+constexpr int RA_X = 64, RA_Y = 4;
+__global__ void __launch_bounds__(RA_X * RA_Y) resample_alpha_kernel(const uint8_t *__restrict__ in, uint8_t *__restrict__ out, int H, int W,
+                                                                     int oH, int oW, float sy, float sx) {
+    pdl_trigger();
+    pdl_wait();
+    const int ox0 = (blockIdx.x * RA_X + threadIdx.x) * 4, oy = blockIdx.y * RA_Y + threadIdx.y;
+    const long b = blockIdx.z;
+    if (ox0 >= oW || oy >= oH) return;
+    int ty[4], tx[4];
+    float wy[4], wx[4];
+    cubic_taps_rn(oy, H, sy, ty, wy);
+    const uint8_t *f = in + b * H * W * 4 + 3;
+    uint32_t word = 0;
+    const int n = min(4, oW - ox0);
+    for (int k = 0; k < n; ++k) {
+        cubic_taps_rn(ox0 + k, W, sx, tx, wx);
+        float a = 0.f;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const uint8_t *row = f + (long)ty[i] * W * 4;
+            float acc = 0.f;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) acc = __fadd_rn(acc, __fmul_rn(u8_to_float(row[tx[j] * 4]), wx[j]));
+            a = __fadd_rn(a, __fmul_rn(acc, wy[i]));
+        }
+        const uint32_t code = (uint32_t)fminf(fmaxf(floorf(__fadd_rn(a, 0.5f)), 0.f), 255.f);
+        word |= code << (8 * k);
+    }
+    uint8_t *o = out + (b * oH + oy) * oW + ox0;
+    if (n == 4 && (reinterpret_cast<uintptr_t>(o) & 3) == 0) {
+        *reinterpret_cast<uint32_t *>(o) = word;
+    } else {
+        for (int k = 0; k < n; ++k) o[k] = (uint8_t)(word >> (8 * k));
     }
 }
 
@@ -1223,16 +1355,18 @@ static bool encode_image_map(CUtensorMap *tm, const void *ptr, int dtype, int B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, const float *res, int rH, int rW, void *out,
-                                    int out_dtype, int B, int outH, int outW, int clamp, void *stream) {
+int tu::bicubic_add_clamp_alpha(const void *x, int in_dtype, int H, int W, const float *res, int rH, int rW, void *out, int out_dtype,
+                                int B, int outH, int outW, int clamp, const uint8_t *alpha, cudaStream_t st) {
     TU_CHECK_ARG(x && out && B > 0 && H > 0 && W > 0 && outH > 0 && outW > 0, "bicubic_add_clamp: bad argument");
     const int layout = dtype_layout(out_dtype);
     out_dtype = dtype_base(out_dtype);
     TU_CHECK_ARG((in_dtype == TU_F32 || in_dtype == TU_BF16 || in_dtype == TU_F16 || in_dtype == TU_U8) &&
                      (out_dtype == TU_F32 || out_dtype == TU_BF16 || out_dtype == TU_F16 || out_dtype == TU_U8),
                  "bicubic_add_clamp: bad dtype");
-    TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout <= 2), "bicubic_add_clamp: interleaved layouts are for uint8 frames");
-    cudaStream_t st = (cudaStream_t)stream;
+    TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout_is_interleaved(layout)), "bicubic_add_clamp: interleaved layouts are for uint8 frames");
+    const bool px4 = layout_is_px4(layout);
+    TU_CHECK_ARG(!px4 || (reinterpret_cast<uintptr_t>(out) & 3) == 0, "bicubic_add_clamp: a 4-byte (RGBA / BGRA) output must be 4-byte aligned");
+    if (!px4) alpha = nullptr;
     const int eb = (int)dtype_size(in_dtype), ob = (int)dtype_size(out_dtype);
     BicubicTileGeom g;
     g.sxh = (float)H / (float)outH; g.sxw = (float)W / (float)outW;
@@ -1254,7 +1388,7 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
         return ok && encode_image_map(&tx, x, in_dtype, B, H, W, g.xr, g.xc) && (!res || encode_image_map(&tr, res, TU_F32, B, rH, rW, g.rr, g.rc));
     };
     // two output columns per thread: TMA tiles, even output width, pair stores aligned
-    const bool pair = g_bicubic_pair && (outW % 2) == 0 && (reinterpret_cast<uintptr_t>(out) % (2 * ob)) == 0 && plan(PAIR_H);
+    const bool pair = g_bicubic_pair && (outW % 2) == 0 && (reinterpret_cast<uintptr_t>(out) % (px4 ? 8 : 2 * ob)) == 0 && plan(PAIR_H);
     // periodic row schedules (x1.5 outputs such as 720p -> 1080p, x3 outputs such as 720p -> 4K): the unrolled circular-window kernel
     const int pat = pair && g_bicubic_pair >= 2 && res && clamp && (in_dtype == TU_BF16 || in_dtype == TU_F16 || in_dtype == TU_U8) &&
                             W <= outW && rW <= outW
@@ -1274,75 +1408,77 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
                   "the vertical table is filled in one pass of the CTA's threads");
     const bool tma = pair || plan(BS_H);
     dim3 grid(ceil_div(outW, BS_W), ceil_div(outH, pair ? PAIR_H : BS_H), B);
-#define TU_BIC_PAIR(TI, TO)                                                                                                     \
+#define TU_BIC_PAIR(TI, TO, PX4)                                                                                                \
     do {                                                                                                                        \
         static PerDeviceFlag attr_done;                                                                                          \
         if (!attr_done.is_set()) {                                                                                                       \
-            cudaError_t e = cudaFuncSetAttribute(bicubic_add_clamp_pair_kernel<TI, TO, true>,                                  \
+            cudaError_t e = cudaFuncSetAttribute(bicubic_add_clamp_pair_kernel<TI, TO, true, PX4>,                             \
                                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);                      \
             if (e == cudaSuccess)                                                                                               \
-                e = cudaFuncSetAttribute(bicubic_add_clamp_pair_kernel<TI, TO, false>,                                         \
+                e = cudaFuncSetAttribute(bicubic_add_clamp_pair_kernel<TI, TO, false, PX4>,                                    \
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);                              \
             if (e != cudaSuccess) return cuda_fail(e, "bicubic smem attribute");                                                \
             attr_done.set();                                                                                                   \
         }                                                                                                                       \
         if (res)                                                                                                                \
-            launch_pdl(bicubic_add_clamp_pair_kernel<TI, TO, true>, grid, dim3(BS_W / 2), tile_bytes + 128, st, tx, tr, g, H, W, rH, rW, \
-                       (TO *)out, outH, outW, clamp, layout);                                                                  \
+            launch_pdl(bicubic_add_clamp_pair_kernel<TI, TO, true, PX4>, grid, dim3(BS_W / 2), tile_bytes + 128, st, tx, tr, g, H, W, rH, \
+                       rW, (TO *)out, outH, outW, clamp, layout, alpha);                                                       \
         else                                                                                                                    \
-            launch_pdl(bicubic_add_clamp_pair_kernel<TI, TO, false>, grid, dim3(BS_W / 2), tile_bytes + 128, st, tx, tr, g, H, W, rH, rW, \
-                       (TO *)out, outH, outW, clamp, layout);                                                                  \
+            launch_pdl(bicubic_add_clamp_pair_kernel<TI, TO, false, PX4>, grid, dim3(BS_W / 2), tile_bytes + 128, st, tx, tr, g, H, W, rH, \
+                       rW, (TO *)out, outH, outW, clamp, layout, alpha);                                                       \
     } while (0)
-#define TU_BIC(TI, TO)                                                                                                          \
+#define TU_BIC(TI, TO, PX4)                                                                                                     \
     do {                                                                                                                        \
         if (tma) {                                                                                                              \
             static PerDeviceFlag attr_done;                                                                                      \
             if (!attr_done.is_set()) {                                                                                                   \
-                cudaError_t e = cudaFuncSetAttribute(bicubic_add_clamp_strip_kernel<TI, TO, 1>,                              \
+                cudaError_t e = cudaFuncSetAttribute(bicubic_add_clamp_strip_kernel<TI, TO, 1, PX4>,                         \
                                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);                  \
                 if (e == cudaSuccess)                                                                                           \
-                    e = cudaFuncSetAttribute(bicubic_add_clamp_strip_kernel<TI, TO, 2>,                                         \
+                    e = cudaFuncSetAttribute(bicubic_add_clamp_strip_kernel<TI, TO, 2, PX4>,                                    \
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);                          \
                 if (e != cudaSuccess) return cuda_fail(e, "bicubic smem attribute");                                            \
                 attr_done.set();                                                                                               \
             }                                                                                                                   \
             if (res)                                                                                                            \
-                launch_pdl(bicubic_add_clamp_strip_kernel<TI, TO, 1>, grid, dim3(BS_W), tile_bytes + 128, st, tx, tr, g, (const TI *)x, H, W, \
-                           res, rH, rW, (TO *)out, outH, outW, clamp, layout);                                              \
+                launch_pdl(bicubic_add_clamp_strip_kernel<TI, TO, 1, PX4>, grid, dim3(BS_W), tile_bytes + 128, st, tx, tr, g, (const TI *)x, \
+                           H, W, res, rH, rW, (TO *)out, outH, outW, clamp, layout, alpha);                                 \
             else                                                                                                                \
-                launch_pdl(bicubic_add_clamp_strip_kernel<TI, TO, 2>, grid, dim3(BS_W), tile_bytes + 128, st, tx, tr, g, (const TI *)x, H, W, \
-                           res, rH, rW, (TO *)out, outH, outW, clamp, layout);                                              \
+                launch_pdl(bicubic_add_clamp_strip_kernel<TI, TO, 2, PX4>, grid, dim3(BS_W), tile_bytes + 128, st, tx, tr, g, (const TI *)x, \
+                           H, W, res, rH, rW, (TO *)out, outH, outW, clamp, layout, alpha);                                 \
         } else {                                                                                                                \
-            bicubic_add_clamp_strip_kernel<TI, TO, 0><<<grid, BS_W, 0, st>>>(tx, tr, g, (const TI *)x, H, W, res, rH, rW,     \
-                                                                                  (TO *)out, outH, outW, clamp, layout);        \
+            bicubic_add_clamp_strip_kernel<TI, TO, 0, PX4><<<grid, BS_W, 0, st>>>(tx, tr, g, (const TI *)x, H, W, res, rH, rW, \
+                                                                                       (TO *)out, outH, outW, clamp, layout, alpha); \
         }                                                                                                                       \
     } while (0)
-#define TU_BIC2(TI, TO)          \
-    do {                         \
-        if (pair) TU_BIC_PAIR(TI, TO); \
-        else TU_BIC(TI, TO);     \
+#define TU_BIC2_A(TI, TO, PX4)        \
+    do {                              \
+        if (pair) TU_BIC_PAIR(TI, TO, PX4); \
+        else TU_BIC(TI, TO, PX4);     \
     } while (0)
-#define TU_BIC_R32_P(TI, TO, PAT, HWC)                                                                                          \
+#define TU_BIC2(TI, TO) TU_BIC2_A(TI, TO, false)
+#define TU_BIC_R32_P(TI, TO, PAT, PX)                                                                                           \
     do {                                                                                                                        \
         static PerDeviceFlag attr_done;                                                                                          \
         if (!attr_done.is_set()) {                                                                                               \
-            cudaError_t e = cudaFuncSetAttribute(bicubic_add_clamp_r32_kernel<TI, TO, PAT, HWC>,                                \
-                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);                       \
+            cudaError_t e = cudaFuncSetAttribute(bicubic_add_clamp_r32_kernel<TI, TO, PAT, PX>,                                 \
+                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (PX == 4 ? 128 : 96) * 1024);     \
             if (e != cudaSuccess) return cuda_fail(e, "bicubic smem attribute");                                                \
             attr_done.set();                                                                                                    \
         }                                                                                                                       \
-        launch_pdl(bicubic_add_clamp_r32_kernel<TI, TO, PAT, HWC>, dim3(grid.x, ceil_div(outH, tile_rows), B), dim3(R32_T),     \
-                   tile_bytes + 128, st, tx, tr, g, H, W, rH, rW, (TO *)out, outH, outW, layout, tile_rows);                    \
+        launch_pdl(bicubic_add_clamp_r32_kernel<TI, TO, PAT, PX>, dim3(grid.x, ceil_div(outH, tile_rows), B), dim3(R32_T),      \
+                   tile_bytes + 128 + (PX == 4 ? px4_stage_bytes<PAT>() + 16 : 0), st, tx, tr, g, H, W, rH, rW, (TO *)out, outH, outW, \
+                   layout, tile_rows, alpha);                                                                                   \
     } while (0)
-#define TU_BIC_R32_L(TI, TO, HWC)                                                                                               \
+#define TU_BIC_R32_L(TI, TO, PX)                                                                                                \
     do {                                                                                                                        \
-        if (pat == 0) TU_BIC_R32_P(TI, TO, 0, HWC);                                                                             \
-        else if (pat == 2) TU_BIC_R32_P(TI, TO, 2, HWC);                                                                        \
-        else if (pat == 3) TU_BIC_R32_P(TI, TO, 3, HWC);                                                                        \
-        else if (pat == 4) TU_BIC_R32_P(TI, TO, 4, HWC);                                                                        \
-        else TU_BIC_R32_P(TI, TO, 6, HWC);                                                                                      \
+        if (pat == 0) TU_BIC_R32_P(TI, TO, 0, PX);                                                                              \
+        else if (pat == 2) TU_BIC_R32_P(TI, TO, 2, PX);                                                                         \
+        else if (pat == 3) TU_BIC_R32_P(TI, TO, 3, PX);                                                                         \
+        else if (pat == 4) TU_BIC_R32_P(TI, TO, 4, PX);                                                                         \
+        else TU_BIC_R32_P(TI, TO, 6, PX);                                                                                       \
     } while (0)
-#define TU_BIC_R32(TI, TO) TU_BIC_R32_L(TI, TO, false)
+#define TU_BIC_R32(TI, TO) TU_BIC_R32_L(TI, TO, 0)
     if (r32 && pat == 0 && layout == 0 && g_bicubic_pair >= 3 && in_dtype != TU_F16 && out_dtype != TU_F16) {
         // streaming variant: strips x segments co-resident (5 CTAs per SM), <= 16 blocks of 12 rows per segment
         const int nblk = outH / 12, strips = (int)grid.x * B;
@@ -1381,10 +1517,19 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
             return TU_OK;
         }
     }
-    if (r32 && layout != 0) {           // interleaved uint8 frames (layouts are accepted for uint8 output only)
-        if (in_dtype == TU_BF16) TU_BIC_R32_L(bf16, uint8_t, true);
-        else if (in_dtype == TU_F16) TU_BIC_R32_L(f16, uint8_t, true);
-        else TU_BIC_R32_L(uint8_t, uint8_t, true);
+    if (r32 && px4) {                   // 4-byte uint8 frames
+        if (in_dtype == TU_BF16) TU_BIC_R32_L(bf16, uint8_t, 4);
+        else if (in_dtype == TU_F16) TU_BIC_R32_L(f16, uint8_t, 4);
+        else TU_BIC_R32_L(uint8_t, uint8_t, 4);
+    } else if (r32 && layout != 0) {    // interleaved uint8 frames (layouts are accepted for uint8 output only)
+        if (in_dtype == TU_BF16) TU_BIC_R32_L(bf16, uint8_t, 3);
+        else if (in_dtype == TU_F16) TU_BIC_R32_L(f16, uint8_t, 3);
+        else TU_BIC_R32_L(uint8_t, uint8_t, 3);
+    } else if (px4) {
+        if (in_dtype == TU_F32) TU_BIC2_A(float, uint8_t, true);
+        else if (in_dtype == TU_BF16) TU_BIC2_A(bf16, uint8_t, true);
+        else if (in_dtype == TU_F16) TU_BIC2_A(f16, uint8_t, true);
+        else TU_BIC2_A(uint8_t, uint8_t, true);
     } else if (r32) {
         if (in_dtype == TU_BF16 && out_dtype == TU_BF16) TU_BIC_R32(bf16, bf16);
         else if (in_dtype == TU_BF16 && out_dtype == TU_F32) TU_BIC_R32(bf16, float);
@@ -1416,6 +1561,7 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
     else if (in_dtype == TU_U8 && out_dtype == TU_F16) TU_BIC2(uint8_t, f16);
     else TU_BIC2(bf16, uint8_t);
 #undef TU_BIC2
+#undef TU_BIC2_A
 #undef TU_BIC_R32
 #undef TU_BIC_R32_P
 #undef TU_BIC_R32_L
@@ -1425,18 +1571,33 @@ extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, c
     return TU_OK;
 }
 
+extern "C" int tu_bicubic_add_clamp(const void *x, int in_dtype, int H, int W, const float *res, int rH, int rW, void *out,
+                                    int out_dtype, int B, int outH, int outW, int clamp, void *stream) {
+    return bicubic_add_clamp_alpha(x, in_dtype, H, W, res, rH, rW, out, out_dtype, B, outH, outW, clamp, nullptr, (cudaStream_t)stream);
+}
+
 extern "C" int tu_bicubic_row_schedule(int H, int rH, int outH) { return H > 0 && rH > 0 && outH > 0 ? row_pattern(H, rH, outH) : -1; }
 
-extern "C" int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out, int out_dtype, int B, int H, int W, int outH, int outW,
-                                        int clamp, void *stream) {
+extern "C" int tu_resize_bilinear_aa_to_alpha(const void *in, int in_dtype, const void *alpha, void *out, int out_dtype, int B, int H, int W,
+                                              int outH, int outW, int clamp, void *stream) {
     TU_CHECK_ARG(in && out && B > 0 && H > 0 && W > 0 && outH > 0 && outW > 0, "resize_bilinear_aa: bad argument");
     const int layout = dtype_layout(out_dtype);
     out_dtype = dtype_base(out_dtype);
-    TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout <= 2), "resize_bilinear_aa: interleaved layouts are for uint8 frames");
+    TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout_is_interleaved(layout)), "resize_bilinear_aa: interleaved layouts are for uint8 frames");
+    const bool px4 = layout_is_px4(layout);
+    TU_CHECK_ARG(!px4 || (reinterpret_cast<uintptr_t>(out) & 3) == 0, "resize_bilinear_aa: a 4-byte (RGBA / BGRA) output must be 4-byte aligned");
+    TU_CHECK_ARG(px4 || !alpha, "resize_bilinear_aa: an alpha plane needs a 4-byte (RGBA / BGRA) output");
+    TU_CHECK_ARG(!px4 || B <= 65535, "resize_bilinear_aa: too many frames");
     cudaStream_t st = (cudaStream_t)stream;
-    dim3 grid(ceil_div(outW, 64), ceil_div(outH, 4), B * 3);
-#define TU_RS(TI, TO) resize_aa_kernel<TI, TO><<<grid, 256, 0, st>>>((const TI *)in, (TO *)out, H, W, outH, outW, clamp, layout)
-    if (in_dtype == TU_F32 && out_dtype == TU_F32) TU_RS(float, float);
+    dim3 grid(ceil_div(outW, 64), ceil_div(outH, 4), px4 ? B : B * 3);
+    const uint8_t *ap = (const uint8_t *)alpha;
+#define TU_RS(TI, TO) resize_aa_kernel<TI, TO><<<grid, 256, 0, st>>>((const TI *)in, (TO *)out, H, W, outH, outW, clamp, layout, nullptr)
+#define TU_RS4(TI) resize_aa_kernel<TI, uint8_t, true><<<grid, 256, 0, st>>>((const TI *)in, (uint8_t *)out, H, W, outH, outW, clamp, layout, ap)
+    if (px4 && in_dtype == TU_F32) TU_RS4(float);
+    else if (px4 && in_dtype == TU_BF16) TU_RS4(bf16);
+    else if (px4 && in_dtype == TU_F16) TU_RS4(f16);
+    else if (px4) TU_CHECK_ARG(false, "resize_bilinear_aa: bad dtype");
+    else if (in_dtype == TU_F32 && out_dtype == TU_F32) TU_RS(float, float);
     else if (in_dtype == TU_BF16 && out_dtype == TU_BF16) TU_RS(bf16, bf16);
     else if (in_dtype == TU_F32 && out_dtype == TU_BF16) TU_RS(float, bf16);
     else if (in_dtype == TU_BF16 && out_dtype == TU_F32) TU_RS(bf16, float);
@@ -1450,8 +1611,14 @@ extern "C" int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out,
     else if (in_dtype == TU_BF16 && out_dtype == TU_F16) TU_RS(bf16, f16);
     else TU_CHECK_ARG(false, "resize_bilinear_aa: bad dtype");
 #undef TU_RS
+#undef TU_RS4
     TU_CHECK_LAUNCH("resize_bilinear_aa");
     return TU_OK;
+}
+
+extern "C" int tu_resize_bilinear_aa_to(const void *in, int in_dtype, void *out, int out_dtype, int B, int H, int W, int outH, int outW,
+                                        int clamp, void *stream) {
+    return tu_resize_bilinear_aa_to_alpha(in, in_dtype, nullptr, out, out_dtype, B, H, W, outH, outW, clamp, stream);
 }
 
 extern "C" int tu_resize_bilinear_aa(const void *in, int dtype, void *out, int B, int H, int W, int outH, int outW,
@@ -1462,12 +1629,27 @@ extern "C" int tu_resize_bilinear_aa(const void *in, int dtype, void *out, int B
 
 extern "C" int tu_frames_to_planar(const void *in, int layout, void *out, int B, int H, int W, void *stream) {
     TU_CHECK_ARG(in && out && B > 0 && H > 0 && W > 0, "frames_to_planar: bad argument");
-    TU_CHECK_ARG(layout == TU_LAYOUT_HWC || layout == TU_LAYOUT_HWC_BGR, "frames_to_planar: layout must be TU_LAYOUT_HWC or TU_LAYOUT_HWC_BGR");
+    TU_CHECK_ARG(layout == TU_LAYOUT_HWC || layout == TU_LAYOUT_HWC_BGR || layout == TU_LAYOUT_RGBA || layout == TU_LAYOUT_BGRA,
+                 "frames_to_planar: layout must be TU_LAYOUT_HWC, TU_LAYOUT_HWC_BGR, TU_LAYOUT_RGBA or TU_LAYOUT_BGRA");
     const long plane = (long)H * W;
     dim3 grid((unsigned)((plane + 1023) / 1024), B);
-    launch_pdl(frames_to_planar_kernel, grid, dim3(256), 0, (cudaStream_t)stream, (const uint8_t *)in, (uint8_t *)out, plane,
-               layout == TU_LAYOUT_HWC_BGR ? 1 : 0);
+    const int swap = layout == TU_LAYOUT_HWC_BGR || layout == TU_LAYOUT_BGRA ? 1 : 0;
+    if (layout_is_px4(layout >> 8))
+        launch_pdl(frames_to_planar_kernel<4>, grid, dim3(256), 0, (cudaStream_t)stream, (const uint8_t *)in, (uint8_t *)out, plane, swap);
+    else
+        launch_pdl(frames_to_planar_kernel<3>, grid, dim3(256), 0, (cudaStream_t)stream, (const uint8_t *)in, (uint8_t *)out, plane, swap);
     TU_CHECK_LAUNCH("frames_to_planar");
+    return TU_OK;
+}
+
+extern "C" int tu_resample_alpha(const void *frames, int code, void *alpha, int B, int H, int W, int outH, int outW, void *stream) {
+    TU_CHECK_ARG(frames && alpha && B > 0 && B <= 65535 && H > 0 && W > 0 && outH > 0 && outW > 0, "resample_alpha: bad argument");
+    TU_CHECK_ARG(dtype_is_px4(code), "resample_alpha: code must be TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA");
+    TU_CHECK_ARG((long)H * W * 4 < (1L << 31) && (long)outH * outW < (1L << 31), "resample_alpha: frame too large");
+    const dim3 grid((unsigned)ceil_div(ceil_div(outW, 4), RA_X), (unsigned)ceil_div(outH, RA_Y), (unsigned)B);
+    launch_pdl(resample_alpha_kernel, grid, dim3(RA_X, RA_Y), 0, (cudaStream_t)stream, (const uint8_t *)frames, (uint8_t *)alpha, H, W, outH,
+               outW, (float)H / (float)outH, (float)W / (float)outW);
+    TU_CHECK_LAUNCH("resample_alpha");
     return TU_OK;
 }
 

@@ -35,11 +35,13 @@ constexpr int NT = 256;
 // body keeps every coefficient a constant-bank operand of exactly one FFMA.
 struct FinFilter { float w[3][81]; float b[3]; };
 
-template <int R, typename TO>
+// PX4: 4-byte uint8 pixels (layout 3 / 5), each written once with its alpha from the plane `alpha` (NULL: 255); the other
+// instantiations never read `alpha`
+template <int R, typename TO, bool PX4 = false>
 __global__ void __launch_bounds__(NT, 4)
 subpixel_tail_kernel(const float *__restrict__ in, const float *__restrict__ wps, const float *__restrict__ bps,
                      const float *__restrict__ addend, TO *__restrict__ out, int H, int W, int clamp, int layout,
-                     const FinFilter fin) {
+                     const FinFilter fin, const uint8_t *__restrict__ alpha) {
     constexpr int NCO = 3 * R * R;
     constexpr int TH = tile_rows<R>(), IR = TH + 2;     // IR = intermediate rows held
     constexpr int NLR = TH / R + 4;            // low-res rows staged: ly0 - 2 .. ly0 + TH/R + 1
@@ -190,7 +192,9 @@ subpixel_tail_kernel(const float *__restrict__ in, const float *__restrict__ wps
             rgb[co] = r;                                                                                    \
             ad[co] = adn[co];                                                                               \
         }                                                                                                   \
-        if (layout == 0) {                                                                                  \
+        if constexpr (PX4) {                                                                                \
+            store_px4(out, (long)b * plane + (long)(oy0 + (ry)) * oW + ox, layout, rgb[0], rgb[1], rgb[2], alpha); \
+        } else if (layout == 0) {                                                                           \
             _Pragma("unroll") for (int co = 0; co < 3; ++co) out[o + co * plane] = from_f<TO>(rgb[co]);     \
         } else {                                                                                            \
             store_rgb<TO>(out, b, plane, (long)(oy0 + (ry)) * oW + ox, layout, rgb[0], rgb[1], rgb[2]);     \
@@ -223,29 +227,29 @@ constexpr size_t tail_smem() {
     return sizeof(float) * (3 * R * R * 28 + ((3 * R * R + 3) & ~3) + 3 * (TH / R + 4) * (TLX + 4) + 3 * IR * 32 * R);
 }
 
-template <int R, typename TO>
+template <int R, typename TO, bool PX4>
 int launch_tail(const float *in, const float *wps, const float *bps, const float *addend, TO *out, int B, int H, int W, int clamp, int layout,
-                const FinFilter &fin, cudaStream_t st) {
+                const FinFilter &fin, const uint8_t *alpha, cudaStream_t st) {
     static PerDeviceFlag attr;
     constexpr size_t smem = tail_smem<R>();
     if (!attr.is_set() && smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(subpixel_tail_kernel<R, TO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(subpixel_tail_kernel<R, TO, PX4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return cuda_fail(e, "subpixel_tail smem attribute");
         attr.set();
     }
     dim3 grid(ceil_div(W, TLX), ceil_div(H * R, tile_rows<R>()), B);
-    launch_pdl(subpixel_tail_kernel<R, TO>, grid, dim3(NT), smem, st, in, wps, bps, addend, out, H, W, clamp, layout, fin);
+    launch_pdl(subpixel_tail_kernel<R, TO, PX4>, grid, dim3(NT), smem, st, in, wps, bps, addend, out, H, W, clamp, layout, fin, alpha);
     TU_CHECK_LAUNCH("subpixel_tail");
     return TU_OK;
 }
 
-template <typename TO>
+template <typename TO, bool PX4 = false>
 int tail_by_r(int r, const float *in, const float *wps, const float *bps, const float *addend, TO *out, int B, int H, int W, int clamp, int layout,
-              const FinFilter &fin, cudaStream_t st) {
+              const FinFilter &fin, cudaStream_t st, const uint8_t *alpha = nullptr) {
     switch (r) {
-        case 2: return launch_tail<2, TO>(in, wps, bps, addend, out, B, H, W, clamp, layout, fin, st);
-        case 3: return launch_tail<3, TO>(in, wps, bps, addend, out, B, H, W, clamp, layout, fin, st);
-        case 6: return launch_tail<6, TO>(in, wps, bps, addend, out, B, H, W, clamp, layout, fin, st);
+        case 2: return launch_tail<2, TO, PX4>(in, wps, bps, addend, out, B, H, W, clamp, layout, fin, alpha, st);
+        case 3: return launch_tail<3, TO, PX4>(in, wps, bps, addend, out, B, H, W, clamp, layout, fin, alpha, st);
+        case 6: return launch_tail<6, TO, PX4>(in, wps, bps, addend, out, B, H, W, clamp, layout, fin, alpha, st);
     }
     set_error("tu: subpixel_conv_add: r must be 2, 3 or 6");
     return TU_ERR_ARG;
@@ -257,22 +261,29 @@ int tail_by_r(int r, const float *in, const float *wps, const float *bps, const 
 
 using namespace tu;
 
-extern "C" int tu_subpixel_conv_add(const float *in, const float *w_ps, const float *b_ps, int r, const float *host_fin_wb,
-                                    const float *addend, void *out, int out_dtype, int B, int H, int W, int clamp, void *stream) {
+int tu::subpixel_conv_add_alpha(const float *in, const float *w_ps, const float *b_ps, int r, const float *host_fin_wb, const float *addend,
+                                void *out, int out_dtype, int B, int H, int W, int clamp, const uint8_t *alpha, cudaStream_t st) {
     TU_CHECK_ARG(in && w_ps && b_ps && host_fin_wb && addend && out && B > 0 && H > 0 && W > 0, "subpixel_conv_add: bad argument");
     TU_CHECK_ARG((long)B * 3 * H * r * W * r < (1L << 31), "subpixel_conv_add: image too large for 32-bit pixel indexing");
     const int layout = dtype_layout(out_dtype);
     out_dtype = dtype_base(out_dtype);
-    TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout <= 2), "subpixel_conv_add: interleaved layouts are for uint8 frames");
+    TU_CHECK_ARG(layout == 0 || (out_dtype == TU_U8 && layout_is_interleaved(layout)), "subpixel_conv_add: interleaved layouts are for uint8 frames");
     TU_CHECK_ARG(out_dtype == TU_F32 || out_dtype == TU_BF16 || out_dtype == TU_U8 || out_dtype == TU_F16, "subpixel_conv_add: bad dtype");
-    cudaStream_t st = (cudaStream_t)stream;
+    const bool px4 = layout_is_px4(layout);
+    TU_CHECK_ARG(!px4 || (reinterpret_cast<uintptr_t>(out) & 3) == 0, "subpixel_conv_add: a 4-byte (RGBA / BGRA) output must be 4-byte aligned");
     FinFilter fin;
     for (int cp = 0; cp < 3; ++cp)
         for (int i = 0; i < 81; ++i) fin.w[cp][i] = host_fin_wb[i];
     for (int i = 0; i < 3; ++i) fin.b[i] = host_fin_wb[81 + i];
+    if (px4) return tail_by_r<uint8_t, true>(r, in, w_ps, b_ps, addend, (uint8_t *)out, B, H, W, clamp, layout, fin, st, alpha);
     if (out_dtype == TU_F32) return tail_by_r<float>(r, in, w_ps, b_ps, addend, (float *)out, B, H, W, clamp, layout, fin, st);
     if (out_dtype == TU_BF16) return tail_by_r<bf16>(r, in, w_ps, b_ps, addend, (bf16 *)out, B, H, W, clamp, layout, fin, st);
     if (out_dtype == TU_U8) return tail_by_r<uint8_t>(r, in, w_ps, b_ps, addend, (uint8_t *)out, B, H, W, clamp, layout, fin, st);
     if (out_dtype == TU_F16) return tail_by_r<f16>(r, in, w_ps, b_ps, addend, (f16 *)out, B, H, W, clamp, layout, fin, st);
     TU_CHECK_ARG(false, "subpixel_conv_add: bad dtype");
+}
+
+extern "C" int tu_subpixel_conv_add(const float *in, const float *w_ps, const float *b_ps, int r, const float *host_fin_wb,
+                                    const float *addend, void *out, int out_dtype, int B, int H, int W, int clamp, void *stream) {
+    return subpixel_conv_add_alpha(in, w_ps, b_ps, r, host_fin_wb, addend, out, out_dtype, B, H, W, clamp, nullptr, (cudaStream_t)stream);
 }

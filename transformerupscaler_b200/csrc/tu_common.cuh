@@ -97,7 +97,14 @@ template <> __device__ __forceinline__ uint8_t from_f<uint8_t>(float v) {
 // TU_U8 | TU_LAYOUT_NV12 (4:2:0 video frames) may add the colour bits TU_YUV_BT601 / TU_YUV_FULL_RANGE in bits 12..13.
 // TU_U16 | TU_LAYOUT_P010 (10-bit 4:2:0 frames) may add the same bits, or TU_YUV_BT2020 (bit 14) instead of TU_YUV_BT601.
 __host__ __device__ __forceinline__ int dtype_base(int d) { return d & 0xFF; }
-__host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }          // 0 planar CHW, 1 HWC RGB, 2 HWC BGR; NV12 / P010: >= 4
+// the layout bits are an enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 8 P010), and dtype_layout keeps the colour bits
+// above them: compare whole values, never bits (0x500 = BGRA shares a bit with NV12, 0x300 = RGBA two bits with HWC / HWC_BGR)
+__host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }
+__host__ __device__ __forceinline__ bool layout_is_px4(int l) { return l == 3 || l == 5; }          // RGBA / BGRA: 4-byte pixels
+__host__ __device__ __forceinline__ bool layout_is_interleaved(int l) { return l == 1 || l == 2 || layout_is_px4(l); }
+__host__ __device__ __forceinline__ bool dtype_is_px4(int d) {                          // TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA
+    return d == (TU_U8 | TU_LAYOUT_RGBA) || d == (TU_U8 | TU_LAYOUT_BGRA);
+}
 __host__ __device__ __forceinline__ bool dtype_is_nv12(int d) {                        // TU_U8 | TU_LAYOUT_NV12 [| colour bits]
     return (d & ~(TU_YUV_BT601 | TU_YUV_FULL_RANGE)) == (TU_U8 | TU_LAYOUT_NV12);
 }
@@ -117,6 +124,20 @@ __device__ __forceinline__ void store_rgb(TO *out, long b, long plane, long pix,
         o[layout == 2 ? 2 : 0] = from_f<TO>(r); o[1] = from_f<TO>(g); o[layout == 2 ? 0 : 2] = from_f<TO>(bl);
     }
 }
+// one 4-byte pixel (layout 3: R G B A, 5: B G R A) at pixel index pix of a (B, H, W, 4) frame batch, written once; its alpha is byte pix of
+// the (B, H, W) plane `alpha`, or 255 when there is none
+__device__ __forceinline__ void store_px4(uint8_t *out, long pix, int layout, float r, float g, float bl, const uint8_t *alpha) {
+    const uint32_t cr = from_f<uint8_t>(r), cg = from_f<uint8_t>(g), cb = from_f<uint8_t>(bl);
+    const uint32_t a = alpha ? (uint32_t)alpha[pix] : 255u;
+    reinterpret_cast<uint32_t *>(out)[pix] = (layout == 5 ? cb | cr << 16 : cr | cb << 16) | cg << 8 | a << 24;
+}
+
+// internal forms of two output ops that also take the alpha plane of a 4-byte output (NULL: alpha 255); the exported functions
+// (tu_bicubic_add_clamp, tu_subpixel_conv_add) are these with NULL
+int bicubic_add_clamp_alpha(const void *x, int in_dtype, int H, int W, const float *res, int rH, int rW, void *out, int out_dtype, int B,
+                            int outH, int outW, int clamp, const uint8_t *alpha, cudaStream_t st);
+int subpixel_conv_add_alpha(const float *in, const float *w_ps, const float *b_ps, int r, const float *host_fin_wb, const float *addend,
+                            void *out, int out_dtype, int B, int H, int W, int clamp, const uint8_t *alpha, cudaStream_t st);
 
 // 4 consecutive elements -> float4 (pointer must be aligned to 4 elements)
 __device__ __forceinline__ float4 load4(const float *p) { return *reinterpret_cast<const float4 *>(p); }

@@ -55,7 +55,7 @@ def _code(dt: torch.dtype) -> int:
 
 
 LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR, "nv12": _lib.TU_LAYOUT_NV12,
-           "p010": _lib.TU_LAYOUT_P010}
+           "p010": _lib.TU_LAYOUT_P010, "rgba": _lib.TU_LAYOUT_RGBA, "bgra": _lib.TU_LAYOUT_BGRA}
 # colour of NV12 and P010 frames: matrix and range
 YUV = {"bt709": 0, "bt601": _lib.TU_YUV_BT601, "bt709_full": _lib.TU_YUV_FULL_RANGE,
        "bt601_full": _lib.TU_YUV_BT601 | _lib.TU_YUV_FULL_RANGE}
@@ -65,7 +65,7 @@ YUV_P010 = {"bt2020": _lib.TU_YUV_BT2020, "bt2020_full": _lib.TU_YUV_BT2020 | _l
 
 def layout_code(name: str) -> int:
     if name not in LAYOUTS:
-        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr', 'nv12' or 'p010'")
+        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr', 'rgba', 'bgra', 'nv12' or 'p010'")
     return LAYOUTS[name]
 
 
@@ -78,6 +78,7 @@ def yuv_code(name: str) -> int:
                      "'bt2020', 'bt2020_full'")
 
 
+# the layout bits 8..11 of a code are an enumeration: compare whole values (0x500 = BGRA shares a bit with NV12's 0x400)
 def _is_nv12(code: int) -> bool:
     return code & 0xF00 == _lib.TU_LAYOUT_NV12
 
@@ -86,12 +87,19 @@ def _is_p010(code: int) -> bool:
     return code & 0xF00 == _lib.TU_LAYOUT_P010
 
 
+def _is_px4(code: int) -> bool:
+    """RGBA / BGRA: 4-byte pixels (B, H, W, 4)"""
+    return code & 0xF00 in (_lib.TU_LAYOUT_RGBA, _lib.TU_LAYOUT_BGRA)
+
+
 def _image_shape(B: int, C_: int, h: int, w: int, code: int) -> Tuple[int, ...]:
-    """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3) or NV12 / P010
-    (B,3h/2,w)"""
+    """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3), 4-byte pixels
+    (B,h,w,4) or NV12 / P010 (B,3h/2,w)"""
     if _is_nv12(code) or _is_p010(code):
         return (B, 3 * h // 2, w)
-    return (B, h, w, 3) if code >> 8 else (B, C_, h, w)
+    if _is_px4(code):
+        return (B, h, w, 4)
+    return (B, h, w, 3) if code & 0xF00 in (_lib.TU_LAYOUT_HWC, _lib.TU_LAYOUT_HWC_BGR) else (B, C_, h, w)
 
 
 def _yuv420_hw(x: torch.Tensor, fmt: str, dtype: torch.dtype) -> Tuple[int, int]:
@@ -171,8 +179,9 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
         x = x.contiguous()
         B = x.shape[0]
     elif in_layout:
-        if x.dim() != 4 or x.shape[3] != 3 or x.dtype != torch.uint8:
-            raise RuntimeError(f"interleaved frames must be uint8 of shape (B,H,W,3), got {x.dtype} {tuple(x.shape)}")
+        px = 4 if _is_px4(in_layout) else 3
+        if x.dim() != 4 or x.shape[3] != px or x.dtype != torch.uint8:
+            raise RuntimeError(f"interleaved frames must be uint8 of shape (B,H,W,{px}), got {x.dtype} {tuple(x.shape)}")
         x = x.contiguous()
         B, H, W, _ = x.shape
     else:
@@ -259,30 +268,52 @@ def _(x, x_planes, out_planes, handle, out_h, out_w, scale, compute_bf16, out_co
 
 
 @torch.library.custom_op("tu::resize_aa", mutates_args=(), device_types="cuda")
-def tu_resize_aa(x: torch.Tensor, out_h: int, out_w: int, clamp: bool, out_code: int = -1) -> torch.Tensor:
-    """antialiased bilinear Resize of a (B,3,H,W) float image; out_code < 0: same dtype as x, else a dtype (| layout) code"""
+def tu_resize_aa(x: torch.Tensor, out_h: int, out_w: int, clamp: bool, out_code: int = -1,
+                 alpha: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """antialiased bilinear Resize of a (B,3,H,W) float image; out_code < 0: same dtype as x, else a dtype (| layout) code.
+    alpha: the (B, out_h, out_w) uint8 alpha plane of an RGBA / BGRA output (tu::resample_alpha); None writes alpha 255"""
     lib = _lib.load()
-    _require_cuda(x)
+    _require_cuda(x, alpha)
     x = x.contiguous()
     B, Cc, H, W = x.shape
     if out_code < 0:
         out_code = _code(x.dtype)
     if Cc != 3 and out_code >> 8:
         raise RuntimeError("interleaved output needs a 3-channel image")
-    shape = (B, out_h, out_w, 3) if out_code >> 8 else (B, Cc, out_h, out_w)
-    out = torch.empty(shape, dtype=_TORCH_DT[out_code & 0xFF], device=x.device)
+    if alpha is not None and (not _is_px4(out_code) or alpha.dtype != torch.uint8 or tuple(alpha.shape) != (B, out_h, out_w)):
+        raise RuntimeError(f"an alpha plane is (B, out_h, out_w) uint8 for an RGBA / BGRA output, got {alpha.dtype} {tuple(alpha.shape)}")
+    out = torch.empty(_image_shape(B, Cc, out_h, out_w, out_code), dtype=_TORCH_DT[out_code & 0xFF], device=x.device)
     with torch.cuda.device(x.device):
-        _lib.check(lib.tu_resize_bilinear_aa_to(x.data_ptr(), _code(x.dtype), out.data_ptr(), out_code, B * Cc // 3, H, W, out_h, out_w,
-                                                int(clamp), _stream()))
+        _lib.check(lib.tu_resize_bilinear_aa_to_alpha(x.data_ptr(), _code(x.dtype), None if alpha is None else alpha.contiguous().data_ptr(),
+                                                      out.data_ptr(), out_code, B * Cc // 3, H, W, out_h, out_w, int(clamp), _stream()))
     return out
 
 
 @tu_resize_aa.register_fake
-def _(x, out_h, out_w, clamp, out_code=-1):
+def _(x, out_h, out_w, clamp, out_code=-1, alpha=None):
     if out_code < 0:
         return x.new_empty((x.shape[0], x.shape[1], out_h, out_w))
-    shape = (x.shape[0], out_h, out_w, 3) if out_code >> 8 else (x.shape[0], x.shape[1], out_h, out_w)
-    return x.new_empty(shape, dtype=_TORCH_DT[out_code & 0xFF])
+    return x.new_empty(_image_shape(x.shape[0], x.shape[1], out_h, out_w, out_code), dtype=_TORCH_DT[out_code & 0xFF])
+
+
+@torch.library.custom_op("tu::resample_alpha", mutates_args=(), device_types="cuda")
+def tu_resample_alpha(x: torch.Tensor, code: int, out_h: int, out_w: int) -> torch.Tensor:
+    """the alpha bytes of RGBA / BGRA frames (B,H,W,4) uint8 resampled (bicubic, tu_resample_alpha) to a (B,out_h,out_w) uint8 plane"""
+    lib = _lib.load()
+    _require_cuda(x)
+    if x.dim() != 4 or x.shape[3] != 4 or x.dtype != torch.uint8:
+        raise RuntimeError(f"resample_alpha takes (B,H,W,4) uint8 frames, got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, H, W, _ = x.shape
+    out = torch.empty((B, out_h, out_w), dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_resample_alpha(x.data_ptr(), code, out.data_ptr(), B, H, W, out_h, out_w, _stream()))
+    return out
+
+
+@tu_resample_alpha.register_fake
+def _(x, code, out_h, out_w):
+    return x.new_empty((x.shape[0], out_h, out_w), dtype=torch.uint8)
 
 
 @torch.library.custom_op("tu::rgb_to_nv12", mutates_args=(), device_types="cuda")
@@ -348,9 +379,11 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
                 require_ratio: bool, compute_bf16: bool, out_dtype: torch.dtype, clamp: bool = True,
                 in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709", out=None):
     """Shape logic of the three reference forwards (W:237-238, F:245-248,323-327, R:121-122) around tu::forward.
-    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'nv12' | 'p010'): uint8 frames may be interleaved (B,H,W,3) or NV12
-    (B,3H/2,W) on either side, and either side may be P010 (B,3H/2,W) uint16 frames; yuv ('bt709' | 'bt601' | 'bt709_full' |
-    'bt601_full', and 'bt2020' | 'bt2020_full' for P010 only) is the colour of the NV12 / P010 side(s).
+    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'rgba' | 'bgra' | 'nv12' | 'p010'): uint8 frames may be interleaved (B,H,W,3),
+    4-byte pixels with alpha (B,H,W,4) or NV12 (B,3H/2,W) on either side, and either side may be P010 (B,3H/2,W) uint16 frames; yuv
+    ('bt709' | 'bt601' | 'bt709_full' | 'bt601_full', and 'bt2020' | 'bt2020_full' for P010 only) is the colour of the NV12 / P010
+    side(s).  An RGBA / BGRA output carries the input alpha resampled to the output size (tu_resample_alpha) when the input is RGBA /
+    BGRA too, else alpha 255; an RGBA / BGRA input going to an output without alpha loses its alpha.
     Frame surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs (see plane_pairs); with out_layout
     'nv12' / 'p010', out= a list of B (y, uv) pairs receives the result and is returned."""
     il, ol = layout_code(in_layout), layout_code(out_layout)
@@ -365,6 +398,12 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
         raise ValueError("out_layout='nv12' writes uint8 frames")
     if p010_out and out_dtype != torch.uint16:
         raise ValueError("out_layout='p010' writes uint16 frames")
+    px4_in, px4_out = in_layout in ("rgba", "bgra"), out_layout in ("rgba", "bgra")
+    if px4_out and out_dtype != torch.uint8:
+        raise ValueError(f"out_layout={out_layout!r} writes uint8 frames")
+    if px4_in and not (isinstance(x, torch.Tensor) and x.dim() == 4 and x.shape[3] == 4 and x.dtype == torch.uint8):
+        got = f"{x.dtype} {tuple(x.shape)}" if isinstance(x, torch.Tensor) else type(x).__name__
+        raise ValueError(f"in_layout={in_layout!r} takes uint8 frames of shape (B, H, W, 4), got {got}")
     il |= yc if nv12_in or p010_in else 0
     planes_in = isinstance(x, (list, tuple))
     if planes_in and not (nv12_in or p010_in):
@@ -432,4 +471,7 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
         return tu_rgb_to_nv12(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16), out_code)
     if p010_out:
         return tu_rgb_to_p010(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F32), out_code)
+    if px4_in and px4_out:
+        # alpha is resampled straight from the input to the requested size, by the rule of every other output path
+        return tu_resize_aa(full, res_out[0], res_out[1], clamp, out_code, tu_resample_alpha(x, _lib.TU_U8 | il, res_out[0], res_out[1]))
     return tu_resize_aa(full, res_out[0], res_out[1], clamp, out_code)

@@ -153,6 +153,10 @@ class EngineModel(nn.Module):
         in_layout / out_layout in {'chw', 'hwc', 'hwc_bgr', 'nv12'} — uint8 frames may arrive / leave interleaved (B,H,W,3), the form PIL
         and OpenCV hold them in (inference.py:65-70, app_overlay.py:382-386), with the channel swap done in the last kernel, or as
         NV12 video frames (B,3H/2,W), the form video decoders hand out and encoders take, converted on the GPU at both ends.
+        'rgba' / 'bgra' on either side: 4-byte uint8 pixels (B,H,W,4) with a straight alpha byte (screen capture, swap chains, PNG),
+        read and written like 'hwc' / 'hwc_bgr'.  The alpha never reaches the network: with RGBA / BGRA on both sides the output
+        alpha is the input alpha resampled bicubically to the output size (rounded to the nearest code), else it is 255; an
+        RGBA / BGRA input going to an output without alpha loses it.
         'p010' on either side: 10-bit P010 video frames (B,3H/2,W) uint16 (HEVC Main10, AV1, VP9 profile 2, HDR), code in the high
         10 bits of each word.  in_layout='p010' takes uint16 frames; out_layout='p010' returns uint16 frames for any frame input
         (uint8 in any layout, or P010), and a P010 input with any other out_layout returns uint8 frames.

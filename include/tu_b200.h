@@ -336,6 +336,12 @@ int tu_transformer_block(float *x, const TuBlockWeights *w, int M, int dim, int 
 /* all window-transformer blocks of a bf16 WindowTransformer / FastTransformer in one fused kernel, in place on the fp32
  * window-ordered token stream (M, dim), M a multiple of 128 (`for block in self.window_blocks`, W:272-273, F:288-289) */
 int tu_window_stack(float *tokens, const TuModelWeights *w, int M, void *stream);
+/* the two fused kernels of one bf16 ResidualTransformer layer (`layer` of w->n_blocks), around its global attention (R:22-50):
+ * tu_resid_pre: LN1 + in_proj of the fp32 tokens (M, 128) -> bf16 q | k | v rows (M, 384) with q pre-scaled by head_dim^-0.5;
+ * tu_resid_post: tokens += out_proj(att), then tokens += fc2(GELU(fc1(LN2(tokens)))) in place, att (M, 128) bf16.
+ * Rows past M are neither read nor written. */
+int tu_resid_pre(const float *tokens, void *qkv, const TuModelWeights *w, int layer, int M, void *stream);
+int tu_resid_post(float *tokens, const void *att, const TuModelWeights *w, int layer, int M, void *stream);
 /* window attention alone: softmax(q k^T + rel_bias) v per 8x8 window and head (head_dim 16) on qkv rows (nWin*64, 3*dim) with q
  * pre-scaled; rel_bias dense (heads,64,64) fp32; out (nWin*64, dim).  WindowTransformer/model.py:104-127 between qkv and proj. */
 int tu_window_attention(const void *qkv, const float *rel_bias, void *out, int nWin, int dim, int heads, int dtype, void *stream);

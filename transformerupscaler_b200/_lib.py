@@ -118,6 +118,8 @@ SIGNATURES = {
     "tu_block_workspace_bytes_for": (sz, [i32, i32, i32, i32, i32]),
     "tu_transformer_block": (i32, [fp, C.POINTER(TuBlockWeights), i32, i32, i32, i32, i32, i32, vp, sz, vp]),
     "tu_window_stack": (i32, [fp, C.POINTER(TuModelWeights), i32, vp]),
+    "tu_resid_pre": (i32, [fp, vp, C.POINTER(TuModelWeights), i32, i32, vp]),
+    "tu_resid_post": (i32, [fp, vp, C.POINTER(TuModelWeights), i32, i32, vp]),
     "tu_global_attention_workspace_bytes": (sz, [i32, i32, i32]),
     "tu_global_attention": (i32, [vp, vp, i32, i32, i32, vp, sz, vp]),
     "tu_window_attention": (i32, [vp, fp, vp, i32, i32, i32, i32, vp]),

@@ -646,6 +646,27 @@ extern "C" int tu_window_stack(float *tokens, const TuModelWeights *w, int M, vo
     return rc;
 }
 
+extern "C" int tu_resid_pre(const float *tokens, void *qkv, const TuModelWeights *w, int layer, int M, void *stream) {
+    TU_CHECK_ARG(tokens && qkv && w && M > 0 && layer >= 0 && layer < w->n_blocks, "resid_pre: bad argument");
+    TU_CHECK_ARG(w->model == TU_MODEL_RESIDUAL && w->dim == 128 && w->stack_w && w->stack_p,
+                 "resid_pre: the model has no fused-layer weights (bf16 ResidualTransformer only)");
+    TU_CHECK_ARG(tc_enabled(), "resid_pre: tcgen05 kernels are unavailable or switched off");
+    int rc = tc_resid_pre(tokens, (bf16 *)qkv, M, layer, w->n_blocks, (const bf16 *)w->stack_w, w->stack_p, (cudaStream_t)stream);
+    TU_CHECK_ARG(rc != TU_TC_UNSUPPORTED, "resid_pre: unsupported alignment (16-byte aligned tokens and qkv) or switched off");
+    return rc;
+}
+
+extern "C" int tu_resid_post(float *tokens, const void *att, const TuModelWeights *w, int layer, int M, void *stream) {
+    TU_CHECK_ARG(tokens && att && w && M > 0 && layer >= 0 && layer < w->n_blocks, "resid_post: bad argument");
+    TU_CHECK_ARG(w->model == TU_MODEL_RESIDUAL && w->dim == 128 && w->stack_w && w->stack_p,
+                 "resid_post: the model has no fused-layer weights (bf16 ResidualTransformer only)");
+    TU_CHECK_ARG(tc_enabled(), "resid_post: tcgen05 kernels are unavailable or switched off");
+    int rc = tc_resid_post(tokens, nullptr, (const bf16 *)att, M, layer, w->n_blocks, (const bf16 *)w->stack_w, w->stack_p,
+                           (cudaStream_t)stream);
+    TU_CHECK_ARG(rc != TU_TC_UNSUPPORTED, "resid_post: unsupported alignment (16-byte aligned tokens and att) or switched off");
+    return rc;
+}
+
 extern "C" int tu_patch_embed(const void *feat, int dtype, const void *w, const float *b, const float *pos_embed,
                               float *tokens, int B, int H, int W, int Ht, int Wt, int dim, int window, int reflect,
                               void *stream) {

@@ -182,19 +182,29 @@ __device__ __forceinline__ int slab_chunk_off(int col, int i) { return (col >> 6
 // LayerNorm of this thread's 48 columns of row i (x already includes the folded offset) -> A32, swizzled
 __device__ __forceinline__ void layernorm_to_a32(f32x2 (&x)[24], const float *gam, const float *bet, float2 *stat, uint8_t *a32, int i,
                                                  int part) {
-    // one exchange: every thread publishes (sum, sum of squares) of its columns; var = E[x^2] - mean^2 in fp32
+    // one exchange: every thread publishes the mean and M2 = sum (x - mean)^2 of its own 48 columns (two passes over registers);
+    // Chan's combination M2 = sum M2_p + 48 sum (mean_p - mean)^2 keeps the variance exact for rows whose channels share an offset
+    // far above their spread, where E[x^2] - mean^2 in fp32 cancels away
     f32x2 s2 = ptx::pk2(0.f, 0.f), q2 = ptx::pk2(0.f, 0.f);
 #pragma unroll
-    for (int j = 0; j < 24; ++j) { s2 = ptx::add2(s2, x[j]); q2 = ptx::fma2(x[j], x[j], q2); }
+    for (int j = 0; j < 24; ++j) s2 = ptx::add2(s2, x[j]);
     float s_lo, s_hi, q_lo, q_hi;
     ptx::up2(s2, s_lo, s_hi);
+    const float pmean = (s_lo + s_hi) * (1.0f / 48);
+    const f32x2 npm = ptx::pk2(-pmean, -pmean);
+#pragma unroll
+    for (int j = 0; j < 24; ++j) {
+        const f32x2 d = ptx::add2(x[j], npm);
+        q2 = ptx::fma2(d, d, q2);
+    }
     ptx::up2(q2, q_lo, q_hi);
-    stat[i * 4 + part] = make_float2(s_lo + s_hi, q_lo + q_hi);
+    stat[i * 4 + part] = make_float2(pmean, q_lo + q_hi);
     asm volatile("bar.sync %0, 128;" ::"r"(2 + (i >> 5)) : "memory");      // only the four warps holding this row's quarters
     const float4 p01 = *reinterpret_cast<const float4 *>(stat + i * 4), p23 = *reinterpret_cast<const float4 *>(stat + i * 4 + 2);
-    const float mean = ((p01.x + p01.z) + (p23.x + p23.z)) * (1.0f / DIM);
-    const float ex2 = ((p01.y + p01.w) + (p23.y + p23.w)) * (1.0f / DIM);
-    const float rstd = rsqrtf(fmaxf(ex2 - mean * mean, 0.f) + 1e-5f);
+    const float mean = ((p01.x + p01.z) + (p23.x + p23.z)) * 0.25f;
+    const float d0 = p01.x - mean, d1 = p01.z - mean, d2 = p23.x - mean, d3 = p23.z - mean;
+    const float m2 = ((p01.y + p01.w) + (p23.y + p23.w)) + 48.0f * ((d0 * d0 + d1 * d1) + (d2 * d2 + d3 * d3));
+    const float rstd = rsqrtf(m2 * (1.0f / DIM) + 1e-5f);
     const f32x2 nmean = ptx::pk2(-mean, -mean), rs = ptx::pk2(rstd, rstd);
 #pragma unroll
     for (int ch = 0; ch < 6; ++ch) {

@@ -11,7 +11,7 @@
  *     synchronises the device, and enqueues all work on `stream` (a cudaStream_t passed as void*);
  *   - return value 0 = success, negative = error; tu_last_error() gives the message (thread-local);
  *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 and TU_F16 = 3 (both image input / output only), TU_U16 = 4 (P010
- *     frames only);
+ *     and yuv444p16 frames only);
  *   - activations inside the engine are NHWC (64 channels); images at the boundary are NCHW, like
  *     the reference's tensors.
  */
@@ -49,7 +49,7 @@ extern "C" {
  * TU_LAYOUT_HWC_BGR read and write them; the alpha bytes never reach the network.  A 4-byte output buffer must be 4-byte aligned.
  * The alpha byte of an output pixel is the input alpha resampled to the output size when the input is 4-byte too (tu_resample_alpha),
  * 255 otherwise; a 4-byte input going to an output without alpha loses its alpha.  TU_U8 only; never with colour bits.
- * The layout bits 8..11 are an enumeration: 0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 8 P010. */
+ * The layout bits 8..11 are an enumeration: 0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010. */
 #define TU_LAYOUT_RGBA 0x300
 #define TU_LAYOUT_BGRA 0x500
 #define TU_U8_RGBA (TU_U8 | TU_LAYOUT_RGBA)
@@ -77,6 +77,26 @@ extern "C" {
 #define TU_LAYOUT_P010 0x800
 #define TU_YUV_BT2020 0x4000        /* BT.2020 non-constant-luminance matrix (Kr, Kb = 0.2627, 0.0593); with TU_LAYOUT_P010 only */
 #define TU_U16_P010 (TU_U16 | TU_LAYOUT_P010)
+/* Planar YUV frames: three separate planes Y, U, V (FFmpeg's yuv420p / yuv444p / yuv444p16, NVDEC's YUV444 / YUV444_16Bit surfaces)
+ * for the image input and / or output of tu_forward / tu_forward_frames, and the code of tu_yuvp_to_rgb / tu_rgb_to_yuvp.
+ *   TU_U8 | TU_LAYOUT_YUV420P (I420): one uint8 buffer of 3HW/2 bytes per frame, (B, 3H/2, W) for a batch: the Y plane (H x W), then
+ *        the U plane (H/2 x W/2), then the V plane (H/2 x W/2), each row-major and contiguous.  H and W even; sited, filtered and
+ *        converted exactly as NV12 (the results are bitwise those of the NV12 frame with U and V interleaved).
+ *   TU_U8 | TU_LAYOUT_YUV444P: (B, 3, H, W) uint8, planes Y, U, V at full resolution; any H and W.
+ *   TU_U16 | TU_LAYOUT_YUV444P (yuv444p16): (B, 3, H, W) little-endian uint16 words with the 10-bit code in the HIGH 10 bits, as P010
+ *        (word >> 6 on read, code << 6 on write); any H and W.
+ * Colour bits: TU_YUV_BT601 and TU_YUV_FULL_RANGE on each; TU_YUV_BT2020 (not with TU_YUV_BT601) on yuv444p16 only.  8-bit frames
+ * convert through planar fp16 RGB, yuv444p16 through planar fp32 RGB.  4:4:4 has no chroma filter: each pixel is converted with its own
+ * (U, V), by NV12's / P010's formulas (u' = (U - mid) / cs, ...; Cb', Cr' from the pixel's own R, G, B).  Buffers and planes need the
+ * alignment of their accesses: 2 bytes for a yuv420p Y plane and its pitch (a pair of luma samples is one access), 2 bytes for every
+ * yuv444p16 plane and pitch; U / V planes of yuv420p and every yuv444p plane may sit at any address.  The 4:4:4 kernels move four
+ * samples per access where a row's four samples are 4-sample aligned (planes and pitches that are multiples of 4 samples, or dense
+ * frames) and single samples elsewhere. */
+#define TU_LAYOUT_YUV420P 0x600
+#define TU_LAYOUT_YUV444P 0x700
+#define TU_U8_YUV420P (TU_U8 | TU_LAYOUT_YUV420P)
+#define TU_U8_YUV444P (TU_U8 | TU_LAYOUT_YUV444P)
+#define TU_U16_YUV444P16 (TU_U16 | TU_LAYOUT_YUV444P)
 
 #define TU_OK 0
 #define TU_ERR_ARG (-1)      /* bad argument (shape / dtype / null pointer)              */
@@ -100,7 +120,7 @@ long long tu_launch_count(void);
  * events on the caller's stream (two event records per forward: cheap enough for the timed region); tu_profile_enable(2)
  * brackets EVERY kernel, tagged with the reference op it implements ("conv1", "conv2" (or "conv1_conv2" when fused), "downsample", "patch_embed",
  * "transformer_blocks", "patch_unembed", "decoder_conv1", "decoder_conv2", "bicubic_add_clamp", "up1", "up1_conv",
- * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
+ * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "yuv420p_to_rgb" / "rgb_to_yuv420p", "yuv444p_to_rgb" / "rgb_to_yuv444p", "yuv444p16_to_rgb" / "rgb_to_yuv444p16" at a planar YUV end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
  * calls in the library that wait on the device): collect sums the milliseconds and launches recorded under `name`
  * (NULL = all); report writes "name total_ms launches\n" lines into buf (returns the needed size when buf is NULL);
  * tu_profile_reset drops the records. */
@@ -230,6 +250,8 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      TU_U8 | TU_LAYOUT_RGBA / TU_LAYOUT_BGRA: (B,H,W,4) frames on either side; an input is read as the same pixels given as
  *      TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR.  With 4-byte frames on BOTH sides the output alpha is the input alpha resampled
  *      (tu_resample_alpha; the workspace of tu_forward_workspace_bytes_io then holds that (B, outH, outW) plane), else 255.
+ *      TU_U8 | TU_LAYOUT_YUV420P / TU_LAYOUT_YUV444P, TU_U16 | TU_LAYOUT_YUV444P (planar YUV, above): as NV12 (8-bit: planar fp16) and
+ *      P010 (16-bit: planar fp32) on either side; the workspace holds the planar RGB frame of each such side.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
@@ -248,13 +270,24 @@ typedef struct TuFramePlanes {
     long long y_pitch;
     long long uv_pitch;
 } TuFramePlanes;
+/* one planar YUV frame (yuv420p / yuv444p / yuv444p16 codes): three planes, each with its own row pitch in bytes, anywhere in device
+ * memory, as an FFmpeg AVFrame (data[0..2], linesize[0..2]) or an NVDEC 4:4:4 surface holds it.
+ *   y:    H rows of W samples;  u, v: H/2 rows of W/2 samples (yuv420p) or H rows of W samples (4:4:4);
+ *   *_pitch: bytes between rows, >= the row's samples.
+ * A YV12 surface (V plane before U) is this descriptor with u and v pointing at its U and V planes.  Alignment: see TU_LAYOUT_YUV420P
+ * above.  A write touches only the valid samples of each row.  The surfaces of one call must not overlap each other or the other side's
+ * buffers; the library does not check that. */
+typedef struct TuFramePlanes3 {
+    void *y, *u, *v;
+    long long y_pitch, u_pitch, v_pitch;
+} TuFramePlanes3;
 
 size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
 /* the same, sized from the packed weights actually used (non-default dim / heads / n_blocks; which fused kernels are packed) */
 size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
-/* the same for the image input / output codes of the call: equal to tu_forward_workspace_bytes_for for every code pair without
- * TU_LAYOUT_NV12 or TU_LAYOUT_P010, larger by the planar fp16 frames of the side(s) that are NV12 and the planar fp32 frames of the
- * side(s) that are P010, and by the (B, outH, outW) alpha plane when both sides are RGBA / BGRA (tu_forward needs it then); 0 for a
+/* the same for the image input / output codes of the call: equal to tu_forward_workspace_bytes_for for every code pair without a YUV
+ * side, larger by the planar fp16 frames of the side(s) that are NV12, yuv420p or yuv444p and the planar fp32 frames of the side(s)
+ * that are P010 or yuv444p16, and by the (B, outH, outW) alpha plane when both sides are RGBA / BGRA (tu_forward needs it then); 0 for a
  * bad code */
 size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale, int compute_dtype,
                                      int in_dtype, int out_dtype);
@@ -271,6 +304,14 @@ int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, 
 int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlanes *x_frames, int in_dtype, void *out,
                       const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
                       int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream);
+/* tu_forward_planes for every kind of YUV side: x_frames / out_frames is a HOST array of B descriptors whose element type the side's
+ * code chooses -- TuFramePlanes for NV12 / P010, TuFramePlanes3 for yuv420p / yuv444p / yuv444p16 -- and otherwise follows the rules of
+ * tu_forward_planes (exactly one of dense buffer and array per side, every descriptor checked before anything is enqueued, workspace of
+ * tu_forward_workspace_bytes_io, results bitwise those of the dense frames).  The two sides are independent: NV12 surfaces in and
+ * yuv444p surfaces out is one call.  tu_forward_planes(...) is this function. */
+int tu_forward_frames(const TuModelWeights *w, const void *x, const void *x_frames, int in_dtype, void *out, const void *out_frames,
+                      int out_dtype, int B, int H, int W, int outH, int outW, int scale, int compute_dtype, int clamp, void *workspace,
+                      size_t workspace_bytes, void *stream);
 
 /* ---- single ops (exported for the per-op parity tests and for composition) ---------------------- */
 /* conv1: 3->64 3x3 p1 + ReLU, NCHW in -> NHWC out.  w64 (optional, bf16 (64,64)) enables the tensor-core kernel
@@ -407,6 +448,13 @@ int tu_rgb_to_p010(const void *rgb_f32, void *p010, int code, int B, int H, int 
  * planar fp32 RGB (8-byte aligned); rgb is a dense (B, 3, H, W) buffer.  Same bits as the dense ops on the same frame contents. */
 int tu_yuv420_planes_to_rgb(const TuFramePlanes *frames, int code, void *rgb, int B, int H, int W, void *stream);
 int tu_rgb_to_yuv420_planes(const void *rgb, const TuFramePlanes *frames, int code, int B, int H, int W, void *stream);
+/* planar YUV frames <-> planar RGB (B, 3, H, W): fp16 RGB for TU_U8 | TU_LAYOUT_YUV420P / TU_LAYOUT_YUV444P codes, fp32 RGB for
+ * TU_U16 | TU_LAYOUT_YUV444P (colour bits as above; anything else, an odd H or W for yuv420p, or B > 65535: TU_ERR_ARG).  Exactly one of
+ * `dense` (the (B, 3H/2, W) or (B, 3, H, W) batch) and `frames` (a HOST array of B TuFramePlanes3, read during the call) is non-NULL.
+ * yuv420p gives the bits of tu_nv12_to_rgb / tu_rgb_to_nv12 on the same samples; 4:4:4 follows the same formulas per pixel without the
+ * chroma filter.  The RGB buffer is 4-byte aligned (yuv420p) or aligned to its element (4:4:4). */
+int tu_yuvp_to_rgb(const void *dense, const TuFramePlanes3 *frames, int code, void *rgb, int B, int H, int W, void *stream);
+int tu_rgb_to_yuvp(const void *rgb, void *dense, const TuFramePlanes3 *frames, int code, int B, int H, int W, void *stream);
 
 #ifdef __cplusplus
 }

@@ -21,6 +21,9 @@ TU_YUV_BT2020 = 0x4000                               # BT.2020 matrix: a colour 
 # OR-ed into TU_U8 for 4-byte pixels with a straight alpha byte, (B, H, W, 4): R G B A / B G R A.  The layout bits 8..11 are an
 # enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 8 P010): compare whole values, never single bits
 TU_LAYOUT_RGBA, TU_LAYOUT_BGRA = 0x300, 0x500
+# planar YUV, three planes Y, U, V: yuv420p (TU_U8, (B, 3H/2, W)), yuv444p (TU_U8, (B, 3, H, W)) and yuv444p16 (TU_U16 | TU_LAYOUT_YUV444P,
+# (B, 3, H, W) words with the code in the high 10 bits)
+TU_LAYOUT_YUV420P, TU_LAYOUT_YUV444P = 0x600, 0x700
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}
 
@@ -81,6 +84,12 @@ class TuFramePlanes(C.Structure):
     _fields_ = [("y", C.c_void_p), ("uv", C.c_void_p), ("y_pitch", C.c_longlong), ("uv_pitch", C.c_longlong)]
 
 
+class TuFramePlanes3(C.Structure):
+    """one planar YUV frame (yuv420p / yuv444p / yuv444p16) as three device planes with row pitches in bytes"""
+    _fields_ = [("y", C.c_void_p), ("u", C.c_void_p), ("v", C.c_void_p), ("y_pitch", C.c_longlong), ("u_pitch", C.c_longlong),
+                ("v_pitch", C.c_longlong)]
+
+
 # name -> (restype, argtypes); must list every symbol include/tu_b200.h declares
 SIGNATURES = {
     "tu_version": (i32, []),
@@ -102,6 +111,8 @@ SIGNATURES = {
     "tu_forward": (i32, [C.POINTER(TuModelWeights), vp, i32, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp, sz, vp]),
     "tu_forward_planes": (i32, [C.POINTER(TuModelWeights), vp, C.POINTER(TuFramePlanes), i32, vp, C.POINTER(TuFramePlanes), i32,
                                 i32, i32, i32, i32, i32, i32, i32, i32, vp, sz, vp]),
+    "tu_forward_frames": (i32, [C.POINTER(TuModelWeights), vp, vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp, sz,
+                                vp]),
     "tu_stem_conv": (i32, [vp, i32, fp, vp, fp, vp, i32, i32, i32, i32, vp]),
     "tu_conv3x3_c64": (i32, [vp, vp, fp, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp]),
     "tu_conv3x3_c64_to3": (i32, [vp, i32, fp, vp, fp, fp, i32, i32, i32, i32, vp]),
@@ -136,6 +147,8 @@ SIGNATURES = {
     "tu_rgb_to_p010": (i32, [vp, vp, i32, i32, i32, i32, vp]),
     "tu_yuv420_planes_to_rgb": (i32, [C.POINTER(TuFramePlanes), i32, vp, i32, i32, i32, vp]),
     "tu_rgb_to_yuv420_planes": (i32, [vp, C.POINTER(TuFramePlanes), i32, i32, i32, i32, vp]),
+    "tu_yuvp_to_rgb": (i32, [vp, C.POINTER(TuFramePlanes3), i32, vp, i32, i32, i32, vp]),
+    "tu_rgb_to_yuvp": (i32, [vp, vp, C.POINTER(TuFramePlanes3), i32, i32, i32, i32, vp]),
 }
 
 

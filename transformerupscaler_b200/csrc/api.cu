@@ -123,11 +123,18 @@ struct Arena {
 };
 
 static int scale_slot(int s) { return s == 2 ? 0 : s == 3 ? 1 : s == 4 ? 2 : s == 6 ? 3 : -1; }
+// profile names of the planar YUV conversions (static strings: the profiler keeps the pointer)
+static const char *yuvp_step(int code, bool to_rgb) {
+    if (dtype_is_yuv420p(code)) return to_rgb ? "yuv420p_to_rgb" : "rgb_to_yuv420p";
+    if (dtype_is_yuv444p(code)) return to_rgb ? "yuv444p_to_rgb" : "rgb_to_yuv444p";
+    return to_rgb ? "yuv444p16_to_rgb" : "rgb_to_yuv444p16";
+}
 
 // Runs (or, with a.dry, only sizes) one forward.  TI/TO are handled by dtype codes in the leaf launchers.
-// xf / of: the input / output frame surfaces of an NV12 / P010 side, or NULL for the dense buffer x / out.
+// xf / of: the input / output frame surfaces of a YUV side (TuFramePlanes for NV12 / P010, TuFramePlanes3 for planar YUV), or NULL for
+// the dense buffer x / out.
 template <typename T>
-static int forward_impl(const TuModelWeights *w, const void *x, const TuFramePlanes *xf, int in_dtype, void *out, const TuFramePlanes *of,
+static int forward_impl(const TuModelWeights *w, const void *x, const void *xf, int in_dtype, void *out, const void *of,
                         int out_dtype, int B, int H, int W, int outH, int outW, int scale, int clamp, Arena &a, cudaStream_t st) {
     const int dt = sizeof(T) == 2 ? TU_BF16 : TU_F32;
     const bool dry = a.dry;
@@ -166,23 +173,33 @@ static int forward_impl(const TuModelWeights *w, const void *x, const TuFramePla
     // included), and the final bicubic reads the same buffer
     if (dtype_is_nv12(in_dtype)) {
         f16 *rgb = (f16 *)a.get((size_t)B * 3 * H * W * sizeof(f16));
-        if (!dry) TU_STEP("nv12_to_rgb", xf ? tu_yuv420_planes_to_rgb(xf, in_dtype, rgb, B, H, W, stv) : tu_nv12_to_rgb(x, in_dtype, rgb, B, H, W, stv));
+        if (!dry) TU_STEP("nv12_to_rgb", xf ? tu_yuv420_planes_to_rgb((const TuFramePlanes *)xf, in_dtype, rgb, B, H, W, stv) : tu_nv12_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F16;
     } else if (dtype_is_p010(in_dtype)) {
         // P010 frames are converted to planar fp32 (fp16 cannot hold every 10-bit step exactly): the forward is then the fp32-input one
         float *rgb = (float *)a.get((size_t)B * 3 * H * W * sizeof(float));
-        if (!dry) TU_STEP("p010_to_rgb", xf ? tu_yuv420_planes_to_rgb(xf, in_dtype, rgb, B, H, W, stv) : tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
+        if (!dry) TU_STEP("p010_to_rgb", xf ? tu_yuv420_planes_to_rgb((const TuFramePlanes *)xf, in_dtype, rgb, B, H, W, stv) : tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F32;
+    } else if (dtype_is_yuvp(in_dtype)) {
+        // planar YUV: 8-bit frames as NV12 (planar fp16), yuv444p16 as P010 (planar fp32)
+        const bool w16 = dtype_base(in_dtype) == TU_U16;
+        void *rgb = a.get((size_t)B * 3 * H * W * (w16 ? sizeof(float) : sizeof(f16)));
+        if (!dry) TU_STEP(yuvp_step(in_dtype, true), tu_yuvp_to_rgb(xf ? nullptr : x, (const TuFramePlanes3 *)xf, in_dtype, rgb, B, H, W, stv));
+        x = rgb;
+        in_dtype = w16 ? TU_F32 : TU_F16;
     }
-    // NV12 / P010 output: the last image kernel writes planar fp16 / fp32 here, and tu_rgb_to_nv12 / tu_rgb_to_p010 writes `out` from it
-    const bool nv12_out = dtype_is_nv12(out_dtype), p010_out = dtype_is_p010(out_dtype);
-    void *img = nv12_out ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
-                : p010_out ? a.get((size_t)B * 3 * outH * outW * sizeof(float)) : out;
-    const int img_dtype = nv12_out ? TU_F16 : p010_out ? TU_F32 : out_dtype;
+    // YUV output: the last image kernel writes planar fp16 (NV12, yuv420p, yuv444p) / fp32 (P010, yuv444p16) here, and the conversion op
+    // writes `out` / `of` from it
+    const bool nv12_out = dtype_is_nv12(out_dtype), p010_out = dtype_is_p010(out_dtype), yuvp_out = dtype_is_yuvp(out_dtype);
+    const bool w16_out = p010_out || (yuvp_out && dtype_base(out_dtype) == TU_U16);
+    void *img = nv12_out || (yuvp_out && !w16_out) ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
+                : w16_out ? a.get((size_t)B * 3 * outH * outW * sizeof(float)) : out;
+    const int img_dtype = dtype_is_yuv(out_dtype) ? (w16_out ? TU_F32 : TU_F16) : out_dtype;
 #define TU_YUV_OUT()                                                                                                    \
-    if (of) TU_STEP(nv12_out ? "rgb_to_nv12" : "rgb_to_p010", tu_rgb_to_yuv420_planes(img, of, out_dtype, B, outH, outW, stv)); \
+    if (yuvp_out) TU_STEP(yuvp_step(out_dtype, false), tu_rgb_to_yuvp(img, of ? nullptr : out, (const TuFramePlanes3 *)of, out_dtype, B, outH, outW, stv)); \
+    else if (of) TU_STEP(nv12_out ? "rgb_to_nv12" : "rgb_to_p010", tu_rgb_to_yuv420_planes(img, (const TuFramePlanes *)of, out_dtype, B, outH, outW, stv)); \
     else if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv));                    \
     else if (p010_out) TU_STEP("rgb_to_p010", tu_rgb_to_p010(img, out, out_dtype, B, outH, outW, stv))
 
@@ -742,38 +759,45 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
 }
 
 // 4:2:0 codes: TU_U8 | TU_LAYOUT_NV12 [| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_P010 [| TU_YUV_BT601 or
-// TU_YUV_BT2020] [| TU_YUV_FULL_RANGE].  TU_U16 is a P010 word and nothing else.  Such frames have an even height and width.
+// TU_YUV_BT2020] [| TU_YUV_FULL_RANGE], and TU_U8 | TU_LAYOUT_YUV420P with NV12's colour bits.  Such frames have an even height and
+// width.  4:4:4 codes: TU_U8 | TU_LAYOUT_YUV444P with NV12's colour bits, TU_U16 | TU_LAYOUT_YUV444P with P010's; any size.  TU_U16
+// is a P010 or yuv444p16 word and nothing else.
 // 4-byte frames: exactly TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA.  Other codes have a layout nibble below 4 and no colour bit.
 static bool plain_code(int d) {
     const int nib = (d >> 8) & 0xF;
     return dtype_is_px4(d) || (!(d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE)) && nib < 4 && dtype_base(d) != TU_U16);
 }
 static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int outH, int outW) {
-    const bool in420 = dtype_is_yuv420(in_dtype), out420 = dtype_is_yuv420(out_dtype);
+    const bool inyuv = dtype_is_yuv(in_dtype), outyuv = dtype_is_yuv(out_dtype);
+    const bool in420 = dtype_is_yuv420(in_dtype) || dtype_is_yuv420p(in_dtype), out420 = dtype_is_yuv420(out_dtype) || dtype_is_yuv420p(out_dtype);
     for (int d : {in_dtype, out_dtype})
         TU_CHECK_ARG(dtype_is_px4(d) || !layout_is_px4((d >> 8) & 0xF),
                      "forward: TU_LAYOUT_RGBA / TU_LAYOUT_BGRA are for uint8 frames (TU_U8) only, without colour bits");
-    TU_CHECK_ARG(in420 || plain_code(in_dtype),
+    TU_CHECK_ARG(inyuv || plain_code(in_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
-                 "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (input)");
-    TU_CHECK_ARG(out420 || plain_code(out_dtype),
+                 "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (input); TU_LAYOUT_YUV420P is "
+                 "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only)");
+    TU_CHECK_ARG(outyuv || plain_code(out_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
-                 "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (output)");
+                 "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (output); TU_LAYOUT_YUV420P is "
+                 "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only)");
     TU_CHECK_ARG(!in420 || (H % 2 == 0 && W % 2 == 0),
-                 std::string("forward: ") + (dtype_is_p010(in_dtype) ? "P010" : "NV12") + " input frames need an even height and width");
+                 std::string("forward: ") + (dtype_is_p010(in_dtype) ? "P010" : dtype_is_nv12(in_dtype) ? "NV12" : "yuv420p") +
+                     " input frames need an even height and width");
     TU_CHECK_ARG(!out420 || (outH % 2 == 0 && outW % 2 == 0),
-                 std::string("forward: ") + (dtype_is_p010(out_dtype) ? "P010" : "NV12") + " output frames need an even height and width");
+                 std::string("forward: ") + (dtype_is_p010(out_dtype) ? "P010" : dtype_is_nv12(out_dtype) ? "NV12" : "yuv420p") +
+                     " output frames need an even height and width");
     return TU_OK;
 }
 
 extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, int H, int W, int outH, int outW, int scale,
                                                 int compute_dtype, int in_dtype, int out_dtype) {
     if (check_forward_args(w, B, H, W, outH, outW, compute_dtype) || check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW)) return 0;
-    // only the NV12 / P010 sides and a 4-byte pair of sides (its alpha plane) change the arena; every other code sizes exactly as
+    // only the YUV sides and a 4-byte pair of sides (its alpha plane) change the arena; every other code sizes exactly as
     // tu_forward_workspace_bytes_for
     const bool alpha_io = dtype_is_px4(in_dtype) && dtype_is_px4(out_dtype);
-    in_dtype = dtype_is_yuv420(in_dtype) || alpha_io ? in_dtype : TU_F32;
-    out_dtype = dtype_is_yuv420(out_dtype) || alpha_io ? out_dtype : TU_F32;
+    in_dtype = dtype_is_yuv(in_dtype) || alpha_io ? in_dtype : TU_F32;
+    out_dtype = dtype_is_yuv(out_dtype) || alpha_io ? out_dtype : TU_F32;
     Arena a{nullptr, 0, 0, true};
     int rc = compute_dtype == TU_F32
                  ? forward_impl<float>(w, nullptr, nullptr, in_dtype, nullptr, nullptr, out_dtype, B, H, W, outH, outW, scale, 1, a, 0)
@@ -781,8 +805,14 @@ extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, 
     return rc == TU_OK ? a.off : 0;
 }
 
-extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlanes *x_frames, int in_dtype, void *out,
-                                 const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
+// frame descriptors of one side: TuFramePlanes (NV12 / P010) or TuFramePlanes3 (planar YUV), by the side's code
+static int check_frames(const void *frames, int code, int B, int H, int W, const char *op) {
+    return dtype_is_yuvp(code) ? check_yuvp_frames((const TuFramePlanes3 *)frames, code, B, H, W, op)
+                               : check_yuv420_planes((const TuFramePlanes *)frames, code, B, H, W, op);
+}
+
+extern "C" int tu_forward_frames(const TuModelWeights *w, const void *x, const void *x_frames, int in_dtype, void *out,
+                                 const void *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
                                  int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream) {
     int rc = check_forward_args(w, B, H, W, outH, outW, compute_dtype);
     if (rc) return rc;
@@ -790,15 +820,17 @@ extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const T
     TU_CHECK_ARG(!(x && x_frames), "forward: give the input as either x or x_frames, not both");
     TU_CHECK_ARG(!(out && out_frames), "forward: give the output as either out or out_frames, not both");
     if ((rc = check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
-    TU_CHECK_ARG(!x_frames || dtype_is_yuv420(in_dtype), "forward: x_frames (frame planes) are for NV12 / P010 input only");
-    TU_CHECK_ARG(!out_frames || dtype_is_yuv420(out_dtype), "forward: out_frames (frame planes) are for NV12 / P010 output only");
+    TU_CHECK_ARG(!x_frames || dtype_is_yuv(in_dtype),
+                 "forward: x_frames (frame planes) are for NV12 / P010 input only (TuFramePlanes), or planar YUV input (TuFramePlanes3)");
+    TU_CHECK_ARG(!out_frames || dtype_is_yuv(out_dtype),
+                 "forward: out_frames (frame planes) are for NV12 / P010 output only (TuFramePlanes), or planar YUV output (TuFramePlanes3)");
     // every descriptor is checked here, before the first kernel of the forward is enqueued
-    if (x_frames && (rc = check_yuv420_planes(x_frames, in_dtype, B, H, W, "forward: x_frames"))) return rc;
-    if (out_frames && (rc = check_yuv420_planes(out_frames, out_dtype, B, outH, outW, "forward: out_frames"))) return rc;
+    if (x_frames && (rc = check_frames(x_frames, in_dtype, B, H, W, "forward: x_frames"))) return rc;
+    if (out_frames && (rc = check_frames(out_frames, out_dtype, B, outH, outW, "forward: out_frames"))) return rc;
     {
         const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype);
-        const int il = dtype_is_yuv420(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_yuv420(out_dtype) ? 0 : dtype_layout(out_dtype);
-        // (TU_U16 has passed check_yuv420_codes only as a P010 word)
+        const int il = dtype_is_yuv(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_yuv(out_dtype) ? 0 : dtype_layout(out_dtype);
+        // (TU_U16 has passed check_yuv420_codes only as a P010 or yuv444p16 word)
         TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8 || ib == TU_U16) &&
                          (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8 || ob == TU_U16),
                      "forward: bad i/o dtype");
@@ -822,6 +854,18 @@ extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const T
     return compute_dtype == TU_F32
                ? forward_impl<float>(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, clamp, a, st)
                : forward_impl<bf16>(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, clamp, a, st);
+}
+
+extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlanes *x_frames, int in_dtype, void *out,
+                                 const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
+                                 int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream) {
+    // TuFramePlanes describe NV12 / P010 frames: tu_forward_frames would read them as TuFramePlanes3 on a planar YUV side
+    TU_CHECK_ARG(!x_frames || !dtype_is_yuvp(in_dtype), "forward_planes: x_frames are TuFramePlanes (NV12 / P010); planar YUV input "
+                                                        "takes TuFramePlanes3 (tu_forward_frames)");
+    TU_CHECK_ARG(!out_frames || !dtype_is_yuvp(out_dtype), "forward_planes: out_frames are TuFramePlanes (NV12 / P010); planar YUV "
+                                                           "output takes TuFramePlanes3 (tu_forward_frames)");
+    return tu_forward_frames(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, compute_dtype, clamp,
+                             workspace, workspace_bytes, stream);
 }
 
 extern "C" int tu_forward(const TuModelWeights *w, const void *x, int in_dtype, void *out, int out_dtype, int B, int H,

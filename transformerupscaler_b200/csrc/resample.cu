@@ -1208,6 +1208,7 @@ template <> struct Yuv420<uint16_t> {
 // Dense: one (B, 3H/2, W) buffer, row pitch W samples, the chroma plane right after the luma plane, frame b at b * 3HW/2.
 template <typename TS> struct Dense420 {
     typedef TS *__restrict__ Param;
+    typedef typename Yuv420<typename std::remove_const<TS>::type>::Pair P;
     TS *y, *uv;
     int W;
     static __device__ __forceinline__ Dense420 frame(Param p, int H, int W) {
@@ -1217,6 +1218,9 @@ template <typename TS> struct Dense420 {
     }
     __device__ __forceinline__ TS *yrow(int r) const { return y + (long)r * W; }
     __device__ __forceinline__ TS *uvrow(int r) const { return uv + (long)r * W; }
+    // the (U, V) pair of chroma sample (r, j): one access to the interleaved row
+    __device__ __forceinline__ P chroma(int r, int j) const { return *reinterpret_cast<const P *>(uvrow(r) + 2 * j); }
+    __device__ __forceinline__ void store_chroma(int r, int j, P c) const { *reinterpret_cast<P *>(uvrow(r) + 2 * j) = c; }
 };
 // Surfaces: frame blockIdx.y of a table of up to kPlanesPerLaunch TuFramePlanes passed by value in the kernel parameters (no copy of
 // descriptors to the device, so a captured graph needs no host memory alive); a larger batch is several launches.  64 x 32 bytes keeps
@@ -1224,6 +1228,7 @@ template <typename TS> struct Dense420 {
 constexpr int kPlanesPerLaunch = 64;
 template <typename TS> struct Planes420 {
     struct Param { TuFramePlanes f[kPlanesPerLaunch]; };
+    typedef typename Yuv420<typename std::remove_const<TS>::type>::Pair P;
     TS *y, *uv;
     long long yp, uvp;
     static __device__ __forceinline__ Planes420 frame(const Param &p, int, int) {
@@ -1232,6 +1237,32 @@ template <typename TS> struct Planes420 {
     }
     __device__ __forceinline__ TS *yrow(int r) const { return (TS *)((char *)y + (long long)r * yp); }
     __device__ __forceinline__ TS *uvrow(int r) const { return (TS *)((char *)uv + (long long)r * uvp); }
+    __device__ __forceinline__ P chroma(int r, int j) const { return *reinterpret_cast<const P *>(uvrow(r) + 2 * j); }
+    __device__ __forceinline__ void store_chroma(int r, int j, P c) const { *reinterpret_cast<P *>(uvrow(r) + 2 * j) = c; }
+};
+// Planar (yuv420p): a table of up to kPlanesPerLaunch TuFramePlanes3 in the kernel parameters, like Planes420; the U and V samples of
+// chroma column j are one sample each of two planes whose rows hold W/2 samples.  A dense (B, 3H/2, W) batch is passed as the table
+// of its frames' planes (row pitches W, W/2, W/2), so this one policy serves dense frames and surfaces.  48-byte descriptors: 64 of
+// them (3,072 bytes) keep a launch's parameters at about 3.1 KB, under the classic 4 KB limit.
+struct Frames3 { TuFramePlanes3 f[kPlanesPerLaunch]; };
+template <typename TS> struct Planar420 {
+    typedef Frames3 Param;
+    typedef typename std::remove_const<TS>::type S;
+    typedef typename Yuv420<S>::Pair P;
+    TS *y, *u, *v;
+    long long yp, up, vp;
+    static __device__ __forceinline__ Planar420 frame(const Param &p, int, int) {
+        const TuFramePlanes3 &d = p.f[blockIdx.y];
+        return {(TS *)d.y, (TS *)d.u, (TS *)d.v, d.y_pitch, d.u_pitch, d.v_pitch};
+    }
+    __device__ __forceinline__ TS *yrow(int r) const { return (TS *)((char *)y + (long long)r * yp); }
+    __device__ __forceinline__ TS *urow(int r) const { return (TS *)((char *)u + (long long)r * up); }
+    __device__ __forceinline__ TS *vrow(int r) const { return (TS *)((char *)v + (long long)r * vp); }
+    __device__ __forceinline__ P chroma(int r, int j) const { return Yuv420<S>::pair(urow(r)[j], vrow(r)[j]); }
+    __device__ __forceinline__ void store_chroma(int r, int j, P c) const {
+        urow(r)[j] = c.x;
+        vrow(r)[j] = c.y;
+    }
 };
 
 __device__ __forceinline__ float clamp01(float v) { return fminf(fmaxf(v, 0.f), 1.f); }
@@ -1258,9 +1289,9 @@ __global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(typename A::Param in
     const long plane = (long)H * W;
     const A f = A::frame(in, H, W);
     const int im = max(i - 1, 0), ip = min(i + 1, Hc - 1), jp = min(j + 1, Wc - 1);
-    const P cm0 = *reinterpret_cast<const P *>(f.uvrow(im) + 2 * j), cm1 = *reinterpret_cast<const P *>(f.uvrow(im) + 2 * jp);
-    const P c00 = *reinterpret_cast<const P *>(f.uvrow(i) + 2 * j), c01 = *reinterpret_cast<const P *>(f.uvrow(i) + 2 * jp);
-    const P cp0 = *reinterpret_cast<const P *>(f.uvrow(ip) + 2 * j), cp1 = *reinterpret_cast<const P *>(f.uvrow(ip) + 2 * jp);
+    const P cm0 = f.chroma(im, j), cm1 = f.chroma(im, jp);
+    const P c00 = f.chroma(i, j), c01 = f.chroma(i, jp);
+    const P cp0 = f.chroma(ip, j), cp1 = f.chroma(ip, jp);
     // vertical sums (x4) of U and V for the top (2i) and bottom (2i+1) luma rows, at chroma columns j and j+1
     const int ut0 = (cm0.x >> s) + 3 * (c00.x >> s), ut1 = (cm1.x >> s) + 3 * (c01.x >> s);
     const int ub0 = 3 * (c00.x >> s) + (cp0.x >> s), ub1 = 3 * (c01.x >> s) + (cp1.x >> s);
@@ -1331,8 +1362,124 @@ __global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict
     const A f = A::frame(out, H, W);
     *reinterpret_cast<P *>(f.yrow(2 * i) + 2 * j) = F::pair(yq[0], yq[1]);
     *reinterpret_cast<P *>(f.yrow(2 * i + 1) + 2 * j) = F::pair(yq[2], yq[3]);
-    *reinterpret_cast<P *>(f.uvrow(i) + 2 * j) =
-        F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid)));
+    f.store_chroma(i, j, F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid))));
+}
+
+// ---- 4:4:4 planar frames (yuv444p / yuv444p16) <-> planar RGB ----------------------------------------------------------------------
+// The per-pixel operation sequence of the 4:2:0 kernels without the chroma filter: u' = (U - mid) / cs (the 4:2:0 kernel's
+// (8U * 0.125 - mid) / cs is the same value: 8U * 0.125 is exact), and Cb', Cr' from the pixel's own R, G, B instead of `bar`.
+// Frame blockIdx.z of a Frames3 table, row blockIdx.y of Hk rows of Wk samples: a frame whose planes are all dense (pitch = W
+// samples) is launched as one row of H * W samples, its RGB planes being dense too.  Each thread converts 4 consecutive samples of a
+// row, with one 4-sample access per plane where the row's 4 samples are aligned to it (every thread of a dense frame whose base
+// addresses are) and single-sample accesses elsewhere (row tails, odd pitches).
+constexpr int k444Threads = 128;
+template <int Bytes> struct QuadWord;            // four consecutive 1-, 2- or 4-byte elements as one access
+template <> struct QuadWord<1> { typedef uint32_t T; };
+template <> struct QuadWord<2> { typedef uint2 T; };
+template <> struct QuadWord<4> { typedef uint4 T; };
+template <typename T> __device__ __forceinline__ bool quad_aligned(const T *p) {
+    return (reinterpret_cast<uintptr_t>(p) & (4 * sizeof(T) - 1)) == 0;
+}
+// n (<= 4) elements at p; one access when vec (then n == 4)
+template <typename T> __device__ __forceinline__ void load_quad(const T *p, bool vec, int n, T (&v)[4]) {
+    if (vec) {
+        const typename QuadWord<sizeof(T)>::T w = *reinterpret_cast<const typename QuadWord<sizeof(T)>::T *>(p);
+        memcpy(v, &w, sizeof(w));
+    } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) v[q] = q < n ? p[q] : v[0];
+    }
+}
+template <typename T> __device__ __forceinline__ void store_quad(T *p, bool vec, int n, const T (&v)[4]) {
+    if (vec) {
+        typename QuadWord<sizeof(T)>::T w;
+        memcpy(&w, v, sizeof(w));
+        *reinterpret_cast<typename QuadWord<sizeof(T)>::T *>(p) = w;
+    } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+            if (q < n) p[q] = v[q];
+    }
+}
+
+template <typename TS, typename TR>
+__global__ void __launch_bounds__(k444Threads) yuv444_to_rgb_kernel(Frames3 in, TR *__restrict__ out, int Hk, int Wk, YuvCoef k) {
+    typedef Yuv420<TS> F;
+    constexpr int s = F::shift;
+    pdl_trigger();
+    pdl_wait();
+    const int c0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+    if (c0 >= Wk) return;
+    const int n = min(4, Wk - c0);
+    const TuFramePlanes3 &d = in.f[blockIdx.z];
+    const long long r = blockIdx.y;
+    const TS *py = (const TS *)((const char *)d.y + r * d.y_pitch) + c0;
+    const TS *pu = (const TS *)((const char *)d.u + r * d.u_pitch) + c0;
+    const TS *pv = (const TS *)((const char *)d.v + r * d.v_pitch) + c0;
+    const long plane = (long)Hk * Wk;
+    TR *o = out + (long)blockIdx.z * 3 * plane + r * Wk + c0;
+    const bool vs = n == 4 && quad_aligned(py) && quad_aligned(pu) && quad_aligned(pv);
+    const bool vr = n == 4 && quad_aligned(o) && (plane & 3) == 0;
+    TS ys[4], us[4], vs4[4];
+    load_quad(py, vs, n, ys);
+    load_quad(pu, vs, n, us);
+    load_quad(pv, vs, n, vs4);
+    float rq[4], gq[4], bq[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const float yn = __fdiv_rn(__fadd_rn((float)(ys[q] >> s), -k.yo), k.ys);
+        const float un = __fdiv_rn(__fadd_rn((float)(us[q] >> s), -F::mid), k.cs);
+        const float vn = __fdiv_rn(__fadd_rn((float)(vs4[q] >> s), -F::mid), k.cs);
+        rq[q] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_rv, vn)));
+        gq[q] = clamp01(__fadd_rn(__fadd_rn(yn, __fmul_rn(k.a_gu, un)), __fmul_rn(k.a_gv, vn)));
+        bq[q] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_bu, un)));
+    }
+    TR ro[4], go[4], bo[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        ro[q] = from_f<TR>(rq[q]);
+        go[q] = from_f<TR>(gq[q]);
+        bo[q] = from_f<TR>(bq[q]);
+    }
+    store_quad(o, vr, n, ro);
+    store_quad(o + plane, vr, n, go);
+    store_quad(o + 2 * plane, vr, n, bo);
+}
+
+template <typename TR, typename TS>
+__global__ void __launch_bounds__(k444Threads) rgb_to_yuv444_kernel(const TR *__restrict__ in, Frames3 out, int Hk, int Wk, YuvCoef k) {
+    typedef Yuv420<TS> F;
+    pdl_trigger();
+    pdl_wait();
+    const int c0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+    if (c0 >= Wk) return;
+    const int n = min(4, Wk - c0);
+    const TuFramePlanes3 &d = out.f[blockIdx.z];
+    const long long r = blockIdx.y;
+    TS *py = (TS *)((char *)d.y + r * d.y_pitch) + c0;
+    TS *pu = (TS *)((char *)d.u + r * d.u_pitch) + c0;
+    TS *pv = (TS *)((char *)d.v + r * d.v_pitch) + c0;
+    const long plane = (long)Hk * Wk;
+    const TR *src = in + (long)blockIdx.z * 3 * plane + r * Wk + c0;
+    const bool vs = n == 4 && quad_aligned(py) && quad_aligned(pu) && quad_aligned(pv);
+    const bool vr = n == 4 && quad_aligned(src) && (plane & 3) == 0;
+    TR px[3][4];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) load_quad(src + c * plane, vr, n, px[c]);
+    TS yq[4], uq[4], vq[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const float R = to_f(px[0][q]), G = to_f(px[1][q]), Bl = to_f(px[2][q]);
+        const float yl = __fadd_rn(__fadd_rn(__fmul_rn(k.kr, R), __fmul_rn(k.kg, G)), __fmul_rn(k.kb, Bl));
+        const float cb = __fadd_rn(__fadd_rn(__fmul_rn(k.cb_r, R), __fmul_rn(k.cb_g, G)), __fmul_rn(0.5f, Bl));
+        const float cr = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, R), __fmul_rn(k.cr_g, G)), __fmul_rn(k.cr_b, Bl));
+        yq[q] = yuv_code<TS>(__fadd_rn(__fmul_rn(k.ys, yl), k.yo));
+        uq[q] = yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid));
+        vq[q] = yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid));
+    }
+    store_quad(py, vs, n, yq);
+    store_quad(pu, vs, n, uq);
+    store_quad(pv, vs, n, vq);
 }
 
 }  // namespace tu
@@ -1776,4 +1923,117 @@ extern "C" int tu_rgb_to_yuv420_planes(const void *rgb, const TuFramePlanes *fra
     cudaStream_t st = (cudaStream_t)stream;
     return p010 ? launch_planes<uint16_t, float, false>(frames, code, (float *)rgb, B, H, W, st, "rgb_to_p010")
                 : launch_planes<uint8_t, f16, false>(frames, code, (f16 *)rgb, B, H, W, st, "rgb_to_nv12");
+}
+
+// ---- planar YUV frames (yuv420p / yuv444p / yuv444p16) ------------------------------------------------------------------------------
+static const char *yuvp_fmt(int code) { return dtype_is_yuv420p(code) ? "yuv420p" : dtype_is_yuv444p(code) ? "yuv444p" : "yuv444p16"; }
+
+// B frames of a planar YUV side: host-side checks of the code, the sizes and every descriptor, made before anything is enqueued
+int tu::check_yuvp_frames(const TuFramePlanes3 *frames, int code, int B, int H, int W, const char *op) {
+    TU_CHECK_ARG(frames && B > 0 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_yuvp(code), std::string(op) + ": TuFramePlanes3 frames are for planar YUV (TU_U8 | TU_LAYOUT_YUV420P, "
+                                                        "TU_U8 | TU_LAYOUT_YUV444P or TU_U16 | TU_LAYOUT_YUV444P [| colour bits]) only");
+    const bool p420 = dtype_is_yuv420p(code), w16 = dtype_base(code) == TU_U16;
+    const std::string fmt = yuvp_fmt(code);
+    TU_CHECK_ARG(!p420 || (H % 2 == 0 && W % 2 == 0), std::string(op) + ": " + fmt + " frames need an even height and width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    TU_CHECK_ARG(p420 || H <= 65535, std::string(op) + ": " + fmt + " frame surfaces have at most 65535 rows");
+    const long long s = w16 ? 2 : 1, yrow = W * s, crow = (p420 ? W / 2 : W) * s;
+    // a pair of luma samples is one access (yuv420p); a 16-bit sample is one word
+    const long long ya = p420 || w16 ? 2 : 1, ca = w16 ? 2 : 1;
+    for (int b = 0; b < B; ++b) {
+        const TuFramePlanes3 &d = frames[b];
+        const std::string at = std::string(op) + ": frame " + std::to_string(b) + ": ";
+        TU_CHECK_ARG(d.y, at + "y is NULL");
+        TU_CHECK_ARG(d.u, at + "u is NULL");
+        TU_CHECK_ARG(d.v, at + "v is NULL");
+        const struct { const char *name; long long pitch, row; } pitches[3] = {{"y_pitch", d.y_pitch, yrow}, {"u_pitch", d.u_pitch, crow},
+                                                                             {"v_pitch", d.v_pitch, crow}};
+        for (const auto &p : pitches)
+            TU_CHECK_ARG(p.pitch >= p.row, at + p.name + " " + std::to_string(p.pitch) + " is smaller than the row's " +
+                                               std::to_string(p.row / s) + " samples (" + std::to_string(p.row) + " bytes)");
+        TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.y) % ya == 0 && d.y_pitch % ya == 0,
+                     at + "y and y_pitch must be multiples of 2 bytes (" + fmt + ")");
+        TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.u) % ca == 0 && d.u_pitch % ca == 0,
+                     at + "u and u_pitch must be multiples of 2 bytes (" + fmt + ")");
+        TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.v) % ca == 0 && d.v_pitch % ca == 0,
+                     at + "v and v_pitch must be multiples of 2 bytes (" + fmt + ")");
+    }
+    return TU_OK;
+}
+
+static int check_yuvp_args(const void *dense, const TuFramePlanes3 *frames, int code, const void *rgb, int B, int H, int W, const char *op) {
+    TU_CHECK_ARG(rgb && B > 0 && B <= 65535 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_yuvp(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_YUV420P or TU_U8 | TU_LAYOUT_YUV444P "
+                                                        "[| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_YUV444P "
+                                                        "[| TU_YUV_BT601 or TU_YUV_BT2020] [| TU_YUV_FULL_RANGE]");
+    TU_CHECK_ARG(!dense != !frames, std::string(op) + ": give exactly one of the dense buffer and the frames array");
+    const bool p420 = dtype_is_yuv420p(code), w16 = dtype_base(code) == TU_U16;
+    const std::string fmt = yuvp_fmt(code);
+    TU_CHECK_ARG(!p420 || (H % 2 == 0 && W % 2 == 0), std::string(op) + ": " + fmt + " frames need an even height and width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    // yuv420p: pairs of luma samples and of fp16 RGB values are one access (as NV12); 4:4:4: one element
+    const uintptr_t ra = p420 ? 4 : w16 ? 4 : 2, fa = p420 || w16 ? 2 : 1;
+    TU_CHECK_ARG((reinterpret_cast<uintptr_t>(rgb) & (ra - 1)) == 0,
+                 std::string(op) + ": the " + (w16 ? "fp32" : "fp16") + " RGB buffer must be " + std::to_string(ra) + "-byte aligned");
+    TU_CHECK_ARG(!dense || (reinterpret_cast<uintptr_t>(dense) & (fa - 1)) == 0,
+                 std::string(op) + ": the dense " + fmt + " buffer must be " + std::to_string(fa) + "-byte aligned");
+    return frames ? check_yuvp_frames(frames, code, B, H, W, op) : TU_OK;
+}
+
+// one launch per kPlanesPerLaunch frames; a dense batch is passed as the table of its frames' planes.  The RGB side is the dense batch,
+// offset to the first frame of the launch
+template <typename TS, typename TR, bool ToRgb>
+static int launch_yuvp(const void *dense, const TuFramePlanes3 *frames, int code, TR *rgb, int B, int H, int W, cudaStream_t st) {
+    const bool p420 = dtype_is_yuv420p(code);
+    const long long s = sizeof(TS), plane = (long long)H * W, crow = p420 ? W / 2 : W, cplane = p420 ? plane / 4 : plane;
+    const YuvCoef k = yuv_coef(code);
+    const std::string what = ToRgb ? std::string(yuvp_fmt(code)) + "_to_rgb" : std::string("rgb_to_") + yuvp_fmt(code);
+    for (int b0 = 0; b0 < B; b0 += kPlanesPerLaunch) {
+        const int nb = std::min(kPlanesPerLaunch, B - b0);
+        Frames3 p = {};
+        bool packed = true;          // every plane of the launch is rows of exactly W samples (4:4:4: one row of H * W samples)
+        for (int b = 0; b < nb; ++b) {
+            if (frames) {
+                p.f[b] = frames[b0 + b];
+            } else {
+                char *f = (char *)dense + (long long)(b0 + b) * (plane + 2 * cplane) * s;
+                p.f[b] = {f, f + plane * s, f + (plane + cplane) * s, W * s, crow * s, crow * s};
+            }
+            packed &= p.f[b].y_pitch == W * s && p.f[b].u_pitch == crow * s && p.f[b].v_pitch == crow * s;
+        }
+        TR *r = rgb + (long long)b0 * 3 * plane;
+        if (p420) {
+            if constexpr (sizeof(TS) == 1) {
+                const dim3 grid((unsigned)ceil_div((int)(plane / 4), 256), nb);
+                if constexpr (ToRgb)
+                    launch_pdl(yuv420_to_rgb_kernel<TS, TR, Planar420<const TS>>, grid, dim3(256), 0, st, p, r, H, W, k);
+                else
+                    launch_pdl(rgb_to_yuv420_kernel<TR, TS, Planar420<TS>>, grid, dim3(256), 0, st, (const TR *)r, p, H, W, k);
+            }
+        } else {
+            const int Hk = packed ? 1 : H, Wk = packed ? H * W : W;
+            const dim3 grid((unsigned)ceil_div(ceil_div(Wk, 4), k444Threads), Hk, nb);
+            if constexpr (ToRgb)
+                launch_pdl(yuv444_to_rgb_kernel<TS, TR>, grid, dim3(k444Threads), 0, st, p, r, Hk, Wk, k);
+            else
+                launch_pdl(rgb_to_yuv444_kernel<TR, TS>, grid, dim3(k444Threads), 0, st, (const TR *)r, p, Hk, Wk, k);
+        }
+        TU_CHECK_LAUNCH(what.c_str());
+    }
+    return TU_OK;
+}
+
+extern "C" int tu_yuvp_to_rgb(const void *dense, const TuFramePlanes3 *frames, int code, void *rgb, int B, int H, int W, void *stream) {
+    if (int rc = check_yuvp_args(dense, frames, code, rgb, B, H, W, "yuvp_to_rgb")) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    return dtype_base(code) == TU_U16 ? launch_yuvp<uint16_t, float, true>(dense, frames, code, (float *)rgb, B, H, W, st)
+                                      : launch_yuvp<uint8_t, f16, true>(dense, frames, code, (f16 *)rgb, B, H, W, st);
+}
+
+extern "C" int tu_rgb_to_yuvp(const void *rgb, void *dense, const TuFramePlanes3 *frames, int code, int B, int H, int W, void *stream) {
+    if (int rc = check_yuvp_args(dense, frames, code, rgb, B, H, W, "rgb_to_yuvp")) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    return dtype_base(code) == TU_U16 ? launch_yuvp<uint16_t, float, false>(dense, frames, code, (float *)rgb, B, H, W, st)
+                                      : launch_yuvp<uint8_t, f16, false>(dense, frames, code, (f16 *)rgb, B, H, W, st);
 }

@@ -55,7 +55,13 @@ def _code(dt: torch.dtype) -> int:
 
 
 LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR, "nv12": _lib.TU_LAYOUT_NV12,
-           "p010": _lib.TU_LAYOUT_P010, "rgba": _lib.TU_LAYOUT_RGBA, "bgra": _lib.TU_LAYOUT_BGRA}
+           "p010": _lib.TU_LAYOUT_P010, "rgba": _lib.TU_LAYOUT_RGBA, "bgra": _lib.TU_LAYOUT_BGRA,
+           "yuv420p": _lib.TU_LAYOUT_YUV420P, "yuv444p": _lib.TU_LAYOUT_YUV444P, "yuv444p16": _lib.TU_LAYOUT_YUV444P}
+# planar YUV layouts (FFmpeg's pix_fmt names) -> frame dtype; yuv444p and yuv444p16 share the layout bits and differ in the dtype
+PLANAR = {"yuv420p": torch.uint8, "yuv444p": torch.uint8, "yuv444p16": torch.uint16}
+# every YUV layout, and the ones of 16-bit words (10-bit codes: the only ones BT.2020 is defined for)
+YUV_LAYOUTS = ("nv12", "p010", *PLANAR)
+YUV16_LAYOUTS = ("p010", "yuv444p16")
 # colour of NV12 and P010 frames: matrix and range
 YUV = {"bt709": 0, "bt601": _lib.TU_YUV_BT601, "bt709_full": _lib.TU_YUV_FULL_RANGE,
        "bt601_full": _lib.TU_YUV_BT601 | _lib.TU_YUV_FULL_RANGE}
@@ -65,7 +71,8 @@ YUV_P010 = {"bt2020": _lib.TU_YUV_BT2020, "bt2020_full": _lib.TU_YUV_BT2020 | _l
 
 def layout_code(name: str) -> int:
     if name not in LAYOUTS:
-        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr', 'rgba', 'bgra', 'nv12' or 'p010'")
+        raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr', 'rgba', 'bgra', 'nv12', 'p010', 'yuv420p', "
+                         "'yuv444p' or 'yuv444p16'")
     return LAYOUTS[name]
 
 
@@ -87,6 +94,20 @@ def _is_p010(code: int) -> bool:
     return code & 0xF00 == _lib.TU_LAYOUT_P010
 
 
+def _is_yuv420p(code: int) -> bool:
+    return code & 0xF00 == _lib.TU_LAYOUT_YUV420P
+
+
+def _is_yuv444p(code: int) -> bool:
+    """yuv444p (TU_U8) or yuv444p16 (TU_U16): (B, 3, H, W)"""
+    return code & 0xF00 == _lib.TU_LAYOUT_YUV444P
+
+
+def _is_yuvp(code: int) -> bool:
+    """planar YUV: frame surfaces are (y, u, v) triples"""
+    return _is_yuv420p(code) or _is_yuv444p(code)
+
+
 def _is_px4(code: int) -> bool:
     """RGBA / BGRA: 4-byte pixels (B, H, W, 4)"""
     return code & 0xF00 in (_lib.TU_LAYOUT_RGBA, _lib.TU_LAYOUT_BGRA)
@@ -94,9 +115,11 @@ def _is_px4(code: int) -> bool:
 
 def _image_shape(B: int, C_: int, h: int, w: int, code: int) -> Tuple[int, ...]:
     """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3), 4-byte pixels
-    (B,h,w,4) or NV12 / P010 (B,3h/2,w)"""
-    if _is_nv12(code) or _is_p010(code):
+    (B,h,w,4), NV12 / P010 / yuv420p (B,3h/2,w) or yuv444p / yuv444p16 (B,3,h,w)"""
+    if _is_nv12(code) or _is_p010(code) or _is_yuv420p(code):
         return (B, 3 * h // 2, w)
+    if _is_yuv444p(code):
+        return (B, 3, h, w)
     if _is_px4(code):
         return (B, h, w, 4)
     return (B, h, w, 3) if code & 0xF00 in (_lib.TU_LAYOUT_HWC, _lib.TU_LAYOUT_HWC_BGR) else (B, C_, h, w)
@@ -154,17 +177,74 @@ def plane_pairs(frames, fmt: str, what: str) -> Tuple[int, int, int]:
     return len(frames), hw[0], hw[1]
 
 
+def _yuv444_hw(x: torch.Tensor, fmt: str, dtype: torch.dtype) -> Tuple[int, int]:
+    """(H, W) of 4:4:4 planar frames (B, 3, H, W); raises ValueError for a shape or dtype that is not one"""
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != dtype:
+        raise ValueError(f"{fmt} frames must be {str(dtype)[6:]} of shape (B, 3, H, W), got {x.dtype} {tuple(x.shape)}")
+    return int(x.shape[2]), int(x.shape[3])
+
+
+def _yuvp_hw(x: torch.Tensor, fmt: str) -> Tuple[int, int]:
+    """(H, W) of dense planar YUV frames of layout name `fmt`"""
+    return _yuv420_hw(x, fmt, torch.uint8) if fmt == "yuv420p" else _yuv444_hw(x, fmt, PLANAR[fmt])
+
+
+def plane_triples(frames, fmt: str, what: str) -> Tuple[int, int, int]:
+    """(B, H, W) of planar YUV frames (fmt 'yuv420p' | 'yuv444p' | 'yuv444p16') given as a list / tuple of B (y, u, v) plane triples --
+    strided views of a decoder's surfaces or an FFmpeg frame's data[0..2]: y (H, W), u and v (H/2, W/2) for yuv420p or (H, W) for 4:4:4,
+    uint8 (uint16 for yuv444p16), unit stride along W, any row stride, all CUDA tensors on one device.  Raises ValueError for anything
+    else."""
+    dtype = PLANAR[fmt]
+    if not isinstance(frames, (list, tuple)) or not frames:
+        raise ValueError(f"{what}: {fmt} frame planes are a non-empty list of (y, u, v) tensor triples")
+    dev, hw = None, None
+    for b, tri in enumerate(frames):
+        if not isinstance(tri, (list, tuple)) or len(tri) != 3 or not all(isinstance(t, torch.Tensor) for t in tri):
+            raise ValueError(f"{what}[{b}] must be a (y, u, v) triple of tensors")
+        for name, t in zip(("y", "u", "v"), tri):
+            if t.dim() != 2 or t.dtype != dtype:
+                raise ValueError(f"{what}[{b}].{name}: {fmt} planes are 2-D {str(dtype)[6:]} tensors, got {t.dtype} {tuple(t.shape)}")
+            if t.stride(1) != 1 and t.shape[1] > 1:
+                raise ValueError(f"{what}[{b}].{name}: a plane needs unit stride along its rows, got strides {t.stride()}")
+            if not t.is_cuda or (dev is not None and t.device != dev):
+                raise ValueError(f"{what}[{b}].{name}: every plane must be a CUDA tensor on one device, got {t.device}")
+            dev = t.device
+        y, u, v = tri
+        H, W = int(y.shape[0]), int(y.shape[1])
+        if fmt == "yuv420p":
+            if H % 2 or W % 2 or tuple(u.shape) != (H // 2, W // 2) or tuple(v.shape) != (H // 2, W // 2):
+                raise ValueError(f"{what}[{b}]: yuv420p planes are y (H, W), u and v (H/2, W/2) with H and W even, got {tuple(y.shape)}, "
+                                 f"{tuple(u.shape)} and {tuple(v.shape)}")
+        elif tuple(u.shape) != (H, W) or tuple(v.shape) != (H, W):
+            raise ValueError(f"{what}[{b}]: {fmt} planes are y, u and v of one size (H, W), got {tuple(y.shape)}, {tuple(u.shape)} and "
+                             f"{tuple(v.shape)}")
+        if hw is not None and hw != (H, W):
+            raise ValueError(f"{what}[{b}]: every frame of a batch has the same size, got {(H, W)} after {hw}")
+        hw = (H, W)
+    return len(frames), hw[0], hw[1]
+
+
+def frame_planes(frames, layout: str, what: str) -> Tuple[int, int, int]:
+    """(B, H, W) of a list of frame planes of layout `layout`: (y, uv) pairs for 'nv12' / 'p010', (y, u, v) triples for planar YUV"""
+    if layout in PLANAR:
+        return plane_triples(frames, layout, what)
+    return plane_pairs(frames, layout.upper(), what)
+
+
 def _flat(frames) -> List[torch.Tensor]:
-    return [t for pair in frames for t in pair]
+    return [t for planes in frames for t in planes]
 
 
-def _descriptors(flat: Sequence[torch.Tensor]):
-    """TuFramePlanes array of the flattened planes [y0, uv0, y1, uv1, ...]; a plane of one row has no meaningful row stride"""
+def _descriptors(flat: Sequence[torch.Tensor], code: int = _lib.TU_U8 | _lib.TU_LAYOUT_NV12):
+    """descriptor array of the flattened planes of a side of code `code`: TuFramePlanes of [y0, uv0, y1, uv1, ...] (NV12 / P010) or
+    TuFramePlanes3 of [y0, u0, v0, y1, ...] (planar YUV); a plane of one row has no meaningful row stride"""
     def pitch(t):
         return (t.stride(0) if t.shape[0] > 1 else t.shape[1]) * t.element_size()
-    n = len(flat) // 2
-    return (_lib.TuFramePlanes * n)(*[_lib.TuFramePlanes(flat[2 * b].data_ptr(), flat[2 * b + 1].data_ptr(), pitch(flat[2 * b]),
-                                                          pitch(flat[2 * b + 1])) for b in range(n)])
+    k = 3 if _is_yuvp(code) else 2
+    S = _lib.TuFramePlanes3 if k == 3 else _lib.TuFramePlanes
+    n = len(flat) // k
+    return (S * n)(*[S(*[flat[k * b + i].data_ptr() for i in range(k)], *[pitch(flat[k * b + i]) for i in range(k)])
+                     for b in range(n)])
 
 
 def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: int, compute_bf16: bool,
@@ -176,6 +256,10 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
     _require_cuda(x)
     if _is_nv12(in_layout) or _is_p010(in_layout):
         H, W = _nv12_hw(x) if _is_nv12(in_layout) else _p010_hw(x)
+        x = x.contiguous()
+        B = x.shape[0]
+    elif _is_yuvp(in_layout):
+        H, W = _yuvp_hw(x, "yuv420p" if _is_yuv420p(in_layout) else "yuv444p16" if x.dtype == torch.uint16 else "yuv444p")
         x = x.contiguous()
         B = x.shape[0]
     elif in_layout:
@@ -191,9 +275,10 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
         B, _, H, W = x.shape
     cdt = _lib.TU_BF16 if compute_bf16 else _lib.TU_F32
     out_shape = _image_shape(B, 3, out_h, out_w, out_code)
-    if _is_p010(out_code) != ((out_code & 0xFF) == _lib.TU_U16):
+    u16_out = (out_code & 0xFF) == _lib.TU_U16
+    if not (_is_yuv444p(out_code) and u16_out) and _is_p010(out_code) != u16_out:
         raise RuntimeError("the P010 output layout is for uint16 frames, and uint16 output is P010 only")
-    if out_code >> 8 and not _is_p010(out_code) and (out_code & 0xFF) != _lib.TU_U8:
+    if out_code >> 8 and not _is_p010(out_code) and not u16_out and (out_code & 0xFF) != _lib.TU_U8:
         raise RuntimeError("interleaved and NV12 output layouts are for uint8 frames")
     out = torch.empty(out_shape, dtype=_TORCH_DT[out_code & 0xFF], device=x.device)
     in_code = _code(x.dtype) | in_layout
@@ -222,8 +307,9 @@ def _(x, handle, out_h, out_w, scale, compute_bf16, out_code, clamp, in_layout=0
 @torch.library.custom_op("tu::forward_planes", mutates_args=("out_planes",), device_types="cuda")
 def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], out_planes: List[torch.Tensor], handle: int, out_h: int,
                       out_w: int, scale: int, compute_bf16: bool, out_code: int, clamp: bool, in_layout: int) -> torch.Tensor:
-    """tu::forward with frame surfaces on an NV12 / P010 side: the input is x (dense) or x_planes ([y0, uv0, y1, uv1, ...]); the output
-    is written into out_planes (and an empty tensor returned), or returned as a new dense tensor when out_planes is empty"""
+    """tu::forward with frame surfaces on a YUV side: the input is x (dense) or x_planes ([y0, uv0, y1, uv1, ...] for NV12 / P010,
+    [y0, u0, v0, y1, ...] for planar YUV); the output is written into out_planes (flattened the same way by out_code; an empty tensor is
+    returned), or returned as a new dense tensor when out_planes is empty"""
     lib = _lib.load()
     pw = _REGISTRY.get(handle)
     if pw is None:
@@ -234,6 +320,9 @@ def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], o
         if _is_nv12(in_layout) or _is_p010(in_layout):
             H, W = _nv12_hw(x) if _is_nv12(in_layout) else _p010_hw(x)
             B = x.shape[0]
+        elif _is_yuvp(in_layout):
+            H, W = _yuvp_hw(x, "yuv420p" if _is_yuv420p(in_layout) else "yuv444p16" if x.dtype == torch.uint16 else "yuv444p")
+            B = x.shape[0]
         elif in_layout:
             B, H, W = x.shape[0], x.shape[1], x.shape[2]
         else:
@@ -241,7 +330,7 @@ def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], o
         x = x.contiguous()
         in_code = _code(x.dtype) | in_layout
     else:
-        B, (H, W) = len(x_planes) // 2, x_planes[0].shape
+        B, (H, W) = len(x_planes) // (3 if _is_yuvp(in_layout) else 2), x_planes[0].shape
         in_code = _code(x_planes[0].dtype) | in_layout
     cdt = _lib.TU_BF16 if compute_bf16 else _lib.TU_F32
     odt = _TORCH_DT[out_code & 0xFF]
@@ -250,10 +339,10 @@ def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], o
     if nbytes == 0:
         _lib.check(_lib.TU_ERR_SCALE if "was not built" in _lib.last_error() else _lib.TU_ERR_ARG)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=ref.device)
-    xd = _descriptors(x_planes) if x is None else None
-    od = _descriptors(out_planes) if out_planes else None
+    xd = _descriptors(x_planes, in_code) if x is None else None
+    od = _descriptors(out_planes, out_code) if out_planes else None
     with torch.cuda.device(ref.device):
-        rc = lib.tu_forward_planes(C.byref(pw.struct), x.data_ptr() if x is not None else None, xd, in_code,
+        rc = lib.tu_forward_frames(C.byref(pw.struct), x.data_ptr() if x is not None else None, xd, in_code,
                                    None if out_planes else out.data_ptr(), od, out_code, B, H, W, out_h, out_w, scale, cdt, int(clamp),
                                    ws.data_ptr(), nbytes, _stream())
     _lib.check(rc)
@@ -263,7 +352,7 @@ def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], o
 @tu_forward_planes.register_fake
 def _(x, x_planes, out_planes, handle, out_h, out_w, scale, compute_bf16, out_code, clamp, in_layout):
     ref = x if x is not None else x_planes[0]
-    B = x.shape[0] if x is not None else len(x_planes) // 2
+    B = x.shape[0] if x is not None else len(x_planes) // (3 if _is_yuvp(in_layout) else 2)
     return ref.new_empty((0,) if out_planes else _image_shape(B, 3, out_h, out_w, out_code), dtype=_TORCH_DT[out_code & 0xFF])
 
 
@@ -375,62 +464,123 @@ def _(x, planes, code):
     return None
 
 
+@torch.library.custom_op("tu::rgb_to_yuvp", mutates_args=(), device_types="cuda")
+def tu_rgb_to_yuvp(x: torch.Tensor, code: int) -> torch.Tensor:
+    """planar RGB (B,3,H,W) -> planar YUV frames: fp16 RGB -> yuv420p (B,3H/2,W) / yuv444p (B,3,H,W) uint8, fp32 RGB -> yuv444p16
+    (B,3,H,W) uint16; code = the frames' TU_U8 / TU_U16 | TU_LAYOUT_YUV420P / TU_LAYOUT_YUV444P | colour bits"""
+    lib = _lib.load()
+    _require_cuda(x)
+    w16 = (code & 0xFF) == _lib.TU_U16
+    want = torch.float32 if w16 else torch.float16
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != want:
+        raise RuntimeError(f"rgb_to_yuvp takes planar {str(want)[6:]} RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    out = torch.empty(_image_shape(B, 3, H, W, code), dtype=torch.uint16 if w16 else torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_yuvp(x.data_ptr(), out.data_ptr(), None, code, B, H, W, _stream()))
+    return out
+
+
+@tu_rgb_to_yuvp.register_fake
+def _(x, code):
+    w16 = (code & 0xFF) == _lib.TU_U16
+    return x.new_empty(_image_shape(x.shape[0], 3, x.shape[2], x.shape[3], code), dtype=torch.uint16 if w16 else torch.uint8)
+
+
+@torch.library.custom_op("tu::rgb_to_yuvp_planes", mutates_args=("planes",), device_types="cuda")
+def tu_rgb_to_yuvp_planes(x: torch.Tensor, planes: List[torch.Tensor], code: int) -> None:
+    """planar RGB (B,3,H,W) -> planar YUV frames (fp16 RGB for 8-bit codes, fp32 for yuv444p16) written into the surfaces
+    [y0, u0, v0, y1, ...]"""
+    lib = _lib.load()
+    _require_cuda(x)
+    want = torch.float32 if (code & 0xFF) == _lib.TU_U16 else torch.float16
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != want:
+        raise RuntimeError(f"rgb_to_yuvp_planes takes planar {str(want)[6:]} RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_yuvp(x.data_ptr(), None, _descriptors(planes, code), code, B, H, W, _stream()))
+
+
+@tu_rgb_to_yuvp_planes.register_fake
+def _(x, planes, code):
+    return None
+
+
 def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale_factor: Optional[int],
                 require_ratio: bool, compute_bf16: bool, out_dtype: torch.dtype, clamp: bool = True,
                 in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709", out=None):
     """Shape logic of the three reference forwards (W:237-238, F:245-248,323-327, R:121-122) around tu::forward.
-    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'rgba' | 'bgra' | 'nv12' | 'p010'): uint8 frames may be interleaved (B,H,W,3),
-    4-byte pixels with alpha (B,H,W,4) or NV12 (B,3H/2,W) on either side, and either side may be P010 (B,3H/2,W) uint16 frames; yuv
-    ('bt709' | 'bt601' | 'bt709_full' | 'bt601_full', and 'bt2020' | 'bt2020_full' for P010 only) is the colour of the NV12 / P010
-    side(s).  An RGBA / BGRA output carries the input alpha resampled to the output size (tu_resample_alpha) when the input is RGBA /
-    BGRA too, else alpha 255; an RGBA / BGRA input going to an output without alpha loses its alpha.
-    Frame surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs (see plane_pairs); with out_layout
-    'nv12' / 'p010', out= a list of B (y, uv) pairs receives the result and is returned."""
+    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'rgba' | 'bgra' | 'nv12' | 'p010' | 'yuv420p' | 'yuv444p' | 'yuv444p16'): uint8
+    frames may be interleaved (B,H,W,3), 4-byte pixels with alpha (B,H,W,4), NV12 or yuv420p (B,3H/2,W) or yuv444p (B,3,H,W) on either
+    side, and either side may be P010 (B,3H/2,W) or yuv444p16 (B,3,H,W) uint16 frames; yuv ('bt709' | 'bt601' | 'bt709_full' |
+    'bt601_full', and 'bt2020' | 'bt2020_full' with a 16-bit YUV side and no 8-bit one) is the colour of the YUV side(s).  An RGBA / BGRA
+    output carries the input alpha resampled to the output size (tu_resample_alpha) when the input is RGBA / BGRA too, else alpha 255; an
+    RGBA / BGRA input going to an output without alpha loses its alpha.
+    Frame surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs (see plane_pairs), with a planar YUV
+    in_layout a list of B (y, u, v) triples (see plane_triples); with a YUV out_layout, out= a list of B such pairs / triples receives the
+    result and is returned."""
     il, ol = layout_code(in_layout), layout_code(out_layout)
     nv12_in, nv12_out = in_layout == "nv12", out_layout == "nv12"
     p010_in, p010_out = in_layout == "p010", out_layout == "p010"
-    if yuv != "bt709" and not (nv12_in or nv12_out or p010_in or p010_out):
+    yuv_in, yuv_out = in_layout in YUV_LAYOUTS, out_layout in YUV_LAYOUTS
+    yuvp_in, yuvp_out = in_layout in PLANAR, out_layout in PLANAR
+    if yuv != "bt709" and not (yuv_in or yuv_out):
         raise ValueError(f"yuv={yuv!r} applies to NV12 / P010 frames only: pass in_layout / out_layout 'nv12' or 'p010'")
     yc = yuv_code(yuv)
-    if yuv in YUV_P010 and (nv12_in or nv12_out or not (p010_in or p010_out)):
-        raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a P010 side and no NV12 side")
+    if yuv in YUV_P010:
+        side16 = in_layout in YUV16_LAYOUTS or out_layout in YUV16_LAYOUTS
+        side8 = (yuv_in and in_layout not in YUV16_LAYOUTS) or (yuv_out and out_layout not in YUV16_LAYOUTS)
+        if (yuvp_in or yuvp_out) and (side8 or not side16):
+            raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a P010 or yuv444p16 side and no 8-bit YUV side "
+                             "(nv12, yuv420p, yuv444p)")
+        if nv12_in or nv12_out or not (p010_in or p010_out or yuvp_in or yuvp_out):
+            raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a P010 side and no NV12 side")
     if nv12_out and out_dtype != torch.uint8:
         raise ValueError("out_layout='nv12' writes uint8 frames")
     if p010_out and out_dtype != torch.uint16:
         raise ValueError("out_layout='p010' writes uint16 frames")
+    if yuvp_out and out_dtype != PLANAR[out_layout]:
+        raise ValueError(f"out_layout={out_layout!r} writes {str(PLANAR[out_layout])[6:]} frames")
     px4_in, px4_out = in_layout in ("rgba", "bgra"), out_layout in ("rgba", "bgra")
     if px4_out and out_dtype != torch.uint8:
         raise ValueError(f"out_layout={out_layout!r} writes uint8 frames")
     if px4_in and not (isinstance(x, torch.Tensor) and x.dim() == 4 and x.shape[3] == 4 and x.dtype == torch.uint8):
         got = f"{x.dtype} {tuple(x.shape)}" if isinstance(x, torch.Tensor) else type(x).__name__
         raise ValueError(f"in_layout={in_layout!r} takes uint8 frames of shape (B, H, W, 4), got {got}")
-    il |= yc if nv12_in or p010_in else 0
+    il |= yc if yuv_in else 0
     planes_in = isinstance(x, (list, tuple))
-    if planes_in and not (nv12_in or p010_in):
+    if planes_in and not yuv_in:
         raise ValueError("a list of (y, uv) frame planes is NV12 / P010 input: pass in_layout='nv12' or 'p010'")
-    if out is not None and not (nv12_out or p010_out):
+    if out is not None and not yuv_out:
         raise ValueError("out= takes NV12 / P010 frame planes: pass out_layout='nv12' or 'p010'")
     if planes_in:
-        B, H, W = plane_pairs(x, "NV12" if nv12_in else "P010", "frames")
+        B, H, W = frame_planes(x, in_layout, "frames")
     elif nv12_in:
         H, W = _nv12_hw(x)
     elif p010_in:
         H, W = _p010_hw(x)
+    elif yuvp_in:
+        H, W = _yuvp_hw(x, in_layout)
     else:
         H, W = (int(x.shape[1]), int(x.shape[2])) if il else (int(x.shape[2]), int(x.shape[3]))
     if upscale_factor is not None:
         res_out = (H * upscale_factor, W * upscale_factor)
     res_out = (int(res_out[0]), int(res_out[1]))
-    out_code = _code(out_dtype) | ol | (yc if nv12_out or p010_out else 0)
+    out_code = _code(out_dtype) | ol | (yc if yuv_out else 0)
 
     def even_out(oh, ow):
         if (nv12_out or p010_out) and (oh % 2 or ow % 2):
             raise ValueError(f"{'NV12' if nv12_out else 'P010'} output frames need an even height and width, got {oh}x{ow}")
+        if out_layout == "yuv420p" and (oh % 2 or ow % 2):
+            raise ValueError(f"yuv420p output frames need an even height and width, got {oh}x{ow}")
         if out is not None:
-            fmt = "NV12" if nv12_out else "P010"
+            fmt = out_layout if yuvp_out else "NV12" if nv12_out else "P010"
             if not isinstance(out, (list, tuple)) or len(out) != (len(x) if planes_in else x.shape[0]):
-                raise ValueError("out= must be a list of one (y, uv) plane pair per input frame")
-            n, h, w = plane_pairs(out, fmt, "out")
+                raise ValueError(f"out= must be a list of one {'(y, u, v) plane triple' if yuvp_out else '(y, uv) plane pair'} per input "
+                                 "frame")
+            n, h, w = frame_planes(out, out_layout, "out")
             dev = (x[0][0] if planes_in else x).device
             if (h, w) != (oh, ow) or out[0][0].device != dev:
                 raise ValueError(f"out= planes must be {fmt} frames of {oh}x{ow} on {dev}, got {h}x{w} on {out[0][0].device}")
@@ -459,18 +609,19 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
     even_out(*res_out)
     # Resize is the last op: the un-clamped full-size image stays in the compute dtype and the Resize kernel writes the requested
     # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store).  fp16 output keeps an fp32
-    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  NV12 output is the fp16 output converted,
-    # P010 output the fp32 output converted
-    mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) and not nv12_out else torch.float32)
+    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  An 8-bit YUV output (NV12, yuv420p, yuv444p) is
+    # the fp16 output converted, a 16-bit one (P010, yuv444p16) the fp32 output converted
+    yuv8_out = yuv_out and out_dtype == torch.uint8
+    mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) and not yuv8_out else torch.float32)
     full = forward(oh, ow, scale, mid_code, False)
-    if out is not None:
-        tu_rgb_to_yuv420_planes(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16 if nv12_out else _lib.TU_F32), _flat(out),
-                                out_code)
-        return out
-    if nv12_out:
-        return tu_rgb_to_nv12(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16), out_code)
-    if p010_out:
-        return tu_rgb_to_p010(tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F32), out_code)
+    if yuv_out:
+        rgb = tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16 if yuv8_out else _lib.TU_F32)
+        if out is not None:
+            (tu_rgb_to_yuvp_planes if yuvp_out else tu_rgb_to_yuv420_planes)(rgb, _flat(out), out_code)
+            return out
+        if yuvp_out:
+            return tu_rgb_to_yuvp(rgb, out_code)
+        return tu_rgb_to_nv12(rgb, out_code) if nv12_out else tu_rgb_to_p010(rgb, out_code)
     if px4_in and px4_out:
         # alpha is resampled straight from the input to the requested size, by the rule of every other output path
         return tu_resize_aa(full, res_out[0], res_out[1], clamp, out_code, tu_resample_alpha(x, _lib.TU_U8 | il, res_out[0], res_out[1]))

@@ -165,11 +165,15 @@ class EngineModel(nn.Module):
         Decoder / encoder surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs -- y (H, W), uv (H/2, W),
         uint8 (NV12) or uint16 (P010), unit stride along W and any row stride (strided views of a pitched surface pool) -- and with
         out_layout 'nv12' / 'p010', out= a list of B such pairs of the output size receives the result and is returned.  Each side is
-        independent of the other; pitch padding and the bytes around the planes are never written."""
+        independent of the other; pitch padding and the bytes around the planes are never written.
+        Planar YUV (FFmpeg's pix_fmt names) on either side: 'yuv420p' (I420) uint8 (B,3H/2,W) -- Y, then U and V of (H/2, W/2) --
+        converted exactly as NV12; 'yuv444p' uint8 and 'yuv444p16' uint16 (B,3,H,W) planes Y, U, V at full resolution, the 16-bit
+        words holding the code in the high 10 bits as P010 (in_layout='yuv444p16' takes uint16 frames; out_layout='yuv444p16' returns
+        uint16 frames for any frame input).  Their surfaces are lists of B (y, u, v) plane triples, in x and in out=."""
         if isinstance(x, (list, tuple)):
-            if in_layout not in ("nv12", "p010"):
+            if in_layout not in engine.YUV_LAYOUTS:
                 raise ValueError("a list of (y, uv) frame planes is NV12 / P010 input: pass in_layout='nv12' or 'p010'")
-            engine.plane_pairs(x, in_layout.upper(), "frames")
+            engine.frame_planes(x, in_layout, "frames")
             return self._forward(x, x[0][0], res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
         return self._forward(x, x, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
 
@@ -184,20 +188,22 @@ class EngineModel(nn.Module):
             raise RuntimeError("transformerupscaler_b200 is forward-only (no autograd): the input requires grad; call under torch.no_grad()")
         # uint8 frames in -> uint8 frames out (ToTensor scaling on read, (out*255).clamp(0,255).to(uint8) on write, fused into
         # the first and last kernels): the video-pipeline entry, an extension of the reference's float-only signature
-        # P010 frames are uint16; any other uint16 tensor is an image like any other and is read as float32
+        # P010 and yuv444p16 frames are uint16; any other uint16 tensor is an image like any other and is read as float32
         if in_layout == "p010" and x0.dtype != torch.uint16:
             raise ValueError(f"in_layout='p010' takes uint16 frames (B, 3H/2, W), got {x0.dtype}")
+        if in_layout == "yuv444p16" and x0.dtype != torch.uint16:
+            raise ValueError(f"in_layout='yuv444p16' takes uint16 frames (B, 3, H, W), got {x0.dtype}")
         frames_u8 = x0.dtype == torch.uint8
-        frames = frames_u8 or in_layout == "p010"
+        frames = frames_u8 or in_layout in engine.YUV16_LAYOUTS
         if x0.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8) and not frames:
             x = x0 = x.float()
         bf16, out_dt = self._select_precision(x0)
         if frames:
-            out_dt = torch.uint16 if out_layout == "p010" else torch.uint8
+            out_dt = torch.uint16 if out_layout in engine.YUV16_LAYOUTS else torch.uint8
         handle = self._packed(bf16, x0.device)
         if (in_layout != "chw" or out_layout != "chw") and not frames:
             raise ValueError("in_layout / out_layout other than 'chw' apply to uint8 / P010 frames only")
-        if out is not None and out_layout not in ("nv12", "p010"):
+        if out is not None and out_layout not in engine.YUV_LAYOUTS:
             raise ValueError("out= takes NV12 / P010 frame planes: pass out_layout='nv12' or 'p010'")
         y = engine.run_forward(handle, self.ENGINE_MODEL, x, res_out, upscale_factor, require_ratio, bf16, out_dt,
                                in_layout=in_layout, out_layout=out_layout, yuv=yuv, out=out)

@@ -10,8 +10,8 @@
  *   - the caller owns every buffer; the library never allocates or frees device memory, never
  *     synchronises the device, and enqueues all work on `stream` (a cudaStream_t passed as void*);
  *   - return value 0 = success, negative = error; tu_last_error() gives the message (thread-local);
- *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 and TU_F16 = 3 (both image input / output only), TU_U16 = 4 (P010
- *     and yuv444p16 frames only);
+ *   - dtype codes: TU_F32 = 0, TU_BF16 = 1, TU_U8 = 2 and TU_F16 = 3 (both image input / output only), TU_U16 = 4 (P010,
+ *     P210, yuv444p16 and the TU_YUV_LSB10 frames only);
  *   - activations inside the engine are NHWC (64 channels); images at the boundary are NCHW, like
  *     the reference's tensors.
  */
@@ -49,7 +49,8 @@ extern "C" {
  * TU_LAYOUT_HWC_BGR read and write them; the alpha bytes never reach the network.  A 4-byte output buffer must be 4-byte aligned.
  * The alpha byte of an output pixel is the input alpha resampled to the output size when the input is 4-byte too (tu_resample_alpha),
  * 255 otherwise; a 4-byte input going to an output without alpha loses its alpha.  TU_U8 only; never with colour bits.
- * The layout bits 8..11 are an enumeration: 0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010. */
+ * The layout bits 8..11 are an enumeration: 0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010, 9 YUV422P,
+ * 10 NV16. */
 #define TU_LAYOUT_RGBA 0x300
 #define TU_LAYOUT_BGRA 0x500
 #define TU_U8_RGBA (TU_U8 | TU_LAYOUT_RGBA)
@@ -97,6 +98,34 @@ extern "C" {
 #define TU_U8_YUV420P (TU_U8 | TU_LAYOUT_YUV420P)
 #define TU_U8_YUV444P (TU_U8 | TU_LAYOUT_YUV444P)
 #define TU_U16_YUV444P16 (TU_U16 | TU_LAYOUT_YUV444P)
+/* 4:2:2 frames (chroma at full height and half width, co-sited with the even luma columns of every row: MPEG-2 / H.264 4:2:2 siting)
+ * and LSB-aligned 10-bit planar frames, for the image input and / or output of tu_forward / tu_forward_frames:
+ *   TU_U8 | TU_LAYOUT_YUV422P (yuv422p, MJPEG's yuvj422p with full-range BT.601): (B, 2H, W) uint8: the Y plane (H x W), then the U and V
+ *        planes (H x W/2 each); surfaces are TuFramePlanes3.
+ *   TU_U8 | TU_LAYOUT_NV16 (nv16): (B, 2H, W) uint8: the Y plane, then H rows of W/2 interleaved (U, V) pairs; surfaces are TuFramePlanes.
+ *   TU_U16 | TU_LAYOUT_NV16 (p210, P216 holding 10-bit content): as nv16 with 16-bit words, the code in the HIGH 10 bits as P010.
+ *   TU_YUV_LSB10, OR-ed into TU_U16 with one of the planar layouts: FFmpeg's yuv420p10le ((B, 3H/2, W), as yuv420p), yuv422p10le
+ *        ((B, 2H, W), as yuv422p) and yuv444p10le ((B, 3, H, W), as yuv444p16): the 10-bit code in the LOW 10 bits of each little-endian
+ *        word.  A word above 1023 reads as 1023 (a stray high bit saturates); a write stores the code with the top 6 bits zero.  Valid
+ *        with TU_U16 and TU_LAYOUT_YUV420P / TU_LAYOUT_YUV422P / TU_LAYOUT_YUV444P only.  TU_U16 | TU_LAYOUT_YUV420P and TU_U16 |
+ *        TU_LAYOUT_YUV422P without it are TU_ERR_ARG; TU_U16 | TU_LAYOUT_YUV444P without it is yuv444p16.
+ * Colour bits: 8-bit codes take NV12's, 16-bit codes P010's (TU_YUV_BT2020 allowed, never with TU_YUV_BT601) and its 10-bit offsets and
+ * scales.  8-bit frames convert through planar fp16 RGB, 16-bit frames through planar fp32 RGB.  4:2:2 needs an even W (any H), yuv420p10le
+ * an even H and W, yuv444p10le takes any size.  4:2:2 is converted with the NV12 formulas on one row instead of a row pair:
+ *   to RGB:  column 2j takes C[j], column 2j+1 (C[j] + C[j+1]) / 2 (j+1 clamped to W/2 - 1), then the NV12 per-pixel sequence;
+ *   to YUV:  Y' per pixel as NV12; per channel bar = ((P[2j-1] + 2 P[2j]) + P[2j+1]) * 0.25 (column 2j-1 clamped at 0), Cb', Cr' from
+ *            bar as NV12.  An image whose rows come in equal pairs gives chroma rows 2i and 2i+1 equal to NV12 chroma row i.
+ * Alignment: a pair of luma samples is one access, so the Y plane and its pitch of nv16 / yuv422p are 2-byte and of the 16-bit 4:2:0 /
+ * 4:2:2 codes 4-byte aligned; an nv16 / p210 (U, V) pair is one access too (2 / 4 bytes); every other 16-bit plane is 2-byte aligned. */
+#define TU_LAYOUT_YUV422P 0x900
+#define TU_LAYOUT_NV16 0xA00
+#define TU_YUV_LSB10 0x10000       /* bit 16 (bit 15, 0x8000, is a flag of no code) */
+#define TU_U8_YUV422P (TU_U8 | TU_LAYOUT_YUV422P)
+#define TU_U8_NV16 (TU_U8 | TU_LAYOUT_NV16)
+#define TU_U16_P210 (TU_U16 | TU_LAYOUT_NV16)
+#define TU_U16_YUV420P10 (TU_U16 | TU_LAYOUT_YUV420P | TU_YUV_LSB10)
+#define TU_U16_YUV422P10 (TU_U16 | TU_LAYOUT_YUV422P | TU_YUV_LSB10)
+#define TU_U16_YUV444P10 (TU_U16 | TU_LAYOUT_YUV444P | TU_YUV_LSB10)
 
 #define TU_OK 0
 #define TU_ERR_ARG (-1)      /* bad argument (shape / dtype / null pointer)              */
@@ -120,7 +149,7 @@ long long tu_launch_count(void);
  * events on the caller's stream (two event records per forward: cheap enough for the timed region); tu_profile_enable(2)
  * brackets EVERY kernel, tagged with the reference op it implements ("conv1", "conv2" (or "conv1_conv2" when fused), "downsample", "patch_embed",
  * "transformer_blocks", "patch_unembed", "decoder_conv1", "decoder_conv2", "bicubic_add_clamp", "up1", "up1_conv",
- * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "yuv420p_to_rgb" / "rgb_to_yuv420p", "yuv444p_to_rgb" / "rgb_to_yuv444p", "yuv444p16_to_rgb" / "rgb_to_yuv444p16" at a planar YUV end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
+ * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "yuv420p_to_rgb" / "rgb_to_yuv420p", "yuv444p_to_rgb" / "rgb_to_yuv444p", "yuv444p16_to_rgb" / "rgb_to_yuv444p16", "yuv420p10le_to_rgb" / "rgb_to_yuv420p10le", "yuv422p_to_rgb" / "rgb_to_yuv422p", "yuv422p10le_to_rgb" / "rgb_to_yuv422p10le", "yuv444p10le_to_rgb" / "rgb_to_yuv444p10le" at a planar YUV end, "nv16_to_rgb" / "rgb_to_nv16", "p210_to_rgb" / "rgb_to_p210" at a semi-planar 4:2:2 end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
  * calls in the library that wait on the device): collect sums the milliseconds and launches recorded under `name`
  * (NULL = all); report writes "name total_ms launches\n" lines into buf (returns the needed size when buf is NULL);
  * tu_profile_reset drops the records. */
@@ -251,7 +280,8 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      TU_LAYOUT_HWC / TU_LAYOUT_HWC_BGR.  With 4-byte frames on BOTH sides the output alpha is the input alpha resampled
  *      (tu_resample_alpha; the workspace of tu_forward_workspace_bytes_io then holds that (B, outH, outW) plane), else 255.
  *      TU_U8 | TU_LAYOUT_YUV420P / TU_LAYOUT_YUV444P, TU_U16 | TU_LAYOUT_YUV444P (planar YUV, above): as NV12 (8-bit: planar fp16) and
- *      P010 (16-bit: planar fp32) on either side; the workspace holds the planar RGB frame of each such side.
+ *      P010 (16-bit: planar fp32) on either side; the workspace holds the planar RGB frame of each such side.  The 4:2:2 codes
+ *      (TU_LAYOUT_YUV422P, TU_LAYOUT_NV16) and the TU_YUV_LSB10 codes (above) likewise.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
@@ -305,7 +335,8 @@ int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlane
                       const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
                       int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream);
 /* tu_forward_planes for every kind of YUV side: x_frames / out_frames is a HOST array of B descriptors whose element type the side's
- * code chooses -- TuFramePlanes for NV12 / P010, TuFramePlanes3 for yuv420p / yuv444p / yuv444p16 -- and otherwise follows the rules of
+ * code chooses -- TuFramePlanes for NV12 / P010 / NV16 / P210 (4:2:2: uv holds H rows), TuFramePlanes3 for the planar codes (yuv420p,
+ * yuv422p, yuv444p, yuv444p16 and the TU_YUV_LSB10 ones; 4:2:2: u and v hold H rows of W/2 samples) -- and otherwise follows the rules of
  * tu_forward_planes (exactly one of dense buffer and array per side, every descriptor checked before anything is enqueued, workspace of
  * tu_forward_workspace_bytes_io, results bitwise those of the dense frames).  The two sides are independent: NV12 surfaces in and
  * yuv444p surfaces out is one call.  tu_forward_planes(...) is this function. */
@@ -455,6 +486,15 @@ int tu_rgb_to_yuv420_planes(const void *rgb, const TuFramePlanes *frames, int co
  * chroma filter.  The RGB buffer is 4-byte aligned (yuv420p) or aligned to its element (4:4:4). */
 int tu_yuvp_to_rgb(const void *dense, const TuFramePlanes3 *frames, int code, void *rgb, int B, int H, int W, void *stream);
 int tu_rgb_to_yuvp(const void *rgb, void *dense, const TuFramePlanes3 *frames, int code, int B, int H, int W, void *stream);
+/* The same two ops also take TU_U8 | TU_LAYOUT_YUV422P (fp16 RGB) and the TU_YUV_LSB10 codes (fp32 RGB): yuv420p10le gives the bits of
+ * P010 with every word shifted left by 6, yuv444p10le those of yuv444p16 likewise; yuv422p follows the 4:2:2 formulas above.  The RGB
+ * buffer is 4-byte (fp16) / 8-byte (fp32) aligned for 4:2:0 and 4:2:2, aligned to its element for 4:4:4.
+ * Semi-planar 4:2:2 frames <-> planar RGB (B, 3, H, W): code TU_U8 | TU_LAYOUT_NV16 with fp16 RGB (4-byte aligned), or TU_U16 |
+ * TU_LAYOUT_NV16 (p210) with fp32 RGB (8-byte aligned), colour bits as above (anything else, an odd W, or B > 65535: TU_ERR_ARG).  Exactly
+ * one of `dense` (the (B, 2H, W) batch) and `frames` (a HOST array of B TuFramePlanes whose uv planes hold H rows, read during the call)
+ * is non-NULL.  yuv422p gives the bits of nv16 on the same samples. */
+int tu_yuv422sp_to_rgb(const void *dense, const TuFramePlanes *frames, int code, void *rgb, int B, int H, int W, void *stream);
+int tu_rgb_to_yuv422sp(const void *rgb, void *dense, const TuFramePlanes *frames, int code, int B, int H, int W, void *stream);
 
 #ifdef __cplusplus
 }

@@ -15,7 +15,7 @@ TU_F32, TU_BF16, TU_U8, TU_F16 = 0, 1, 2, 3      # TU_U8 and TU_F16: image input
 TU_LAYOUT_HWC, TU_LAYOUT_HWC_BGR = 0x100, 0x200      # OR-ed into TU_U8 for interleaved uint8 frames
 TU_LAYOUT_NV12 = 0x400                               # OR-ed into TU_U8 for NV12 (4:2:0) video frames, (B, 3H/2, W)
 TU_YUV_BT601, TU_YUV_FULL_RANGE = 0x1000, 0x2000     # colour bits of an NV12 code; neither = BT.709 limited range
-TU_U16 = 4                                           # 16-bit frame words: valid only as TU_U16 | TU_LAYOUT_P010
+TU_U16 = 4                                           # 16-bit frame words: valid only with a 16-bit YUV layout (P010, ...)
 TU_LAYOUT_P010 = 0x800                               # OR-ed into TU_U16 for P010 (10-bit 4:2:0) video frames, (B, 3H/2, W)
 TU_YUV_BT2020 = 0x4000                               # BT.2020 matrix: a colour bit of P010 codes only (not with TU_YUV_BT601)
 # OR-ed into TU_U8 for 4-byte pixels with a straight alpha byte, (B, H, W, 4): R G B A / B G R A.  The layout bits 8..11 are an
@@ -24,6 +24,9 @@ TU_LAYOUT_RGBA, TU_LAYOUT_BGRA = 0x300, 0x500
 # planar YUV, three planes Y, U, V: yuv420p (TU_U8, (B, 3H/2, W)), yuv444p (TU_U8, (B, 3, H, W)) and yuv444p16 (TU_U16 | TU_LAYOUT_YUV444P,
 # (B, 3, H, W) words with the code in the high 10 bits)
 TU_LAYOUT_YUV420P, TU_LAYOUT_YUV444P = 0x600, 0x700
+# 4:2:2: yuv422p (TU_U8, three planes, (B, 2H, W)) and NV16 (TU_U8) / P210 (TU_U16, code in the high 10 bits): Y then interleaved (U, V) rows
+TU_LAYOUT_YUV422P, TU_LAYOUT_NV16 = 0x900, 0xA00
+TU_YUV_LSB10 = 0x10000                               # with TU_U16 and a planar layout: yuv420p10le / yuv422p10le / yuv444p10le
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}
 
@@ -149,6 +152,8 @@ SIGNATURES = {
     "tu_rgb_to_yuv420_planes": (i32, [vp, C.POINTER(TuFramePlanes), i32, i32, i32, i32, vp]),
     "tu_yuvp_to_rgb": (i32, [vp, C.POINTER(TuFramePlanes3), i32, vp, i32, i32, i32, vp]),
     "tu_rgb_to_yuvp": (i32, [vp, vp, C.POINTER(TuFramePlanes3), i32, i32, i32, i32, vp]),
+    "tu_yuv422sp_to_rgb": (i32, [vp, C.POINTER(TuFramePlanes), i32, vp, i32, i32, i32, vp]),
+    "tu_rgb_to_yuv422sp": (i32, [vp, vp, C.POINTER(TuFramePlanes), i32, i32, i32, i32, vp]),
 }
 
 

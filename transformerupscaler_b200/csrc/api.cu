@@ -127,12 +127,21 @@ static int scale_slot(int s) { return s == 2 ? 0 : s == 3 ? 1 : s == 4 ? 2 : s =
 static const char *yuvp_step(int code, bool to_rgb) {
     if (dtype_is_yuv420p(code)) return to_rgb ? "yuv420p_to_rgb" : "rgb_to_yuv420p";
     if (dtype_is_yuv444p(code)) return to_rgb ? "yuv444p_to_rgb" : "rgb_to_yuv444p";
+    if (dtype_is_yuv422p(code)) return to_rgb ? "yuv422p_to_rgb" : "rgb_to_yuv422p";
+    if (dtype_is_yuv420p10(code)) return to_rgb ? "yuv420p10le_to_rgb" : "rgb_to_yuv420p10le";
+    if (dtype_is_yuv422p10(code)) return to_rgb ? "yuv422p10le_to_rgb" : "rgb_to_yuv422p10le";
+    if (dtype_is_yuv444p10(code)) return to_rgb ? "yuv444p10le_to_rgb" : "rgb_to_yuv444p10le";
     return to_rgb ? "yuv444p16_to_rgb" : "rgb_to_yuv444p16";
+}
+// and of the semi-planar 4:2:2 ones
+static const char *yuv422sp_step(int code, bool to_rgb) {
+    if (dtype_is_p210(code)) return to_rgb ? "p210_to_rgb" : "rgb_to_p210";
+    return to_rgb ? "nv16_to_rgb" : "rgb_to_nv16";
 }
 
 // Runs (or, with a.dry, only sizes) one forward.  TI/TO are handled by dtype codes in the leaf launchers.
-// xf / of: the input / output frame surfaces of a YUV side (TuFramePlanes for NV12 / P010, TuFramePlanes3 for planar YUV), or NULL for
-// the dense buffer x / out.
+// xf / of: the input / output frame surfaces of a YUV side (TuFramePlanes for NV12 / P010 / NV16 / P210, TuFramePlanes3 for planar YUV),
+// or NULL for the dense buffer x / out.
 template <typename T>
 static int forward_impl(const TuModelWeights *w, const void *x, const void *xf, int in_dtype, void *out, const void *of,
                         int out_dtype, int B, int H, int W, int outH, int outW, int scale, int clamp, Arena &a, cudaStream_t st) {
@@ -182,23 +191,28 @@ static int forward_impl(const TuModelWeights *w, const void *x, const void *xf, 
         if (!dry) TU_STEP("p010_to_rgb", xf ? tu_yuv420_planes_to_rgb((const TuFramePlanes *)xf, in_dtype, rgb, B, H, W, stv) : tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F32;
-    } else if (dtype_is_yuvp(in_dtype)) {
-        // planar YUV: 8-bit frames as NV12 (planar fp16), yuv444p16 as P010 (planar fp32)
+    } else if (dtype_is_yuvp(in_dtype) || dtype_is_yuv422sp(in_dtype)) {
+        // planar YUV and semi-planar 4:2:2: 8-bit frames as NV12 (planar fp16), 16-bit frames as P010 (planar fp32)
         const bool w16 = dtype_base(in_dtype) == TU_U16;
         void *rgb = a.get((size_t)B * 3 * H * W * (w16 ? sizeof(float) : sizeof(f16)));
-        if (!dry) TU_STEP(yuvp_step(in_dtype, true), tu_yuvp_to_rgb(xf ? nullptr : x, (const TuFramePlanes3 *)xf, in_dtype, rgb, B, H, W, stv));
+        if (!dry && dtype_is_yuvp(in_dtype))
+            TU_STEP(yuvp_step(in_dtype, true), tu_yuvp_to_rgb(xf ? nullptr : x, (const TuFramePlanes3 *)xf, in_dtype, rgb, B, H, W, stv));
+        else if (!dry)
+            TU_STEP(yuv422sp_step(in_dtype, true), tu_yuv422sp_to_rgb(xf ? nullptr : x, (const TuFramePlanes *)xf, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = w16 ? TU_F32 : TU_F16;
     }
-    // YUV output: the last image kernel writes planar fp16 (NV12, yuv420p, yuv444p) / fp32 (P010, yuv444p16) here, and the conversion op
-    // writes `out` / `of` from it
+    // YUV output: the last image kernel writes planar fp16 (8-bit codes) / fp32 (16-bit codes) here, and the conversion op writes `out` /
+    // `of` from it
     const bool nv12_out = dtype_is_nv12(out_dtype), p010_out = dtype_is_p010(out_dtype), yuvp_out = dtype_is_yuvp(out_dtype);
-    const bool w16_out = p010_out || (yuvp_out && dtype_base(out_dtype) == TU_U16);
-    void *img = nv12_out || (yuvp_out && !w16_out) ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
+    const bool sp422_out = dtype_is_yuv422sp(out_dtype);
+    const bool w16_out = p010_out || ((yuvp_out || sp422_out) && dtype_base(out_dtype) == TU_U16);
+    void *img = nv12_out || ((yuvp_out || sp422_out) && !w16_out) ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
                 : w16_out ? a.get((size_t)B * 3 * outH * outW * sizeof(float)) : out;
     const int img_dtype = dtype_is_yuv(out_dtype) ? (w16_out ? TU_F32 : TU_F16) : out_dtype;
 #define TU_YUV_OUT()                                                                                                    \
     if (yuvp_out) TU_STEP(yuvp_step(out_dtype, false), tu_rgb_to_yuvp(img, of ? nullptr : out, (const TuFramePlanes3 *)of, out_dtype, B, outH, outW, stv)); \
+    else if (sp422_out) TU_STEP(yuv422sp_step(out_dtype, false), tu_rgb_to_yuv422sp(img, of ? nullptr : out, (const TuFramePlanes *)of, out_dtype, B, outH, outW, stv)); \
     else if (of) TU_STEP(nv12_out ? "rgb_to_nv12" : "rgb_to_p010", tu_rgb_to_yuv420_planes(img, (const TuFramePlanes *)of, out_dtype, B, outH, outW, stv)); \
     else if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv));                    \
     else if (p010_out) TU_STEP("rgb_to_p010", tu_rgb_to_p010(img, out, out_dtype, B, outH, outW, stv))
@@ -763,30 +777,42 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
 // width.  4:4:4 codes: TU_U8 | TU_LAYOUT_YUV444P with NV12's colour bits, TU_U16 | TU_LAYOUT_YUV444P with P010's; any size.  TU_U16
 // is a P010 or yuv444p16 word and nothing else.
 // 4-byte frames: exactly TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA.  Other codes have a layout nibble below 4 and no colour bit.
+// 4:2:2 codes: TU_U8 | TU_LAYOUT_YUV422P / TU_LAYOUT_NV16 with NV12's colour bits, TU_U16 | TU_LAYOUT_NV16 with P010's; an even width.
+// TU_YUV_LSB10 goes with TU_U16 and a planar layout only (yuv420p10le: an even height and width, yuv422p10le: an even width).
 static bool plain_code(int d) {
     const int nib = (d >> 8) & 0xF;
-    return dtype_is_px4(d) || (!(d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE)) && nib < 4 && dtype_base(d) != TU_U16);
+    return dtype_is_px4(d) ||
+           (!(d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE | TU_YUV_LSB10)) && nib < 4 && dtype_base(d) != TU_U16);
 }
 static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int outH, int outW) {
     const bool inyuv = dtype_is_yuv(in_dtype), outyuv = dtype_is_yuv(out_dtype);
-    const bool in420 = dtype_is_yuv420(in_dtype) || dtype_is_yuv420p(in_dtype), out420 = dtype_is_yuv420(out_dtype) || dtype_is_yuv420p(out_dtype);
+    const bool in420 = dtype_is_yuv420(in_dtype) || dtype_is_yuv420p(in_dtype) || dtype_is_yuv420p10(in_dtype);
+    const bool out420 = dtype_is_yuv420(out_dtype) || dtype_is_yuv420p(out_dtype) || dtype_is_yuv420p10(out_dtype);
+    const bool in422 = dtype_is_yuv422p(in_dtype) || dtype_is_yuv422p10(in_dtype) || dtype_is_yuv422sp(in_dtype);
+    const bool out422 = dtype_is_yuv422p(out_dtype) || dtype_is_yuv422p10(out_dtype) || dtype_is_yuv422sp(out_dtype);
     for (int d : {in_dtype, out_dtype})
         TU_CHECK_ARG(dtype_is_px4(d) || !layout_is_px4((d >> 8) & 0xF),
                      "forward: TU_LAYOUT_RGBA / TU_LAYOUT_BGRA are for uint8 frames (TU_U8) only, without colour bits");
     TU_CHECK_ARG(inyuv || plain_code(in_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
                  "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (input); TU_LAYOUT_YUV420P is "
-                 "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only)");
+                 "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only); TU_LAYOUT_YUV422P "
+                 "is for uint8 frames, TU_LAYOUT_NV16 for uint8 frames or 16-bit words (P210), TU_YUV_LSB10 for 16-bit words of a planar "
+                 "layout only");
     TU_CHECK_ARG(outyuv || plain_code(out_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
                  "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (output); TU_LAYOUT_YUV420P is "
-                 "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only)");
+                 "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only); TU_LAYOUT_YUV422P "
+                 "is for uint8 frames, TU_LAYOUT_NV16 for uint8 frames or 16-bit words (P210), TU_YUV_LSB10 for 16-bit words of a planar "
+                 "layout only");
     TU_CHECK_ARG(!in420 || (H % 2 == 0 && W % 2 == 0),
-                 std::string("forward: ") + (dtype_is_p010(in_dtype) ? "P010" : dtype_is_nv12(in_dtype) ? "NV12" : "yuv420p") +
+                 std::string("forward: ") + (dtype_is_p010(in_dtype) ? "P010" : dtype_is_nv12(in_dtype) ? "NV12" : dtype_is_yuv420p(in_dtype) ? "yuv420p" : "yuv420p10le") +
                      " input frames need an even height and width");
+    TU_CHECK_ARG(!in422 || W % 2 == 0, "forward: 4:2:2 input frames need an even width");
     TU_CHECK_ARG(!out420 || (outH % 2 == 0 && outW % 2 == 0),
-                 std::string("forward: ") + (dtype_is_p010(out_dtype) ? "P010" : dtype_is_nv12(out_dtype) ? "NV12" : "yuv420p") +
+                 std::string("forward: ") + (dtype_is_p010(out_dtype) ? "P010" : dtype_is_nv12(out_dtype) ? "NV12" : dtype_is_yuv420p(out_dtype) ? "yuv420p" : "yuv420p10le") +
                      " output frames need an even height and width");
+    TU_CHECK_ARG(!out422 || outW % 2 == 0, "forward: 4:2:2 output frames need an even width");
     return TU_OK;
 }
 
@@ -805,10 +831,11 @@ extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, 
     return rc == TU_OK ? a.off : 0;
 }
 
-// frame descriptors of one side: TuFramePlanes (NV12 / P010) or TuFramePlanes3 (planar YUV), by the side's code
+// frame descriptors of one side: TuFramePlanes (NV12 / P010 / NV16 / P210) or TuFramePlanes3 (planar YUV), by the side's code
 static int check_frames(const void *frames, int code, int B, int H, int W, const char *op) {
-    return dtype_is_yuvp(code) ? check_yuvp_frames((const TuFramePlanes3 *)frames, code, B, H, W, op)
-                               : check_yuv420_planes((const TuFramePlanes *)frames, code, B, H, W, op);
+    if (dtype_is_yuvp(code)) return check_yuvp_frames((const TuFramePlanes3 *)frames, code, B, H, W, op);
+    if (dtype_is_yuv422sp(code)) return check_yuv422sp_frames((const TuFramePlanes *)frames, code, B, H, W, op);
+    return check_yuv420_planes((const TuFramePlanes *)frames, code, B, H, W, op);
 }
 
 extern "C" int tu_forward_frames(const TuModelWeights *w, const void *x, const void *x_frames, int in_dtype, void *out,
@@ -821,16 +848,16 @@ extern "C" int tu_forward_frames(const TuModelWeights *w, const void *x, const v
     TU_CHECK_ARG(!(out && out_frames), "forward: give the output as either out or out_frames, not both");
     if ((rc = check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
     TU_CHECK_ARG(!x_frames || dtype_is_yuv(in_dtype),
-                 "forward: x_frames (frame planes) are for NV12 / P010 input only (TuFramePlanes), or planar YUV input (TuFramePlanes3)");
+                 "forward: x_frames (frame planes) are for NV12 / P010 input only (TuFramePlanes, as are NV16 / P210), or planar YUV input (TuFramePlanes3)");
     TU_CHECK_ARG(!out_frames || dtype_is_yuv(out_dtype),
-                 "forward: out_frames (frame planes) are for NV12 / P010 output only (TuFramePlanes), or planar YUV output (TuFramePlanes3)");
+                 "forward: out_frames (frame planes) are for NV12 / P010 output only (TuFramePlanes, as are NV16 / P210), or planar YUV output (TuFramePlanes3)");
     // every descriptor is checked here, before the first kernel of the forward is enqueued
     if (x_frames && (rc = check_frames(x_frames, in_dtype, B, H, W, "forward: x_frames"))) return rc;
     if (out_frames && (rc = check_frames(out_frames, out_dtype, B, outH, outW, "forward: out_frames"))) return rc;
     {
         const int ib = dtype_base(in_dtype), ob = dtype_base(out_dtype);
         const int il = dtype_is_yuv(in_dtype) ? 0 : dtype_layout(in_dtype), ol = dtype_is_yuv(out_dtype) ? 0 : dtype_layout(out_dtype);
-        // (TU_U16 has passed check_yuv420_codes only as a P010 or yuv444p16 word)
+        // (TU_U16 has passed check_yuv420_codes only as the word of a YUV code)
         TU_CHECK_ARG((ib == TU_F32 || ib == TU_BF16 || ib == TU_F16 || ib == TU_U8 || ib == TU_U16) &&
                          (ob == TU_F32 || ob == TU_BF16 || ob == TU_F16 || ob == TU_U8 || ob == TU_U16),
                      "forward: bad i/o dtype");
@@ -859,7 +886,7 @@ extern "C" int tu_forward_frames(const TuModelWeights *w, const void *x, const v
 extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlanes *x_frames, int in_dtype, void *out,
                                  const TuFramePlanes *out_frames, int out_dtype, int B, int H, int W, int outH, int outW, int scale,
                                  int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream) {
-    // TuFramePlanes describe NV12 / P010 frames: tu_forward_frames would read them as TuFramePlanes3 on a planar YUV side
+    // TuFramePlanes describe NV12 / P010 / NV16 / P210 frames: tu_forward_frames would read them as TuFramePlanes3 on a planar YUV side
     TU_CHECK_ARG(!x_frames || !dtype_is_yuvp(in_dtype), "forward_planes: x_frames are TuFramePlanes (NV12 / P010); planar YUV input "
                                                         "takes TuFramePlanes3 (tu_forward_frames)");
     TU_CHECK_ARG(!out_frames || !dtype_is_yuvp(out_dtype), "forward_planes: out_frames are TuFramePlanes (NV12 / P010); planar YUV "

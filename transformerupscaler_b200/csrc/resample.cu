@@ -1187,19 +1187,34 @@ static YuvCoef yuv_coef(int code) {
     return k;
 }
 
-// sample formats: NV12 holds one 8-bit code per byte; P010 one 10-bit code in the high bits of a little-endian uint16 word (the low
-// 6 bits are ignored on read and zero on write).  A pair of samples (two luma, or U then V) is one 2-byte / 4-byte access.
+// Sample formats, the key of these traits: uint8_t is one 8-bit code per byte (NV12, NV16, yuv420p, yuv422p, yuv444p); uint16_t one
+// 10-bit code in the high bits of a little-endian word (P010, P210, yuv444p16: the low 6 bits are ignored on read and zero on write);
+// Lsb10 one 10-bit code in the low bits of a word (yuv4xxp10le: a word above 1023 reads as 1023, the top 6 bits are zero on write).
+// T is the storage type; a pair of samples (two luma, or U then V) is one 2-byte / 4-byte access.
+struct Lsb10;
 template <typename TS> struct Yuv420;
 template <> struct Yuv420<uint8_t> {
+    typedef uint8_t T;
     typedef uchar2 Pair;
     static constexpr int shift = 0;
     static constexpr float mid = 128.f, cmax = 255.f;
+    static __device__ __forceinline__ int code(T w) { return w; }
     static __device__ __forceinline__ Pair pair(uint8_t a, uint8_t b) { return make_uchar2(a, b); }
 };
 template <> struct Yuv420<uint16_t> {
+    typedef uint16_t T;
     typedef ushort2 Pair;
     static constexpr int shift = 6;
     static constexpr float mid = 512.f, cmax = 1023.f;
+    static __device__ __forceinline__ int code(T w) { return w >> shift; }
+    static __device__ __forceinline__ Pair pair(uint16_t a, uint16_t b) { return make_ushort2(a, b); }
+};
+template <> struct Yuv420<Lsb10> {
+    typedef uint16_t T;
+    typedef ushort2 Pair;
+    static constexpr int shift = 0;
+    static constexpr float mid = 512.f, cmax = 1023.f;
+    static __device__ __forceinline__ int code(T w) { return min((int)w, 1023); }
     static __device__ __forceinline__ Pair pair(uint16_t a, uint16_t b) { return make_ushort2(a, b); }
 };
 
@@ -1279,7 +1294,6 @@ template <typename TS, typename TR, typename A>
 __global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(typename A::Param in, TR *__restrict__ out, int H, int W, YuvCoef k) {
     typedef Yuv420<TS> F;
     typedef typename F::Pair P;
-    constexpr int s = F::shift;
     pdl_trigger();
     pdl_wait();
     const int Hc = H >> 1, Wc = W >> 1;
@@ -1293,14 +1307,14 @@ __global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(typename A::Param in
     const P c00 = f.chroma(i, j), c01 = f.chroma(i, jp);
     const P cp0 = f.chroma(ip, j), cp1 = f.chroma(ip, jp);
     // vertical sums (x4) of U and V for the top (2i) and bottom (2i+1) luma rows, at chroma columns j and j+1
-    const int ut0 = (cm0.x >> s) + 3 * (c00.x >> s), ut1 = (cm1.x >> s) + 3 * (c01.x >> s);
-    const int ub0 = 3 * (c00.x >> s) + (cp0.x >> s), ub1 = 3 * (c01.x >> s) + (cp1.x >> s);
-    const int vt0 = (cm0.y >> s) + 3 * (c00.y >> s), vt1 = (cm1.y >> s) + 3 * (c01.y >> s);
-    const int vb0 = 3 * (c00.y >> s) + (cp0.y >> s), vb1 = 3 * (c01.y >> s) + (cp1.y >> s);
+    const int ut0 = F::code(cm0.x) + 3 * F::code(c00.x), ut1 = F::code(cm1.x) + 3 * F::code(c01.x);
+    const int ub0 = 3 * F::code(c00.x) + F::code(cp0.x), ub1 = 3 * F::code(c01.x) + F::code(cp1.x);
+    const int vt0 = F::code(cm0.y) + 3 * F::code(c00.y), vt1 = F::code(cm1.y) + 3 * F::code(c01.y);
+    const int vb0 = 3 * F::code(c00.y) + F::code(cp0.y), vb1 = 3 * F::code(c01.y) + F::code(cp1.y);
     const int us[4] = {2 * ut0, ut0 + ut1, 2 * ub0, ub0 + ub1}, vs[4] = {2 * vt0, vt0 + vt1, 2 * vb0, vb0 + vb1};   // x8
     const P y0 = *reinterpret_cast<const P *>(f.yrow(2 * i) + 2 * j);
     const P y1 = *reinterpret_cast<const P *>(f.yrow(2 * i + 1) + 2 * j);
-    const int ys[4] = {y0.x >> s, y0.y >> s, y1.x >> s, y1.y >> s};
+    const int ys[4] = {F::code(y0.x), F::code(y0.y), F::code(y1.x), F::code(y1.y)};
     float r[4], g[4], bl[4];
 #pragma unroll
     for (int p = 0; p < 4; ++p) {
@@ -1321,8 +1335,8 @@ __global__ void __launch_bounds__(256) yuv420_to_rgb_kernel(typename A::Param in
 }
 
 template <typename TS>
-__device__ __forceinline__ TS yuv_code(float v) {         // min(max(floor(v + 0.5), 0), cmax), stored << shift
-    return (TS)((int)fminf(fmaxf(floorf(__fadd_rn(v, 0.5f)), 0.f), Yuv420<TS>::cmax) << Yuv420<TS>::shift);
+__device__ __forceinline__ typename Yuv420<TS>::T yuv_code(float v) {         // min(max(floor(v + 0.5), 0), cmax), stored << shift
+    return (typename Yuv420<TS>::T)((int)fminf(fmaxf(floorf(__fadd_rn(v, 0.5f)), 0.f), Yuv420<TS>::cmax) << Yuv420<TS>::shift);
 }
 
 // One thread per chroma sample (i, j): its (U, V) pair and its 2x2 luma block.  Chroma filter (type-0 siting): the column sums
@@ -1351,7 +1365,7 @@ __global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict
         px[c][0] = a.x; px[c][1] = a.y; px[c][2] = b.x; px[c][3] = b.y;
         bar[c] = __fmul_rn(__fadd_rn(__fadd_rn(v0, __fmul_rn(2.f, v1)), v2), 0.125f);
     }
-    TS yq[4];
+    typename F::T yq[4];
 #pragma unroll
     for (int p = 0; p < 4; ++p) {
         const float yl = __fadd_rn(__fadd_rn(__fmul_rn(k.kr, px[0][p]), __fmul_rn(k.kg, px[1][p])), __fmul_rn(k.kb, px[2][p]));
@@ -1362,6 +1376,82 @@ __global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict
     const A f = A::frame(out, H, W);
     *reinterpret_cast<P *>(f.yrow(2 * i) + 2 * j) = F::pair(yq[0], yq[1]);
     *reinterpret_cast<P *>(f.yrow(2 * i + 1) + 2 * j) = F::pair(yq[2], yq[3]);
+    f.store_chroma(i, j, F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid))));
+}
+
+// ---- 4:2:2 frames (NV16 / P210 semi-planar, yuv422p / yuv422p10le planar) <-> planar RGB --------------------------------------------
+// Chroma row r belongs to luma row r (co-sited with the even luma columns).  The addressing policies of the 4:2:0 kernels serve: Planes420
+// (a TuFramePlanes table; a dense (B, 2H, W) batch is passed as the table of its frames' planes) and Planar420 (a Frames3 table).  Only the
+// number of chroma rows differs, and the policies never see it.
+// One thread per chroma sample (i, j): luma row i, columns 2j, 2j+1.  Column 2j takes chroma column j, column 2j+1 the mean of j and j+1
+// (clamped): integer sums (at most 2 * 1023) times 1/2, exact in fp32; then the per-pixel sequence of yuv420_to_rgb_kernel.
+template <typename TS, typename TR, typename A>
+__global__ void __launch_bounds__(256) yuv422_to_rgb_kernel(typename A::Param in, TR *__restrict__ out, int H, int W, YuvCoef k) {
+    typedef Yuv420<TS> F;
+    typedef typename F::Pair P;
+    pdl_trigger();
+    pdl_wait();
+    const int Wc = W >> 1;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= H * Wc) return;
+    const int i = t / Wc, j = t - i * Wc;
+    const long plane = (long)H * W;
+    const A f = A::frame(in, H, W);
+    const P c0 = f.chroma(i, j), c1 = f.chroma(i, min(j + 1, Wc - 1));
+    const int u0 = F::code(c0.x), v0 = F::code(c0.y);
+    const int us[2] = {2 * u0, u0 + F::code(c1.x)}, vs[2] = {2 * v0, v0 + F::code(c1.y)};   // x2
+    const P y = *reinterpret_cast<const P *>(f.yrow(i) + 2 * j);
+    const int ys[2] = {F::code(y.x), F::code(y.y)};
+    float r[2], g[2], bl[2];
+#pragma unroll
+    for (int p = 0; p < 2; ++p) {
+        const float yn = __fdiv_rn(__fadd_rn((float)ys[p], -k.yo), k.ys);
+        const float un = __fdiv_rn(__fadd_rn(__fmul_rn((float)us[p], 0.5f), -F::mid), k.cs);
+        const float vn = __fdiv_rn(__fadd_rn(__fmul_rn((float)vs[p], 0.5f), -F::mid), k.cs);
+        r[p] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_rv, vn)));
+        g[p] = clamp01(__fadd_rn(__fadd_rn(yn, __fmul_rn(k.a_gu, un)), __fmul_rn(k.a_gv, vn)));
+        bl[p] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_bu, un)));
+    }
+    TR *o = out + (long)blockIdx.y * 3 * plane + (long)i * W + 2 * j;
+    store_rgb2(o, r[0], r[1]);
+    store_rgb2(o + plane, g[0], g[1]);
+    store_rgb2(o + 2 * plane, bl[0], bl[1]);
+}
+
+// One thread per chroma sample (i, j): its (U, V) pair and its luma pair.  Chroma filter: the 4:2:0 filter on one row instead of a row-pair
+// sum, bar = ((P[2j-1] + 2 P[2j]) + P[2j+1]) * 0.25 (column 2j-1 clamped at 0), per channel.  On rows that come in equal pairs the 4:2:0
+// sums are exactly twice these, and * 0.125 on them rounds as * 0.25 here: the chroma of both rows equals the 4:2:0 chroma row.
+template <typename TR, typename TS, typename A>
+__global__ void __launch_bounds__(256) rgb_to_yuv422_kernel(const TR *__restrict__ in, typename A::Param out, int H, int W, YuvCoef k) {
+    typedef Yuv420<TS> F;
+    typedef typename F::Pair P;
+    pdl_trigger();
+    pdl_wait();
+    const int Wc = W >> 1;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= H * Wc) return;
+    const int i = t / Wc, j = t - i * Wc;
+    const long plane = (long)H * W;
+    const TR *src = in + (long)blockIdx.y * 3 * plane + (long)i * W;
+    const int cl = max(2 * j - 1, 0);
+    float px[3][2], bar[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const TR *s = src + c * plane;
+        const float2 a = load_rgb2(s + 2 * j);
+        px[c][0] = a.x; px[c][1] = a.y;
+        bar[c] = __fmul_rn(__fadd_rn(__fadd_rn(to_f(s[cl]), __fmul_rn(2.f, a.x)), a.y), 0.25f);
+    }
+    typename F::T yq[2];
+#pragma unroll
+    for (int p = 0; p < 2; ++p) {
+        const float yl = __fadd_rn(__fadd_rn(__fmul_rn(k.kr, px[0][p]), __fmul_rn(k.kg, px[1][p])), __fmul_rn(k.kb, px[2][p]));
+        yq[p] = yuv_code<TS>(__fadd_rn(__fmul_rn(k.ys, yl), k.yo));
+    }
+    const float cb = __fadd_rn(__fadd_rn(__fmul_rn(k.cb_r, bar[0]), __fmul_rn(k.cb_g, bar[1])), __fmul_rn(0.5f, bar[2]));
+    const float cr = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, bar[0]), __fmul_rn(k.cr_g, bar[1])), __fmul_rn(k.cr_b, bar[2]));
+    const A f = A::frame(out, H, W);
+    *reinterpret_cast<P *>(f.yrow(i) + 2 * j) = F::pair(yq[0], yq[1]);
     f.store_chroma(i, j, F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid))));
 }
 
@@ -1405,7 +1495,7 @@ template <typename T> __device__ __forceinline__ void store_quad(T *p, bool vec,
 template <typename TS, typename TR>
 __global__ void __launch_bounds__(k444Threads) yuv444_to_rgb_kernel(Frames3 in, TR *__restrict__ out, int Hk, int Wk, YuvCoef k) {
     typedef Yuv420<TS> F;
-    constexpr int s = F::shift;
+    typedef typename F::T S;
     pdl_trigger();
     pdl_wait();
     const int c0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
@@ -1413,23 +1503,23 @@ __global__ void __launch_bounds__(k444Threads) yuv444_to_rgb_kernel(Frames3 in, 
     const int n = min(4, Wk - c0);
     const TuFramePlanes3 &d = in.f[blockIdx.z];
     const long long r = blockIdx.y;
-    const TS *py = (const TS *)((const char *)d.y + r * d.y_pitch) + c0;
-    const TS *pu = (const TS *)((const char *)d.u + r * d.u_pitch) + c0;
-    const TS *pv = (const TS *)((const char *)d.v + r * d.v_pitch) + c0;
+    const S *py = (const S *)((const char *)d.y + r * d.y_pitch) + c0;
+    const S *pu = (const S *)((const char *)d.u + r * d.u_pitch) + c0;
+    const S *pv = (const S *)((const char *)d.v + r * d.v_pitch) + c0;
     const long plane = (long)Hk * Wk;
     TR *o = out + (long)blockIdx.z * 3 * plane + r * Wk + c0;
     const bool vs = n == 4 && quad_aligned(py) && quad_aligned(pu) && quad_aligned(pv);
     const bool vr = n == 4 && quad_aligned(o) && (plane & 3) == 0;
-    TS ys[4], us[4], vs4[4];
+    S ys[4], us[4], vs4[4];
     load_quad(py, vs, n, ys);
     load_quad(pu, vs, n, us);
     load_quad(pv, vs, n, vs4);
     float rq[4], gq[4], bq[4];
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-        const float yn = __fdiv_rn(__fadd_rn((float)(ys[q] >> s), -k.yo), k.ys);
-        const float un = __fdiv_rn(__fadd_rn((float)(us[q] >> s), -F::mid), k.cs);
-        const float vn = __fdiv_rn(__fadd_rn((float)(vs4[q] >> s), -F::mid), k.cs);
+        const float yn = __fdiv_rn(__fadd_rn((float)F::code(ys[q]), -k.yo), k.ys);
+        const float un = __fdiv_rn(__fadd_rn((float)F::code(us[q]), -F::mid), k.cs);
+        const float vn = __fdiv_rn(__fadd_rn((float)F::code(vs4[q]), -F::mid), k.cs);
         rq[q] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_rv, vn)));
         gq[q] = clamp01(__fadd_rn(__fadd_rn(yn, __fmul_rn(k.a_gu, un)), __fmul_rn(k.a_gv, vn)));
         bq[q] = clamp01(__fadd_rn(yn, __fmul_rn(k.a_bu, un)));
@@ -1449,6 +1539,7 @@ __global__ void __launch_bounds__(k444Threads) yuv444_to_rgb_kernel(Frames3 in, 
 template <typename TR, typename TS>
 __global__ void __launch_bounds__(k444Threads) rgb_to_yuv444_kernel(const TR *__restrict__ in, Frames3 out, int Hk, int Wk, YuvCoef k) {
     typedef Yuv420<TS> F;
+    typedef typename F::T S;
     pdl_trigger();
     pdl_wait();
     const int c0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
@@ -1456,9 +1547,9 @@ __global__ void __launch_bounds__(k444Threads) rgb_to_yuv444_kernel(const TR *__
     const int n = min(4, Wk - c0);
     const TuFramePlanes3 &d = out.f[blockIdx.z];
     const long long r = blockIdx.y;
-    TS *py = (TS *)((char *)d.y + r * d.y_pitch) + c0;
-    TS *pu = (TS *)((char *)d.u + r * d.u_pitch) + c0;
-    TS *pv = (TS *)((char *)d.v + r * d.v_pitch) + c0;
+    S *py = (S *)((char *)d.y + r * d.y_pitch) + c0;
+    S *pu = (S *)((char *)d.u + r * d.u_pitch) + c0;
+    S *pv = (S *)((char *)d.v + r * d.v_pitch) + c0;
     const long plane = (long)Hk * Wk;
     const TR *src = in + (long)blockIdx.z * 3 * plane + r * Wk + c0;
     const bool vs = n == 4 && quad_aligned(py) && quad_aligned(pu) && quad_aligned(pv);
@@ -1466,7 +1557,7 @@ __global__ void __launch_bounds__(k444Threads) rgb_to_yuv444_kernel(const TR *__
     TR px[3][4];
 #pragma unroll
     for (int c = 0; c < 3; ++c) load_quad(src + c * plane, vr, n, px[c]);
-    TS yq[4], uq[4], vq[4];
+    S yq[4], uq[4], vq[4];
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
         const float R = to_f(px[0][q]), G = to_f(px[1][q]), Bl = to_f(px[2][q]);
@@ -1856,6 +1947,7 @@ extern "C" int tu_rgb_to_p010(const void *rgb_f32, void *p010, int code, int B, 
 
 // B frame surfaces of an NV12 (code TU_U8 | TU_LAYOUT_NV12 ...) or P010 (TU_U16 | TU_LAYOUT_P010 ...) side: host-side checks of the
 // code, the sizes and every descriptor, made before anything is enqueued (tu_forward_planes runs them ahead of its first kernel)
+static int check_sp_descriptors(const TuFramePlanes *frames, bool w16, int B, int W, const char *op, const char *fmt);
 int tu::check_yuv420_planes(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op) {
     TU_CHECK_ARG(frames && B > 0 && H > 0 && W > 0, std::string(op) + ": bad argument");
     TU_CHECK_ARG(dtype_is_yuv420(code), std::string(op) + ": frame planes are for NV12 (TU_U8 | TU_LAYOUT_NV12 [| colour bits]) or P010 "
@@ -1864,9 +1956,25 @@ int tu::check_yuv420_planes(const TuFramePlanes *frames, int code, int B, int H,
     const std::string fmt = p010 ? "P010" : "NV12";
     TU_CHECK_ARG(H % 2 == 0 && W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even height and width");
     TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
-    const long long row = (long long)W * (p010 ? 2 : 1);
-    const uintptr_t al = p010 ? 4 : 2;                              // a pair of samples is one access
-    const char *al_msg = p010 ? "a multiple of 4 bytes (P010)" : "a multiple of 2 bytes (NV12)";
+    return check_sp_descriptors(frames, p010, B, W, op, p010 ? "P010" : "NV12");
+}
+
+// B frames of a semi-planar 4:2:2 side (NV16 / P210): the checks of check_yuv420_planes with H chroma rows, so any H
+int tu::check_yuv422sp_frames(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op) {
+    TU_CHECK_ARG(frames && B > 0 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_yuv422sp(code), std::string(op) + ": frame planes are for NV16 (TU_U8 | TU_LAYOUT_NV16 [| colour bits]) or P210 "
+                                                            "(TU_U16 | TU_LAYOUT_NV16 [| colour bits]) frames only");
+    const bool p210 = dtype_is_p210(code);
+    TU_CHECK_ARG(W % 2 == 0, std::string(op) + ": " + (p210 ? "P210" : "NV16") + " frames need an even width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    return check_sp_descriptors(frames, p210, B, W, op, p210 ? "P210" : "NV16");
+}
+
+// the descriptors of B semi-planar frames (y, and uv of interleaved (U, V) pairs): pointers, pitches and their alignment
+static int check_sp_descriptors(const TuFramePlanes *frames, bool w16, int B, int W, const char *op, const char *fmt) {
+    const long long row = (long long)W * (w16 ? 2 : 1);
+    const uintptr_t al = w16 ? 4 : 2;                               // a pair of samples is one access
+    const std::string al_msg = std::string("a multiple of ") + (w16 ? "4" : "2") + " bytes (" + fmt + ")";
     for (int b = 0; b < B; ++b) {
         const TuFramePlanes &d = frames[b];
         const std::string at = std::string(op) + ": frame " + std::to_string(b) + ": ";
@@ -1925,22 +2033,30 @@ extern "C" int tu_rgb_to_yuv420_planes(const void *rgb, const TuFramePlanes *fra
                 : launch_planes<uint8_t, f16, false>(frames, code, (f16 *)rgb, B, H, W, st, "rgb_to_nv12");
 }
 
-// ---- planar YUV frames (yuv420p / yuv444p / yuv444p16) ------------------------------------------------------------------------------
-static const char *yuvp_fmt(int code) { return dtype_is_yuv420p(code) ? "yuv420p" : dtype_is_yuv444p(code) ? "yuv444p" : "yuv444p16"; }
+// ---- planar YUV frames (yuv420p / yuv422p / yuv444p, yuv444p16, and the LSB 10-bit yuv420p10le / yuv422p10le / yuv444p10le) ----------
+static const char *yuvp_fmt(int code) {
+    return dtype_is_yuv420p(code) ? "yuv420p" : dtype_is_yuv444p(code) ? "yuv444p" : dtype_is_yuv444p16(code) ? "yuv444p16"
+           : dtype_is_yuv422p(code) ? "yuv422p" : dtype_is_yuv420p10(code) ? "yuv420p10le" : dtype_is_yuv422p10(code) ? "yuv422p10le"
+                                                                                                                       : "yuv444p10le";
+}
+static bool yuvp_is_420(int code) { return dtype_is_yuv420p(code) || dtype_is_yuv420p10(code); }
+static bool yuvp_is_422(int code) { return dtype_is_yuv422p(code) || dtype_is_yuv422p10(code); }
 
 // B frames of a planar YUV side: host-side checks of the code, the sizes and every descriptor, made before anything is enqueued
 int tu::check_yuvp_frames(const TuFramePlanes3 *frames, int code, int B, int H, int W, const char *op) {
     TU_CHECK_ARG(frames && B > 0 && H > 0 && W > 0, std::string(op) + ": bad argument");
     TU_CHECK_ARG(dtype_is_yuvp(code), std::string(op) + ": TuFramePlanes3 frames are for planar YUV (TU_U8 | TU_LAYOUT_YUV420P, "
-                                                        "TU_U8 | TU_LAYOUT_YUV444P or TU_U16 | TU_LAYOUT_YUV444P [| colour bits]) only");
-    const bool p420 = dtype_is_yuv420p(code), w16 = dtype_base(code) == TU_U16;
+                                                        "TU_U8 | TU_LAYOUT_YUV422P, TU_U8 | TU_LAYOUT_YUV444P, TU_U16 | TU_LAYOUT_YUV444P, "
+                                                        "or TU_U16 | one of them | TU_YUV_LSB10 [| colour bits]) only");
+    const bool p420 = yuvp_is_420(code), p422 = yuvp_is_422(code), w16 = dtype_base(code) == TU_U16;
     const std::string fmt = yuvp_fmt(code);
     TU_CHECK_ARG(!p420 || (H % 2 == 0 && W % 2 == 0), std::string(op) + ": " + fmt + " frames need an even height and width");
+    TU_CHECK_ARG(!p422 || W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even width");
     TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
-    TU_CHECK_ARG(p420 || H <= 65535, std::string(op) + ": " + fmt + " frame surfaces have at most 65535 rows");
-    const long long s = w16 ? 2 : 1, yrow = W * s, crow = (p420 ? W / 2 : W) * s;
-    // a pair of luma samples is one access (yuv420p); a 16-bit sample is one word
-    const long long ya = p420 || w16 ? 2 : 1, ca = w16 ? 2 : 1;
+    TU_CHECK_ARG(p420 || p422 || H <= 65535, std::string(op) + ": " + fmt + " frame surfaces have at most 65535 rows");
+    const long long s = w16 ? 2 : 1, yrow = W * s, crow = (p420 || p422 ? W / 2 : W) * s;
+    // a pair of luma samples is one access (4:2:0, 4:2:2); a 16-bit sample is one word
+    const long long ya = p420 || p422 ? 2 * s : s, ca = s;
     for (int b = 0; b < B; ++b) {
         const TuFramePlanes3 &d = frames[b];
         const std::string at = std::string(op) + ": frame " + std::to_string(b) + ": ";
@@ -1953,7 +2069,7 @@ int tu::check_yuvp_frames(const TuFramePlanes3 *frames, int code, int B, int H, 
             TU_CHECK_ARG(p.pitch >= p.row, at + p.name + " " + std::to_string(p.pitch) + " is smaller than the row's " +
                                                std::to_string(p.row / s) + " samples (" + std::to_string(p.row) + " bytes)");
         TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.y) % ya == 0 && d.y_pitch % ya == 0,
-                     at + "y and y_pitch must be multiples of 2 bytes (" + fmt + ")");
+                     at + "y and y_pitch must be multiples of " + std::to_string(ya) + " bytes (" + fmt + ")");
         TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.u) % ca == 0 && d.u_pitch % ca == 0,
                      at + "u and u_pitch must be multiples of 2 bytes (" + fmt + ")");
         TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.v) % ca == 0 && d.v_pitch % ca == 0,
@@ -1964,16 +2080,18 @@ int tu::check_yuvp_frames(const TuFramePlanes3 *frames, int code, int B, int H, 
 
 static int check_yuvp_args(const void *dense, const TuFramePlanes3 *frames, int code, const void *rgb, int B, int H, int W, const char *op) {
     TU_CHECK_ARG(rgb && B > 0 && B <= 65535 && H > 0 && W > 0, std::string(op) + ": bad argument");
-    TU_CHECK_ARG(dtype_is_yuvp(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_YUV420P or TU_U8 | TU_LAYOUT_YUV444P "
-                                                        "[| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_YUV444P "
+    TU_CHECK_ARG(dtype_is_yuvp(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_YUV420P, TU_LAYOUT_YUV422P or TU_LAYOUT_YUV444P "
+                                                        "[| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_YUV444P, or TU_U16 | "
+                                                        "TU_LAYOUT_YUV420P, TU_LAYOUT_YUV422P or TU_LAYOUT_YUV444P | TU_YUV_LSB10 "
                                                         "[| TU_YUV_BT601 or TU_YUV_BT2020] [| TU_YUV_FULL_RANGE]");
     TU_CHECK_ARG(!dense != !frames, std::string(op) + ": give exactly one of the dense buffer and the frames array");
-    const bool p420 = dtype_is_yuv420p(code), w16 = dtype_base(code) == TU_U16;
+    const bool p420 = yuvp_is_420(code), p422 = yuvp_is_422(code), w16 = dtype_base(code) == TU_U16;
     const std::string fmt = yuvp_fmt(code);
     TU_CHECK_ARG(!p420 || (H % 2 == 0 && W % 2 == 0), std::string(op) + ": " + fmt + " frames need an even height and width");
+    TU_CHECK_ARG(!p422 || W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even width");
     TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
-    // yuv420p: pairs of luma samples and of fp16 RGB values are one access (as NV12); 4:4:4: one element
-    const uintptr_t ra = p420 ? 4 : w16 ? 4 : 2, fa = p420 || w16 ? 2 : 1;
+    // 4:2:0 / 4:2:2: pairs of luma samples and of RGB values are one access (as NV12 / P010); 4:4:4: one element
+    const uintptr_t ra = (p420 || p422 ? 2 : 1) * (w16 ? 4 : 2), fa = (p420 || p422 ? 2 : 1) * (w16 ? 2 : 1);
     TU_CHECK_ARG((reinterpret_cast<uintptr_t>(rgb) & (ra - 1)) == 0,
                  std::string(op) + ": the " + (w16 ? "fp32" : "fp16") + " RGB buffer must be " + std::to_string(ra) + "-byte aligned");
     TU_CHECK_ARG(!dense || (reinterpret_cast<uintptr_t>(dense) & (fa - 1)) == 0,
@@ -1982,11 +2100,13 @@ static int check_yuvp_args(const void *dense, const TuFramePlanes3 *frames, int 
 }
 
 // one launch per kPlanesPerLaunch frames; a dense batch is passed as the table of its frames' planes.  The RGB side is the dense batch,
-// offset to the first frame of the launch
-template <typename TS, typename TR, bool ToRgb>
+// offset to the first frame of the launch.  F is the sample format (uint8_t, uint16_t: yuv444p16 only, Lsb10)
+template <typename F, typename TR, bool ToRgb>
 static int launch_yuvp(const void *dense, const TuFramePlanes3 *frames, int code, TR *rgb, int B, int H, int W, cudaStream_t st) {
-    const bool p420 = dtype_is_yuv420p(code);
-    const long long s = sizeof(TS), plane = (long long)H * W, crow = p420 ? W / 2 : W, cplane = p420 ? plane / 4 : plane;
+    typedef typename Yuv420<F>::T S;
+    const bool p420 = yuvp_is_420(code), p422 = yuvp_is_422(code);
+    const long long s = sizeof(S), plane = (long long)H * W, crow = p420 || p422 ? W / 2 : W;
+    const long long cplane = p420 ? plane / 4 : p422 ? plane / 2 : plane;
     const YuvCoef k = yuv_coef(code);
     const std::string what = ToRgb ? std::string(yuvp_fmt(code)) + "_to_rgb" : std::string("rgb_to_") + yuvp_fmt(code);
     for (int b0 = 0; b0 < B; b0 += kPlanesPerLaunch) {
@@ -2003,21 +2123,28 @@ static int launch_yuvp(const void *dense, const TuFramePlanes3 *frames, int code
             packed &= p.f[b].y_pitch == W * s && p.f[b].u_pitch == crow * s && p.f[b].v_pitch == crow * s;
         }
         TR *r = rgb + (long long)b0 * 3 * plane;
-        if (p420) {
-            if constexpr (sizeof(TS) == 1) {
-                const dim3 grid((unsigned)ceil_div((int)(plane / 4), 256), nb);
-                if constexpr (ToRgb)
-                    launch_pdl(yuv420_to_rgb_kernel<TS, TR, Planar420<const TS>>, grid, dim3(256), 0, st, p, r, H, W, k);
-                else
-                    launch_pdl(rgb_to_yuv420_kernel<TR, TS, Planar420<TS>>, grid, dim3(256), 0, st, (const TR *)r, p, H, W, k);
+        if (p420 || p422) {
+            if constexpr (!std::is_same<F, uint16_t>::value) {      // no MSB-word 4:2:0 / 4:2:2 planar format exists
+                const dim3 grid((unsigned)ceil_div((int)(p420 ? plane / 4 : plane / 2), 256), nb);
+                if (p420) {
+                    if constexpr (ToRgb)
+                        launch_pdl(yuv420_to_rgb_kernel<F, TR, Planar420<const S>>, grid, dim3(256), 0, st, p, r, H, W, k);
+                    else
+                        launch_pdl(rgb_to_yuv420_kernel<TR, F, Planar420<S>>, grid, dim3(256), 0, st, (const TR *)r, p, H, W, k);
+                } else {
+                    if constexpr (ToRgb)
+                        launch_pdl(yuv422_to_rgb_kernel<F, TR, Planar420<const S>>, grid, dim3(256), 0, st, p, r, H, W, k);
+                    else
+                        launch_pdl(rgb_to_yuv422_kernel<TR, F, Planar420<S>>, grid, dim3(256), 0, st, (const TR *)r, p, H, W, k);
+                }
             }
         } else {
             const int Hk = packed ? 1 : H, Wk = packed ? H * W : W;
             const dim3 grid((unsigned)ceil_div(ceil_div(Wk, 4), k444Threads), Hk, nb);
             if constexpr (ToRgb)
-                launch_pdl(yuv444_to_rgb_kernel<TS, TR>, grid, dim3(k444Threads), 0, st, p, r, Hk, Wk, k);
+                launch_pdl(yuv444_to_rgb_kernel<F, TR>, grid, dim3(k444Threads), 0, st, p, r, Hk, Wk, k);
             else
-                launch_pdl(rgb_to_yuv444_kernel<TR, TS>, grid, dim3(k444Threads), 0, st, (const TR *)r, p, Hk, Wk, k);
+                launch_pdl(rgb_to_yuv444_kernel<TR, F>, grid, dim3(k444Threads), 0, st, (const TR *)r, p, Hk, Wk, k);
         }
         TU_CHECK_LAUNCH(what.c_str());
     }
@@ -2027,6 +2154,7 @@ static int launch_yuvp(const void *dense, const TuFramePlanes3 *frames, int code
 extern "C" int tu_yuvp_to_rgb(const void *dense, const TuFramePlanes3 *frames, int code, void *rgb, int B, int H, int W, void *stream) {
     if (int rc = check_yuvp_args(dense, frames, code, rgb, B, H, W, "yuvp_to_rgb")) return rc;
     cudaStream_t st = (cudaStream_t)stream;
+    if (dtype_is_lsb10(code)) return launch_yuvp<Lsb10, float, true>(dense, frames, code, (float *)rgb, B, H, W, st);
     return dtype_base(code) == TU_U16 ? launch_yuvp<uint16_t, float, true>(dense, frames, code, (float *)rgb, B, H, W, st)
                                       : launch_yuvp<uint8_t, f16, true>(dense, frames, code, (f16 *)rgb, B, H, W, st);
 }
@@ -2034,6 +2162,70 @@ extern "C" int tu_yuvp_to_rgb(const void *dense, const TuFramePlanes3 *frames, i
 extern "C" int tu_rgb_to_yuvp(const void *rgb, void *dense, const TuFramePlanes3 *frames, int code, int B, int H, int W, void *stream) {
     if (int rc = check_yuvp_args(dense, frames, code, rgb, B, H, W, "rgb_to_yuvp")) return rc;
     cudaStream_t st = (cudaStream_t)stream;
+    if (dtype_is_lsb10(code)) return launch_yuvp<Lsb10, float, false>(dense, frames, code, (float *)rgb, B, H, W, st);
     return dtype_base(code) == TU_U16 ? launch_yuvp<uint16_t, float, false>(dense, frames, code, (float *)rgb, B, H, W, st)
                                       : launch_yuvp<uint8_t, f16, false>(dense, frames, code, (f16 *)rgb, B, H, W, st);
+}
+
+// ---- semi-planar 4:2:2 frames (NV16 / P210) ----------------------------------------------------------------------------------------
+static int check_yuv422sp_args(const void *dense, const TuFramePlanes *frames, int code, const void *rgb, int B, int H, int W,
+                               const char *op) {
+    TU_CHECK_ARG(rgb && B > 0 && B <= 65535 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_yuv422sp(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_NV16 [| TU_YUV_BT601] [| TU_YUV_FULL_RANGE], "
+                                                             "or TU_U16 | TU_LAYOUT_NV16 [| TU_YUV_BT601 or TU_YUV_BT2020] [| TU_YUV_FULL_RANGE]");
+    TU_CHECK_ARG(!dense != !frames, std::string(op) + ": give exactly one of the dense buffer and the frames array");
+    const bool p210 = dtype_is_p210(code);
+    const std::string fmt = p210 ? "P210" : "NV16";
+    TU_CHECK_ARG(W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    const uintptr_t ra = p210 ? 8 : 4, fa = p210 ? 4 : 2;      // a pair of RGB values / of samples is one access
+    TU_CHECK_ARG((reinterpret_cast<uintptr_t>(rgb) & (ra - 1)) == 0,
+                 std::string(op) + ": the " + (p210 ? "fp32" : "fp16") + " RGB buffer must be " + std::to_string(ra) + "-byte aligned");
+    TU_CHECK_ARG(!dense || (reinterpret_cast<uintptr_t>(dense) & (fa - 1)) == 0,
+                 std::string(op) + ": the dense " + fmt + " buffer must be " + std::to_string(fa) + "-byte aligned");
+    return frames ? check_yuv422sp_frames(frames, code, B, H, W, op) : TU_OK;
+}
+
+// one launch per kPlanesPerLaunch frames, the dense (B, 2H, W) batch passed as the table of its frames' planes (Y, then H chroma rows)
+template <typename TS, typename TR, bool ToRgb>
+static int launch_yuv422sp(const void *dense, const TuFramePlanes *frames, int code, TR *rgb, int B, int H, int W, cudaStream_t st) {
+    typedef Planes420<typename std::conditional<ToRgb, const TS, TS>::type> A;
+    const long long s = sizeof(TS), plane = (long long)H * W;
+    const YuvCoef k = yuv_coef(code);
+    const char *what = dtype_is_p210(code) ? (ToRgb ? "p210_to_rgb" : "rgb_to_p210") : (ToRgb ? "nv16_to_rgb" : "rgb_to_nv16");
+    const dim3 block(256);
+    for (int b0 = 0; b0 < B; b0 += kPlanesPerLaunch) {
+        const int nb = std::min(kPlanesPerLaunch, B - b0);
+        typename A::Param p = {};
+        for (int b = 0; b < nb; ++b) {
+            if (frames) {
+                p.f[b] = frames[b0 + b];
+            } else {
+                char *f = (char *)dense + (long long)(b0 + b) * 2 * plane * s;
+                p.f[b] = {f, f + plane * s, W * s, W * s};
+            }
+        }
+        TR *r = rgb + (long long)b0 * 3 * plane;
+        const dim3 grid((unsigned)ceil_div((int)(plane / 2), 256), nb);
+        if constexpr (ToRgb)
+            launch_pdl(yuv422_to_rgb_kernel<TS, TR, A>, grid, block, 0, st, p, r, H, W, k);
+        else
+            launch_pdl(rgb_to_yuv422_kernel<TR, TS, A>, grid, block, 0, st, (const TR *)r, p, H, W, k);
+        TU_CHECK_LAUNCH(what);
+    }
+    return TU_OK;
+}
+
+extern "C" int tu_yuv422sp_to_rgb(const void *dense, const TuFramePlanes *frames, int code, void *rgb, int B, int H, int W, void *stream) {
+    if (int rc = check_yuv422sp_args(dense, frames, code, rgb, B, H, W, "yuv422sp_to_rgb")) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    return dtype_is_p210(code) ? launch_yuv422sp<uint16_t, float, true>(dense, frames, code, (float *)rgb, B, H, W, st)
+                               : launch_yuv422sp<uint8_t, f16, true>(dense, frames, code, (f16 *)rgb, B, H, W, st);
+}
+
+extern "C" int tu_rgb_to_yuv422sp(const void *rgb, void *dense, const TuFramePlanes *frames, int code, int B, int H, int W, void *stream) {
+    if (int rc = check_yuv422sp_args(dense, frames, code, rgb, B, H, W, "rgb_to_yuv422sp")) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    return dtype_is_p210(code) ? launch_yuv422sp<uint16_t, float, false>(dense, frames, code, (float *)rgb, B, H, W, st)
+                               : launch_yuv422sp<uint8_t, f16, false>(dense, frames, code, (f16 *)rgb, B, H, W, st);
 }

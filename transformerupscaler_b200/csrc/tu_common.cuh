@@ -21,8 +21,10 @@ int cuda_fail(cudaError_t e, const char *what);
 void count_launch();   // every kernel launch of the library is counted (tu_launch_count)
 // checks B NV12 / P010 frame surfaces (resample.cu): TU_ERR_ARG with the frame index and field in the message
 int check_yuv420_planes(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op);
-// the same for B planar YUV frames (yuv420p / yuv444p / yuv444p16: TuFramePlanes3)
+// the same for B planar YUV frames (every planar code: TuFramePlanes3)
 int check_yuvp_frames(const TuFramePlanes3 *frames, int code, int B, int H, int W, const char *op);
+// the same for B semi-planar 4:2:2 frames (NV16 / P210: TuFramePlanes with H chroma rows)
+int check_yuv422sp_frames(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op);
 
 #define TU_CHECK_ARG(cond, msg)                         \
     do {                                                \
@@ -99,7 +101,7 @@ template <> __device__ __forceinline__ uint8_t from_f<uint8_t>(float v) {
 // TU_U8 | TU_LAYOUT_NV12 (4:2:0 video frames) may add the colour bits TU_YUV_BT601 / TU_YUV_FULL_RANGE in bits 12..13.
 // TU_U16 | TU_LAYOUT_P010 (10-bit 4:2:0 frames) may add the same bits, or TU_YUV_BT2020 (bit 14) instead of TU_YUV_BT601.
 __host__ __device__ __forceinline__ int dtype_base(int d) { return d & 0xFF; }
-// the layout bits are an enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010), and dtype_layout keeps the colour bits
+// the layout bits are an enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010, 9 YUV422P, 10 NV16), and dtype_layout keeps the colour bits
 // above them: compare whole values, never bits (0x500 = BGRA shares a bit with NV12, 0x300 = RGBA two bits with HWC / HWC_BGR)
 __host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }
 __host__ __device__ __forceinline__ bool layout_is_px4(int l) { return l == 3 || l == 5; }          // RGBA / BGRA: 4-byte pixels
@@ -127,9 +129,28 @@ __host__ __device__ __forceinline__ bool dtype_is_yuv444p16(int d) {            
     const int c = d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE);
     return (d & ~c) == (TU_U16 | TU_LAYOUT_YUV444P) && (c & (TU_YUV_BT601 | TU_YUV_BT2020)) != (TU_YUV_BT601 | TU_YUV_BT2020);
 }
-__host__ __device__ __forceinline__ bool dtype_is_yuvp(int d) { return dtype_is_yuv420p(d) || dtype_is_yuv444p(d) || dtype_is_yuv444p16(d); }
+// 4:2:2 (layout 9 yuv422p: three planes, 10 NV16: Y then interleaved (U, V) rows) and the LSB-aligned 10-bit planar codes (TU_U16 |
+// planar layout | TU_YUV_LSB10: the code in the low 10 bits).  8-bit codes take NV12's colour bits, 16-bit codes P010's
+__host__ __device__ __forceinline__ bool yuv8_code_is(int d, int base) { return (d & ~(TU_YUV_BT601 | TU_YUV_FULL_RANGE)) == base; }
+__host__ __device__ __forceinline__ bool yuv16_code_is(int d, int base) {
+    const int c = d & (TU_YUV_BT601 | TU_YUV_BT2020 | TU_YUV_FULL_RANGE);
+    return (d & ~c) == base && (c & (TU_YUV_BT601 | TU_YUV_BT2020)) != (TU_YUV_BT601 | TU_YUV_BT2020);
+}
+__host__ __device__ __forceinline__ bool dtype_is_yuv422p(int d) { return yuv8_code_is(d, TU_U8 | TU_LAYOUT_YUV422P); }
+__host__ __device__ __forceinline__ bool dtype_is_nv16(int d) { return yuv8_code_is(d, TU_U8 | TU_LAYOUT_NV16); }
+__host__ __device__ __forceinline__ bool dtype_is_p210(int d) { return yuv16_code_is(d, TU_U16 | TU_LAYOUT_NV16); }
+__host__ __device__ __forceinline__ bool dtype_is_yuv420p10(int d) { return yuv16_code_is(d, TU_U16 | TU_LAYOUT_YUV420P | TU_YUV_LSB10); }
+__host__ __device__ __forceinline__ bool dtype_is_yuv422p10(int d) { return yuv16_code_is(d, TU_U16 | TU_LAYOUT_YUV422P | TU_YUV_LSB10); }
+__host__ __device__ __forceinline__ bool dtype_is_yuv444p10(int d) { return yuv16_code_is(d, TU_U16 | TU_LAYOUT_YUV444P | TU_YUV_LSB10); }
+__host__ __device__ __forceinline__ bool dtype_is_lsb10(int d) { return dtype_is_yuv420p10(d) || dtype_is_yuv422p10(d) || dtype_is_yuv444p10(d); }
+// semi-planar 4:2:2 (TuFramePlanes surfaces with H chroma rows)
+__host__ __device__ __forceinline__ bool dtype_is_yuv422sp(int d) { return dtype_is_nv16(d) || dtype_is_p210(d); }
+// every planar code (TuFramePlanes3 surfaces)
+__host__ __device__ __forceinline__ bool dtype_is_yuvp(int d) {
+    return dtype_is_yuv420p(d) || dtype_is_yuv444p(d) || dtype_is_yuv444p16(d) || dtype_is_yuv422p(d) || dtype_is_lsb10(d);
+}
 // every YUV frame code: converted to / from a planar fp16 (8-bit) or fp32 (16-bit) RGB frame at the ends of the forward
-__host__ __device__ __forceinline__ bool dtype_is_yuv(int d) { return dtype_is_yuv420(d) || dtype_is_yuvp(d); }
+__host__ __device__ __forceinline__ bool dtype_is_yuv(int d) { return dtype_is_yuv420(d) || dtype_is_yuvp(d) || dtype_is_yuv422sp(d); }
 // one RGB pixel of frame b -> out, in the requested layout.  pix = y * W + x, plane = H * W
 template <typename TO>
 __device__ __forceinline__ void store_rgb(TO *out, long b, long plane, long pix, int layout, float r, float g, float bl) {

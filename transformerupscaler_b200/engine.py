@@ -56,12 +56,19 @@ def _code(dt: torch.dtype) -> int:
 
 LAYOUTS = {"chw": 0, "hwc": _lib.TU_LAYOUT_HWC, "hwc_bgr": _lib.TU_LAYOUT_HWC_BGR, "nv12": _lib.TU_LAYOUT_NV12,
            "p010": _lib.TU_LAYOUT_P010, "rgba": _lib.TU_LAYOUT_RGBA, "bgra": _lib.TU_LAYOUT_BGRA,
-           "yuv420p": _lib.TU_LAYOUT_YUV420P, "yuv444p": _lib.TU_LAYOUT_YUV444P, "yuv444p16": _lib.TU_LAYOUT_YUV444P}
-# planar YUV layouts (FFmpeg's pix_fmt names) -> frame dtype; yuv444p and yuv444p16 share the layout bits and differ in the dtype
-PLANAR = {"yuv420p": torch.uint8, "yuv444p": torch.uint8, "yuv444p16": torch.uint16}
+           "yuv420p": _lib.TU_LAYOUT_YUV420P, "yuv444p": _lib.TU_LAYOUT_YUV444P, "yuv444p16": _lib.TU_LAYOUT_YUV444P,
+           "yuv420p10le": _lib.TU_LAYOUT_YUV420P | _lib.TU_YUV_LSB10, "yuv422p": _lib.TU_LAYOUT_YUV422P,
+           "yuv422p10le": _lib.TU_LAYOUT_YUV422P | _lib.TU_YUV_LSB10, "yuv444p10le": _lib.TU_LAYOUT_YUV444P | _lib.TU_YUV_LSB10,
+           "nv16": _lib.TU_LAYOUT_NV16, "p210": _lib.TU_LAYOUT_NV16}
+# planar YUV layouts (FFmpeg's pix_fmt names) -> frame dtype; yuv444p and yuv444p16 share the layout bits and differ in the dtype, the
+# *p10le layouts carry TU_YUV_LSB10 (the code in the low 10 bits of each word)
+PLANAR = {"yuv420p": torch.uint8, "yuv444p": torch.uint8, "yuv444p16": torch.uint16, "yuv420p10le": torch.uint16,
+          "yuv422p": torch.uint8, "yuv422p10le": torch.uint16, "yuv444p10le": torch.uint16}
+# semi-planar 4:2:2 layouts -> frame dtype (nv16 and p210 share the layout bits and differ in the dtype)
+SEMI422 = {"nv16": torch.uint8, "p210": torch.uint16}
 # every YUV layout, and the ones of 16-bit words (10-bit codes: the only ones BT.2020 is defined for)
-YUV_LAYOUTS = ("nv12", "p010", *PLANAR)
-YUV16_LAYOUTS = ("p010", "yuv444p16")
+YUV_LAYOUTS = ("nv12", "p010", *PLANAR, *SEMI422)
+YUV16_LAYOUTS = ("p010", "yuv444p16", "yuv420p10le", "yuv422p10le", "yuv444p10le", "p210")
 # colour of NV12 and P010 frames: matrix and range
 YUV = {"bt709": 0, "bt601": _lib.TU_YUV_BT601, "bt709_full": _lib.TU_YUV_FULL_RANGE,
        "bt601_full": _lib.TU_YUV_BT601 | _lib.TU_YUV_FULL_RANGE}
@@ -72,7 +79,7 @@ YUV_P010 = {"bt2020": _lib.TU_YUV_BT2020, "bt2020_full": _lib.TU_YUV_BT2020 | _l
 def layout_code(name: str) -> int:
     if name not in LAYOUTS:
         raise ValueError(f"unknown frame layout {name!r}: use 'chw', 'hwc', 'hwc_bgr', 'rgba', 'bgra', 'nv12', 'p010', 'yuv420p', "
-                         "'yuv444p' or 'yuv444p16'")
+                         "'yuv444p', 'yuv444p16', 'yuv420p10le', 'yuv422p', 'yuv422p10le', 'yuv444p10le', 'nv16' or 'p210'")
     return LAYOUTS[name]
 
 
@@ -103,9 +110,31 @@ def _is_yuv444p(code: int) -> bool:
     return code & 0xF00 == _lib.TU_LAYOUT_YUV444P
 
 
+def _is_yuv422p(code: int) -> bool:
+    """yuv422p (TU_U8) or yuv422p10le (TU_U16 | TU_YUV_LSB10): (B, 2H, W)"""
+    return code & 0xF00 == _lib.TU_LAYOUT_YUV422P
+
+
+def _is_nv16(code: int) -> bool:
+    """nv16 (TU_U8) or p210 (TU_U16): (B, 2H, W), frame surfaces are (y, uv) pairs"""
+    return code & 0xF00 == _lib.TU_LAYOUT_NV16
+
+
 def _is_yuvp(code: int) -> bool:
     """planar YUV: frame surfaces are (y, u, v) triples"""
-    return _is_yuv420p(code) or _is_yuv444p(code)
+    return _is_yuv420p(code) or _is_yuv444p(code) or _is_yuv422p(code)
+
+
+def _yuv_name(code: int, dtype: torch.dtype) -> str:
+    """layout name of a planar or 4:2:2 YUV code whose frames have dtype `dtype`"""
+    lsb = code & _lib.TU_YUV_LSB10
+    if _is_yuv420p(code):
+        return "yuv420p10le" if lsb else "yuv420p"
+    if _is_yuv422p(code):
+        return "yuv422p10le" if lsb else "yuv422p"
+    if _is_nv16(code):
+        return "p210" if dtype == torch.uint16 else "nv16"
+    return "yuv444p10le" if lsb else "yuv444p16" if dtype == torch.uint16 else "yuv444p"
 
 
 def _is_px4(code: int) -> bool:
@@ -115,11 +144,13 @@ def _is_px4(code: int) -> bool:
 
 def _image_shape(B: int, C_: int, h: int, w: int, code: int) -> Tuple[int, ...]:
     """shape of a (B, C_, h, w) image stored with dtype (| layout) code `code`: planar, interleaved (B,h,w,3), 4-byte pixels
-    (B,h,w,4), NV12 / P010 / yuv420p (B,3h/2,w) or yuv444p / yuv444p16 (B,3,h,w)"""
+    (B,h,w,4), NV12 / P010 / yuv420p[10le] (B,3h/2,w), 4:2:2 (B,2h,w) or 4:4:4 (B,3,h,w)"""
     if _is_nv12(code) or _is_p010(code) or _is_yuv420p(code):
         return (B, 3 * h // 2, w)
     if _is_yuv444p(code):
         return (B, 3, h, w)
+    if _is_yuv422p(code) or _is_nv16(code):
+        return (B, 2 * h, w)
     if _is_px4(code):
         return (B, h, w, 4)
     return (B, h, w, 3) if code & 0xF00 in (_lib.TU_LAYOUT_HWC, _lib.TU_LAYOUT_HWC_BGR) else (B, C_, h, w)
@@ -148,10 +179,11 @@ def _p010_hw(x: torch.Tensor) -> Tuple[int, int]:
 
 
 def plane_pairs(frames, fmt: str, what: str) -> Tuple[int, int, int]:
-    """(B, H, W) of 4:2:0 frames given as a list / tuple of B (y, uv) plane pairs -- strided views of a decoder's or encoder's pitched
-    surfaces: y (H, W) and uv (H/2, W), uint8 for NV12 and uint16 for P010, unit stride along W, any row stride, all CUDA tensors on
-    one device.  Raises ValueError for anything else."""
-    dtype = torch.uint8 if fmt == "NV12" else torch.uint16
+    """(B, H, W) of semi-planar frames given as a list / tuple of B (y, uv) plane pairs -- strided views of a decoder's or encoder's
+    pitched surfaces: y (H, W) and uv (H/2, W) for 4:2:0 or (H, W) for 4:2:2, uint8 for NV12 / NV16 and uint16 for P010 / P210, unit
+    stride along W, any row stride, all CUDA tensors on one device.  Raises ValueError for anything else."""
+    dtype = torch.uint8 if fmt in ("NV12", "NV16") else torch.uint16
+    sub = fmt in ("NV12", "P010")
     if not isinstance(frames, (list, tuple)) or not frames:
         raise ValueError(f"{what}: {fmt} frame planes are a non-empty list of (y, uv) tensor pairs")
     dev, hw = None, None
@@ -168,8 +200,11 @@ def plane_pairs(frames, fmt: str, what: str) -> Tuple[int, int, int]:
             dev = t.device
         y, uv = pair
         H, W = int(y.shape[0]), int(y.shape[1])
-        if H % 2 or W % 2 or tuple(uv.shape) != (H // 2, W):
+        if sub and (H % 2 or W % 2 or tuple(uv.shape) != (H // 2, W)):
             raise ValueError(f"{what}[{b}]: {fmt} planes are y (H, W) and uv (H/2, W) with H and W even, got {tuple(y.shape)} and "
+                             f"{tuple(uv.shape)}")
+        if not sub and (W % 2 or tuple(uv.shape) != (H, W)):
+            raise ValueError(f"{what}[{b}]: {fmt} planes are y and uv of one size (H, W) with W even, got {tuple(y.shape)} and "
                              f"{tuple(uv.shape)}")
         if hw is not None and hw != (H, W):
             raise ValueError(f"{what}[{b}]: every frame of a batch has the same size, got {(H, W)} after {hw}")
@@ -184,16 +219,26 @@ def _yuv444_hw(x: torch.Tensor, fmt: str, dtype: torch.dtype) -> Tuple[int, int]
     return int(x.shape[2]), int(x.shape[3])
 
 
+def _yuv422_hw(x: torch.Tensor, fmt: str, dtype: torch.dtype) -> Tuple[int, int]:
+    """(H, W) of 4:2:2 frames (B, 2H, W); raises ValueError for a shape or dtype that is not one"""
+    if x.dim() != 3 or x.dtype != dtype:
+        raise ValueError(f"{fmt} frames must be {str(dtype)[6:]} of shape (B, 2H, W), got {x.dtype} {tuple(x.shape)}")
+    if x.shape[1] % 2 or x.shape[2] % 2:
+        raise ValueError(f"{fmt} frames (B, 2H, W) need an even row count and an even width, got {tuple(x.shape)}")
+    return int(x.shape[1]) // 2, int(x.shape[2])
+
+
 def _yuvp_hw(x: torch.Tensor, fmt: str) -> Tuple[int, int]:
-    """(H, W) of dense planar YUV frames of layout name `fmt`"""
-    return _yuv420_hw(x, fmt, torch.uint8) if fmt == "yuv420p" else _yuv444_hw(x, fmt, PLANAR[fmt])
+    """(H, W) of dense planar or semi-planar 4:2:2 YUV frames of layout name `fmt`"""
+    if fmt in SEMI422 or fmt.startswith("yuv422p"):
+        return _yuv422_hw(x, fmt, SEMI422.get(fmt) or PLANAR[fmt])
+    return _yuv420_hw(x, fmt, PLANAR[fmt]) if fmt.startswith("yuv420p") else _yuv444_hw(x, fmt, PLANAR[fmt])
 
 
 def plane_triples(frames, fmt: str, what: str) -> Tuple[int, int, int]:
-    """(B, H, W) of planar YUV frames (fmt 'yuv420p' | 'yuv444p' | 'yuv444p16') given as a list / tuple of B (y, u, v) plane triples --
-    strided views of a decoder's surfaces or an FFmpeg frame's data[0..2]: y (H, W), u and v (H/2, W/2) for yuv420p or (H, W) for 4:4:4,
-    uint8 (uint16 for yuv444p16), unit stride along W, any row stride, all CUDA tensors on one device.  Raises ValueError for anything
-    else."""
+    """(B, H, W) of planar YUV frames (fmt: a key of PLANAR) given as a list / tuple of B (y, u, v) plane triples -- strided views of a
+    decoder's surfaces or an FFmpeg frame's data[0..2]: y (H, W), u and v (H/2, W/2) for 4:2:0, (H, W/2) for 4:2:2 or (H, W) for 4:4:4,
+    of the layout's dtype, unit stride along W, any row stride, all CUDA tensors on one device.  Raises ValueError for anything else."""
     dtype = PLANAR[fmt]
     if not isinstance(frames, (list, tuple)) or not frames:
         raise ValueError(f"{what}: {fmt} frame planes are a non-empty list of (y, u, v) tensor triples")
@@ -211,9 +256,13 @@ def plane_triples(frames, fmt: str, what: str) -> Tuple[int, int, int]:
             dev = t.device
         y, u, v = tri
         H, W = int(y.shape[0]), int(y.shape[1])
-        if fmt == "yuv420p":
+        if fmt.startswith("yuv420p"):
             if H % 2 or W % 2 or tuple(u.shape) != (H // 2, W // 2) or tuple(v.shape) != (H // 2, W // 2):
-                raise ValueError(f"{what}[{b}]: yuv420p planes are y (H, W), u and v (H/2, W/2) with H and W even, got {tuple(y.shape)}, "
+                raise ValueError(f"{what}[{b}]: {fmt} planes are y (H, W), u and v (H/2, W/2) with H and W even, got {tuple(y.shape)}, "
+                                 f"{tuple(u.shape)} and {tuple(v.shape)}")
+        elif fmt.startswith("yuv422p"):
+            if W % 2 or tuple(u.shape) != (H, W // 2) or tuple(v.shape) != (H, W // 2):
+                raise ValueError(f"{what}[{b}]: {fmt} planes are y (H, W), u and v (H, W/2) with W even, got {tuple(y.shape)}, "
                                  f"{tuple(u.shape)} and {tuple(v.shape)}")
         elif tuple(u.shape) != (H, W) or tuple(v.shape) != (H, W):
             raise ValueError(f"{what}[{b}]: {fmt} planes are y, u and v of one size (H, W), got {tuple(y.shape)}, {tuple(u.shape)} and "
@@ -236,7 +285,7 @@ def _flat(frames) -> List[torch.Tensor]:
 
 
 def _descriptors(flat: Sequence[torch.Tensor], code: int = _lib.TU_U8 | _lib.TU_LAYOUT_NV12):
-    """descriptor array of the flattened planes of a side of code `code`: TuFramePlanes of [y0, uv0, y1, uv1, ...] (NV12 / P010) or
+    """descriptor array of the flattened planes of a side of code `code`: TuFramePlanes of [y0, uv0, y1, uv1, ...] (NV12 / P010 / NV16 / P210) or
     TuFramePlanes3 of [y0, u0, v0, y1, ...] (planar YUV); a plane of one row has no meaningful row stride"""
     def pitch(t):
         return (t.stride(0) if t.shape[0] > 1 else t.shape[1]) * t.element_size()
@@ -258,8 +307,8 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
         H, W = _nv12_hw(x) if _is_nv12(in_layout) else _p010_hw(x)
         x = x.contiguous()
         B = x.shape[0]
-    elif _is_yuvp(in_layout):
-        H, W = _yuvp_hw(x, "yuv420p" if _is_yuv420p(in_layout) else "yuv444p16" if x.dtype == torch.uint16 else "yuv444p")
+    elif _is_yuvp(in_layout) or _is_nv16(in_layout):
+        H, W = _yuvp_hw(x, _yuv_name(in_layout, x.dtype))
         x = x.contiguous()
         B = x.shape[0]
     elif in_layout:
@@ -276,7 +325,8 @@ def _forward_impl(x: torch.Tensor, handle: int, out_h: int, out_w: int, scale: i
     cdt = _lib.TU_BF16 if compute_bf16 else _lib.TU_F32
     out_shape = _image_shape(B, 3, out_h, out_w, out_code)
     u16_out = (out_code & 0xFF) == _lib.TU_U16
-    if not (_is_yuv444p(out_code) and u16_out) and _is_p010(out_code) != u16_out:
+    u16_layout = _is_yuv444p(out_code) or _is_nv16(out_code) or out_code & _lib.TU_YUV_LSB10
+    if (u16_out and not (u16_layout or _is_p010(out_code))) or (_is_p010(out_code) and not u16_out):
         raise RuntimeError("the P010 output layout is for uint16 frames, and uint16 output is P010 only")
     if out_code >> 8 and not _is_p010(out_code) and not u16_out and (out_code & 0xFF) != _lib.TU_U8:
         raise RuntimeError("interleaved and NV12 output layouts are for uint8 frames")
@@ -320,8 +370,8 @@ def tu_forward_planes(x: Optional[torch.Tensor], x_planes: List[torch.Tensor], o
         if _is_nv12(in_layout) or _is_p010(in_layout):
             H, W = _nv12_hw(x) if _is_nv12(in_layout) else _p010_hw(x)
             B = x.shape[0]
-        elif _is_yuvp(in_layout):
-            H, W = _yuvp_hw(x, "yuv420p" if _is_yuv420p(in_layout) else "yuv444p16" if x.dtype == torch.uint16 else "yuv444p")
+        elif _is_yuvp(in_layout) or _is_nv16(in_layout):
+            H, W = _yuvp_hw(x, _yuv_name(in_layout, x.dtype))
             B = x.shape[0]
         elif in_layout:
             B, H, W = x.shape[0], x.shape[1], x.shape[2]
@@ -466,8 +516,9 @@ def _(x, planes, code):
 
 @torch.library.custom_op("tu::rgb_to_yuvp", mutates_args=(), device_types="cuda")
 def tu_rgb_to_yuvp(x: torch.Tensor, code: int) -> torch.Tensor:
-    """planar RGB (B,3,H,W) -> planar YUV frames: fp16 RGB -> yuv420p (B,3H/2,W) / yuv444p (B,3,H,W) uint8, fp32 RGB -> yuv444p16
-    (B,3,H,W) uint16; code = the frames' TU_U8 / TU_U16 | TU_LAYOUT_YUV420P / TU_LAYOUT_YUV444P | colour bits"""
+    """planar RGB (B,3,H,W) -> planar YUV frames: fp16 RGB -> yuv420p (B,3H/2,W) / yuv422p (B,2H,W) / yuv444p (B,3,H,W) uint8, fp32 RGB
+    -> yuv444p16 or the *p10le frames of those shapes, uint16; code = the frames' TU_U8 / TU_U16 | planar layout [| TU_YUV_LSB10] |
+    colour bits"""
     lib = _lib.load()
     _require_cuda(x)
     w16 = (code & 0xFF) == _lib.TU_U16
@@ -490,7 +541,7 @@ def _(x, code):
 
 @torch.library.custom_op("tu::rgb_to_yuvp_planes", mutates_args=("planes",), device_types="cuda")
 def tu_rgb_to_yuvp_planes(x: torch.Tensor, planes: List[torch.Tensor], code: int) -> None:
-    """planar RGB (B,3,H,W) -> planar YUV frames (fp16 RGB for 8-bit codes, fp32 for yuv444p16) written into the surfaces
+    """planar RGB (B,3,H,W) -> planar YUV frames (fp16 RGB for 8-bit codes, fp32 for 16-bit ones) written into the surfaces
     [y0, u0, v0, y1, ...]"""
     lib = _lib.load()
     _require_cuda(x)
@@ -508,17 +559,62 @@ def _(x, planes, code):
     return None
 
 
+@torch.library.custom_op("tu::rgb_to_yuv422sp", mutates_args=(), device_types="cuda")
+def tu_rgb_to_yuv422sp(x: torch.Tensor, code: int) -> torch.Tensor:
+    """planar RGB (B,3,H,W) -> semi-planar 4:2:2 frames (B,2H,W): fp16 RGB -> nv16 uint8, fp32 RGB -> p210 uint16; code = the frames'
+    TU_U8 / TU_U16 | TU_LAYOUT_NV16 | colour bits"""
+    lib = _lib.load()
+    _require_cuda(x)
+    w16 = (code & 0xFF) == _lib.TU_U16
+    want = torch.float32 if w16 else torch.float16
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != want:
+        raise RuntimeError(f"rgb_to_yuv422sp takes planar {str(want)[6:]} RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    out = torch.empty(_image_shape(B, 3, H, W, code), dtype=torch.uint16 if w16 else torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_yuv422sp(x.data_ptr(), out.data_ptr(), None, code, B, H, W, _stream()))
+    return out
+
+
+@tu_rgb_to_yuv422sp.register_fake
+def _(x, code):
+    w16 = (code & 0xFF) == _lib.TU_U16
+    return x.new_empty(_image_shape(x.shape[0], 3, x.shape[2], x.shape[3], code), dtype=torch.uint16 if w16 else torch.uint8)
+
+
+@torch.library.custom_op("tu::rgb_to_yuv422sp_planes", mutates_args=("planes",), device_types="cuda")
+def tu_rgb_to_yuv422sp_planes(x: torch.Tensor, planes: List[torch.Tensor], code: int) -> None:
+    """planar RGB (B,3,H,W) -> semi-planar 4:2:2 frames (fp16 RGB for nv16, fp32 for p210) written into the surfaces [y0, uv0, y1, ...]"""
+    lib = _lib.load()
+    _require_cuda(x)
+    want = torch.float32 if (code & 0xFF) == _lib.TU_U16 else torch.float16
+    if x.dim() != 4 or x.shape[1] != 3 or x.dtype != want:
+        raise RuntimeError(f"rgb_to_yuv422sp_planes takes planar {str(want)[6:]} RGB (B,3,H,W), got {x.dtype} {tuple(x.shape)}")
+    x = x.contiguous()
+    B, _, H, W = x.shape
+    with torch.cuda.device(x.device):
+        _lib.check(lib.tu_rgb_to_yuv422sp(x.data_ptr(), None, _descriptors(planes, code), code, B, H, W, _stream()))
+
+
+@tu_rgb_to_yuv422sp_planes.register_fake
+def _(x, planes, code):
+    return None
+
+
 def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale_factor: Optional[int],
                 require_ratio: bool, compute_bf16: bool, out_dtype: torch.dtype, clamp: bool = True,
                 in_layout: str = "chw", out_layout: str = "chw", yuv: str = "bt709", out=None):
     """Shape logic of the three reference forwards (W:237-238, F:245-248,323-327, R:121-122) around tu::forward.
-    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'rgba' | 'bgra' | 'nv12' | 'p010' | 'yuv420p' | 'yuv444p' | 'yuv444p16'): uint8
-    frames may be interleaved (B,H,W,3), 4-byte pixels with alpha (B,H,W,4), NV12 or yuv420p (B,3H/2,W) or yuv444p (B,3,H,W) on either
-    side, and either side may be P010 (B,3H/2,W) or yuv444p16 (B,3,H,W) uint16 frames; yuv ('bt709' | 'bt601' | 'bt709_full' |
+    in_layout / out_layout ('chw' | 'hwc' | 'hwc_bgr' | 'rgba' | 'bgra' | 'nv12' | 'p010' | 'yuv420p' | 'yuv444p' | 'yuv444p16' |
+    'yuv420p10le' | 'yuv422p' | 'yuv422p10le' | 'yuv444p10le' | 'nv16' | 'p210'): uint8 frames may be interleaved (B,H,W,3), 4-byte
+    pixels with alpha (B,H,W,4), NV12 or yuv420p (B,3H/2,W), yuv422p or nv16 (B,2H,W) or yuv444p (B,3,H,W) on either side, and either side
+    may be P010 or yuv420p10le (B,3H/2,W), yuv422p10le or p210 (B,2H,W), or yuv444p16 or yuv444p10le (B,3,H,W) uint16 frames (the *p10le
+    words hold the code in their low 10 bits, the others in their high 10 bits); yuv ('bt709' | 'bt601' | 'bt709_full' |
     'bt601_full', and 'bt2020' | 'bt2020_full' with a 16-bit YUV side and no 8-bit one) is the colour of the YUV side(s).  An RGBA / BGRA
     output carries the input alpha resampled to the output size (tu_resample_alpha) when the input is RGBA / BGRA too, else alpha 255; an
     RGBA / BGRA input going to an output without alpha loses its alpha.
-    Frame surfaces: with in_layout 'nv12' / 'p010', x may be a list of B (y, uv) plane pairs (see plane_pairs), with a planar YUV
+    Frame surfaces: with in_layout 'nv12' / 'p010' / 'nv16' / 'p210', x may be a list of B (y, uv) plane pairs (see plane_pairs), with a planar YUV
     in_layout a list of B (y, u, v) triples (see plane_triples); with a YUV out_layout, out= a list of B such pairs / triples receives the
     result and is returned."""
     il, ol = layout_code(in_layout), layout_code(out_layout)
@@ -526,16 +622,17 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
     p010_in, p010_out = in_layout == "p010", out_layout == "p010"
     yuv_in, yuv_out = in_layout in YUV_LAYOUTS, out_layout in YUV_LAYOUTS
     yuvp_in, yuvp_out = in_layout in PLANAR, out_layout in PLANAR
+    sp422_in, sp422_out = in_layout in SEMI422, out_layout in SEMI422
     if yuv != "bt709" and not (yuv_in or yuv_out):
         raise ValueError(f"yuv={yuv!r} applies to NV12 / P010 frames only: pass in_layout / out_layout 'nv12' or 'p010'")
     yc = yuv_code(yuv)
     if yuv in YUV_P010:
         side16 = in_layout in YUV16_LAYOUTS or out_layout in YUV16_LAYOUTS
         side8 = (yuv_in and in_layout not in YUV16_LAYOUTS) or (yuv_out and out_layout not in YUV16_LAYOUTS)
-        if (yuvp_in or yuvp_out) and (side8 or not side16):
-            raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a P010 or yuv444p16 side and no 8-bit YUV side "
-                             "(nv12, yuv420p, yuv444p)")
-        if nv12_in or nv12_out or not (p010_in or p010_out or yuvp_in or yuvp_out):
+        if (yuvp_in or yuvp_out or sp422_in or sp422_out) and (side8 or not side16):
+            raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a 16-bit YUV side ({', '.join(YUV16_LAYOUTS)}) "
+                             "and no 8-bit YUV side (nv12, nv16, yuv420p, yuv422p, yuv444p)")
+        if nv12_in or nv12_out or not (p010_in or p010_out or yuvp_in or yuvp_out or sp422_in or sp422_out):
             raise ValueError(f"yuv={yuv!r} (BT.2020) is defined for 10-bit frames: it needs a P010 side and no NV12 side")
     if nv12_out and out_dtype != torch.uint8:
         raise ValueError("out_layout='nv12' writes uint8 frames")
@@ -543,6 +640,8 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
         raise ValueError("out_layout='p010' writes uint16 frames")
     if yuvp_out and out_dtype != PLANAR[out_layout]:
         raise ValueError(f"out_layout={out_layout!r} writes {str(PLANAR[out_layout])[6:]} frames")
+    if sp422_out and out_dtype != SEMI422[out_layout]:
+        raise ValueError(f"out_layout={out_layout!r} writes {str(SEMI422[out_layout])[6:]} frames")
     px4_in, px4_out = in_layout in ("rgba", "bgra"), out_layout in ("rgba", "bgra")
     if px4_out and out_dtype != torch.uint8:
         raise ValueError(f"out_layout={out_layout!r} writes uint8 frames")
@@ -561,7 +660,7 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
         H, W = _nv12_hw(x)
     elif p010_in:
         H, W = _p010_hw(x)
-    elif yuvp_in:
+    elif yuvp_in or sp422_in:
         H, W = _yuvp_hw(x, in_layout)
     else:
         H, W = (int(x.shape[1]), int(x.shape[2])) if il else (int(x.shape[2]), int(x.shape[3]))
@@ -573,10 +672,12 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
     def even_out(oh, ow):
         if (nv12_out or p010_out) and (oh % 2 or ow % 2):
             raise ValueError(f"{'NV12' if nv12_out else 'P010'} output frames need an even height and width, got {oh}x{ow}")
-        if out_layout == "yuv420p" and (oh % 2 or ow % 2):
-            raise ValueError(f"yuv420p output frames need an even height and width, got {oh}x{ow}")
+        if out_layout in ("yuv420p", "yuv420p10le") and (oh % 2 or ow % 2):
+            raise ValueError(f"{out_layout} output frames need an even height and width, got {oh}x{ow}")
+        if out_layout in ("yuv422p", "yuv422p10le", *SEMI422) and ow % 2:
+            raise ValueError(f"{out_layout} output frames need an even width, got {oh}x{ow}")
         if out is not None:
-            fmt = out_layout if yuvp_out else "NV12" if nv12_out else "P010"
+            fmt = out_layout if yuvp_out or sp422_out else "NV12" if nv12_out else "P010"
             if not isinstance(out, (list, tuple)) or len(out) != (len(x) if planes_in else x.shape[0]):
                 raise ValueError(f"out= must be a list of one {'(y, u, v) plane triple' if yuvp_out else '(y, uv) plane pair'} per input "
                                  "frame")
@@ -609,18 +710,21 @@ def run_forward(pw_handle: int, model: str, x, res_out: Tuple[int, int], upscale
     even_out(*res_out)
     # Resize is the last op: the un-clamped full-size image stays in the compute dtype and the Resize kernel writes the requested
     # output dtype / layout (uint8 frames: (out*255).clamp(0,255).to(uint8) fused into its store).  fp16 output keeps an fp32
-    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  An 8-bit YUV output (NV12, yuv420p, yuv444p) is
-    # the fp16 output converted, a 16-bit one (P010, yuv444p16) the fp32 output converted
+    # intermediate, so that it is the fp32 result rounded once, at the Resize's store.  An 8-bit YUV output (NV12, NV16, yuv420p, yuv422p,
+    # yuv444p) is the fp16 output converted, a 16-bit one (P010, P210, yuv444p16, *p10le) the fp32 output converted
     yuv8_out = yuv_out and out_dtype == torch.uint8
     mid_code = _code(torch.bfloat16 if compute_bf16 and out_dtype in (torch.bfloat16, torch.uint8) and not yuv8_out else torch.float32)
     full = forward(oh, ow, scale, mid_code, False)
     if yuv_out:
         rgb = tu_resize_aa(full, res_out[0], res_out[1], clamp, _lib.TU_F16 if yuv8_out else _lib.TU_F32)
         if out is not None:
-            (tu_rgb_to_yuvp_planes if yuvp_out else tu_rgb_to_yuv420_planes)(rgb, _flat(out), out_code)
+            (tu_rgb_to_yuvp_planes if yuvp_out else tu_rgb_to_yuv422sp_planes if sp422_out else tu_rgb_to_yuv420_planes)(rgb, _flat(out),
+                                                                                                                  out_code)
             return out
         if yuvp_out:
             return tu_rgb_to_yuvp(rgb, out_code)
+        if sp422_out:
+            return tu_rgb_to_yuv422sp(rgb, out_code)
         return tu_rgb_to_nv12(rgb, out_code) if nv12_out else tu_rgb_to_p010(rgb, out_code)
     if px4_in and px4_out:
         # alpha is resampled straight from the input to the requested size, by the rule of every other output path

@@ -169,7 +169,11 @@ class EngineModel(nn.Module):
         Planar YUV (FFmpeg's pix_fmt names) on either side: 'yuv420p' (I420) uint8 (B,3H/2,W) -- Y, then U and V of (H/2, W/2) --
         converted exactly as NV12; 'yuv444p' uint8 and 'yuv444p16' uint16 (B,3,H,W) planes Y, U, V at full resolution, the 16-bit
         words holding the code in the high 10 bits as P010 (in_layout='yuv444p16' takes uint16 frames; out_layout='yuv444p16' returns
-        uint16 frames for any frame input).  Their surfaces are lists of B (y, u, v) plane triples, in x and in out=."""
+        uint16 frames for any frame input).  Their surfaces are lists of B (y, u, v) plane triples, in x and in out=.
+        4:2:2 and LSB-aligned 10-bit frames: 'yuv422p' uint8 (B,2H,W) -- Y, then U and V of (H, W/2) -- and 'nv16' uint8 / 'p210' uint16
+        (B,2H,W) -- Y, then H rows of (U, V) pairs, p210 words holding the code in the high 10 bits; 'yuv420p10le' (B,3H/2,W),
+        'yuv422p10le' (B,2H,W) and 'yuv444p10le' (B,3,H,W) uint16 with the code in the LOW 10 bits of each word (FFmpeg's software
+        10-bit formats).  Surfaces: (y, uv) pairs for nv16 / p210, (y, u, v) triples for the planar ones."""
         if isinstance(x, (list, tuple)):
             if in_layout not in engine.YUV_LAYOUTS:
                 raise ValueError("a list of (y, uv) frame planes is NV12 / P010 input: pass in_layout='nv12' or 'p010'")
@@ -188,11 +192,13 @@ class EngineModel(nn.Module):
             raise RuntimeError("transformerupscaler_b200 is forward-only (no autograd): the input requires grad; call under torch.no_grad()")
         # uint8 frames in -> uint8 frames out (ToTensor scaling on read, (out*255).clamp(0,255).to(uint8) on write, fused into
         # the first and last kernels): the video-pipeline entry, an extension of the reference's float-only signature
-        # P010 and yuv444p16 frames are uint16; any other uint16 tensor is an image like any other and is read as float32
+        # 16-bit YUV frames are uint16; any other uint16 tensor is an image like any other and is read as float32
         if in_layout == "p010" and x0.dtype != torch.uint16:
             raise ValueError(f"in_layout='p010' takes uint16 frames (B, 3H/2, W), got {x0.dtype}")
         if in_layout == "yuv444p16" and x0.dtype != torch.uint16:
             raise ValueError(f"in_layout='yuv444p16' takes uint16 frames (B, 3, H, W), got {x0.dtype}")
+        if in_layout in engine.YUV16_LAYOUTS and x0.dtype != torch.uint16:
+            raise ValueError(f"in_layout={in_layout!r} takes uint16 frames, got {x0.dtype}")
         frames_u8 = x0.dtype == torch.uint8
         frames = frames_u8 or in_layout in engine.YUV16_LAYOUTS
         if x0.dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.uint8) and not frames:

@@ -50,7 +50,7 @@ extern "C" {
  * The alpha byte of an output pixel is the input alpha resampled to the output size when the input is 4-byte too (tu_resample_alpha),
  * 255 otherwise; a 4-byte input going to an output without alpha loses its alpha.  TU_U8 only; never with colour bits.
  * The layout bits 8..11 are an enumeration: 0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010, 9 YUV422P,
- * 10 NV16. */
+ * 10 NV16, 11 YUYV, 12 UYVY. */
 #define TU_LAYOUT_RGBA 0x300
 #define TU_LAYOUT_BGRA 0x500
 #define TU_U8_RGBA (TU_U8 | TU_LAYOUT_RGBA)
@@ -126,6 +126,23 @@ extern "C" {
 #define TU_U16_YUV420P10 (TU_U16 | TU_LAYOUT_YUV420P | TU_YUV_LSB10)
 #define TU_U16_YUV422P10 (TU_U16 | TU_LAYOUT_YUV422P | TU_YUV_LSB10)
 #define TU_U16_YUV444P10 (TU_U16 | TU_LAYOUT_YUV444P | TU_YUV_LSB10)
+/* Packed 4:2:2 frames (luma and chroma interleaved in one plane, as webcams, capture cards and D3D11 / VAAPI decoders hand them out), for
+ * the image input and / or output of tu_forward / tu_forward_frames and the code of tu_packed422_to_rgb / tu_rgb_to_packed422:
+ *   TU_U8 | TU_LAYOUT_YUYV (yuyv422, YUY2): (B, H, W, 2) uint8, each row W/2 macropixels of the bytes Y0 U Y1 V.
+ *   TU_U8 | TU_LAYOUT_UYVY (uyvy422, UYVY, DeckLink's 8-bit YUV): (B, H, W, 2) uint8, macropixels U Y0 V Y1.
+ *   TU_U16 | TU_LAYOUT_YUYV (y210, DXGI_FORMAT_Y210): (B, H, W, 2) little-endian uint16 words Y0 U Y1 V, the 10-bit code in the HIGH
+ *        10 bits as P010 (word >> 6 on read: the low 6 bits are ignored; code << 6 on write: the low 6 bits are zero).
+ * Every other code with these layouts is TU_ERR_ARG (TU_U16 | TU_LAYOUT_UYVY, float dtypes, TU_YUV_LSB10).  Colour bits: the 8-bit codes
+ * take NV12's, y210 P010's (TU_YUV_BT2020 allowed, never with TU_YUV_BT601).  A packed frame holds the samples of an nv16 (8-bit) or p210
+ * (y210) frame -- macropixel j of row i is Y[i][2j], Y[i][2j+1], U[i][j], V[i][j] -- and converts bitwise as that frame does, in both
+ * directions: 4:2:2 siting and formulas as above, planar fp16 RGB for the 8-bit codes and planar fp32 RGB for y210.  W even, any H.
+ * A macropixel is one access: the buffer (dense) or each frame's data pointer and pitch (TuFramePacked) are multiples of 4 bytes (8-bit)
+ * or 8 bytes (y210).  A write touches only the 2W samples of each row. */
+#define TU_LAYOUT_YUYV 0xB00
+#define TU_LAYOUT_UYVY 0xC00
+#define TU_U8_YUYV422 (TU_U8 | TU_LAYOUT_YUYV)
+#define TU_U8_UYVY422 (TU_U8 | TU_LAYOUT_UYVY)
+#define TU_U16_Y210 (TU_U16 | TU_LAYOUT_YUYV)
 
 #define TU_OK 0
 #define TU_ERR_ARG (-1)      /* bad argument (shape / dtype / null pointer)              */
@@ -149,7 +166,7 @@ long long tu_launch_count(void);
  * events on the caller's stream (two event records per forward: cheap enough for the timed region); tu_profile_enable(2)
  * brackets EVERY kernel, tagged with the reference op it implements ("conv1", "conv2" (or "conv1_conv2" when fused), "downsample", "patch_embed",
  * "transformer_blocks", "patch_unembed", "decoder_conv1", "decoder_conv2", "bicubic_add_clamp", "up1", "up1_conv",
- * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "yuv420p_to_rgb" / "rgb_to_yuv420p", "yuv444p_to_rgb" / "rgb_to_yuv444p", "yuv444p16_to_rgb" / "rgb_to_yuv444p16", "yuv420p10le_to_rgb" / "rgb_to_yuv420p10le", "yuv422p_to_rgb" / "rgb_to_yuv422p", "yuv422p10le_to_rgb" / "rgb_to_yuv422p10le", "yuv444p10le_to_rgb" / "rgb_to_yuv444p10le" at a planar YUV end, "nv16_to_rgb" / "rgb_to_nv16", "p210_to_rgb" / "rgb_to_p210" at a semi-planar 4:2:2 end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
+ * "final_upscale", "final_conv_add", and "nv12_to_rgb" / "rgb_to_nv12" at an NV12 end, "p010_to_rgb" / "rgb_to_p010" at a P010 end, "yuv420p_to_rgb" / "rgb_to_yuv420p", "yuv444p_to_rgb" / "rgb_to_yuv444p", "yuv444p16_to_rgb" / "rgb_to_yuv444p16", "yuv420p10le_to_rgb" / "rgb_to_yuv420p10le", "yuv422p_to_rgb" / "rgb_to_yuv422p", "yuv422p10le_to_rgb" / "rgb_to_yuv422p10le", "yuv444p10le_to_rgb" / "rgb_to_yuv444p10le" at a planar YUV end, "nv16_to_rgb" / "rgb_to_nv16", "p210_to_rgb" / "rgb_to_p210" at a semi-planar 4:2:2 end, "yuyv422_to_rgb" / "rgb_to_yuyv422", "uyvy422_to_rgb" / "rgb_to_uyvy422", "y210_to_rgb" / "rgb_to_y210" at a packed 4:2:2 end, "resample_alpha" when both ends are RGBA / BGRA).  tu_profile_collect / tu_profile_report synchronise those events (the only
  * calls in the library that wait on the device): collect sums the milliseconds and launches recorded under `name`
  * (NULL = all); report writes "name total_ms launches\n" lines into buf (returns the needed size when buf is NULL);
  * tu_profile_reset drops the records. */
@@ -281,7 +298,8 @@ int tu_pack_weights(int model, const TuNamedTensor *tensors, int n_tensors, int 
  *      (tu_resample_alpha; the workspace of tu_forward_workspace_bytes_io then holds that (B, outH, outW) plane), else 255.
  *      TU_U8 | TU_LAYOUT_YUV420P / TU_LAYOUT_YUV444P, TU_U16 | TU_LAYOUT_YUV444P (planar YUV, above): as NV12 (8-bit: planar fp16) and
  *      P010 (16-bit: planar fp32) on either side; the workspace holds the planar RGB frame of each such side.  The 4:2:2 codes
- *      (TU_LAYOUT_YUV422P, TU_LAYOUT_NV16) and the TU_YUV_LSB10 codes (above) likewise.
+ *      (TU_LAYOUT_YUV422P, TU_LAYOUT_NV16), the TU_YUV_LSB10 codes and the packed 4:2:2 codes (TU_LAYOUT_YUYV, TU_LAYOUT_UYVY; above)
+ *      likewise.
  * scale: FastTransformer integer factor (ignored by the others).  For FastTransformer the library
  *      writes the (scale*H, scale*W) image; an antialiased Resize to res_out, when required, is
  *      tu_resize_bilinear_aa.
@@ -311,6 +329,14 @@ typedef struct TuFramePlanes3 {
     void *y, *u, *v;
     long long y_pitch, u_pitch, v_pitch;
 } TuFramePlanes3;
+/* one packed 4:2:2 frame (yuyv422 / uyvy422 / y210 codes): one plane of H rows of 2W samples (W/2 macropixels), row r starting at
+ * data + r * pitch bytes, as a V4L2 / Media Foundation buffer, a DeckLink / NDI frame or a D3D11 / VAAPI surface holds it.  pitch >= 2W
+ * samples; data and pitch are multiples of 4 bytes (8-bit) or 8 bytes (y210).  A write touches only the 2W samples of each row.  The
+ * surfaces of one call must not overlap each other or the other side's buffers; the library does not check that. */
+typedef struct TuFramePacked {
+    void *data;
+    long long pitch;
+} TuFramePacked;
 
 size_t tu_forward_workspace_bytes(int model, int B, int H, int W, int outH, int outW, int scale, int compute_dtype);
 /* the same, sized from the packed weights actually used (non-default dim / heads / n_blocks; which fused kernels are packed) */
@@ -336,7 +362,8 @@ int tu_forward_planes(const TuModelWeights *w, const void *x, const TuFramePlane
                       int compute_dtype, int clamp, void *workspace, size_t workspace_bytes, void *stream);
 /* tu_forward_planes for every kind of YUV side: x_frames / out_frames is a HOST array of B descriptors whose element type the side's
  * code chooses -- TuFramePlanes for NV12 / P010 / NV16 / P210 (4:2:2: uv holds H rows), TuFramePlanes3 for the planar codes (yuv420p,
- * yuv422p, yuv444p, yuv444p16 and the TU_YUV_LSB10 ones; 4:2:2: u and v hold H rows of W/2 samples) -- and otherwise follows the rules of
+ * yuv422p, yuv444p, yuv444p16 and the TU_YUV_LSB10 ones; 4:2:2: u and v hold H rows of W/2 samples), TuFramePacked for yuyv422 /
+ * uyvy422 / y210 (tu_forward_planes rejects a frames array on such a side) -- and otherwise follows the rules of
  * tu_forward_planes (exactly one of dense buffer and array per side, every descriptor checked before anything is enqueued, workspace of
  * tu_forward_workspace_bytes_io, results bitwise those of the dense frames).  The two sides are independent: NV12 surfaces in and
  * yuv444p surfaces out is one call.  tu_forward_planes(...) is this function. */
@@ -495,6 +522,13 @@ int tu_rgb_to_yuvp(const void *rgb, void *dense, const TuFramePlanes3 *frames, i
  * is non-NULL.  yuv422p gives the bits of nv16 on the same samples. */
 int tu_yuv422sp_to_rgb(const void *dense, const TuFramePlanes *frames, int code, void *rgb, int B, int H, int W, void *stream);
 int tu_rgb_to_yuv422sp(const void *rgb, void *dense, const TuFramePlanes *frames, int code, int B, int H, int W, void *stream);
+/* Packed 4:2:2 frames <-> planar RGB (B, 3, H, W): code TU_U8 | TU_LAYOUT_YUYV / TU_LAYOUT_UYVY with fp16 RGB (4-byte aligned), or
+ * TU_U16 | TU_LAYOUT_YUYV (y210) with fp32 RGB (8-byte aligned), colour bits as above (anything else, an odd W, B > 65535, a NULL or a
+ * misaligned buffer: TU_ERR_ARG, before any launch).  Exactly one of `dense` (the (B, H, W, 2) batch) and `frames` (a HOST array of B
+ * TuFramePacked, read during the call) is non-NULL.  Bitwise tu_yuv422sp_to_rgb / tu_rgb_to_yuv422sp on the nv16 / p210 frame of the
+ * same samples. */
+int tu_packed422_to_rgb(const void *dense, const TuFramePacked *frames, int code, void *rgb, int B, int H, int W, void *stream);
+int tu_rgb_to_packed422(const void *rgb, void *dense, const TuFramePacked *frames, int code, int B, int H, int W, void *stream);
 
 #ifdef __cplusplus
 }

@@ -27,6 +27,9 @@ TU_LAYOUT_YUV420P, TU_LAYOUT_YUV444P = 0x600, 0x700
 # 4:2:2: yuv422p (TU_U8, three planes, (B, 2H, W)) and NV16 (TU_U8) / P210 (TU_U16, code in the high 10 bits): Y then interleaved (U, V) rows
 TU_LAYOUT_YUV422P, TU_LAYOUT_NV16 = 0x900, 0xA00
 TU_YUV_LSB10 = 0x10000                               # with TU_U16 and a planar layout: yuv420p10le / yuv422p10le / yuv444p10le
+# packed 4:2:2, one plane (B, H, W, 2): YUYV (TU_U8: yuyv422 / YUY2 bytes Y0 U Y1 V; TU_U16: y210 words, code in the high 10 bits) and
+# UYVY (TU_U8 only: uyvy422 bytes U Y0 V Y1)
+TU_LAYOUT_YUYV, TU_LAYOUT_UYVY = 0xB00, 0xC00
 TU_ERR_ARG, TU_ERR_SCALE, TU_ERR_TOKENS, TU_ERR_WORKSPACE, TU_ERR_CUDA = -1, -2, -3, -4, -5
 MODEL_IDS = {"WindowTransformer": 0, "FastTransformer": 1, "ResidualTransformer": 2}
 
@@ -93,6 +96,11 @@ class TuFramePlanes3(C.Structure):
                 ("v_pitch", C.c_longlong)]
 
 
+class TuFramePacked(C.Structure):
+    """one packed 4:2:2 frame (yuyv422 / uyvy422 / y210) as one device plane with its row pitch in bytes"""
+    _fields_ = [("data", C.c_void_p), ("pitch", C.c_longlong)]
+
+
 # name -> (restype, argtypes); must list every symbol include/tu_b200.h declares
 SIGNATURES = {
     "tu_version": (i32, []),
@@ -154,6 +162,8 @@ SIGNATURES = {
     "tu_rgb_to_yuvp": (i32, [vp, vp, C.POINTER(TuFramePlanes3), i32, i32, i32, i32, vp]),
     "tu_yuv422sp_to_rgb": (i32, [vp, C.POINTER(TuFramePlanes), i32, vp, i32, i32, i32, vp]),
     "tu_rgb_to_yuv422sp": (i32, [vp, vp, C.POINTER(TuFramePlanes), i32, i32, i32, i32, vp]),
+    "tu_packed422_to_rgb": (i32, [vp, C.POINTER(TuFramePacked), i32, vp, i32, i32, i32, vp]),
+    "tu_rgb_to_packed422": (i32, [vp, vp, C.POINTER(TuFramePacked), i32, i32, i32, i32, vp]),
 }
 
 

@@ -138,10 +138,16 @@ static const char *yuv422sp_step(int code, bool to_rgb) {
     if (dtype_is_p210(code)) return to_rgb ? "p210_to_rgb" : "rgb_to_p210";
     return to_rgb ? "nv16_to_rgb" : "rgb_to_nv16";
 }
+// and of the packed 4:2:2 ones
+static const char *packed422_step(int code, bool to_rgb) {
+    if (dtype_is_y210(code)) return to_rgb ? "y210_to_rgb" : "rgb_to_y210";
+    if (dtype_is_uyvy422(code)) return to_rgb ? "uyvy422_to_rgb" : "rgb_to_uyvy422";
+    return to_rgb ? "yuyv422_to_rgb" : "rgb_to_yuyv422";
+}
 
 // Runs (or, with a.dry, only sizes) one forward.  TI/TO are handled by dtype codes in the leaf launchers.
-// xf / of: the input / output frame surfaces of a YUV side (TuFramePlanes for NV12 / P010 / NV16 / P210, TuFramePlanes3 for planar YUV),
-// or NULL for the dense buffer x / out.
+// xf / of: the input / output frame surfaces of a YUV side (TuFramePlanes for NV12 / P010 / NV16 / P210, TuFramePlanes3 for planar YUV,
+// TuFramePacked for packed 4:2:2), or NULL for the dense buffer x / out.
 template <typename T>
 static int forward_impl(const TuModelWeights *w, const void *x, const void *xf, int in_dtype, void *out, const void *of,
                         int out_dtype, int B, int H, int W, int outH, int outW, int scale, int clamp, Arena &a, cudaStream_t st) {
@@ -191,12 +197,14 @@ static int forward_impl(const TuModelWeights *w, const void *x, const void *xf, 
         if (!dry) TU_STEP("p010_to_rgb", xf ? tu_yuv420_planes_to_rgb((const TuFramePlanes *)xf, in_dtype, rgb, B, H, W, stv) : tu_p010_to_rgb(x, in_dtype, rgb, B, H, W, stv));
         x = rgb;
         in_dtype = TU_F32;
-    } else if (dtype_is_yuvp(in_dtype) || dtype_is_yuv422sp(in_dtype)) {
-        // planar YUV and semi-planar 4:2:2: 8-bit frames as NV12 (planar fp16), 16-bit frames as P010 (planar fp32)
+    } else if (dtype_is_yuvp(in_dtype) || dtype_is_yuv422sp(in_dtype) || dtype_is_packed422(in_dtype)) {
+        // planar YUV, semi-planar and packed 4:2:2: 8-bit frames as NV12 (planar fp16), 16-bit frames as P010 (planar fp32)
         const bool w16 = dtype_base(in_dtype) == TU_U16;
         void *rgb = a.get((size_t)B * 3 * H * W * (w16 ? sizeof(float) : sizeof(f16)));
         if (!dry && dtype_is_yuvp(in_dtype))
             TU_STEP(yuvp_step(in_dtype, true), tu_yuvp_to_rgb(xf ? nullptr : x, (const TuFramePlanes3 *)xf, in_dtype, rgb, B, H, W, stv));
+        else if (!dry && dtype_is_packed422(in_dtype))
+            TU_STEP(packed422_step(in_dtype, true), tu_packed422_to_rgb(xf ? nullptr : x, (const TuFramePacked *)xf, in_dtype, rgb, B, H, W, stv));
         else if (!dry)
             TU_STEP(yuv422sp_step(in_dtype, true), tu_yuv422sp_to_rgb(xf ? nullptr : x, (const TuFramePlanes *)xf, in_dtype, rgb, B, H, W, stv));
         x = rgb;
@@ -205,14 +213,15 @@ static int forward_impl(const TuModelWeights *w, const void *x, const void *xf, 
     // YUV output: the last image kernel writes planar fp16 (8-bit codes) / fp32 (16-bit codes) here, and the conversion op writes `out` /
     // `of` from it
     const bool nv12_out = dtype_is_nv12(out_dtype), p010_out = dtype_is_p010(out_dtype), yuvp_out = dtype_is_yuvp(out_dtype);
-    const bool sp422_out = dtype_is_yuv422sp(out_dtype);
-    const bool w16_out = p010_out || ((yuvp_out || sp422_out) && dtype_base(out_dtype) == TU_U16);
-    void *img = nv12_out || ((yuvp_out || sp422_out) && !w16_out) ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
+    const bool sp422_out = dtype_is_yuv422sp(out_dtype), pk422_out = dtype_is_packed422(out_dtype);
+    const bool w16_out = p010_out || ((yuvp_out || sp422_out || pk422_out) && dtype_base(out_dtype) == TU_U16);
+    void *img = nv12_out || ((yuvp_out || sp422_out || pk422_out) && !w16_out) ? a.get((size_t)B * 3 * outH * outW * sizeof(f16))
                 : w16_out ? a.get((size_t)B * 3 * outH * outW * sizeof(float)) : out;
     const int img_dtype = dtype_is_yuv(out_dtype) ? (w16_out ? TU_F32 : TU_F16) : out_dtype;
 #define TU_YUV_OUT()                                                                                                    \
     if (yuvp_out) TU_STEP(yuvp_step(out_dtype, false), tu_rgb_to_yuvp(img, of ? nullptr : out, (const TuFramePlanes3 *)of, out_dtype, B, outH, outW, stv)); \
     else if (sp422_out) TU_STEP(yuv422sp_step(out_dtype, false), tu_rgb_to_yuv422sp(img, of ? nullptr : out, (const TuFramePlanes *)of, out_dtype, B, outH, outW, stv)); \
+    else if (pk422_out) TU_STEP(packed422_step(out_dtype, false), tu_rgb_to_packed422(img, of ? nullptr : out, (const TuFramePacked *)of, out_dtype, B, outH, outW, stv)); \
     else if (of) TU_STEP(nv12_out ? "rgb_to_nv12" : "rgb_to_p010", tu_rgb_to_yuv420_planes(img, (const TuFramePlanes *)of, out_dtype, B, outH, outW, stv)); \
     else if (nv12_out) TU_STEP("rgb_to_nv12", tu_rgb_to_nv12(img, out, out_dtype, B, outH, outW, stv));                    \
     else if (p010_out) TU_STEP("rgb_to_p010", tu_rgb_to_p010(img, out, out_dtype, B, outH, outW, stv))
@@ -779,6 +788,7 @@ extern "C" size_t tu_forward_workspace_bytes_for(const TuModelWeights *w, int B,
 // 4-byte frames: exactly TU_U8 | TU_LAYOUT_RGBA or TU_U8 | TU_LAYOUT_BGRA.  Other codes have a layout nibble below 4 and no colour bit.
 // 4:2:2 codes: TU_U8 | TU_LAYOUT_YUV422P / TU_LAYOUT_NV16 with NV12's colour bits, TU_U16 | TU_LAYOUT_NV16 with P010's; an even width.
 // TU_YUV_LSB10 goes with TU_U16 and a planar layout only (yuv420p10le: an even height and width, yuv422p10le: an even width).
+// Packed 4:2:2 codes: TU_U8 | TU_LAYOUT_YUYV / TU_LAYOUT_UYVY with NV12's colour bits, TU_U16 | TU_LAYOUT_YUYV with P010's; an even width.
 static bool plain_code(int d) {
     const int nib = (d >> 8) & 0xF;
     return dtype_is_px4(d) ||
@@ -788,8 +798,8 @@ static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int out
     const bool inyuv = dtype_is_yuv(in_dtype), outyuv = dtype_is_yuv(out_dtype);
     const bool in420 = dtype_is_yuv420(in_dtype) || dtype_is_yuv420p(in_dtype) || dtype_is_yuv420p10(in_dtype);
     const bool out420 = dtype_is_yuv420(out_dtype) || dtype_is_yuv420p(out_dtype) || dtype_is_yuv420p10(out_dtype);
-    const bool in422 = dtype_is_yuv422p(in_dtype) || dtype_is_yuv422p10(in_dtype) || dtype_is_yuv422sp(in_dtype);
-    const bool out422 = dtype_is_yuv422p(out_dtype) || dtype_is_yuv422p10(out_dtype) || dtype_is_yuv422sp(out_dtype);
+    const bool in422 = dtype_is_yuv422p(in_dtype) || dtype_is_yuv422p10(in_dtype) || dtype_is_yuv422sp(in_dtype) || dtype_is_packed422(in_dtype);
+    const bool out422 = dtype_is_yuv422p(out_dtype) || dtype_is_yuv422p10(out_dtype) || dtype_is_yuv422sp(out_dtype) || dtype_is_packed422(out_dtype);
     for (int d : {in_dtype, out_dtype})
         TU_CHECK_ARG(dtype_is_px4(d) || !layout_is_px4((d >> 8) & 0xF),
                      "forward: TU_LAYOUT_RGBA / TU_LAYOUT_BGRA are for uint8 frames (TU_U8) only, without colour bits");
@@ -798,13 +808,13 @@ static int check_yuv420_codes(int in_dtype, int out_dtype, int H, int W, int out
                  "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (input); TU_LAYOUT_YUV420P is "
                  "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only); TU_LAYOUT_YUV422P "
                  "is for uint8 frames, TU_LAYOUT_NV16 for uint8 frames or 16-bit words (P210), TU_YUV_LSB10 for 16-bit words of a planar "
-                 "layout only");
+                 "layout only; TU_LAYOUT_YUYV is for uint8 frames or 16-bit words (Y210), TU_LAYOUT_UYVY for uint8 frames");
     TU_CHECK_ARG(outyuv || plain_code(out_dtype),
                  "forward: TU_LAYOUT_NV12 is for uint8 frames (TU_U8), TU_LAYOUT_P010 for 16-bit words (TU_U16, P010 only), and the "
                  "colour bits TU_YUV_* go with them only (TU_YUV_BT2020 with P010, never with TU_YUV_BT601) (output); TU_LAYOUT_YUV420P is "
                  "for uint8 frames, TU_LAYOUT_YUV444P for uint8 frames or 16-bit words (TU_YUV_BT2020 with 16-bit words only); TU_LAYOUT_YUV422P "
                  "is for uint8 frames, TU_LAYOUT_NV16 for uint8 frames or 16-bit words (P210), TU_YUV_LSB10 for 16-bit words of a planar "
-                 "layout only");
+                 "layout only; TU_LAYOUT_YUYV is for uint8 frames or 16-bit words (Y210), TU_LAYOUT_UYVY for uint8 frames");
     TU_CHECK_ARG(!in420 || (H % 2 == 0 && W % 2 == 0),
                  std::string("forward: ") + (dtype_is_p010(in_dtype) ? "P010" : dtype_is_nv12(in_dtype) ? "NV12" : dtype_is_yuv420p(in_dtype) ? "yuv420p" : "yuv420p10le") +
                      " input frames need an even height and width");
@@ -831,11 +841,20 @@ extern "C" size_t tu_forward_workspace_bytes_io(const TuModelWeights *w, int B, 
     return rc == TU_OK ? a.off : 0;
 }
 
-// frame descriptors of one side: TuFramePlanes (NV12 / P010 / NV16 / P210) or TuFramePlanes3 (planar YUV), by the side's code
+// frame descriptors of one side: TuFramePlanes (NV12 / P010 / NV16 / P210), TuFramePlanes3 (planar YUV) or TuFramePacked (packed
+// 4:2:2), by the side's code
 static int check_frames(const void *frames, int code, int B, int H, int W, const char *op) {
     if (dtype_is_yuvp(code)) return check_yuvp_frames((const TuFramePlanes3 *)frames, code, B, H, W, op);
+    if (dtype_is_packed422(code)) return check_packed422_frames((const TuFramePacked *)frames, code, B, H, W, op);
     if (dtype_is_yuv422sp(code)) return check_yuv422sp_frames((const TuFramePlanes *)frames, code, B, H, W, op);
     return check_yuv420_planes((const TuFramePlanes *)frames, code, B, H, W, op);
+}
+
+static int check_packed422_dense(const void *buf, int code, const char *side) {
+    const uintptr_t al = dtype_is_y210(code) ? 8 : 4;
+    TU_CHECK_ARG(!buf || !dtype_is_packed422(code) || reinterpret_cast<uintptr_t>(buf) % al == 0,
+                 std::string("forward: the dense packed 4:2:2 ") + side + " buffer must be " + std::to_string(al) + "-byte aligned");
+    return TU_OK;
 }
 
 extern "C" int tu_forward_frames(const TuModelWeights *w, const void *x, const void *x_frames, int in_dtype, void *out,
@@ -848,9 +867,12 @@ extern "C" int tu_forward_frames(const TuModelWeights *w, const void *x, const v
     TU_CHECK_ARG(!(out && out_frames), "forward: give the output as either out or out_frames, not both");
     if ((rc = check_yuv420_codes(in_dtype, out_dtype, H, W, outH, outW))) return rc;
     TU_CHECK_ARG(!x_frames || dtype_is_yuv(in_dtype),
-                 "forward: x_frames (frame planes) are for NV12 / P010 input only (TuFramePlanes, as are NV16 / P210), or planar YUV input (TuFramePlanes3)");
+                 "forward: x_frames (frame planes) are for NV12 / P010 input only (TuFramePlanes, as are NV16 / P210), or planar YUV input (TuFramePlanes3), or packed 4:2:2 input (TuFramePacked)");
     TU_CHECK_ARG(!out_frames || dtype_is_yuv(out_dtype),
-                 "forward: out_frames (frame planes) are for NV12 / P010 output only (TuFramePlanes, as are NV16 / P210), or planar YUV output (TuFramePlanes3)");
+                 "forward: out_frames (frame planes) are for NV12 / P010 output only (TuFramePlanes, as are NV16 / P210), or planar YUV output (TuFramePlanes3), or packed 4:2:2 output (TuFramePacked)");
+    // a dense packed 4:2:2 buffer is read / written one macropixel at a time: its alignment is checked here too, before anything is
+    // enqueued (the output's conversion op is the last step of the forward)
+    if ((rc = check_packed422_dense(x, in_dtype, "input")) || (rc = check_packed422_dense(out, out_dtype, "output"))) return rc;
     // every descriptor is checked here, before the first kernel of the forward is enqueued
     if (x_frames && (rc = check_frames(x_frames, in_dtype, B, H, W, "forward: x_frames"))) return rc;
     if (out_frames && (rc = check_frames(out_frames, out_dtype, B, outH, outW, "forward: out_frames"))) return rc;
@@ -891,6 +913,11 @@ extern "C" int tu_forward_planes(const TuModelWeights *w, const void *x, const T
                                                         "takes TuFramePlanes3 (tu_forward_frames)");
     TU_CHECK_ARG(!out_frames || !dtype_is_yuvp(out_dtype), "forward_planes: out_frames are TuFramePlanes (NV12 / P010); planar YUV "
                                                            "output takes TuFramePlanes3 (tu_forward_frames)");
+    // nor can they describe a one-plane packed 4:2:2 frame (TuFramePacked)
+    TU_CHECK_ARG(!x_frames || !dtype_is_packed422(in_dtype), "forward_planes: x_frames are TuFramePlanes (NV12 / P010); packed 4:2:2 input "
+                                                             "takes TuFramePacked (tu_forward_frames)");
+    TU_CHECK_ARG(!out_frames || !dtype_is_packed422(out_dtype), "forward_planes: out_frames are TuFramePlanes (NV12 / P010); packed 4:2:2 "
+                                                                "output takes TuFramePacked (tu_forward_frames)");
     return tu_forward_frames(w, x, x_frames, in_dtype, out, out_frames, out_dtype, B, H, W, outH, outW, scale, compute_dtype, clamp,
                              workspace, workspace_bytes, stream);
 }

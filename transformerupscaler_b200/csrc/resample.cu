@@ -1254,6 +1254,12 @@ template <typename TS> struct Planes420 {
     __device__ __forceinline__ TS *uvrow(int r) const { return (TS *)((char *)uv + (long long)r * uvp); }
     __device__ __forceinline__ P chroma(int r, int j) const { return *reinterpret_cast<const P *>(uvrow(r) + 2 * j); }
     __device__ __forceinline__ void store_chroma(int r, int j, P c) const { *reinterpret_cast<P *>(uvrow(r) + 2 * j) = c; }
+    // the luma pair (r, 2j..2j+1) and, for 4:2:2, the pair with its chroma sample (r, j): one access per plane
+    __device__ __forceinline__ P luma(int r, int j) const { return *reinterpret_cast<const P *>(yrow(r) + 2 * j); }
+    __device__ __forceinline__ void store_422(int r, int j, P y, P c) const {
+        *reinterpret_cast<P *>(yrow(r) + 2 * j) = y;
+        store_chroma(r, j, c);
+    }
 };
 // Planar (yuv420p): a table of up to kPlanesPerLaunch TuFramePlanes3 in the kernel parameters, like Planes420; the U and V samples of
 // chroma column j are one sample each of two planes whose rows hold W/2 samples.  A dense (B, 3H/2, W) batch is passed as the table
@@ -1277,6 +1283,47 @@ template <typename TS> struct Planar420 {
     __device__ __forceinline__ void store_chroma(int r, int j, P c) const {
         urow(r)[j] = c.x;
         vrow(r)[j] = c.y;
+    }
+    __device__ __forceinline__ P luma(int r, int j) const { return *reinterpret_cast<const P *>(yrow(r) + 2 * j); }
+    __device__ __forceinline__ void store_422(int r, int j, P y, P c) const {
+        *reinterpret_cast<P *>(yrow(r) + 2 * j) = y;
+        store_chroma(r, j, c);
+    }
+};
+// Packed 4:2:2 (yuyv422 / uyvy422 / y210): a table of up to kPlanesPerLaunch TuFramePacked in the kernel parameters (64 x 16 bytes), like
+// Planes420; a dense (B, H, W, 2) batch is passed as the table of its frames (pitch 2W samples).  Chroma sample (r, j) and the luma pair
+// (r, 2j..2j+1) are the one macropixel j of row r: four samples Y0 U Y1 V (YUYV) or U Y0 V Y1 (UYVY), read as one aligned 4- / 8-byte
+// load (the kernel's chroma and luma reads of the same macropixel are the same load) and written as one aligned store.
+enum class PackedOrder { YUYV, UYVY };
+struct FramesPacked { TuFramePacked f[kPlanesPerLaunch]; };
+template <typename TS, PackedOrder O> struct Packed422 {
+    typedef FramesPacked Param;
+    typedef typename std::remove_const<TS>::type S;
+    typedef typename Yuv420<S>::Pair P;
+    // one macropixel as one integer word, sample k in bits [k * 8 sizeof(S), ...): a word rather than a uchar4 / ushort4, whose fields
+    // the compiler would load one by one where the kernel uses only two of them (the neighbour's chroma)
+    typedef typename std::conditional<sizeof(S) == 1, uint32_t, unsigned long long>::type Word;
+    static constexpr int kBits = 8 * sizeof(S);
+    static constexpr int kY0 = O == PackedOrder::YUYV ? 0 : 1, kC0 = 1 - kY0;        // sample index of Y0 and of U; Y1, V are 2 further
+    TS *p;
+    long long pitch;
+    static __device__ __forceinline__ Packed422 frame(const Param &t, int, int) {
+        const TuFramePacked &d = t.f[blockIdx.y];
+        return {(TS *)d.data, d.pitch};
+    }
+    __device__ __forceinline__ Word *word(int r, int j) const { return reinterpret_cast<Word *>((char *)p + (long long)r * pitch) + j; }
+    static __device__ __forceinline__ S sample(Word w, int k) { return (S)(w >> (k * kBits)); }
+    __device__ __forceinline__ P chroma(int r, int j) const {
+        const Word w = *word(r, j);
+        return Yuv420<S>::pair(sample(w, kC0), sample(w, kC0 + 2));
+    }
+    __device__ __forceinline__ P luma(int r, int j) const {
+        const Word w = *word(r, j);
+        return Yuv420<S>::pair(sample(w, kY0), sample(w, kY0 + 2));
+    }
+    __device__ __forceinline__ void store_422(int r, int j, P y, P c) const {
+        *word(r, j) = (Word)y.x << (kY0 * kBits) | (Word)c.x << (kC0 * kBits) | (Word)y.y << ((kY0 + 2) * kBits) |
+                      (Word)c.y << ((kC0 + 2) * kBits);
     }
 };
 
@@ -1379,10 +1426,11 @@ __global__ void __launch_bounds__(256) rgb_to_yuv420_kernel(const TR *__restrict
     f.store_chroma(i, j, F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid))));
 }
 
-// ---- 4:2:2 frames (NV16 / P210 semi-planar, yuv422p / yuv422p10le planar) <-> planar RGB --------------------------------------------
+// ---- 4:2:2 frames (NV16 / P210 semi-planar, yuv422p / yuv422p10le planar, yuyv422 / uyvy422 / y210 packed) <-> planar RGB ------------
 // Chroma row r belongs to luma row r (co-sited with the even luma columns).  The addressing policies of the 4:2:0 kernels serve: Planes420
 // (a TuFramePlanes table; a dense (B, 2H, W) batch is passed as the table of its frames' planes) and Planar420 (a Frames3 table).  Only the
-// number of chroma rows differs, and the policies never see it.
+// number of chroma rows differs, and the policies never see it.  Packed422 serves the packed frames.  The luma pair and the whole sample
+// (luma pair and chroma pair, on the way out) go through the policy: one macropixel access in the packed one.
 // One thread per chroma sample (i, j): luma row i, columns 2j, 2j+1.  Column 2j takes chroma column j, column 2j+1 the mean of j and j+1
 // (clamped): integer sums (at most 2 * 1023) times 1/2, exact in fp32; then the per-pixel sequence of yuv420_to_rgb_kernel.
 template <typename TS, typename TR, typename A>
@@ -1400,7 +1448,7 @@ __global__ void __launch_bounds__(256) yuv422_to_rgb_kernel(typename A::Param in
     const P c0 = f.chroma(i, j), c1 = f.chroma(i, min(j + 1, Wc - 1));
     const int u0 = F::code(c0.x), v0 = F::code(c0.y);
     const int us[2] = {2 * u0, u0 + F::code(c1.x)}, vs[2] = {2 * v0, v0 + F::code(c1.y)};   // x2
-    const P y = *reinterpret_cast<const P *>(f.yrow(i) + 2 * j);
+    const P y = f.luma(i, j);
     const int ys[2] = {F::code(y.x), F::code(y.y)};
     float r[2], g[2], bl[2];
 #pragma unroll
@@ -1451,8 +1499,8 @@ __global__ void __launch_bounds__(256) rgb_to_yuv422_kernel(const TR *__restrict
     const float cb = __fadd_rn(__fadd_rn(__fmul_rn(k.cb_r, bar[0]), __fmul_rn(k.cb_g, bar[1])), __fmul_rn(0.5f, bar[2]));
     const float cr = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, bar[0]), __fmul_rn(k.cr_g, bar[1])), __fmul_rn(k.cr_b, bar[2]));
     const A f = A::frame(out, H, W);
-    *reinterpret_cast<P *>(f.yrow(i) + 2 * j) = F::pair(yq[0], yq[1]);
-    f.store_chroma(i, j, F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid))));
+    f.store_422(i, j, F::pair(yq[0], yq[1]),
+                F::pair(yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cb), F::mid)), yuv_code<TS>(__fadd_rn(__fmul_rn(k.cs, cr), F::mid))));
 }
 
 // ---- 4:4:4 planar frames (yuv444p / yuv444p16) <-> planar RGB ----------------------------------------------------------------------
@@ -2228,4 +2276,90 @@ extern "C" int tu_rgb_to_yuv422sp(const void *rgb, void *dense, const TuFramePla
     cudaStream_t st = (cudaStream_t)stream;
     return dtype_is_p210(code) ? launch_yuv422sp<uint16_t, float, false>(dense, frames, code, (float *)rgb, B, H, W, st)
                                : launch_yuv422sp<uint8_t, f16, false>(dense, frames, code, (f16 *)rgb, B, H, W, st);
+}
+
+// ---- packed 4:2:2 frames (yuyv422 / uyvy422 / y210) -------------------------------------------------------------------------------
+static const char *packed422_fmt(int code) { return dtype_is_y210(code) ? "y210" : dtype_is_uyvy422(code) ? "uyvy422" : "yuyv422"; }
+
+// B frames of a packed 4:2:2 side: host-side checks of the code, the sizes and every descriptor, made before anything is enqueued
+int tu::check_packed422_frames(const TuFramePacked *frames, int code, int B, int H, int W, const char *op) {
+    TU_CHECK_ARG(frames && B > 0 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_packed422(code), std::string(op) + ": TuFramePacked frames are for packed 4:2:2 (TU_U8 | TU_LAYOUT_YUYV, TU_U8 | "
+                                                               "TU_LAYOUT_UYVY or TU_U16 | TU_LAYOUT_YUYV [| colour bits]) only");
+    const std::string fmt = packed422_fmt(code);
+    TU_CHECK_ARG(W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    const long long s = dtype_is_y210(code) ? 2 : 1, row = 2LL * W * s, al = 4 * s;      // a macropixel is one access
+    for (int b = 0; b < B; ++b) {
+        const TuFramePacked &d = frames[b];
+        const std::string at = std::string(op) + ": frame " + std::to_string(b) + ": ";
+        TU_CHECK_ARG(d.data, at + "data is NULL");
+        TU_CHECK_ARG(d.pitch >= row, at + "pitch " + std::to_string(d.pitch) + " is smaller than the row's " + std::to_string(2LL * W) +
+                                         " samples (" + std::to_string(row) + " bytes)");
+        TU_CHECK_ARG(reinterpret_cast<uintptr_t>(d.data) % al == 0, at + "data must be a multiple of " + std::to_string(al) + " bytes (" + fmt + ")");
+        TU_CHECK_ARG(d.pitch % al == 0, at + "pitch must be a multiple of " + std::to_string(al) + " bytes (" + fmt + ")");
+    }
+    return TU_OK;
+}
+
+static int check_packed422_args(const void *dense, const TuFramePacked *frames, int code, const void *rgb, int B, int H, int W,
+                                const char *op) {
+    TU_CHECK_ARG(rgb && B > 0 && B <= 65535 && H > 0 && W > 0, std::string(op) + ": bad argument");
+    TU_CHECK_ARG(dtype_is_packed422(code), std::string(op) + ": code must be TU_U8 | TU_LAYOUT_YUYV or TU_LAYOUT_UYVY [| TU_YUV_BT601] "
+                                                              "[| TU_YUV_FULL_RANGE], or TU_U16 | TU_LAYOUT_YUYV [| TU_YUV_BT601 or "
+                                                              "TU_YUV_BT2020] [| TU_YUV_FULL_RANGE]");
+    TU_CHECK_ARG(!dense != !frames, std::string(op) + ": give exactly one of the dense buffer and the frames array");
+    const bool y210 = dtype_is_y210(code);
+    const std::string fmt = packed422_fmt(code);
+    TU_CHECK_ARG(W % 2 == 0, std::string(op) + ": " + fmt + " frames need an even width");
+    TU_CHECK_ARG((long)H * W * 3 < (1L << 31), std::string(op) + ": frame too large");
+    const uintptr_t ra = y210 ? 8 : 4, fa = y210 ? 8 : 4;       // a pair of RGB values / a macropixel is one access
+    TU_CHECK_ARG((reinterpret_cast<uintptr_t>(rgb) & (ra - 1)) == 0,
+                 std::string(op) + ": the " + (y210 ? "fp32" : "fp16") + " RGB buffer must be " + std::to_string(ra) + "-byte aligned");
+    TU_CHECK_ARG(!dense || (reinterpret_cast<uintptr_t>(dense) & (fa - 1)) == 0,
+                 std::string(op) + ": the dense " + fmt + " buffer must be " + std::to_string(fa) + "-byte aligned");
+    return frames ? check_packed422_frames(frames, code, B, H, W, op) : TU_OK;
+}
+
+// one launch per kPlanesPerLaunch frames, the dense (B, H, W, 2) batch passed as the table of its frames (pitch 2W samples)
+template <typename TS, typename TR, PackedOrder O, bool ToRgb>
+static int launch_packed422(const void *dense, const TuFramePacked *frames, int code, TR *rgb, int B, int H, int W, cudaStream_t st) {
+    typedef Packed422<typename std::conditional<ToRgb, const TS, TS>::type, O> A;
+    const long long s = sizeof(TS), plane = (long long)H * W;
+    const YuvCoef k = yuv_coef(code);
+    const std::string what = ToRgb ? std::string(packed422_fmt(code)) + "_to_rgb" : std::string("rgb_to_") + packed422_fmt(code);
+    for (int b0 = 0; b0 < B; b0 += kPlanesPerLaunch) {
+        const int nb = std::min(kPlanesPerLaunch, B - b0);
+        typename A::Param p = {};
+        for (int b = 0; b < nb; ++b)
+            p.f[b] = frames ? frames[b0 + b] : TuFramePacked{(char *)dense + (long long)(b0 + b) * 2 * plane * s, 2 * W * s};
+        TR *r = rgb + (long long)b0 * 3 * plane;
+        const dim3 grid((unsigned)ceil_div((int)(plane / 2), 256), nb);
+        if constexpr (ToRgb)
+            launch_pdl(yuv422_to_rgb_kernel<TS, TR, A>, grid, dim3(256), 0, st, p, r, H, W, k);
+        else
+            launch_pdl(rgb_to_yuv422_kernel<TR, TS, A>, grid, dim3(256), 0, st, (const TR *)r, p, H, W, k);
+        TU_CHECK_LAUNCH(what.c_str());
+    }
+    return TU_OK;
+}
+
+template <bool ToRgb>
+static int packed422_op(const void *dense, const TuFramePacked *frames, int code, void *rgb, int B, int H, int W, void *stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype_is_y210(code))
+        return launch_packed422<uint16_t, float, PackedOrder::YUYV, ToRgb>(dense, frames, code, (float *)rgb, B, H, W, st);
+    if (dtype_is_uyvy422(code))
+        return launch_packed422<uint8_t, f16, PackedOrder::UYVY, ToRgb>(dense, frames, code, (f16 *)rgb, B, H, W, st);
+    return launch_packed422<uint8_t, f16, PackedOrder::YUYV, ToRgb>(dense, frames, code, (f16 *)rgb, B, H, W, st);
+}
+
+extern "C" int tu_packed422_to_rgb(const void *dense, const TuFramePacked *frames, int code, void *rgb, int B, int H, int W, void *stream) {
+    if (int rc = check_packed422_args(dense, frames, code, rgb, B, H, W, "packed422_to_rgb")) return rc;
+    return packed422_op<true>(dense, frames, code, rgb, B, H, W, stream);
+}
+
+extern "C" int tu_rgb_to_packed422(const void *rgb, void *dense, const TuFramePacked *frames, int code, int B, int H, int W, void *stream) {
+    if (int rc = check_packed422_args(dense, frames, code, rgb, B, H, W, "rgb_to_packed422")) return rc;
+    return packed422_op<false>(dense, frames, code, (void *)rgb, B, H, W, stream);
 }

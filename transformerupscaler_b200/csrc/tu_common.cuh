@@ -25,6 +25,8 @@ int check_yuv420_planes(const TuFramePlanes *frames, int code, int B, int H, int
 int check_yuvp_frames(const TuFramePlanes3 *frames, int code, int B, int H, int W, const char *op);
 // the same for B semi-planar 4:2:2 frames (NV16 / P210: TuFramePlanes with H chroma rows)
 int check_yuv422sp_frames(const TuFramePlanes *frames, int code, int B, int H, int W, const char *op);
+// the same for B packed 4:2:2 frames (yuyv422 / uyvy422 / y210: TuFramePacked)
+int check_packed422_frames(const TuFramePacked *frames, int code, int B, int H, int W, const char *op);
 
 #define TU_CHECK_ARG(cond, msg)                         \
     do {                                                \
@@ -101,7 +103,8 @@ template <> __device__ __forceinline__ uint8_t from_f<uint8_t>(float v) {
 // TU_U8 | TU_LAYOUT_NV12 (4:2:0 video frames) may add the colour bits TU_YUV_BT601 / TU_YUV_FULL_RANGE in bits 12..13.
 // TU_U16 | TU_LAYOUT_P010 (10-bit 4:2:0 frames) may add the same bits, or TU_YUV_BT2020 (bit 14) instead of TU_YUV_BT601.
 __host__ __device__ __forceinline__ int dtype_base(int d) { return d & 0xFF; }
-// the layout bits are an enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010, 9 YUV422P, 10 NV16), and dtype_layout keeps the colour bits
+// the layout bits are an enumeration (0 CHW, 1 HWC, 2 HWC_BGR, 3 RGBA, 4 NV12, 5 BGRA, 6 YUV420P, 7 YUV444P, 8 P010, 9 YUV422P, 10 NV16,
+// 11 YUYV, 12 UYVY), and dtype_layout keeps the colour bits
 // above them: compare whole values, never bits (0x500 = BGRA shares a bit with NV12, 0x300 = RGBA two bits with HWC / HWC_BGR)
 __host__ __device__ __forceinline__ int dtype_layout(int d) { return d >> 8; }
 __host__ __device__ __forceinline__ bool layout_is_px4(int l) { return l == 3 || l == 5; }          // RGBA / BGRA: 4-byte pixels
@@ -149,8 +152,16 @@ __host__ __device__ __forceinline__ bool dtype_is_yuv422sp(int d) { return dtype
 __host__ __device__ __forceinline__ bool dtype_is_yuvp(int d) {
     return dtype_is_yuv420p(d) || dtype_is_yuv444p(d) || dtype_is_yuv444p16(d) || dtype_is_yuv422p(d) || dtype_is_lsb10(d);
 }
+// packed 4:2:2 (layout 11 YUYV: Y0 U Y1 V, 12 UYVY: U Y0 V Y1; one plane, TuFramePacked surfaces): yuyv422 and uyvy422 (TU_U8, NV12's
+// colour bits) and y210 (TU_U16 | TU_LAYOUT_YUYV, the code in the high 10 bits, P010's colour bits)
+__host__ __device__ __forceinline__ bool dtype_is_yuyv422(int d) { return yuv8_code_is(d, TU_U8 | TU_LAYOUT_YUYV); }
+__host__ __device__ __forceinline__ bool dtype_is_uyvy422(int d) { return yuv8_code_is(d, TU_U8 | TU_LAYOUT_UYVY); }
+__host__ __device__ __forceinline__ bool dtype_is_y210(int d) { return yuv16_code_is(d, TU_U16 | TU_LAYOUT_YUYV); }
+__host__ __device__ __forceinline__ bool dtype_is_packed422(int d) { return dtype_is_yuyv422(d) || dtype_is_uyvy422(d) || dtype_is_y210(d); }
 // every YUV frame code: converted to / from a planar fp16 (8-bit) or fp32 (16-bit) RGB frame at the ends of the forward
-__host__ __device__ __forceinline__ bool dtype_is_yuv(int d) { return dtype_is_yuv420(d) || dtype_is_yuvp(d) || dtype_is_yuv422sp(d); }
+__host__ __device__ __forceinline__ bool dtype_is_yuv(int d) {
+    return dtype_is_yuv420(d) || dtype_is_yuvp(d) || dtype_is_yuv422sp(d) || dtype_is_packed422(d);
+}
 // one RGB pixel of frame b -> out, in the requested layout.  pix = y * W + x, plane = H * W
 template <typename TO>
 __device__ __forceinline__ void store_rgb(TO *out, long b, long plane, long pix, int layout, float r, float g, float bl) {

@@ -173,12 +173,17 @@ class EngineModel(nn.Module):
         4:2:2 and LSB-aligned 10-bit frames: 'yuv422p' uint8 (B,2H,W) -- Y, then U and V of (H, W/2) -- and 'nv16' uint8 / 'p210' uint16
         (B,2H,W) -- Y, then H rows of (U, V) pairs, p210 words holding the code in the high 10 bits; 'yuv420p10le' (B,3H/2,W),
         'yuv422p10le' (B,2H,W) and 'yuv444p10le' (B,3,H,W) uint16 with the code in the LOW 10 bits of each word (FFmpeg's software
-        10-bit formats).  Surfaces: (y, uv) pairs for nv16 / p210, (y, u, v) triples for the planar ones."""
+        10-bit formats).  Surfaces: (y, uv) pairs for nv16 / p210, (y, u, v) triples for the planar ones.
+        Packed 4:2:2 (FFmpeg's names), luma and chroma interleaved in one plane, (B,H,W,2) with W even: 'yuyv422' (YUY2: webcams, V4L2,
+        Media Foundation) and 'uyvy422' (UYVY: capture cards, DeckLink, NDI) uint8, 'y210' uint16 words Y0 U Y1 V with the code in the
+        high 10 bits (D3D11 / QSV / VAAPI 4:2:2 10-bit decoders).  Converted bitwise as the nv16 / p210 frame of the same samples.
+        Surfaces: lists of B (H, W, 2) tensors with strides (row pitch, 2, 1), in x and in out=."""
         if isinstance(x, (list, tuple)):
             if in_layout not in engine.YUV_LAYOUTS:
                 raise ValueError("a list of (y, uv) frame planes is NV12 / P010 input: pass in_layout='nv12' or 'p010'")
             engine.frame_planes(x, in_layout, "frames")
-            return self._forward(x, x[0][0], res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
+            x0 = x[0] if isinstance(x[0], torch.Tensor) else x[0][0]        # a packed 4:2:2 frame is one surface
+            return self._forward(x, x0, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
         return self._forward(x, x, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out)
 
     def _forward(self, x, x0: torch.Tensor, res_out, upscale_factor, require_ratio, in_layout, out_layout, yuv, out):
